@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Flux-VAE HDR decode throughput on B200 (BASELINE.json metric: megapixels/s).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -24,6 +24,10 @@ aux_c4_4096 / aux_c4_rows : BASELINE config C4 (1x16x512x512 -> 4096^2, "aggress
         row-tiled over the N GPUs of the job (strong scaling), outside the headline's timed region.
 --impl reference : the reference node's CPU path (oracle port, TWO decoder passes + conv_out per call as the
         reference does) on the host cores: every step is ONE image of the C2 batch at its full 1024^2 size.
+--dump-outputs DIR : after the timed steps, the IMAGE the last timed step returned is written as DIR/image.npy
+        (float32 [4, 1024, 1024, 3]; --impl reference: [1, 1024, 1024, 3]; N > 1: DIR/image_rank<r>.npy per rank, a fixed
+        sample of its pixels where the files together would pass 64 MB).  Weights and latents are seeded, so two builds
+        run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -46,6 +50,7 @@ CONV_MFLOP_PER_PX = 9.4628          # SURVEY.md §8d: 3x3/1x1 convs of the decod
 PER_GPU_BATCH, LATENT = 4, 128      # config C2
 MODE = "moderate"
 C4_ROOFLINE_MP_S = 76.8             # SURVEY.md §8d: 17.851 MFLOP/px at 4096^2 against the sustained bf16 peak, per GPU
+DUMP_BYTES = 64 * 10 ** 6           # --dump-outputs: at most this many bytes over all files of all ranks
 
 
 def workload_config(world: int) -> dict:
@@ -166,11 +171,11 @@ class ClockSampler:
                 "samples": len(sm), "source": self.src}
 
 
-def cpu_reference_run(steps: int, warmup: int, sample_latent: int = 64, budget_s: float = 0.0, dec=None):
+def cpu_reference_run(steps: int, warmup: int, sample_latent: int = 64, dec=None):
     """The reference node's CPU path (oracle port: fp32 PyTorch eager decoder + the restated HDR math, with the
     reference's real call structure: TWO decoder passes + a third conv_out per call, hdr_vae_decode.py:859,876,1022)
-    on all host cores.  One 1x16xSxS latent per step; budget_s > 0 stops early once the projected time of another
-    step would exceed it (never fewer than 2 timed steps)."""
+    on all host cores.  One 1x16xSxS latent per step, `steps` timed steps.
+    -> (summary dict, seconds per step, the image the last timed step returned)."""
     import torch
     from oracle import hdr_oracle as ho
     from oracle.flux_decoder import build_decoder, make_latent
@@ -179,7 +184,6 @@ def cpu_reference_run(steps: int, warmup: int, sample_latent: int = 64, budget_s
     dec = dec if dec is not None else build_decoder(0)
     z = make_latent(1, sample_latent, sample_latent, seed=1234)
     times = []
-    t_begin = time.perf_counter()
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
@@ -188,35 +192,35 @@ def cpu_reference_run(steps: int, warmup: int, sample_latent: int = 64, budget_s
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
-            if budget_s > 0 and len(times) >= 2 and (time.perf_counter() - t_begin) + dt > budget_s:
-                break
     mp = (8 * sample_latent) ** 2 / 1e6
     per = sum(times) / len(times)
     return {"value": mp / per, "unit": UNIT, "cores": cores, "kind": "port",
             "sample": f"{len(times)} x (1x16x{sample_latent}x{sample_latent} latent -> {8 * sample_latent}^2, {MODE}; "
                       f"2 decoder passes + conv_out as the reference node does), {per:.2f} s per call, fp32 torch CPU, "
-                      f"{cores} threads"}, per, len(times)
+                      f"{cores} threads"}, per, out
 
 
 def run_reference_arm(args):
     """`--impl reference`: the reference's CPU implementation of the path on the box's host cores, on the B200 arm's
     config.  Every step decodes ONE image of the C2 batch at its full size (1x16x128x128 -> 1024^2, "moderate") with
     the reference node's call structure; MP/s is per pixel, so one image of the batch is a bounded sample of the
-    4-image step.  Warm-up is a single C2-sized call; the timed steps stop once REF_BUDGET_S (default 240 s) would be
-    exceeded (reported in `steps`, the request in `steps_requested`).  Three C1-sized calls (1x16x64x64 -> 512^2,
-    BASELINE configs[0], the reference's own CPU-runnable case) are timed as well and reported in cpu_baseline."""
+    4-image step.  Warm-up is a single C2-sized call, then exactly --steps timed calls (each takes seconds to minutes
+    on the host cores).  Three C1-sized calls (1x16x64x64 -> 512^2, BASELINE configs[0], the reference's own
+    CPU-runnable case) are timed as well and reported in cpu_baseline.  --dump-outputs: the image of the last timed call,
+    DIR/image.npy (float32 [1, 1024, 1024, 3])."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     from oracle.flux_decoder import build_decoder
     dec = build_decoder(0)
-    budget = float(os.environ.get("REF_BUDGET_S", "240"))
-    c1, c1_per, c1_n = cpu_reference_run(3, 1, 64, dec=dec)
-    base, per, done = cpu_reference_run(max(2, args.steps), 1, LATENT, budget_s=budget, dec=dec)
-    base["c1_512"] = {"value": c1["value"], "unit": UNIT, "s_per_call": c1_per, "calls": c1_n,
+    c1, c1_per, _ = cpu_reference_run(3, 1, 64, dec=dec)
+    base, per, last_out = cpu_reference_run(args.steps, 1, LATENT, dec=dec)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "image", last_out, DUMP_BYTES)
+    base["c1_512"] = {"value": c1["value"], "unit": UNIT, "s_per_call": c1_per, "calls": 3,
                       "workload": "C1: 1x16x64x64 latent -> 512x512, reference node call structure"}
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus,
-            "steps": done, "steps_requested": args.steps, "warmup": 1, "ms_per_step": per * 1e3, "higher_is_better": True,
+            "steps": args.steps, "warmup": 1, "ms_per_step": per * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(args.gpus),
             "reference_step": f"one image of the C2 batch at full size: 1x16x{LATENT}x{LATENT} -> {8 * LATENT}^2, {MODE}, "
@@ -297,6 +301,22 @@ def emit(line: dict) -> None:
     out.flush()
 
 
+def dump_output(dirname: str, name: str, t, budget: int) -> None:
+    """Write tensor `t` as dirname/name.npy in float32.  When it would exceed `budget` bytes, a fixed sample of its pixels
+    (rows of the last dimension, drawn with seed 0 and kept in order) is written instead, [n_sampled, last dim]: the same
+    pixels on every run for the same shape."""
+    import numpy as np
+    import torch
+    t = t.detach().float()
+    if t.numel() * 4 + 128 > budget:                          # 128: the .npy header
+        rows = t.reshape(-1, t.shape[-1])
+        keep = (budget - 128) // (4 * rows.shape[1])
+        idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        t = rows[idx.to(rows.device)]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy())
+
+
 def main():
     guard_stdout()
     ap = argparse.ArgumentParser()
@@ -307,7 +327,11 @@ def main():
     ap.add_argument("--no-aux", action="store_true", help="skip the auxiliary 4096^2 single-GPU measurement")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager", action="store_true", help="skip the PyTorch-eager-on-the-same-GPU comparator")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the image of the last timed step to DIR/image.npy (float32) for output comparisons")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -358,11 +382,15 @@ def main():
     with ClockSampler(local_rank) as clocks:
         barrier()
         e0.record()
-        for _ in range(args.steps):
+        for _ in range(args.steps - 1):
             step_device()
+        last_out, _ = step_device()
         e1.record()
         barrier()
     launches = lib.hdrvae_launch_count() - n0
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "image" if world == 1 else f"image_rank{rank}", last_out, DUMP_BYTES // world)
+    del last_out
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle.ref_loader import reference_available
 from vae_decode_hdr_b200 import NODE_CLASS_MAPPINGS
 from vae_decode_hdr_b200.linear_exr_export import (LinearEXRExport, highest_version, write_exr_scanlines,
                                                    write_radiance_hdr)
@@ -23,21 +24,26 @@ def test_node_surface_equals_reference():
     assert cls is LinearEXRExport
     assert (cls.RETURN_TYPES, cls.RETURN_NAMES, cls.FUNCTION, cls.CATEGORY, cls.OUTPUT_NODE) == \
         (("STRING",), ("filepath",), "export_linear_exr", "image", True)
-    from oracle.ref_loader import reference_available
-    if reference_available():
-        import importlib.util, sys, types
-        for name in ("pyexr", "imageio", "imageio.v3", "folder_paths"):
-            sys.modules.setdefault(name, types.ModuleType(name))
-        spec = importlib.util.spec_from_file_location("_ref_linear_exr_export", "/root/reference/linear_exr_export.py")
-        mod = importlib.util.module_from_spec(spec)
-        try:
-            spec.loader.exec_module(mod)
-        except Exception as e:      # the reference needs cv2 at import time
-            pytest.skip(f"reference exporter not importable here: {e}")
-        ref = mod.LinearEXRExport
-        assert cls.INPUT_TYPES() == ref.INPUT_TYPES()
-        import inspect
-        assert list(inspect.signature(cls.export_linear_exr).parameters) == list(inspect.signature(ref.export_linear_exr).parameters)
+
+
+@pytest.mark.skipif(not reference_available(), reason="unmodified reference source not present (HDRVAE_REFERENCE_ROOT)")
+def test_node_surface_equals_reference_tree():
+    """Same INPUT_TYPES and export_linear_exr() parameters as the unmodified reference class."""
+    import importlib.util, inspect, sys, types
+    from oracle.ref_loader import REFERENCE_ROOT
+    cls = NODE_CLASS_MAPPINGS["LinearEXRExport"]
+    for name in ("pyexr", "imageio", "imageio.v3", "folder_paths"):
+        sys.modules.setdefault(name, types.ModuleType(name))
+    spec = importlib.util.spec_from_file_location("_ref_linear_exr_export",
+                                                  os.path.join(REFERENCE_ROOT, "linear_exr_export.py"))
+    mod = importlib.util.module_from_spec(spec)
+    try:
+        spec.loader.exec_module(mod)
+    except Exception as e:      # the reference needs cv2 at import time
+        pytest.skip(f"reference exporter not importable here: {e}")
+    ref = mod.LinearEXRExport
+    assert cls.INPUT_TYPES() == ref.INPUT_TYPES()
+    assert list(inspect.signature(cls.export_linear_exr).parameters) == list(inspect.signature(ref.export_linear_exr).parameters)
 
 
 @pytest.mark.skipif(cv2 is None, reason="cv2 not importable")
