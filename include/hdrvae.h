@@ -1,5 +1,5 @@
 /*
- * hdrvae.h — C ABI of libhdrvae.so: the B200 (sm_100a) Flux-VAE HDR decode path.
+ * hdrvae.h — C ABI of libhdrvae.so: the B200 (sm_100a) HDR decode path for Flux.1 and SD1.x / SDXL VAEs.
  *
  * The reference (netocg/vae-decode-hdr) has no native code and no FFI: the whole
  * path is PyTorch eager driven from hdr_vae_decode.py.  Each entry point below
@@ -144,11 +144,19 @@ int hdrvae_profile_end(const char* path_or_null);
 /* Replaces the reference's reads of vae.first_stage_model.decoder.* modules
  * (hdr_vae_decode.py:448,505-516,842,855,876): one-time repack of the state
  * dict into K-major bf16 GEMM operands (3x3 taps, upsample phase weights,
- * fused q/k/v) owned by the context. */
+ * fused q/k/v) owned by the context.
+ * The decoder's latent channel count C_z is the input-channel count of conv_in.weight (Flux.1: 16, SD1.x / SDXL: 4;
+ * 1..64).  Optionally the descriptors "post_quant_conv.weight" [C_z, C_lat, 1, 1] and "post_quant_conv.bias" [C_z]
+ * (both or neither; 1 <= C_lat <= 64): the 1x1 conv of vae.first_stage_model that SD-family AutoencoderKL applies to the
+ * latent before the decoder.  The decode entry points then take latents of C_lat channels and apply it first. */
 int hdrvae_load_weights(hdrvae_ctx* ctx, const hdrvae_weight_desc* descs, int n, int precision);
 
+/* Channels C_lat of the latents the decode entry points take (post_quant_conv's input channels, else conv_in's):
+ * 16 for Flux.1, 4 for SD1.x / SDXL.  <0 before hdrvae_load_weights succeeded. */
+int hdrvae_latent_channels(const hdrvae_ctx* ctx);
+
 /* Bytes of caller-provided device workspace hdrvae_decode needs for a latent
- * batch [B,16,h,w].  The workspace pointer must be 256-byte aligned (what
+ * batch [B,C_lat,h,w].  The workspace pointer must be 256-byte aligned (what
  * cudaMalloc and torch's allocator return). */
 int hdrvae_workspace_bytes(hdrvae_ctx* ctx, int B, int h, int w, size_t* bytes);
 
@@ -156,7 +164,7 @@ int hdrvae_workspace_bytes(hdrvae_ctx* ctx, int B, int h, int w, size_t* bytes);
  * Replaces HDRVAEDecode.simple_hdr_decode's happy path (hdr_vae_decode.py:62-195):
  * analyze_conv_out (:837) + intelligent_hdr_decode (:1009) + multiplier (:180) +
  * _format_tensor passthrough (:209-212,:354), with ONE decoder pass.
- *   latent_nchw : device float32 [B,16,h,w]            (:78)
+ *   latent_nchw : device float32 [B,C_lat,h,w]         (:78; C_lat = hdrvae_latent_channels)
  *   out_bhwc    : device float32 [B,8h,8w,3] contiguous (:195)
  *   expansion_factor : smart_hdr_expansion factor (1.0 for "conservative" as the
  *                 reference calls it, 3.0 for the README "moderate" alias)
@@ -208,7 +216,7 @@ typedef struct hdrvae_exchange {
 typedef struct hdrvae_rows hdrvae_rows;
 
 int hdrvae_rows_workspace_bytes(hdrvae_ctx* ctx, int h, int w, int world, size_t* bytes);
-/* latent_full_nchw: device float32 [1,16,h,w] (the whole latent, every rank has it; 16 MB at 4096^2);
+/* latent_full_nchw: device float32 [1,C_lat,h,w] (the whole latent, every rank has it; 16 MB at 4096^2 for Flux);
  * out_rows: device float32 [1, 8h/world, 8w, 3] = this rank's rows of the IMAGE. */
 int hdrvae_rows_begin(hdrvae_ctx* ctx, const float* latent_full_nchw, int h, int w, int rank, int world, int mode,
                       float expansion_factor, float ev_multiplier, float* out_rows, void* workspace,

@@ -73,6 +73,7 @@ SIGNATURES = {
     "hdrvae_profile_begin": (_i, []),
     "hdrvae_profile_end": (_i, [C.c_char_p]),
     "hdrvae_load_weights": (_i, [_vp, C.POINTER(HdrvaeWeightDesc), _i, _i]),
+    "hdrvae_latent_channels": (_i, [_vp]),
     "hdrvae_workspace_bytes": (_i, [_vp, _i, _i, _i, C.POINTER(_sz)]),
     "hdrvae_decode": (_i, [_vp, _vp, _i, _i, _i, _i, _f, _f, _vp, C.POINTER(HdrvaeStats), _vp, _sz, _vp]),
     "hdrvae_decode_begin": (_i, [_vp, _vp, _i, _i, _i, _vp, _sz, C.POINTER(_vp), _vp]),

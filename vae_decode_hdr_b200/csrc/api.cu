@@ -269,7 +269,8 @@ struct Plan {
 static constexpr long long kScoreBudgetElems = 1024ll << 20;  // fp32 score chunk <= 4 GiB (K and V^T are re-read once per chunk)
 static constexpr int kSplitRowsBudget = 65536;                // rows x splits of fp32 PV partials (128 MiB)
 
-static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = false, bool attn_scratch = true) {
+// c_lat: channels of the caller's latent (sizes the graph-input copy)
+static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = false, bool attn_scratch = true, int c_lat = 16) {
   Plan pl;
   const size_t km = high ? 3 : 1;                              // hi|lo|hi operands are 3x as wide
   pl.B = B; pl.h = h; pl.w = w;
@@ -310,7 +311,7 @@ static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = f
   pl.kpart_bytes = attn_only && ksp > 1 ? (size_t)B * pl.T * (512 + 2) * 4 * ksp : 0;
   pl.off_kpart = take(pl.kpart_bytes);
   pl.off_epi = take(attn_only ? 0 : epilogue_scratch_bytes(B, 8 * h, 8 * w));
-  pl.off_lat_in = take(attn_only ? 0 : (size_t)B * 16 * pl.T * 4);          // graph input: fp32 latent copy
+  pl.off_lat_in = take(attn_only ? 0 : (size_t)B * c_lat * pl.T * 4);       // graph input: fp32 latent copy
   pl.off_img = take(attn_only ? 0 : (size_t)B * 64 * pl.T * 3 * 4);        // graph output: fp32 BHWC image
   pl.total = off;
   return pl;
@@ -671,10 +672,10 @@ static int run_decoder(hdrvae_ctx* ctx, const float* latent, const Plan& pl, uin
 
   if (ctx->high) {
     float* latf = reinterpret_cast<float*>(ws + pl.off_f32) + (size_t)pl.Tp * 1536;
-    HDRVAE_TRY(launch_latent_to_nhwc(latent, latf, DT_F32, B, 16, H * W, 64, s));
+    HDRVAE_TRY(launch_latent_to_nhwc(latent, latf, DT_F32, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
     HDRVAE_TRY(launch_split3(latf, 64, lat, 192, (long long)B * H * W, 64, 1.f, 0, s));
   } else {
-    HDRVAE_TRY(launch_latent_to_nhwc(latent, lat, dt, B, 16, H * W, 64, s));
+    HDRVAE_TRY(launch_latent_to_nhwc(latent, lat, dt, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
   }
   {
     ConvIO io; io.x = lat; io.y = st.x; io.stats = stats_ptr(ctx, &st); io.stats_chunks = &st.pending;
@@ -990,7 +991,8 @@ static int build_rows_program(hdrvae_rows* st) {
     float* x = st->x;
     rows_compute(st, [=](cudaStream_t s) {
       // latent rows of this rank plus one neighbour row each side (rows outside the image are zero)
-      HDRVAE_TRY(launch_latent_rows_to_nhwc(latent, lat, dt, 16, pl.h, pl.w, rank * pl.hl - 1, pl.hl + 2, 64, s));
+      HDRVAE_TRY(launch_latent_rows_to_nhwc(latent, lat, dt, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, pl.h, pl.w,
+                                            rank * pl.hl - 1, pl.hl + 2, 64, s));
       HDRVAE_TRY(gn_scratch_reset(stats, 1, pl.gn_chunks, s));
       ConvIO io; io.x = lat; io.y = x; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
       if (x16) { io.y_dtype = x_dt; io.y_scale = x_scale; }
@@ -1153,6 +1155,11 @@ int hdrvae_set_conv_impl(hdrvae_ctx* ctx, int impl) {
   return 0;
 }
 
+int hdrvae_latent_channels(const hdrvae_ctx* ctx) {
+  HDRVAE_REQUIRE(ctx != nullptr && ctx->loaded, "hdrvae_latent_channels: weights not loaded");
+  return ctx->c_lat;
+}
+
 int hdrvae_operand_dtype(hdrvae_ctx* ctx) { return ctx ? ctx->op_dtype : -1; }
 int hdrvae_features_dtype(hdrvae_ctx* ctx) { return ctx ? (ctx->high ? DT_F32 : ctx->op_dtype) : -1; }
 
@@ -1228,7 +1235,27 @@ int hdrvae_load_weights(hdrvae_ctx* ctx, const hdrvae_weight_desc* descs, int n,
     return 0;
   };
 
-  HDRVAE_TRY(conv("conv_in", 512, 16, 3, false, op, &ctx->conv_in));
+  {
+    // latent channels from the weights: conv_in's input (Flux 16, SD1.x / SDXL 4), and post_quant_conv's input when the
+    // first-stage model has one (a 1x1 conv with bias that SD-family AutoencoderKL applies to the latent before the decoder)
+    auto it = ctx->shapes.find("conv_in.weight");
+    const int cz = it != ctx->shapes.end() && it->second.size() == 4 ? (int)it->second[1] : 16;
+    HDRVAE_REQUIRE(cz >= 1 && cz <= 64, "conv_in.weight has %d input channels (latent channels must be 1..64)", cz);
+    HDRVAE_TRY(conv("conv_in", 512, cz, 3, false, op, &ctx->conv_in));
+    ctx->c_z = ctx->c_lat = cz;
+    const bool pw = ctx->shapes.count("post_quant_conv.weight") != 0, pb = ctx->shapes.count("post_quant_conv.bias") != 0;
+    HDRVAE_REQUIRE(pw == pb, "post_quant_conv needs both weight and bias (got only its %s)", pw ? "weight" : "bias");
+    if (pw) {
+      const auto& sw = ctx->shapes["post_quant_conv.weight"];
+      const auto& sb = ctx->shapes["post_quant_conv.bias"];
+      const int cl = sw.size() == 4 ? (int)sw[1] : 0;
+      HDRVAE_REQUIRE(sw.size() == 4 && sw[0] == cz && cl >= 1 && cl <= 64 && sw[2] == 1 && sw[3] == 1 && sb.size() == 1 && sb[0] == cz,
+                     "post_quant_conv has the wrong shape (want weight [%d,C,1,1] with 1 <= C <= 64 and bias [%d])", cz, cz);
+      ctx->c_lat = cl;
+      ctx->pq_w = W("post_quant_conv.weight");
+      ctx->pq_b = W("post_quant_conv.bias");
+    }
+  }
   HDRVAE_TRY(res("mid.block_1", 512, 512, &ctx->mid1));
   HDRVAE_TRY(res("mid.block_2", 512, 512, &ctx->mid2));
   HDRVAE_TRY(norm("mid.attn_1.norm", 512, &ctx->attn_norm));
@@ -1286,8 +1313,8 @@ int hdrvae_load_weights(hdrvae_ctx* ctx, const hdrvae_weight_desc* descs, int n,
 
 int hdrvae_workspace_bytes(hdrvae_ctx* ctx, int B, int h, int w, size_t* bytes) {
   HDRVAE_REQUIRE(ctx != nullptr && bytes != nullptr, "hdrvae_workspace_bytes: null argument");
-  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_workspace_bytes: empty latent batch [%d,16,%d,%d]", B, h, w);
-  *bytes = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx)).total;
+  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_workspace_bytes: empty latent batch [%d,%d,%d,%d]", B, ctx->c_lat, h, w);
+  *bytes = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat).total;
   return 0;
 }
 
@@ -1344,9 +1371,9 @@ static int run_segment(hdrvae_ctx* ctx, hdrvae_ctx::GraphEntry key, cudaStream_t
 int hdrvae_decode_begin(hdrvae_ctx* ctx, const float* latent, int B, int h, int w, void* workspace, size_t ws_bytes,
                         void** raw_stats_dev, void* stream) {
   HDRVAE_REQUIRE(ctx != nullptr && latent != nullptr, "hdrvae_decode: null argument");
-  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode: empty latent batch [%d,16,%d,%d]", B, h, w);
+  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode: empty latent batch [%d,%d,%d,%d]", B, ctx->c_lat, h, w);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx));
+  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
@@ -1358,7 +1385,7 @@ int hdrvae_decode_begin(hdrvae_ctx* ctx, const float* latent, int B, int h, int 
   };
   if (graphs_enabled(ctx, s)) {
     float* lat_in = reinterpret_cast<float*>(ws + pl.off_lat_in);
-    HDRVAE_CUDA_OK(cudaMemcpyAsync(lat_in, latent, (size_t)B * 16 * pl.T * 4, cudaMemcpyDeviceToDevice, s));
+    HDRVAE_CUDA_OK(cudaMemcpyAsync(lat_in, latent, (size_t)B * ctx->c_lat * pl.T * 4, cudaMemcpyDeviceToDevice, s));
     hdrvae_ctx::GraphEntry key{0, B, h, w, 0, ctx->conv_impl, ctx->cta_group, 0.f, 0.f, workspace, nullptr, 0};
     HDRVAE_TRY(run_segment(ctx, key, s, [&]() { return body(lat_in); }));
   } else {
@@ -1373,7 +1400,7 @@ int hdrvae_decode_finish(hdrvae_ctx* ctx, int B, int h, int w, int mode, float e
   HDRVAE_REQUIRE(ctx != nullptr && out_bhwc != nullptr, "hdrvae_decode: null argument");
   HDRVAE_REQUIRE(mode >= 0 && mode <= 3, "hdrvae_decode: bad mode %d", mode);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx));
+  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
@@ -1400,7 +1427,7 @@ int hdrvae_decode(hdrvae_ctx* ctx, const float* latent, int B, int h, int w, int
                   float ev_multiplier, float* out_bhwc, hdrvae_stats* stats, void* workspace, size_t ws_bytes,
                   void* stream) {
   HDRVAE_REQUIRE(ctx != nullptr && latent != nullptr && out_bhwc != nullptr, "hdrvae_decode: null argument");
-  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode: empty latent batch [%d,16,%d,%d]", B, h, w);
+  HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode: empty latent batch [%d,%d,%d,%d]", B, ctx->c_lat, h, w);
   HDRVAE_REQUIRE(mode >= 0 && mode <= 3, "hdrvae_decode: bad mode %d", mode);
   HDRVAE_TRY(hdrvae_decode_begin(ctx, latent, B, h, w, workspace, ws_bytes, nullptr, stream));
   return hdrvae_decode_finish(ctx, B, h, w, mode, expansion_factor, ev_multiplier, out_bhwc, stats, workspace, ws_bytes, stream);
@@ -1584,7 +1611,7 @@ int hdrvae_decode_features(hdrvae_ctx* ctx, const float* latent, int B, int h, i
   HDRVAE_REQUIRE(ctx != nullptr && latent != nullptr && features != nullptr, "hdrvae_decode_features: null argument");
   HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode_features: empty latent batch");
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx));
+  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   void* feat = nullptr;

@@ -19,9 +19,12 @@ int launch_pack_weight(const float* w, void* out, int out_dtype, int cout, int c
 int launch_add_vectors(const float* a, const float* b, float* c, int n, cudaStream_t s);
 int launch_split3(const float* x, long long x_ld, void* out, long long out_ld, long long n, int C, float scale, int order,
                   cudaStream_t s);
-int launch_latent_to_nhwc(const float* z, void* out, int out_dtype, int B, int C, int HW, int cpad, cudaStream_t s);
-int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, int h, int w, int y0, int rows, int cpad,
-                               cudaStream_t s);
+// Latent staging: z [B][C_lat][HW] fp32 -> NHWC [B][HW][cpad] holding C channels, with post_quant_conv applied when
+// pq_w ([C][C_lat]) and pq_b ([C]) are given (otherwise C_lat == C and z is copied).
+int launch_latent_to_nhwc(const float* z, void* out, int out_dtype, int B, int C, int C_lat, const float* pq_w,
+                          const float* pq_b, int HW, int cpad, cudaStream_t s);
+int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, int C_lat, const float* pq_w,
+                               const float* pq_b, int h, int w, int y0, int rows, int cpad, cudaStream_t s);
 int launch_softmax_rows(const float* s, void* p, int p_dtype, float* inv_sum, int n_rows, int n_valid, int n_pad,
                         long long s_ld, long long p_ld, cudaStream_t st);
 int launch_attn_row_parts(const float* part, int rows, int parts, int mode, float* out, cudaStream_t st);
@@ -160,6 +163,10 @@ struct hdrvae_ctx {
   std::vector<void*> owned;                       // every device allocation of the context
   std::map<std::string, float*> raw;              // fp32 device copies of the state dict
   std::map<std::string, std::vector<int64_t>> shapes;
+  int c_z = 16;                                   // input channels of conv_in (Flux 16, SD1.x / SDXL 4)
+  int c_lat = 16;                                 // channels of the caller's latent: post_quant_conv's input, else c_z
+  const float* pq_w = nullptr;                    // post_quant_conv (1x1, fp32 [c_z][c_lat] + bias [c_z]) or null
+  const float* pq_b = nullptr;
   PackedConv conv_in, qk, vproj, proj_out;
   NormW attn_norm, norm_out;
   ResW mid1, mid2, up[4][3];

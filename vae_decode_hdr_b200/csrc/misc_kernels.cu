@@ -99,34 +99,49 @@ int launch_pack_weight(const float* w, void* out, int out_dtype, int cout, int c
 }
 
 // ------------------------------------------------------------------ latent NCHW fp32 -> NHWC bf16 (channels zero-padded)
+// Channel c of one latent pixel as conv_in sees it.  zp points at the pixel's channel 0, channels `cstride` apart.  With
+// post_quant_conv (SD1.x / SDXL first-stage models): y[c] = b[c] + sum_c' W[c][c'] z[c'] in fp32, fmaf in the fixed order
+// c' = 0 .. C_lat-1; without it the latent itself.
+__device__ __forceinline__ float staged_latent(const float* __restrict__ zp, long long cstride, int c, int C_lat,
+                                               const float* __restrict__ pq_w, const float* __restrict__ pq_b) {
+  if (pq_w == nullptr) return zp[c * cstride];
+  float v = pq_b[c];
+  for (int k = 0; k < C_lat; ++k) v = fmaf(pq_w[c * C_lat + k], zp[k * cstride], v);
+  return v;
+}
+
 __global__ void latent_to_nhwc_kernel(const float* __restrict__ z, void* __restrict__ out, int out_dtype, int B, int C,
-                                      int HW, int cpad) {
+                                      int C_lat, const float* __restrict__ pq_w, const float* __restrict__ pq_b, int HW,
+                                      int cpad) {
   const long long total = (long long)B * HW * cpad;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int c = (int)(i % cpad);
     const long long p = i / cpad;
     const int hw = (int)(p % HW);
     const int b = (int)(p / HW);
-    const float v = c < C ? z[((long long)b * C + c) * HW + hw] : 0.f;
+    const float v = c < C ? staged_latent(z + (long long)b * C_lat * HW + hw, HW, c, C_lat, pq_w, pq_b) : 0.f;
     if (out_dtype == DT_F32) reinterpret_cast<float*>(out)[i] = v;
     else if (out_dtype == DT_BF16) reinterpret_cast<__nv_bfloat16*>(out)[i] = __float2bfloat16_rn(v);
     else reinterpret_cast<__half*>(out)[i] = __float2half_rn(v);
   }
 }
-int launch_latent_to_nhwc(const float* z, void* out, int out_dtype, int B, int C, int HW, int cpad, cudaStream_t s) {
+int launch_latent_to_nhwc(const float* z, void* out, int out_dtype, int B, int C, int C_lat, const float* pq_w,
+                          const float* pq_b, int HW, int cpad, cudaStream_t s) {
   const long long total = (long long)B * HW * cpad;
   int grid = ceil_div(total, 256);
   if (grid > 2368) grid = 2368;
-  latent_to_nhwc_kernel<<<grid, 256, 0, s>>>(z, out, out_dtype, B, C, HW, cpad);
+  latent_to_nhwc_kernel<<<grid, 256, 0, s>>>(z, out, out_dtype, B, C, C_lat, pq_w, pq_b, HW, cpad);
   HDRVAE_LAUNCHED();
   HDRVAE_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
 // ------------------------------------------------------------------ latent row slab (row tiling)
-// full latent NCHW fp32 [C][h][w] -> NHWC 16-bit slab [rows][w][cpad] holding latent rows y0 .. y0+rows-1;
-// rows outside the image and the padding channels are zero.
+// full latent NCHW fp32 [C_lat][h][w] -> NHWC 16-bit slab [rows][w][cpad] holding latent rows y0 .. y0+rows-1 (after
+// post_quant_conv, if any); rows outside the image and the padding channels are zero — conv_in's zero padding applies
+// to post_quant_conv's output, so its bias must not reach those rows.
 __global__ void latent_rows_to_nhwc_kernel(const float* __restrict__ z, void* __restrict__ out, int out_dtype, int C,
+                                           int C_lat, const float* __restrict__ pq_w, const float* __restrict__ pq_b,
                                            int h, int w, int y0, int rows, int cpad) {
   const long long total = (long long)rows * w * cpad;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -134,17 +149,18 @@ __global__ void latent_rows_to_nhwc_kernel(const float* __restrict__ z, void* __
     const long long p = i / cpad;
     const int x = (int)(p % w);
     const int y = y0 + (int)(p / w);
-    const float v = (c < C && y >= 0 && y < h) ? z[((long long)c * h + y) * w + x] : 0.f;
+    const float v = (c < C && y >= 0 && y < h) ? staged_latent(z + (long long)y * w + x, (long long)h * w, c, C_lat, pq_w, pq_b)
+                                               : 0.f;
     if (out_dtype == DT_BF16) reinterpret_cast<__nv_bfloat16*>(out)[i] = __float2bfloat16_rn(v);
     else reinterpret_cast<__half*>(out)[i] = __float2half_rn(v);
   }
 }
-int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, int h, int w, int y0, int rows, int cpad,
-                               cudaStream_t s) {
+int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, int C_lat, const float* pq_w,
+                               const float* pq_b, int h, int w, int y0, int rows, int cpad, cudaStream_t s) {
   const long long total = (long long)rows * w * cpad;
   int grid = ceil_div(total, 256);
   if (grid > 2368) grid = 2368;
-  latent_rows_to_nhwc_kernel<<<grid, 256, 0, s>>>(z, out, out_dtype, C, h, w, y0, rows, cpad);
+  latent_rows_to_nhwc_kernel<<<grid, 256, 0, s>>>(z, out, out_dtype, C, C_lat, pq_w, pq_b, h, w, y0, rows, cpad);
   HDRVAE_LAUNCHED();
   HDRVAE_CUDA_OK(cudaGetLastError());
   return 0;

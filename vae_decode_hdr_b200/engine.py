@@ -89,6 +89,9 @@ class HdrVaeEngine:
             N.check(self.lib.hdrvae_load_weights(self._ctx, arr, len(descs), PRECISIONS[self.precision]),
                     "hdrvae_load_weights")
         self.operand_dtype = _ID_DTYPE[self.lib.hdrvae_operand_dtype(self._ctx)]
+        # channels of the latents this engine decodes: 16 for Flux.1, 4 for SD1.x / SDXL (post_quant_conv's input when the
+        # state dict carries post_quant_conv.{weight,bias}, else conv_in's)
+        self.latent_channels = self.lib.hdrvae_latent_channels(self._ctx)
         self.features_dtype = _ID_DTYPE[self.lib.hdrvae_features_dtype(self._ctx)]
 
     def set_conv_impl(self, impl: int) -> None:
@@ -119,10 +122,9 @@ class HdrVaeEngine:
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
 
-    @staticmethod
-    def _check_latent(latent: torch.Tensor) -> Tuple[int, int, int]:
-        if latent.dim() != 4 or latent.shape[1] != 16:
-            raise ValueError(f"expected a Flux latent [B,16,h,w], got {tuple(latent.shape)}")
+    def _check_latent(self, latent: torch.Tensor) -> Tuple[int, int, int]:
+        if latent.dim() != 4 or latent.shape[1] != self.latent_channels:
+            raise ValueError(f"expected a latent [B,{self.latent_channels},h,w] for this VAE, got {tuple(latent.shape)}")
         B, _, h, w = latent.shape
         if B == 0 or h == 0 or w == 0:
             raise ValueError(f"empty latent batch {tuple(latent.shape)}")
@@ -131,7 +133,7 @@ class HdrVaeEngine:
     # -- the hot path ----------------------------------------------------------------------------
     def decode(self, latent: torch.Tensor, hdr_mode: str = DEFAULT_MODE, ev_multiplier: float = 1.0,
                want_stats: bool = True, out: Optional[torch.Tensor] = None):
-        """latent: float32 [B,16,h,w] on this engine's device -> (float32 [B,8h,8w,3], stats dict|None)."""
+        """latent: float32 [B,latent_channels,h,w] on this engine's device -> (float32 [B,8h,8w,3], stats dict|None)."""
         B, h, w = self._check_latent(latent)
         mode, factor = resolve_mode(hdr_mode)
         with torch.cuda.device(self.device):

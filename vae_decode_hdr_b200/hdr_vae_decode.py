@@ -33,13 +33,35 @@ def _decoder_of(vae: Any):
     try:
         return vae.first_stage_model.decoder          # hdr_vae_decode.py:842
     except AttributeError as e:
-        raise RuntimeError("HDRVAEDecode: vae.first_stage_model.decoder not found (not a Flux/SD-style VAE)") from e
+        raise RuntimeError("HDRVAEDecode: vae.first_stage_model.decoder not found (not a Flux.1 / SD1.x / SDXL-style "
+                           "AutoencoderKL VAE)") from e
 
 
-def _weights_key(decoder) -> Tuple:
-    """Identity + in-place-modification fingerprint of EVERY parameter (storage address, version counter, size).  The
-    id() half is safe against reuse because an engine never outlives its decoder (weakref.finalize below)."""
-    ps = list(decoder.parameters())
+def _post_quant_conv_of(vae: Any) -> Optional[torch.nn.Module]:
+    """SD1.x / SDXL first-stage models apply post_quant_conv (1x1 conv, 4 -> 4 channels) to the latent before the decoder;
+    Flux's has none (absent, None or nn.Identity)."""
+    m = getattr(getattr(vae, "first_stage_model", None), "post_quant_conv", None)
+    w = getattr(m, "weight", None)
+    if isinstance(m, torch.nn.Module) and isinstance(w, torch.Tensor) and w.dim() == 4:
+        return m
+    return None
+
+
+def _engine_state_dict(decoder, pqc: Optional[torch.nn.Module]) -> Dict[str, torch.Tensor]:
+    """The decoder's state dict plus post_quant_conv.{weight,bias} (a bias-less conv sends zeros)."""
+    sd = dict(decoder.state_dict())
+    if pqc is not None:
+        sd["post_quant_conv.weight"] = pqc.weight.detach()
+        b = pqc.bias
+        sd["post_quant_conv.bias"] = b.detach() if b is not None else pqc.weight.new_zeros(pqc.weight.shape[0])
+    return sd
+
+
+def _weights_key(decoder, pqc: Optional[torch.nn.Module] = None) -> Tuple:
+    """Identity + in-place-modification fingerprint of EVERY parameter of the decoder and of post_quant_conv (storage
+    address, version counter, size).  The id() half is safe against reuse because an engine never outlives its decoder
+    (weakref.finalize below)."""
+    ps = list(decoder.parameters()) + (list(pqc.parameters()) if pqc is not None else [])
     return (id(decoder), len(ps), hash(tuple((p.data_ptr(), p._version, p.numel()) for p in ps)))
 
 
@@ -117,13 +139,13 @@ class HDRVAEDecode:
 
     @classmethod
     def _engine_for(cls, vae: Any, device: torch.device) -> HdrVaeEngine:
-        decoder = _decoder_of(vae)
-        key = (_weights_key(decoder), str(device))
+        decoder, pqc = _decoder_of(vae), _post_quant_conv_of(vae)
+        key = (_weights_key(decoder, pqc), str(device))
         eng = cls._engines.get(key)
         if eng is None:
             for k in [k for k in cls._engines if k[0][0] == id(decoder) and k[1] == str(device)]:
                 cls._evict(k)                          # weights changed in place: repack
-            eng = HdrVaeEngine(decoder.state_dict(), device)
+            eng = HdrVaeEngine(_engine_state_dict(decoder, pqc), device)
             cls._register(decoder, key, eng)
         else:
             cls._engines.move_to_end(key)
@@ -142,9 +164,10 @@ class HDRVAEDecode:
 
     @classmethod
     def adopt_engine(cls, vae: Any, device, engine: HdrVaeEngine) -> None:
-        """Register an already-built engine for this vae's decoder weights (avoids a second repack)."""
+        """Register an already-built engine for this vae's decoder (and post_quant_conv) weights (avoids a second
+        repack)."""
         decoder = _decoder_of(vae)
-        cls._register(decoder, (_weights_key(decoder), str(torch.device(device))), engine)
+        cls._register(decoder, (_weights_key(decoder, _post_quant_conv_of(vae)), str(torch.device(device))), engine)
 
     @classmethod
     def release_memory(cls, keep_weights: bool = True) -> None:

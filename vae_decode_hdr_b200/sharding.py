@@ -117,9 +117,10 @@ def decode_batch_sharded(engine, latent_local: torch.Tensor, hdr_mode: str, ev_m
     distributed = dist.is_initialized() and dist.get_world_size(group) > 1
     if distributed:
         _validate_across_ranks(latent_local, hdr_mode, ev_multiplier, group)
+    # after the validation: every rank holds the same shape, so either all ranks raise here or none does
+    if latent_local.dim() != 4 or latent_local.shape[1] != engine.latent_channels:
+        raise ValueError(f"expected a latent [B,{engine.latent_channels},h,w] for this VAE, got {tuple(latent_local.shape)}")
     if latent_local.shape[0] == 0:
-        if latent_local.dim() != 4 or latent_local.shape[1] != 16:
-            raise ValueError(f"expected a Flux latent [B,16,h,w], got {tuple(latent_local.shape)}")
         if distributed:
             exchange_raw_stats_block(identity_raw_block(engine.device), engine.lib, group)
         h, w = latent_local.shape[2:]

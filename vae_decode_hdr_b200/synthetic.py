@@ -5,15 +5,16 @@ for real checkpoints (BASELINE.json: "random-init Flux AE weights and synthetic 
 from __future__ import annotations
 
 import math
-from typing import Dict, Iterator, List, Tuple
+from typing import Dict, Iterator, List, Optional, Tuple
 
 import torch
 
 CH, CH_MULT, Z = 128, (1, 2, 4, 4), 16
 
 
-def decoder_param_shapes() -> List[Tuple[str, Tuple[int, ...]]]:
-    """State-dict keys/shapes of the Flux.1 AE decoder (BFL / ComfyUI naming; SURVEY.md §8b)."""
+def decoder_param_shapes(z_channels: int = Z) -> List[Tuple[str, Tuple[int, ...]]]:
+    """State-dict keys/shapes of the Flux.1 AE decoder (BFL / ComfyUI naming; SURVEY.md §8b); z_channels = 4 gives the
+    SD1.x / SDXL decoder (same graph, conv_in 4 -> 512)."""
     out: List[Tuple[str, Tuple[int, ...]]] = []
 
     def conv(name, cout, cin, k):
@@ -31,7 +32,7 @@ def decoder_param_shapes() -> List[Tuple[str, Tuple[int, ...]]]:
             conv(f"{name}.nin_shortcut", cout, cin, 1)
 
     top = CH * CH_MULT[-1]
-    conv("conv_in", top, Z, 3)
+    conv("conv_in", top, z_channels, 3)
     res("mid.block_1", top, top)
     norm("mid.attn_1.norm", top)
     for n in ("q", "k", "v", "proj_out"):
@@ -50,12 +51,12 @@ def decoder_param_shapes() -> List[Tuple[str, Tuple[int, ...]]]:
     return out
 
 
-def random_decoder_state_dict(seed: int = 0) -> Dict[str, torch.Tensor]:
+def random_decoder_state_dict(seed: int = 0, z_channels: int = Z) -> Dict[str, torch.Tensor]:
     """PyTorch-default-style init (conv weight/bias ~ U(+-1/sqrt(fan_in)), GroupNorm 1/0), fp32, CPU."""
     g = torch.Generator(device="cpu").manual_seed(seed)
     sd: Dict[str, torch.Tensor] = {}
     fan_in = 1
-    for name, shape in decoder_param_shapes():
+    for name, shape in decoder_param_shapes(z_channels):
         if len(shape) == 4:
             fan_in = shape[1] * shape[2] * shape[3]
             bound = 1.0 / math.sqrt(fan_in)
@@ -82,16 +83,20 @@ class _DecoderBag(torch.nn.Module):
 
 
 class _FirstStage:
-    def __init__(self, decoder):
+    def __init__(self, decoder, post_quant_conv=None):
         self.decoder = decoder
+        if post_quant_conv is not None:
+            self.post_quant_conv = post_quant_conv
 
 
 class SyntheticVAE:
     """The attributes of comfy.sd.VAE the node touches; ``output_device`` is where the IMAGE lands
-    (ComfyUI: the intermediate device, normally CPU)."""
+    (ComfyUI: the intermediate device, normally CPU).  ``post_quant_conv``: the 1x1 conv an SD1.x / SDXL first-stage
+    model applies to the latent before the decoder (Flux: None)."""
 
-    def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda", output_device="cpu"):
-        self.first_stage_model = _FirstStage(_DecoderBag(state_dict))
+    def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda", output_device="cpu",
+                 post_quant_conv: Optional[torch.nn.Module] = None):
+        self.first_stage_model = _FirstStage(_DecoderBag(state_dict), post_quant_conv)
         self.device = torch.device(device)
         self.output_device = torch.device(output_device)
 
