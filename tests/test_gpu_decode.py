@@ -263,17 +263,42 @@ torch.save({"img": img.cpu(), "feat": feat.cpu()}, sys.argv[1])
 """
 
 
-def _decode_in_child(tmp_path, name, env_extra):
+_ROWS_CHILD = r"""
+import sys, torch
+sys.path.insert(0, ".")
+from oracle.flux_decoder import build_decoder, make_latent
+from vae_decode_hdr_b200.engine import HdrVaeEngine
+from vae_decode_hdr_b200.sharding import decode_rows_emulated
+eng = HdrVaeEngine(build_decoder(0).state_dict(), "cuda:0")
+z = make_latent(1, 32, 8, seed=43).to("cuda:0")
+tiled, _ = decode_rows_emulated(eng, z, 2, "moderate")
+whole, _ = eng.decode(z, "moderate")
+torch.save({"tiled": tiled.cpu(), "whole": whole.cpu()}, sys.argv[1])
+"""
+
+
+def _decode_in_child(tmp_path, name, env_extra, script=_SWITCH_CHILD):
     """The numeric-plan switches are read once per process, so the other setting runs in a child process."""
     import os
     import subprocess
     import sys
     out = tmp_path / name
     env = dict(os.environ, **env_extra)
-    r = subprocess.run([sys.executable, "-c", _SWITCH_CHILD, str(out)], env=env, capture_output=True, text=True, timeout=300,
+    r = subprocess.run([sys.executable, "-c", script, str(out)], env=env, capture_output=True, text=True, timeout=300,
                        cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     assert r.returncode == 0, r.stderr[-2000:]
     return torch.load(out)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("env", [{}, {"HDRVAE_FUSE_GN": "0"}, {"HDRVAE_X16": "0"}, {"HDRVAE_FUSE_NIN": "0"}, {"HDRVAE_H16": "0"}],
+                         ids=["default", "fuse_gn_0", "x16_0", "fuse_nin_0", "h16_0"])
+def test_row_tiled_decode_equals_single_gpu_under_each_numeric_plan(tmp_path, env):
+    """Row tiling must store every tensor as the single-GPU decode does under every numeric-plan setting: on the exact-tiling
+    shape of test_row_tiled_decode_equals_single_gpu (32x8 latent on 2 virtual ranks) the images agree to the same 1e-6."""
+    r = _decode_in_child(tmp_path, "rows.pt", env, _ROWS_CHILD)
+    assert r["tiled"].shape == r["whole"].shape
+    assert _rel(r["tiled"], r["whole"]) < 1e-6, _rel(r["tiled"], r["whole"])
 
 
 @pytest.mark.gpu

@@ -3,11 +3,14 @@
 // drives through vae.decode (hdr_vae_decode.py:859,:1022; graph in SURVEY.md §8 a3).
 //
 // Numeric plan (DESIGN.md "Precision"): tensor-core operands are 16-bit (fp16 by default, bf16 selectable)
-// for everything that is normalised or bounded (GroupNorm outputs, weights, attention q/k/v/probabilities);
-// the un-normalised residual stream x and the conv1 outputs h stay fp32 in HBM; the five convs that consume
-// the raw stream (3 upsample convs, 2 nin_shortcuts) read a 16-bit copy of it scaled by 2^-4 that the producing
-// conv's epilogue writes next to the fp32 tensor (kind::tf32 on the fp32 tensor itself is also implemented in
-// gemm_tc.cu and reachable through hdrvae_conv2d, at half the MMA rate).
+// for everything that is normalised or bounded (GroupNorm outputs, weights, attention q/k/v/probabilities).
+// The un-normalised tensors are stored in the 16-bit operand type scaled by 2^-4 on the tcgen05 kernels: the conv1
+// outputs h (h_is_16bit), and with fp16 operands the residual stream x too (x_is_16bit), which the five convs that
+// consume the raw stream (3 upsample convs, 2 nin_shortcuts fused into conv2) then read directly.  An fp32 x (bf16 and
+// high precision, the validation kernels, HDRVAE_X16=0) comes with a scaled 16-bit copy that the producing conv's
+// epilogue writes next to it for those convs (kind::tf32 on the fp32 tensor itself is also implemented in gemm_tc.cu and
+// reachable through hdrvae_conv2d, at half the MMA rate).  The single-GPU and the row-tiled decode are issued by one
+// layer program (Decoder below).
 #include <stdarg.h>
 #include <string.h>
 
@@ -269,6 +272,20 @@ struct Plan {
 static constexpr long long kScoreBudgetElems = 1024ll << 20;  // fp32 score chunk <= 4 GiB (K and V^T are re-read once per chunk)
 static constexpr int kSplitRowsBudget = 65536;                // rows x splits of fp32 PV partials (128 MiB)
 
+// Rows of one score / probability chunk of the GEMM-level attention (n_q query rows against Tp keys), and the GroupNorm
+// partial chunks per image that the decoder's convs can write for an h x w latent (convs == false: no convs).
+static void chunk_sizes(int n_q, int Tp, int h, int w, bool convs, int* s_rows, int* gn_chunks) {
+  long long rows = kScoreBudgetElems / Tp;
+  rows = rows / 128 * 128;
+  if (rows < 128) rows = 128;
+  const long long q128 = (n_q + 127) / 128 * 128;
+  if (rows > q128) rows = q128;
+  *s_rows = (int)rows;
+  *gn_chunks = 1184;
+  if (convs)
+    for (int l = 1; l <= 8; l *= 2) *gn_chunks = std::max(*gn_chunks, 4 * tiles_for(l * h, l * w));
+}
+
 // c_lat: channels of the caller's latent (sizes the graph-input copy)
 static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = false, bool attn_scratch = true, int c_lat = 16) {
   Plan pl;
@@ -276,15 +293,7 @@ static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = f
   pl.B = B; pl.h = h; pl.w = w;
   pl.T = h * w;
   pl.Tp = (pl.T + 63) / 64 * 64;
-  long long rows = kScoreBudgetElems / pl.Tp;
-  rows = rows / 128 * 128;
-  if (rows < 128) rows = 128;
-  const long long t128 = (pl.T + 127) / 128 * 128;
-  if (rows > t128) rows = t128;
-  pl.s_rows = (int)rows;
-  pl.gn_chunks = 1184;
-  if (!attn_only)
-    for (int l = 1; l <= 8; l *= 2) pl.gn_chunks = std::max(pl.gn_chunks, 4 * tiles_for(l * h, l * w));
+  chunk_sizes(pl.T, pl.Tp, h, w, !attn_only, &pl.s_rows, &pl.gn_chunks);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes, 1024); return o; };
   const size_t widest = attn_only ? 0 : (size_t)B * pl.T * 64 * 256;   // elements of [B, 8h, 8w, 256]
@@ -317,35 +326,11 @@ static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = f
   return pl;
 }
 
-// ---- decoder layer program ------------------------------------------------------------------------
+// ---- numeric plan ---------------------------------------------------------------------------------
 // Un-normalised tensors that feed a conv directly (upsample convs, nin_shortcuts) are handed over as a
 // 16-bit copy scaled by 2^-4: fp16 then covers |x| < 1e6 (no overflow for any sane activation) and loses
 // precision only below 1e-3 (absolute error < 5e-7); the consuming conv multiplies its accumulator by 2^4.
 static constexpr float kRawOperandScale = 1.0f / 16.0f;
-
-struct DecState {
-  void* xa16;      // scaled 16-bit copy of a level's last ResBlock output = operand of the level's upsample conv
-  void* xb16;      // scaled 16-bit copy of an upsample conv's output = operand of the next block's nin_shortcut
-  float* x;        // residual stream (fp32)
-  float* hbuf;     // block-internal fp32 tensor
-  void* t;         // 16-bit operand buffer
-  void* gn;        // GroupNorm scratch (partials | scale | shift)
-  int gn_chunks;   // capacity of the partial area (chunks per image)
-  int pending;     // partial chunks per image currently valid for the tensor about to be normalised
-  int x_dt = DT_F32;      // element type of the residual stream: fp32, or the operand type scaled by x_scale (x_is_16bit)
-  float x_scale = 1.f;
-};
-
-static int run_gn(hdrvae_ctx* ctx, const void* x, int x_dtype, void* y, int B, int HW, const NormW& nw, bool silu,
-                  DecState* st, cudaStream_t s, int y_dtype = -1, float in_scale = 1.f) {
-  char pname[64];
-  snprintf(pname, sizeof pname, "groupnorm%s C=%d @%dx%d", silu ? "+silu" : "", nw.C, B, HW);
-  ProfScope prof(pname, 0.0, (double)B * HW * nw.C * (dt_bytes(x_dtype) * (st->pending > 0 ? 1 : 2) + 2.0), s);
-  const int partials = st->pending;
-  st->pending = 0;
-  return launch_groupnorm(x, x_dtype, y, y_dtype >= 0 ? y_dtype : (ctx->high ? DT_F16X3 : ctx->op_dtype), B, HW, nw.C, nw.gamma,
-                          nw.beta, silu, st->gn, st->gn_chunks, partials, s, in_scale);
-}
 
 // The block-internal tensor h = conv1(...) is never on the residual path: it is stored ONLY as the scaled 16-bit operand
 // type (2 B instead of 4 written by conv1, 2 instead of 4 read by norm2; its GroupNorm statistics still come from the
@@ -392,80 +377,6 @@ static bool gn_is_fused(hdrvae_ctx* ctx, const PackedConv& pc, const ConvIO& io,
   return on && x_is_16bit(ctx) && x_dtype == DT_F16 && pc.w_dtype == DT_F16 && pc.kmul == 1 && !pc.upsample && pc.ks == 3 &&
          pc.cout_pad >= 256 && pc.cin_pad % 64 == 0 && ctx->cta_group != 1 && io.x2 == nullptr && io.y_dtype == DT_F16 &&
          io.stats != nullptr && conv_takes_slab(pc, io, H, W, ctx->conv_impl);
-}
-
-static float* stats_ptr(hdrvae_ctx* ctx, DecState* st) {
-  return ctx->conv_impl == HDRVAE_CONV_TCGEN05 ? reinterpret_cast<float*>(st->gn) : nullptr;
-}
-
-// GroupNorm + SiLU in front of a conv: the streaming kernel x -> t (16-bit operand, or hi|lo|hi in the high-precision mode).
-// (Round 1 also carried an experimental variant that normalised inside the conv's operand path — correct but 10 % slower,
-// DESIGN.md §8 — removed in round 2; last present in commit 93846d6.)
-static int gn_before_conv(hdrvae_ctx* ctx, const void* x, const NormW& nw, const PackedConv& pc, ConvIO* io, DecState* st,
-                          int B, int H, int W, cudaStream_t s, int x_dtype = DT_F32, float x_scale = 1.f) {
-  if (gn_is_fused(ctx, pc, *io, x_dtype, H, W)) {
-    // only the reduction of the producer's partials runs as a kernel (-> per-(image, channel) scale / shift); the conv's
-    // transform warps normalise the scaled fp16 tensor as it lands in shared memory: no normalised copy in HBM
-    char pname[64];
-    snprintf(pname, sizeof pname, "groupnorm statistics C=%d @%dx%d", nw.C, B, H * W);
-    ProfScope prof(pname, 0.0, 0.0, s);
-    const int partials = st->pending;
-    st->pending = 0;
-    const float* scale = nullptr; const float* shift = nullptr;
-    HDRVAE_TRY(launch_gn_scale_shift(B, H * W, nw.C, nw.gamma, nw.beta, st->gn, st->gn_chunks, partials, s, &scale, &shift));
-    io->x = x; io->xf_scale = scale; io->xf_shift = shift; io->xf_in_scale = x_scale;
-    return 0;
-  }
-  HDRVAE_TRY(run_gn(ctx, x, x_dtype, st->t, B, H * W, nw, true, st, s, -1, x_scale));
-  io->x = st->t;
-  return 0;
-}
-
-static int run_res(hdrvae_ctx* ctx, const ResW& rw, DecState* st, int B, int H, int W, cudaStream_t s) {
-  const int impl = ctx->conv_impl;
-  const bool h16 = h_is_16bit(ctx);
-  const int h_dt = h16 ? ctx->op_dtype : DT_F32;
-  const float h_scale = h16 ? kRawOperandScale : 1.f;
-  {
-    ConvIO io; io.y = st->hbuf; io.stats = stats_ptr(ctx, st); io.stats_chunks = &st->pending;
-    io.y_dtype = h_dt; io.y_scale = h_scale;
-    HDRVAE_TRY(gn_before_conv(ctx, st->x, rw.n1, rw.c1, &io, st, B, H, W, s, st->x_dt, 1.f / st->x_scale));
-    HDRVAE_TRY(run_conv(ctx, rw.c1, io, B, H, W, impl, s));
-  }
-  const bool x16 = st->x_dt != DT_F32;
-  ConvIO io; io.stats = stats_ptr(ctx, st); io.stats_chunks = &st->pending;
-  if (x16) { io.y_dtype = st->x_dt; io.y_scale = st->x_scale; }
-  else if (rw.dual_out) { io.y2 = st->xa16; io.y2_dtype = ctx->op_dtype; io.y2_scale = kRawOperandScale; }
-  if (rw.has_nin) {
-    // norm2 as a separate pass (conv1's output lives in hbuf, which the shortcut is about to overwrite); then the
-    // shortcut on the scaled 16-bit copy of x into hbuf, and conv2 accumulates onto it in place
-    HDRVAE_TRY(run_gn(ctx, st->hbuf, h_dt, st->t, B, H * W, rw.n2, true, st, s, -1, 1.f / h_scale));
-    io.x = st->t;
-    if (nin_is_fused(ctx, rw, H, W)) {
-      // x_new = conv2(t) + nin(x): ONE launch, written over the old x (whose scaled 16-bit copy is what the shortcut reads)
-      io.x2 = st->xb16; io.pc2 = &rw.nin_x16; io.bias = rw.bias_c2_nin; io.y = st->x;
-      if (x16) {
-        // the shortcut reads the 16-bit stream itself; Cin != Cout, so the new stream goes to the other buffer
-        io.x2 = st->x; io.y = st->hbuf;
-        HDRVAE_TRY(run_conv(ctx, rw.c2, io, B, H, W, impl, s));
-        std::swap(st->x, st->hbuf);
-        return 0;
-      }
-      return run_conv(ctx, rw.c2, io, B, H, W, impl, s);
-    }
-    HDRVAE_REQUIRE(!x16, "the 16-bit residual stream needs the fused shortcut");
-    ConvIO sc; sc.x = st->xb16; sc.y = st->hbuf; sc.alpha = 1.0f / kRawOperandScale;
-    HDRVAE_TRY(run_conv(ctx, rw.nin, sc, B, H, W, impl, s));
-    io.y = st->hbuf; io.residual = st->hbuf;
-    HDRVAE_TRY(run_conv(ctx, rw.c2, io, B, H, W, impl, s));
-    std::swap(st->x, st->hbuf);
-  } else {
-    io.y = st->x; io.residual = st->x;                  // x += conv2(t), in place
-    if (x16) { io.res_dtype = st->x_dt; io.res_scale = 1.f / st->x_scale; }
-    HDRVAE_TRY(gn_before_conv(ctx, st->hbuf, rw.n2, rw.c2, &io, st, B, H, W, s, h_dt, 1.f / h_scale));
-    HDRVAE_TRY(run_conv(ctx, rw.c2, io, B, H, W, impl, s));
-  }
-  return 0;
 }
 
 // HDRVAE_ATTN_FUSED=0 selects the GEMM-level form (QK^T twice with the soft-max fused into the GEMM epilogues, P through
@@ -651,96 +562,6 @@ static int run_attention_core(hdrvae_ctx* ctx, const Plan& pl, uint8_t* ws, cons
   return 0;
 }
 
-static int run_decoder(hdrvae_ctx* ctx, const float* latent, const Plan& pl, uint8_t* ws, void** features,
-                       cudaStream_t s) {
-  HDRVAE_REQUIRE(ctx->loaded, "hdrvae: weights not loaded");
-  const int B = pl.B, impl = ctx->conv_impl, dt = ctx->op_dtype;
-  int H = pl.h, W = pl.w;
-  void* lat = ws + pl.off_lat;
-  DecState st;
-  st.xa16 = ws + pl.off_x16;
-  st.xb16 = ws + pl.off_x16b;
-  st.x = reinterpret_cast<float*>(ws + pl.off_x);
-  st.hbuf = reinterpret_cast<float*>(ws + pl.off_h);
-  st.t = ws + pl.off_t;
-  st.gn = ws + pl.off_gn;
-  st.gn_chunks = pl.gn_chunks;
-  st.pending = 0;
-  const bool x16 = x_is_16bit(ctx);
-  if (x16) { st.x_dt = dt; st.x_scale = kRawOperandScale; }
-  HDRVAE_TRY(gn_scratch_reset(st.gn, B, pl.gn_chunks, s));
-
-  if (ctx->high) {
-    float* latf = reinterpret_cast<float*>(ws + pl.off_f32) + (size_t)pl.Tp * 1536;
-    HDRVAE_TRY(launch_latent_to_nhwc(latent, latf, DT_F32, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
-    HDRVAE_TRY(launch_split3(latf, 64, lat, 192, (long long)B * H * W, 64, 1.f, 0, s));
-  } else {
-    HDRVAE_TRY(launch_latent_to_nhwc(latent, lat, dt, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
-  }
-  {
-    ConvIO io; io.x = lat; io.y = st.x; io.stats = stats_ptr(ctx, &st); io.stats_chunks = &st.pending;
-    if (x16) { io.y_dtype = st.x_dt; io.y_scale = st.x_scale; }
-    HDRVAE_TRY(run_conv(ctx, ctx->conv_in, io, B, H, W, impl, s));
-  }
-  HDRVAE_TRY(run_res(ctx, ctx->mid1, &st, B, H, W, s));
-  {
-    // mid.attn_1: x += proj_out(softmax(q k^T / sqrt(c)) v), q,k,v = 1x1 convs of GroupNorm(x) (no SiLU)
-    void* qk = ws + pl.off_qk;
-    void* vt = ws + pl.off_vt;
-    void* o = ws + pl.off_o;
-    HDRVAE_TRY(run_gn(ctx, st.x, st.x_dt, st.t, B, H * W, ctx->attn_norm, false, &st, s, -1, 1.f / st.x_scale));
-    if (ctx->high) {
-      ProfScope prof("attention (high precision, GEMM form)", 4.0 * B * (double)pl.T * pl.T * 512 * 3, 0.0, s);
-      for (int b = 0; b < B; ++b)
-        HDRVAE_TRY(run_attention_high(ctx, pl, ws, reinterpret_cast<const uint16_t*>(st.t) + (size_t)b * pl.T * 1536,
-                                      reinterpret_cast<uint16_t*>(o) + (size_t)b * pl.T * 1536, s));
-    } else {
-    if (pl.Tp != pl.T) HDRVAE_CUDA_OK(cudaMemsetAsync(qk, 0, (size_t)B * pl.Tp * 1024 * 2, s));
-    {
-      ProfScope pq("attention q|k and v^T projections", 2.0 * B * (double)pl.T * 512 * 1536, 0.0, s);
-      for (int b = 0; b < B; ++b) {
-        const uint16_t* tb = reinterpret_cast<const uint16_t*>(st.t) + (size_t)b * pl.T * 512;
-        // [q*scale | k] = t Wqk^T + bqk : [T][1024]
-        HDRVAE_TRY(run_gemm(ctx, dt, tb, 512, pl.T, 512, ctx->qk.w[0], 512, 1024, 1024,
-                            reinterpret_cast<uint16_t*>(qk) + (size_t)b * pl.Tp * 1024, 1024, dt, ctx->qk.bias, false, 1.0f,
-                            nullptr, impl, s));
-        // v^T = Wv t^T + bv : [512][Tp]  (operand roles swapped so PV sees a K-major B operand)
-        HDRVAE_TRY(run_gemm(ctx, dt, ctx->vproj.w[0], 512, 512, 512, tb, 512, pl.T, pl.Tp,
-                            reinterpret_cast<uint16_t*>(vt) + (size_t)b * 512 * pl.Tp, pl.Tp, dt, ctx->vproj.bias, true, 1.0f,
-                            nullptr, impl, s));
-      }
-    }
-    {
-      ProfScope prof("attention core (QK^T, softmax, PV)", 4.0 * B * (double)pl.T * pl.T * 512, 10.0 * B * (double)pl.T * pl.Tp, s);
-      // key-split partials borrow the block-internal fp32 buffer: nothing of a ResnetBlock is live across mid.attn_1
-      HDRVAE_TRY(run_attention_core(ctx, pl, ws, qk, vt, o, 1.0f, st.hbuf, (size_t)B * pl.T * 64 * 256 * 4, s));
-    }
-    }
-    ConvIO io; io.x = o; io.y = st.x; io.residual = st.x; io.stats = stats_ptr(ctx, &st); io.stats_chunks = &st.pending;
-    if (x16) { io.y_dtype = st.x_dt; io.y_scale = st.x_scale; io.res_dtype = st.x_dt; io.res_scale = 1.f / st.x_scale; }
-    HDRVAE_TRY(run_conv(ctx, ctx->proj_out, io, B, H, W, impl, s));
-  }
-  HDRVAE_TRY(run_res(ctx, ctx->mid2, &st, B, H, W, s));
-  for (int lvl = 3; lvl >= 0; --lvl) {
-    for (int i = 0; i < 3; ++i) HDRVAE_TRY(run_res(ctx, ctx->up[lvl][i], &st, B, H, W, s));
-    if (lvl != 0) {
-      // operand: the scaled 16-bit copy written by the level's last ResBlock; levels 2 and 1 feed a nin_shortcut
-      // one block later, so their output gets a scaled copy too
-      ConvIO io; io.x = st.xa16; io.y = st.hbuf; io.alpha = 1.0f / kRawOperandScale;
-      if (x16) { io.x = st.x; io.y_dtype = st.x_dt; io.y_scale = st.x_scale; }     // the stream is its own operand copy
-      else if (lvl <= 2) { io.y2 = st.xb16; io.y2_dtype = dt; io.y2_scale = kRawOperandScale; }
-      io.stats = stats_ptr(ctx, &st); io.stats_chunks = &st.pending;
-      HDRVAE_TRY(run_conv(ctx, ctx->upsample[lvl], io, B, H, W, impl, s));
-      std::swap(st.x, st.hbuf);
-      H *= 2; W *= 2;
-    }
-  }
-  // the tensor the reference's hook captures: 16-bit operand of conv_out, or fp32 in the high-precision mode
-  HDRVAE_TRY(run_gn(ctx, st.x, st.x_dt, st.t, B, H * W, ctx->norm_out, true, &st, s, ctx->high ? DT_F32 : -1, 1.f / st.x_scale));
-  *features = st.t;
-  return 0;
-}
-
 static int check_ws(const Plan& pl, void* ws, size_t bytes) {
   HDRVAE_REQUIRE(ws != nullptr && bytes >= pl.total, "hdrvae: workspace too small (%zu < %zu bytes)", bytes, pl.total);
   // every plan offset is a multiple of 1024; TMA and the vector loads need 16 bytes, cudaMalloc gives 256 and torch's
@@ -765,14 +586,7 @@ static RowsPlan make_rows_plan(int h, int w, int world, bool attn_scratch = true
   pl.h = h; pl.w = w; pl.world = world; pl.hl = h / world;
   pl.T = h * w; pl.Tl = pl.hl * w;
   pl.Tp = (pl.T + 63) / 64 * 64;
-  long long rows = kScoreBudgetElems / pl.Tp;
-  rows = rows / 128 * 128;
-  if (rows < 128) rows = 128;
-  const long long t128 = (pl.Tl + 127) / 128 * 128;
-  if (rows > t128) rows = t128;
-  pl.s_rows = (int)rows;
-  pl.gn_chunks = 1184;
-  for (int l = 1; l <= 8; l *= 2) pl.gn_chunks = std::max(pl.gn_chunks, 4 * tiles_for(l * pl.hl, l * w));
+  chunk_sizes(pl.Tl, pl.Tp, pl.hl, w, true, &pl.s_rows, &pl.gn_chunks);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes, 1024); return o; };
   const size_t widest = (size_t)(8 * pl.hl + 2) * 8 * w * 256;           // slab elements incl. halo rows
@@ -812,9 +626,7 @@ struct hdrvae_rows {
   struct Op { bool exchange; std::function<int(cudaStream_t)> fn; hdrvae_exchange ex; };
   std::vector<Op> ops;
   size_t pc = 0;
-  // layer-program state while the op list is being built
-  float* x = nullptr; float* hbuf = nullptr;
-  int H = 0, W = 0, pending = 0;
+  int pending = 0;          // GroupNorm partial chunks of the last conv, written and read while the ops run
   // every rank's workspace as mapped into this process (hdrvae_peer_open; own pointer at [rank]): hdrvae_rows_set_peers
   uint8_t* peers[kRowsMaxRanks] = {};
   bool peers_set = false;
@@ -822,10 +634,6 @@ struct hdrvae_rows {
 
 namespace hdrvae {
 
-static void rows_compute(hdrvae_rows* st, std::function<int(cudaStream_t)> fn) {
-  hdrvae_rows::Op op; op.exchange = false; op.fn = std::move(fn); memset(&op.ex, 0, sizeof op.ex);
-  st->ops.push_back(std::move(op));
-}
 static void rows_exchange(hdrvae_rows* st, const hdrvae_exchange& ex) {
   hdrvae_rows::Op op; op.exchange = true; op.ex = ex;
   st->ops.push_back(std::move(op));
@@ -853,231 +661,367 @@ static int zero_border_halos(hdrvae_rows* st, void* slab, int H, int W, int C, i
   return 0;
 }
 
-// conv epilogue emitted this rank's GroupNorm partials: fold them, then (exchange) all-reduce the sums
-static void rows_stats_and_halo(hdrvae_rows* st, const void* slab_f32, int H, int W, int C, const void* slab16, int C16,
-                                int eb = 4) {
-  hdrvae_ctx* ctx = st->ctx;
-  void* gn = st->ws + st->pl.off_gn;
-  const int gn_chunks = st->pl.gn_chunks;
-  int* pending = &st->pending;
-  rows_compute(st, [=](cudaStream_t s) { return launch_gn_reduce_partials(gn, 1, 512, gn_chunks, *pending, s); });
+// ---- decoder layer program ----------------------------------------------------------------------------------------
+// The decoder graph is written once and issued against a Decoder, which says where the tensors live and how a step is
+// issued: the single-GPU decode launches each step for B dense images as it is issued; the row-tiled decode (rows set)
+// records the steps of one image, stored as slabs with one halo row above and below, into hdrvae_rows::ops together
+// with the exchanges between them.  Only step, norm and conv depend on the target; the storage decisions of the numeric
+// plan are made here once for both.
+struct Decoder {
+  hdrvae_ctx* ctx;
+  hdrvae_rows* rows;     // null: single-GPU decode
+  cudaStream_t s;        // single-GPU decode: the stream the steps are launched on
+  int B;                 // images
+  int pad;               // halo rows stored above and below each image: 0 dense, 1 slab
+  void* lat;             // staged latent: conv_in's operand
+  float* x;              // residual stream (stored as x_dt)
+  float* hbuf;           // block-internal tensor h (stored as h_dt); also the stream's second buffer
+  void* t;               // GroupNorm outputs: 16-bit operand buffer
+  void* xa16;            // scaled 16-bit copy of a level's last ResBlock output = operand of the level's upsample conv
+  void* xb16;            // scaled 16-bit copy of an upsample conv's output = operand of the next block's nin_shortcut
+  void* gn;              // GroupNorm scratch (partials | scale | shift | sums)
+  int gn_chunks;         // capacity of the partial area (chunks per image)
+  int* pending;          // partial chunks per image valid for the tensor about to be normalised (read when a step runs)
+  int x_dt, h_dt;        // element types of x and h: fp32, or the operand type holding the value times x_scale / h_scale
+  float x_scale, h_scale;
+};
+
+static Decoder make_decoder(hdrvae_ctx* ctx, hdrvae_rows* rows, cudaStream_t s, int B, int* pending) {
+  Decoder d;
+  memset(&d, 0, sizeof d);
+  d.ctx = ctx; d.rows = rows; d.s = s; d.B = B; d.pad = rows != nullptr ? 1 : 0; d.pending = pending;
+  const bool x16 = x_is_16bit(ctx), h16 = h_is_16bit(ctx);
+  d.x_dt = x16 ? ctx->op_dtype : DT_F32; d.x_scale = x16 ? kRawOperandScale : 1.f;
+  d.h_dt = h16 ? ctx->op_dtype : DT_F32; d.h_scale = h16 ? kRawOperandScale : 1.f;
+  return d;
+}
+
+// Runs fn now (single-GPU) or appends it to the row-tiled program, which runs it from hdrvae_rows_run: steps capture by
+// value what they read.
+static int step(Decoder& d, std::function<int(cudaStream_t)> fn) {
+  if (d.rows == nullptr) return fn(d.s);
+  hdrvae_rows::Op op; op.exchange = false; op.fn = std::move(fn); memset(&op.ex, 0, sizeof op.ex);
+  d.rows->ops.push_back(std::move(op));
+  return 0;
+}
+
+// t = [SiLU](GroupNorm(x)), x stored as x_dt holding the value times x_scale; y_dt: element type of t (-1: operand type).
+// Single-GPU: the streaming kernel on the producing conv's partials.  Row tiling: from the all-reduced sums, over the whole
+// slab (halo rows included: GroupNorm is elementwise once the global statistics are known), then the zero padding at the
+// image borders is restored.
+static int norm(Decoder& d, const void* x, int x_dt, float x_scale, const NormW& nw, bool silu, int H, int W, int y_dt = -1) {
+  const int ydt = y_dt >= 0 ? y_dt : (d.ctx->high ? DT_F16X3 : d.ctx->op_dtype);
+  if (d.rows == nullptr) {
+    char pname[64];
+    snprintf(pname, sizeof pname, "groupnorm%s C=%d @%dx%d", silu ? "+silu" : "", nw.C, d.B, H * W);
+    ProfScope prof(pname, 0.0, (double)d.B * H * W * nw.C * (dt_bytes(x_dt) * (*d.pending > 0 ? 1 : 2) + 2.0), d.s);
+    const int partials = *d.pending;
+    *d.pending = 0;
+    return launch_groupnorm(x, x_dt, d.t, ydt, d.B, H * W, nw.C, nw.gamma, nw.beta, silu, d.gn, d.gn_chunks, partials, d.s,
+                            1.f / x_scale);
+  }
+  const NormW n = nw;
+  const double count = (double)H * d.rows->pl.world * (double)W * (double)(n.C / 32);
+  return step(d, [=](cudaStream_t s) {
+    const long long slab = (long long)(H + 2) * W * n.C;
+    HDRVAE_TRY(launch_gn_apply_from_sums(x, x_dt, slab, d.t, ydt, slab, 1, (H + 2) * W, n.C, n.gamma, n.beta, silu, d.gn,
+                                         d.gn_chunks, count, s, 1.f / x_scale));
+    return zero_border_halos(d.rows, d.t, H, W, n.C, 2, s);
+  });
+}
+
+static float* stats_ptr(const Decoder& d) {
+  return d.ctx->conv_impl == HDRVAE_CONV_TCGEN05 ? reinterpret_cast<float*>(d.gn) : nullptr;
+}
+
+// conv flags
+constexpr int kNoStats = 1;      // no GroupNorm statistics (the separate nin_shortcut: its output is conv2's residual)
+constexpr int kZeroHalos = 2;    // row tiling: y is the 16-bit stream, read raw by later 3x3 convs: zero its border halo rows
+constexpr int kDenseInput = 4;   // x is dense, not a slab (proj_out reads the attention output)
+
+// Issues run_conv with the target's halo rows and the GroupNorm statistics of y.  xf: GroupNorm + SiLU of io.x applied
+// inside the conv (norm_conv), its scale / shift computed right before the conv.  Row tiling, after a conv with
+// statistics: fold this rank's partials, then one exchange all-reduces the sums and fills the halo rows of y and of its
+// scaled copy in xa16 (the upsample conv's 3x3 operand).
+static int conv(Decoder& d, const PackedConv& pc, ConvIO io, int H, int W, int flags = 0, const NormW* xf = nullptr) {
+  hdrvae_rows* rows = d.rows;
+  io.x_pad = (flags & kDenseInput) ? 0 : d.pad;
+  io.y_pad = d.pad;
+  if (!(flags & kNoStats)) { io.stats = stats_ptr(d); io.stats_chunks = d.pending; }
+  if (xf != nullptr && rows != nullptr) {     // a border rank's outer halo row is padding, not an image row
+    io.xf_y_lo = rows->rank == 0 ? 0 : -1;
+    io.xf_y_hi = rows->rank == rows->pl.world - 1 ? H : H + 1;
+  }
+  const int OH = pc.upsample ? 2 * H : H, OW = pc.upsample ? 2 * W : W;
+  const PackedConv* p = &pc;
+  const bool zero_y = rows != nullptr && (flags & kZeroHalos);
+  const bool xa_copy = rows != nullptr && io.y2 != nullptr && io.y2 == d.xa16;
+  HDRVAE_TRY(step(d, [=](cudaStream_t s) mutable {
+    if (xf != nullptr && rows == nullptr) {
+      // only the reduction of the producer's partials runs as a kernel (-> per-(image, channel) scale / shift); the conv's
+      // transform warps normalise the scaled fp16 tensor as it lands in shared memory: no normalised copy in HBM
+      char pname[64];
+      snprintf(pname, sizeof pname, "groupnorm statistics C=%d @%dx%d", xf->C, d.B, H * W);
+      ProfScope prof(pname, 0.0, 0.0, s);
+      const int partials = *d.pending;
+      *d.pending = 0;
+      HDRVAE_TRY(launch_gn_scale_shift(d.B, H * W, xf->C, xf->gamma, xf->beta, d.gn, d.gn_chunks, partials, s, &io.xf_scale,
+                                       &io.xf_shift));
+    } else if (xf != nullptr) {
+      HDRVAE_TRY(launch_gn_scale_shift_from_sums(1, xf->C, xf->gamma, xf->beta, d.gn, d.gn_chunks,
+                                                 (double)H * rows->pl.world * (double)W * (double)(xf->C / 32), s,
+                                                 &io.xf_scale, &io.xf_shift));
+    }
+    HDRVAE_TRY(run_conv(d.ctx, *p, io, d.B, H, W, d.ctx->conv_impl, s));
+    if (zero_y) HDRVAE_TRY(zero_border_halos(rows, io.y, OH, OW, p->cout, 2, s));
+    if (xa_copy) HDRVAE_TRY(zero_border_halos(rows, io.y2, OH, OW, p->cout, 2, s));
+    return 0;
+  }));
+  if (rows == nullptr || io.stats == nullptr) return 0;
+  HDRVAE_TRY(step(d, [=](cudaStream_t s) { return launch_gn_reduce_partials(d.gn, 1, 512, d.gn_chunks, *d.pending, s); }));
   hdrvae_exchange ex;
   memset(&ex, 0, sizeof ex);
-  add_halo(st, &ex, slab_f32, H, W, C, eb);
-  if (slab16 != nullptr) add_halo(st, &ex, slab16, H, W, C16, 2);
+  add_halo(rows, &ex, io.y, OH, OW, pc.cout, dt_bytes(io.y_dtype));
+  if (xa_copy) add_halo(rows, &ex, io.y2, OH, OW, pc.cout, 2);
   ex.kind |= HDRVAE_EX_ALLREDUCE_F64;
-  ex.allreduce_off = ws_off(st, gn_sums_ptr(gn, 1, 512, gn_chunks));
+  ex.allreduce_off = ws_off(rows, gn_sums_ptr(d.gn, 1, 512, d.gn_chunks));
   ex.allreduce_count = 32 * 2;
-  rows_exchange(st, ex);
-  (void)ctx;
+  rows_exchange(rows, ex);
+  return 0;
 }
 
-// t = [silu](GroupNorm(x)) over the whole slab (halo rows included: GroupNorm is elementwise once the global
-// statistics are known), then restore the zero padding at the image borders
-static void rows_gn(hdrvae_rows* st, const void* x_slab, const NormW& nw, bool silu, int H, int W, int x_dtype = DT_F32,
-                    float in_scale = 1.f) {
-  hdrvae_ctx* ctx = st->ctx;
-  void* gn = st->ws + st->pl.off_gn;
-  void* t = st->ws + st->pl.off_t;
-  const int gn_chunks = st->pl.gn_chunks;
-  const double count = (double)H * st->pl.world * (double)W * (double)(nw.C / 32);
-  const NormW n = nw;
-  rows_compute(st, [=](cudaStream_t s) {
-    const long long slab = (long long)(H + 2) * W * n.C;
-    HDRVAE_TRY(launch_gn_apply_from_sums(x_slab, x_dtype, slab, t, ctx->op_dtype, slab, 1, (H + 2) * W, n.C, n.gamma, n.beta,
-                                         silu, gn, gn_chunks, count, s, in_scale));
-    return zero_border_halos(st, t, H, W, n.C, 2, s);
-  });
+// conv(SiLU(GroupNorm(x))): the GroupNorm is applied inside the conv when gn_is_fused allows it for the conv as issued,
+// otherwise by norm into t.
+static int norm_conv(Decoder& d, const void* x, int x_dt, float x_scale, const NormW& nw, const PackedConv& pc, ConvIO io,
+                     int H, int W, int flags = 0) {
+  io.stats = stats_ptr(d);                       // what conv sets: the decision sees the conv as issued
+  if (!gn_is_fused(d.ctx, pc, io, x_dt, H, W)) {
+    HDRVAE_TRY(norm(d, x, x_dt, x_scale, nw, true, H, W));
+    io.x = d.t;
+    return conv(d, pc, io, H, W, flags);
+  }
+  io.x = x; io.xf_in_scale = 1.f / x_scale;
+  return conv(d, pc, io, H, W, flags, &nw);
 }
 
-static void rows_res(hdrvae_rows* st, const ResW& rw, int H, int W) {
-  hdrvae_ctx* ctx = st->ctx;
-  void* t = st->ws + st->pl.off_t;
-  void* xa = st->ws + st->pl.off_xa;
-  void* xb = st->ws + st->pl.off_xb;
-  float* stats = reinterpret_cast<float*>(st->ws + st->pl.off_gn);
-  int* pending = &st->pending;
-  float* x = st->x; float* hb = st->hbuf;
-  const ResW* r = &rw;
-  const bool h16 = h_is_16bit(ctx);                    // same storage rules as the single-GPU program (bit-identical results)
-  const int h_dt = h16 ? ctx->op_dtype : DT_F32;
-  const float h_scale = h16 ? kRawOperandScale : 1.f;
-  const bool x16 = x_is_16bit(ctx);
-  const int x_dt = x16 ? ctx->op_dtype : DT_F32;
-  const float x_scale = x16 ? kRawOperandScale : 1.f;
-  // GroupNorm applied inside the conv (same rule as the single-GPU program): the conv reads the scaled fp16 slab itself,
-  // halo rows included; a border rank's outer halo row is padding, not an image row
-  void* gn = st->ws + st->pl.off_gn;
-  const int gn_chunks = st->pl.gn_chunks;
-  const int y_lo = st->rank == 0 ? 0 : -1, y_hi = st->rank == st->pl.world - 1 ? H : H + 1;
-  const double world_rows = (double)H * st->pl.world;
-  ConvIO probe1; probe1.y = hb; probe1.y_dtype = h_dt; probe1.stats = stats;
-  const bool f1 = gn_is_fused(ctx, rw.c1, probe1, x_dt, H, W);
-  if (!f1) rows_gn(st, x, rw.n1, true, H, W, x_dt, 1.f / x_scale);
-  rows_compute(st, [=](cudaStream_t s) {
-    ConvIO io; io.x = t; io.y = hb; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
-    io.y_dtype = h_dt; io.y_scale = h_scale;
-    if (f1) {
-      HDRVAE_TRY(launch_gn_scale_shift_from_sums(1, r->n1.C, r->n1.gamma, r->n1.beta, gn, gn_chunks,
-                                                 world_rows * (double)W * (double)(r->n1.C / 32), s, &io.xf_scale, &io.xf_shift));
-      io.x = x; io.xf_in_scale = 1.f / x_scale; io.xf_y_lo = y_lo; io.xf_y_hi = y_hi;
-    }
-    return run_conv(ctx, r->c1, io, 1, H, W, HDRVAE_CONV_TCGEN05, s);
-  });
-  rows_stats_and_halo(st, hb, H, W, rw.c1.cout, nullptr, 0, h16 ? 2 : 4);
-  const bool fused_nin = nin_is_fused(ctx, rw, H, W);
-  float* out = (rw.has_nin && (!fused_nin || x16)) ? hb : x;      // 16-bit stream: the shortcut reads x itself, so not in place
-  ConvIO probe2; probe2.y = out; probe2.residual = rw.has_nin ? nullptr : out; probe2.y_dtype = x_dt; probe2.stats = stats;
-  const bool f2 = !rw.has_nin && gn_is_fused(ctx, rw.c2, probe2, h_dt, H, W);     // (a shortcut block writes over h: not fused)
-  if (!f2) rows_gn(st, hb, rw.n2, true, H, W, h_dt, 1.f / h_scale);
-  rows_compute(st, [=](cudaStream_t s) {
-    if (x16) {
-      // the residual stream is the scaled 16-bit tensor (see x_is_16bit): in place with a 16-bit residual, or — with a
-      // shortcut — from x into the other buffer; its border halo rows are conv padding for the raw-stream convs
-      ConvIO io; io.x = t; io.y = out; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
-      io.y_dtype = x_dt; io.y_scale = x_scale;
-      if (fused_nin) { io.x2 = x; io.pc2 = &r->nin_x16; io.bias = r->bias_c2_nin; }
-      else { io.residual = out; io.res_dtype = x_dt; io.res_scale = 1.f / x_scale; }
-      if (f2) {
-        HDRVAE_TRY(launch_gn_scale_shift_from_sums(1, r->n2.C, r->n2.gamma, r->n2.beta, gn, gn_chunks,
-                                                   world_rows * (double)W * (double)(r->n2.C / 32), s, &io.xf_scale, &io.xf_shift));
-        io.x = hb; io.xf_in_scale = 1.f / h_scale; io.xf_y_lo = y_lo; io.xf_y_hi = y_hi;
-      }
-      HDRVAE_TRY(run_conv(ctx, r->c2, io, 1, H, W, HDRVAE_CONV_TCGEN05, s));
-      return zero_border_halos(st, out, H, W, r->c2.cout, 2, s);
-    }
-    if (fused_nin) {
-      ConvIO io; io.x = t; io.y = out; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
-      io.x2 = xb; io.pc2 = &r->nin_x16; io.bias = r->bias_c2_nin;
-      return run_conv(ctx, r->c2, io, 1, H, W, HDRVAE_CONV_TCGEN05, s);
-    }
-    if (r->has_nin) {
-      ConvIO sc; sc.x = xb; sc.y = hb; sc.alpha = 1.0f / kRawOperandScale; sc.x_pad = sc.y_pad = 1;
-      HDRVAE_TRY(run_conv(ctx, r->nin, sc, 1, H, W, HDRVAE_CONV_TCGEN05, s));
-    }
-    ConvIO io; io.x = t; io.y = out; io.residual = out; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
-    if (r->dual_out) { io.y2 = xa; io.y2_dtype = ctx->op_dtype; io.y2_scale = kRawOperandScale; }
-    HDRVAE_TRY(run_conv(ctx, r->c2, io, 1, H, W, HDRVAE_CONV_TCGEN05, s));
-    if (r->dual_out) HDRVAE_TRY(zero_border_halos(st, xa, H, W, r->c2.cout, 2, s));
+static int decode_res(Decoder& d, const ResW& rw, int H, int W) {
+  hdrvae_ctx* ctx = d.ctx;
+  const bool x16 = d.x_dt != DT_F32;
+  const int stream_flags = x16 ? kZeroHalos : 0;
+  {
+    ConvIO io; io.y = d.hbuf; io.y_dtype = d.h_dt; io.y_scale = d.h_scale;
+    HDRVAE_TRY(norm_conv(d, d.x, d.x_dt, d.x_scale, rw.n1, rw.c1, io, H, W));
+  }
+  ConvIO io;
+  if (x16) { io.y_dtype = d.x_dt; io.y_scale = d.x_scale; }
+  else if (rw.dual_out) { io.y2 = d.xa16; io.y2_dtype = ctx->op_dtype; io.y2_scale = kRawOperandScale; }
+  if (!rw.has_nin) {
+    io.y = d.x; io.residual = d.x;                  // x += conv2(t), in place
+    io.res_dtype = d.x_dt; io.res_scale = 1.f / d.x_scale;
+    return norm_conv(d, d.hbuf, d.h_dt, d.h_scale, rw.n2, rw.c2, io, H, W, stream_flags);
+  }
+  // norm2 as a separate pass (conv1's output lives in hbuf, which the shortcut is about to overwrite); then the
+  // shortcut on the scaled 16-bit copy of x into hbuf, and conv2 accumulates onto it in place
+  HDRVAE_TRY(norm(d, d.hbuf, d.h_dt, d.h_scale, rw.n2, true, H, W));
+  io.x = d.t;
+  if (nin_is_fused(ctx, rw, H, W)) {
+    // x_new = conv2(t) + nin(x): ONE launch, written over the old x (whose scaled 16-bit copy is what the shortcut reads)
+    io.x2 = d.xb16; io.pc2 = &rw.nin_x16; io.bias = rw.bias_c2_nin; io.y = d.x;
+    if (!x16) return conv(d, rw.c2, io, H, W);
+    // the shortcut reads the 16-bit stream itself; Cin != Cout, so the new stream goes to the other buffer
+    io.x2 = d.x; io.y = d.hbuf;
+    HDRVAE_TRY(conv(d, rw.c2, io, H, W, stream_flags));
+    std::swap(d.x, d.hbuf);
     return 0;
+  }
+  HDRVAE_REQUIRE(!x16, "the 16-bit residual stream needs the fused shortcut");
+  ConvIO sc; sc.x = d.xb16; sc.y = d.hbuf; sc.alpha = 1.0f / kRawOperandScale;
+  HDRVAE_TRY(conv(d, rw.nin, sc, H, W, kNoStats));
+  io.y = d.hbuf; io.residual = d.hbuf;
+  HDRVAE_TRY(conv(d, rw.c2, io, H, W));
+  std::swap(d.x, d.hbuf);
+  return 0;
+}
+
+// conv_in on the staged latent, mid.block_1 and mid.attn_1's GroupNorm (no SiLU) into t
+static int decode_to_attention(Decoder& d, int H, int W) {
+  ConvIO io; io.x = d.lat; io.y = d.x; io.y_dtype = d.x_dt; io.y_scale = d.x_scale;
+  HDRVAE_TRY(conv(d, d.ctx->conv_in, io, H, W, d.x_dt != DT_F32 ? kZeroHalos : 0));
+  HDRVAE_TRY(decode_res(d, d.ctx->mid1, H, W));
+  return norm(d, d.x, d.x_dt, d.x_scale, d.ctx->attn_norm, false, H, W);
+}
+
+// x += proj_out(o), mid.block_2, the up levels and norm_out (+ SiLU) into t: the tensor the reference's hook captures
+// (16-bit operand of conv_out, or fp32 in the high-precision mode)
+static int decode_from_attention(Decoder& d, const void* o, int H, int W) {
+  hdrvae_ctx* ctx = d.ctx;
+  const bool x16 = d.x_dt != DT_F32;
+  {
+    // proj_out adds in place and writes no halo rows: the stream's border halos stay zero
+    ConvIO io; io.x = o; io.y = d.x; io.residual = d.x;
+    io.y_dtype = d.x_dt; io.y_scale = d.x_scale; io.res_dtype = d.x_dt; io.res_scale = 1.f / d.x_scale;
+    HDRVAE_TRY(conv(d, ctx->proj_out, io, H, W, kDenseInput));
+  }
+  HDRVAE_TRY(decode_res(d, ctx->mid2, H, W));
+  for (int lvl = 3; lvl >= 0; --lvl) {
+    for (int i = 0; i < 3; ++i) HDRVAE_TRY(decode_res(d, ctx->up[lvl][i], H, W));
+    if (lvl != 0) {
+      // operand: the scaled 16-bit copy written by the level's last ResBlock; levels 2 and 1 feed a nin_shortcut
+      // one block later, so their output gets a scaled copy too
+      ConvIO io; io.x = d.xa16; io.y = d.hbuf; io.alpha = 1.0f / kRawOperandScale;
+      if (x16) { io.x = d.x; io.y_dtype = d.x_dt; io.y_scale = d.x_scale; }     // the stream is its own operand copy
+      else if (lvl <= 2) { io.y2 = d.xb16; io.y2_dtype = ctx->op_dtype; io.y2_scale = kRawOperandScale; }
+      HDRVAE_TRY(conv(d, ctx->upsample[lvl], io, H, W, x16 ? kZeroHalos : 0));
+      std::swap(d.x, d.hbuf);
+      H *= 2; W *= 2;
+    }
+  }
+  return norm(d, d.x, d.x_dt, d.x_scale, ctx->norm_out, true, H, W, ctx->high ? DT_F32 : -1);
+}
+
+// mid.attn_1 between its GroupNorm (t) and proj_out, single-GPU: per-image q|k and v^T projections, then the attention
+// core over all images; the high-precision mode takes the GEMM-level form on hi / lo operands.  *o: proj_out's operand.
+static int attend_dense(Decoder& d, const Plan& pl, uint8_t* ws, const void** o_out) {
+  hdrvae_ctx* ctx = d.ctx;
+  const int B = d.B, impl = ctx->conv_impl, dt = ctx->op_dtype;
+  cudaStream_t s = d.s;
+  void* qk = ws + pl.off_qk;
+  void* vt = ws + pl.off_vt;
+  void* o = ws + pl.off_o;
+  *o_out = o;
+  if (ctx->high) {
+    ProfScope prof("attention (high precision, GEMM form)", 4.0 * B * (double)pl.T * pl.T * 512 * 3, 0.0, s);
+    for (int b = 0; b < B; ++b)
+      HDRVAE_TRY(run_attention_high(ctx, pl, ws, reinterpret_cast<const uint16_t*>(d.t) + (size_t)b * pl.T * 1536,
+                                    reinterpret_cast<uint16_t*>(o) + (size_t)b * pl.T * 1536, s));
+    return 0;
+  }
+  if (pl.Tp != pl.T) HDRVAE_CUDA_OK(cudaMemsetAsync(qk, 0, (size_t)B * pl.Tp * 1024 * 2, s));
+  {
+    ProfScope pq("attention q|k and v^T projections", 2.0 * B * (double)pl.T * 512 * 1536, 0.0, s);
+    for (int b = 0; b < B; ++b) {
+      const uint16_t* tb = reinterpret_cast<const uint16_t*>(d.t) + (size_t)b * pl.T * 512;
+      // [q*scale | k] = t Wqk^T + bqk : [T][1024]
+      HDRVAE_TRY(run_gemm(ctx, dt, tb, 512, pl.T, 512, ctx->qk.w[0], 512, 1024, 1024,
+                          reinterpret_cast<uint16_t*>(qk) + (size_t)b * pl.Tp * 1024, 1024, dt, ctx->qk.bias, false, 1.0f,
+                          nullptr, impl, s));
+      // v^T = Wv t^T + bv : [512][Tp]  (operand roles swapped so PV sees a K-major B operand)
+      HDRVAE_TRY(run_gemm(ctx, dt, ctx->vproj.w[0], 512, 512, 512, tb, 512, pl.T, pl.Tp,
+                          reinterpret_cast<uint16_t*>(vt) + (size_t)b * 512 * pl.Tp, pl.Tp, dt, ctx->vproj.bias, true, 1.0f,
+                          nullptr, impl, s));
+    }
+  }
+  ProfScope prof("attention core (QK^T, softmax, PV)", 4.0 * B * (double)pl.T * pl.T * 512, 10.0 * B * (double)pl.T * pl.Tp, s);
+  // key-split partials borrow the block-internal fp32 buffer: nothing of a ResnetBlock is live across mid.attn_1
+  return run_attention_core(ctx, pl, ws, qk, vt, o, 1.0f, d.hbuf, (size_t)B * pl.T * 64 * 256 * 4, s);
+}
+
+static int run_decoder(hdrvae_ctx* ctx, const float* latent, const Plan& pl, uint8_t* ws, void** features,
+                       cudaStream_t s) {
+  HDRVAE_REQUIRE(ctx->loaded, "hdrvae: weights not loaded");
+  const int B = pl.B, H = pl.h, W = pl.w;
+  int pending = 0;
+  Decoder d = make_decoder(ctx, nullptr, s, B, &pending);
+  d.lat = ws + pl.off_lat;
+  d.x = reinterpret_cast<float*>(ws + pl.off_x);
+  d.hbuf = reinterpret_cast<float*>(ws + pl.off_h);
+  d.t = ws + pl.off_t;
+  d.xa16 = ws + pl.off_x16;
+  d.xb16 = ws + pl.off_x16b;
+  d.gn = ws + pl.off_gn;
+  d.gn_chunks = pl.gn_chunks;
+  HDRVAE_TRY(gn_scratch_reset(d.gn, B, pl.gn_chunks, s));
+  if (ctx->high) {
+    float* latf = reinterpret_cast<float*>(ws + pl.off_f32) + (size_t)pl.Tp * 1536;
+    HDRVAE_TRY(launch_latent_to_nhwc(latent, latf, DT_F32, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
+    HDRVAE_TRY(launch_split3(latf, 64, d.lat, 192, (long long)B * H * W, 64, 1.f, 0, s));
+  } else {
+    HDRVAE_TRY(launch_latent_to_nhwc(latent, d.lat, ctx->op_dtype, B, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, H * W, 64, s));
+  }
+  HDRVAE_TRY(decode_to_attention(d, H, W));
+  const void* o = nullptr;
+  HDRVAE_TRY(attend_dense(d, pl, ws, &o));
+  HDRVAE_TRY(decode_from_attention(d, o, H, W));
+  *features = d.t;
+  return 0;
+}
+
+// mid.attn_1 between its GroupNorm (t) and proj_out, row tiling: q|k and v of this rank's tokens, all-gathered, then this
+// rank's queries attend to all keys.  *o: proj_out's operand (dense [Tl][512]).
+static void attend_rows(Decoder& d, int W, const void** o_out) {
+  hdrvae_rows* st = d.rows;
+  hdrvae_ctx* ctx = d.ctx;
+  const RowsPlan& pl = st->pl;
+  uint8_t* ws = st->ws;
+  const int rank = st->rank, dt = ctx->op_dtype;
+  uint16_t* qk = reinterpret_cast<uint16_t*>(ws + pl.off_qk);
+  uint16_t* vb = reinterpret_cast<uint16_t*>(ws + pl.off_v);
+  uint16_t* vt = reinterpret_cast<uint16_t*>(ws + pl.off_vt);
+  uint16_t* o = reinterpret_cast<uint16_t*>(ws + pl.off_o);
+  *o_out = o;
+  const uint16_t* tl = reinterpret_cast<const uint16_t*>(d.t) + (size_t)W * 512;      // interior rows of the slab
+  float* hscr = d.hbuf;                                   // idle across the attention: lends its memory to the key-split partials
+  const size_t hscr_bytes = (size_t)(8 * pl.hl + 2) * 8 * pl.w * 256 * 4;
+  step(d, [=](cudaStream_t s) {
+    if (pl.Tp != pl.T) {
+      HDRVAE_CUDA_OK(cudaMemsetAsync(qk, 0, (size_t)pl.Tp * 1024 * 2, s));
+      HDRVAE_CUDA_OK(cudaMemsetAsync(vt, 0, (size_t)512 * pl.Tp * 2, s));
+    }
+    HDRVAE_TRY(run_gemm(ctx, dt, tl, 512, pl.Tl, 512, ctx->qk.w[0], 512, 1024, 1024, qk + (size_t)rank * pl.Tl * 1024, 1024, dt,
+                        ctx->qk.bias, false, 1.0f, nullptr, HDRVAE_CONV_TCGEN05, s));
+    return run_gemm(ctx, dt, tl, 512, pl.Tl, 512, ctx->vproj.w[0], 512, 512, 512, vb + (size_t)rank * pl.Tl * 512, 512, dt,
+                    ctx->vproj.bias, false, 1.0f, nullptr, HDRVAE_CONV_TCGEN05, s);
   });
-  if (x16) rows_stats_and_halo(st, out, H, W, rw.c2.cout, nullptr, 0, 2);
-  else rows_stats_and_halo(st, out, H, W, rw.c2.cout, rw.dual_out ? xa : nullptr, rw.c2.cout);
-  if (rw.has_nin && (!fused_nin || x16)) std::swap(st->x, st->hbuf);
+  hdrvae_exchange ex;
+  memset(&ex, 0, sizeof ex);
+  ex.kind = HDRVAE_EX_ALLGATHER;
+  ex.n_gather = 2;
+  ex.gather_off[0] = pl.off_qk; ex.gather_bytes_per_rank[0] = (size_t)pl.Tl * 1024 * 2;
+  ex.gather_off[1] = pl.off_v;  ex.gather_bytes_per_rank[1] = (size_t)pl.Tl * 512 * 2;
+  rows_exchange(st, ex);
+  step(d, [=](cudaStream_t s) {
+    HDRVAE_TRY(launch_transpose_pad(vb, vt, pl.T, 512, pl.Tp, s));
+    return attention_rows(ctx, ws, pl.off_s, pl.off_p, pl.off_inv, pl.off_part, hscr, hscr_bytes, pl.s_rows,
+                          qk + (size_t)rank * pl.Tl * 1024, pl.Tl, qk + 512, vt, pl.T, pl.Tp, o, 1.0f, s);
+  });
 }
 
 static int build_rows_program(hdrvae_rows* st) {
   hdrvae_ctx* ctx = st->ctx;
   const RowsPlan& pl = st->pl;
-  const int dt = ctx->op_dtype;
   uint8_t* ws = st->ws;
-  void* lat = ws + pl.off_lat;
-  void* t = ws + pl.off_t;
-  void* xa = ws + pl.off_xa;
-  void* xb = ws + pl.off_xb;
-  float* stats = reinterpret_cast<float*>(ws + pl.off_gn);
-  int* pending = &st->pending;
-  st->x = reinterpret_cast<float*>(ws + pl.off_x);
-  st->hbuf = reinterpret_cast<float*>(ws + pl.off_h);
-  int H = pl.hl, W = pl.w;
-  const int rank = st->rank;
-  const float* latent = st->latent;
-  const bool x16 = x_is_16bit(ctx);                    // residual stream stored like the single-GPU program stores it
-  const int x_dt = x16 ? dt : DT_F32;
-  const float x_scale = x16 ? kRawOperandScale : 1.f;
-  const int x_eb = x16 ? 2 : 4;
-
-  {
-    float* x = st->x;
-    rows_compute(st, [=](cudaStream_t s) {
-      // latent rows of this rank plus one neighbour row each side (rows outside the image are zero)
-      HDRVAE_TRY(launch_latent_rows_to_nhwc(latent, lat, dt, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, pl.h, pl.w,
-                                            rank * pl.hl - 1, pl.hl + 2, 64, s));
-      HDRVAE_TRY(gn_scratch_reset(stats, 1, pl.gn_chunks, s));
-      ConvIO io; io.x = lat; io.y = x; io.stats = stats; io.stats_chunks = pending; io.x_pad = io.y_pad = 1;
-      if (x16) { io.y_dtype = x_dt; io.y_scale = x_scale; }
-      HDRVAE_TRY(run_conv(ctx, ctx->conv_in, io, 1, H, W, HDRVAE_CONV_TCGEN05, s));
-      return x16 ? zero_border_halos(st, x, H, W, 512, 2, s) : 0;
-    });
-    rows_stats_and_halo(st, x, H, W, 512, nullptr, 0, x_eb);
-  }
-  rows_res(st, ctx->mid1, H, W);
-  {
-    // mid.attn_1 is global: q for this rank's tokens, K and V of all tokens (all-gather)
-    uint16_t* qk = reinterpret_cast<uint16_t*>(ws + pl.off_qk);
-    uint16_t* vb = reinterpret_cast<uint16_t*>(ws + pl.off_v);
-    uint16_t* vt = reinterpret_cast<uint16_t*>(ws + pl.off_vt);
-    uint16_t* o = reinterpret_cast<uint16_t*>(ws + pl.off_o);
-    float* x = st->x;
-    float* hscr = st->hbuf;                                   // idle across the attention: lends its memory to the key-split partials
-    const size_t hscr_bytes = (size_t)(8 * pl.hl + 2) * 8 * pl.w * 256 * 4;
-    rows_gn(st, x, ctx->attn_norm, false, H, W, x_dt, 1.f / x_scale);
-    rows_compute(st, [=](cudaStream_t s) {
-      const uint16_t* tl = reinterpret_cast<const uint16_t*>(t) + (size_t)W * 512;      // interior rows of the slab
-      if (pl.Tp != pl.T) {
-        HDRVAE_CUDA_OK(cudaMemsetAsync(qk, 0, (size_t)pl.Tp * 1024 * 2, s));
-        HDRVAE_CUDA_OK(cudaMemsetAsync(vt, 0, (size_t)512 * pl.Tp * 2, s));
-      }
-      HDRVAE_TRY(run_gemm(ctx, dt, tl, 512, pl.Tl, 512, ctx->qk.w[0], 512, 1024, 1024, qk + (size_t)rank * pl.Tl * 1024, 1024, dt,
-                          ctx->qk.bias, false, 1.0f, nullptr, HDRVAE_CONV_TCGEN05, s));
-      return run_gemm(ctx, dt, tl, 512, pl.Tl, 512, ctx->vproj.w[0], 512, 512, 512, vb + (size_t)rank * pl.Tl * 512, 512, dt,
-                      ctx->vproj.bias, false, 1.0f, nullptr, HDRVAE_CONV_TCGEN05, s);
-    });
-    hdrvae_exchange ex;
-    memset(&ex, 0, sizeof ex);
-    ex.kind = HDRVAE_EX_ALLGATHER;
-    ex.n_gather = 2;
-    ex.gather_off[0] = pl.off_qk; ex.gather_bytes_per_rank[0] = (size_t)pl.Tl * 1024 * 2;
-    ex.gather_off[1] = pl.off_v;  ex.gather_bytes_per_rank[1] = (size_t)pl.Tl * 512 * 2;
-    rows_exchange(st, ex);
-    rows_compute(st, [=](cudaStream_t s) {
-      HDRVAE_TRY(launch_transpose_pad(vb, vt, pl.T, 512, pl.Tp, s));
-      HDRVAE_TRY(attention_rows(ctx, ws, pl.off_s, pl.off_p, pl.off_inv, pl.off_part, hscr, hscr_bytes, pl.s_rows,
-                                qk + (size_t)rank * pl.Tl * 1024, pl.Tl, qk + 512, vt, pl.T, pl.Tp, o, 1.0f, s));
-      ConvIO io; io.x = o; io.y = x; io.residual = x; io.stats = stats; io.stats_chunks = pending; io.x_pad = 0; io.y_pad = 1;
-      if (x16) { io.y_dtype = x_dt; io.y_scale = x_scale; io.res_dtype = x_dt; io.res_scale = 1.f / x_scale; }
-      return run_conv(ctx, ctx->proj_out, io, 1, H, W, HDRVAE_CONV_TCGEN05, s);
-    });
-    rows_stats_and_halo(st, x, H, W, 512, nullptr, 0, x_eb);
-  }
-  rows_res(st, ctx->mid2, H, W);
-  for (int lvl = 3; lvl >= 0; --lvl) {
-    for (int i = 0; i < 3; ++i) rows_res(st, ctx->up[lvl][i], H, W);
-    if (lvl != 0) {
-      float* hb = st->hbuf;
-      float* xs = st->x;
-      const PackedConv* up = &ctx->upsample[lvl];
-      const int Hc = H, Wc = W;
-      rows_compute(st, [=](cudaStream_t s) {
-        ConvIO io; io.x = xa; io.y = hb; io.alpha = 1.0f / kRawOperandScale; io.x_pad = io.y_pad = 1;
-        if (x16) { io.x = xs; io.y_dtype = x_dt; io.y_scale = x_scale; }
-        else if (lvl <= 2) { io.y2 = xb; io.y2_dtype = dt; io.y2_scale = kRawOperandScale; }
-        io.stats = stats; io.stats_chunks = pending;
-        HDRVAE_TRY(run_conv(ctx, *up, io, 1, Hc, Wc, HDRVAE_CONV_TCGEN05, s));
-        return x16 ? zero_border_halos(st, hb, 2 * Hc, 2 * Wc, up->cout, 2, s) : 0;
-      });
-      H *= 2; W *= 2;
-      rows_stats_and_halo(st, hb, H, W, up->cout, nullptr, 0, x_eb);
-      std::swap(st->x, st->hbuf);
-    }
-  }
-  {
-    float* x = st->x;
-    rows_gn(st, x, ctx->norm_out, true, H, W, x_dt, 1.f / x_scale);
-    void* epi = ws + pl.off_epi;
-    float* hscratch = st->hbuf;                       // the other fp32 stream buffer is free by now
-    rows_compute(st, [=](cudaStream_t s) {
-      return run_phase_a(ctx, t, 1, H, W, 1, hscratch, epi, s);
-    });
-    hdrvae_exchange ex;
-    memset(&ex, 0, sizeof ex);
-    ex.kind = HDRVAE_EX_RAW_STATS;
-    ex.raw_stats_off = ws_off(st, epilogue_raw_stats_ptr(epi, 1, H, W));
-    rows_exchange(st, ex);
-    rows_compute(st, [=](cudaStream_t s) {
-      return launch_epilogue_phase_b(1, H, W, st->mode, st->factor, st->ev, st->out, nullptr, epi, s);
-    });
-  }
+  const int H = pl.hl, W = pl.w, rank = st->rank;
+  Decoder d = make_decoder(ctx, st, nullptr, 1, &st->pending);
+  d.lat = ws + pl.off_lat;
+  d.x = reinterpret_cast<float*>(ws + pl.off_x);
+  d.hbuf = reinterpret_cast<float*>(ws + pl.off_h);
+  d.t = ws + pl.off_t;
+  d.xa16 = ws + pl.off_xa;
+  d.xb16 = ws + pl.off_xb;
+  d.gn = ws + pl.off_gn;
+  d.gn_chunks = pl.gn_chunks;
+  step(d, [=](cudaStream_t s) {
+    // latent rows of this rank plus one neighbour row each side (rows outside the image are zero)
+    HDRVAE_TRY(launch_latent_rows_to_nhwc(st->latent, d.lat, ctx->op_dtype, ctx->c_z, ctx->c_lat, ctx->pq_w, ctx->pq_b, pl.h,
+                                          pl.w, rank * pl.hl - 1, pl.hl + 2, 64, s));
+    return gn_scratch_reset(d.gn, 1, pl.gn_chunks, s);
+  });
+  HDRVAE_TRY(decode_to_attention(d, H, W));
+  const void* o = nullptr;
+  attend_rows(d, W, &o);
+  HDRVAE_TRY(decode_from_attention(d, o, H, W));
+  // epilogue: phase A on this rank's rows, the HDR statistics all-reduced, phase B
+  void* epi = ws + pl.off_epi;
+  // conv_out's scratch: the other stream buffer is free by now
+  step(d, [=](cudaStream_t s) { return run_phase_a(ctx, d.t, 1, 8 * H, 8 * W, 1, d.hbuf, epi, s); });
+  hdrvae_exchange ex;
+  memset(&ex, 0, sizeof ex);
+  ex.kind = HDRVAE_EX_RAW_STATS;
+  ex.raw_stats_off = ws_off(st, epilogue_raw_stats_ptr(epi, 1, 8 * H, 8 * W));
+  rows_exchange(st, ex);
+  step(d, [=](cudaStream_t s) {
+    return launch_epilogue_phase_b(1, 8 * H, 8 * W, st->mode, st->factor, st->ev, st->out, nullptr, epi, s);
+  });
   return 0;
 }
 
