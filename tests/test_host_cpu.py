@@ -353,3 +353,27 @@ def test_public_header_is_plain_c():
     hdr = os.path.join(ROOT, "include", "hdrvae.h")
     r = subprocess.run(["gcc", "-std=c99", "-Wall", "-fsyntax-only", "-x", "c", hdr], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
+
+
+def test_environment_is_read_only_by_the_switch_table():
+    """The library reads its environment switches in one place, switches() in csrc/api.cu, and DESIGN.md §6 lists exactly
+    the switches read there: no getenv elsewhere in csrc/, every getenv there names its variable literally."""
+    csrc = os.path.join(ROOT, "vae_decode_hdr_b200", "csrc")
+    api = open(os.path.join(csrc, "api.cu")).read()
+    m = re.search(r"^const Switches& switches\(\) \{\n.*?^\}\n", api, flags=re.S | re.M)
+    assert m, "switches() not found in csrc/api.cu"
+    table = m.group(0)
+    for fn in sorted(os.listdir(csrc)):
+        if fn.endswith((".cu", ".cuh", ".h")):
+            src = open(os.path.join(csrc, fn)).read()
+            if fn == "api.cu":
+                src = src.replace(table, "")
+            assert "getenv" not in src, f"csrc/{fn} reads the environment outside switches()"
+    names = re.findall(r"getenv\(\"(HDRVAE_[A-Z0-9_]+)\"\)", table)
+    assert len(names) == table.count("getenv(") and len(set(names)) == len(names), table
+    design = open(os.path.join(ROOT, "DESIGN.md")).read()
+    sec = re.search(r"^## 6\..*?(?=^## 7\.)", design, flags=re.S | re.M)
+    assert sec, "DESIGN.md has no section 6"
+    para = re.search(r"^\*\*Switches\*\*.*?(?=\n\n)", sec.group(0), flags=re.S | re.M)
+    assert para, "DESIGN.md §6 has no **Switches** paragraph"
+    assert sorted(set(re.findall(r"HDRVAE_[A-Z0-9_]+", para.group(0)))) == sorted(names)

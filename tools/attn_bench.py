@@ -1,6 +1,6 @@
 """Attention core alone (hdrvae_attention: q, k, v 16-bit [B, T, 512]): device time of the whole test entry (which also
-allocates its workspace and transposes / interleaves the operands) and, for the fused kernel, of the kernel itself
-(library profile scope).  HDRVAE_ATTN_FUSED=0|1 HDRVAE_ATTN_CG=1|2 python tools/attn_bench.py [BxT ...]"""
+allocates its workspace and transposes / interleaves the operands) and of the fused kernel itself (library profile
+scope).  python tools/attn_bench.py [BxT ...]"""
 import os
 import sys
 import tempfile
@@ -40,4 +40,4 @@ for B, T in cases:
         if ln.startswith("attention fused kernel"):
             kms = float(ln.split("\t")[1].split()[0])
             kern = f"  kernel alone {kms:.3f} ms = {4.0 * B * T * T * 512 / (kms / 1e3) / 1e12:.1f} TFLOP/s"
-    print(f"fused={os.environ.get('HDRVAE_ATTN_FUSED', '1')} cg={os.environ.get('HDRVAE_ATTN_CG', '-')} B={B} T={T}: entry {ms:.3f} ms  {tf:.1f} TFLOP/s effective{kern}", flush=True)
+    print(f"B={B} T={T}: entry {ms:.3f} ms  {tf:.1f} TFLOP/s effective{kern}", flush=True)

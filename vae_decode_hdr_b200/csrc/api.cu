@@ -39,6 +39,26 @@ void set_error(const char* fmt, ...) {
 bool g_prof_on = false;
 std::vector<ProfEntry> g_prof;
 
+// ---- environment switches: the only place the library reads the environment ---------------------
+const Switches& switches() {
+  static const Switches sw = [] {
+    auto off = [](const char* e) { return e != nullptr && atoi(e) == 0; };
+    Switches w;
+    w.h16 = !off(getenv("HDRVAE_H16"));
+    w.x16 = !off(getenv("HDRVAE_X16"));
+    w.fuse_nin = !off(getenv("HDRVAE_FUSE_NIN"));
+    w.fuse_gn = !off(getenv("HDRVAE_FUSE_GN"));
+    const char* no_graph = getenv("HDRVAE_NO_GRAPH");
+    w.graphs = !(no_graph != nullptr && atoi(no_graph) != 0);
+    const char* impl = getenv("HDRVAE_CONV_IMPL");
+    w.conv_direct = impl != nullptr && strcmp(impl, "direct") == 0;
+    const char* dbg = getenv("HDRVAE_GEMM_DBG");
+    w.gemm_dbg = dbg != nullptr ? atoi(dbg) : 0;
+    return w;
+  }();
+  return sw;
+}
+
 }  // namespace hdrvae
 
 using namespace hdrvae;
@@ -225,22 +245,14 @@ int run_conv(hdrvae_ctx* ctx, const PackedConv& pc, const ConvIO& io, int B, int
 // conv (same-box A/B of the C2 step: 44.3 -> 43.4 ms; the chip runs at its power cap, so the 4x lower L2 -> SM operand
 // traffic also buys clock).  The 128-column convs that add the residual in place were the exception in round 1 (8 x 16
 // tiles: 1.76 vs 1.57 ms, their epilogue was the bound); with the round-2 epilogue the slab form wins there too
-// (1.21 vs 1.44 ms).  HDRVAE_SLAB=0 keeps the tap-reload form everywhere; HDRVAE_SLAB_MAXN / HDRVAE_SLAB_RES=0 move
-// the thresholds for experiments.
+// (1.21 vs 1.44 ms).
+static constexpr int kSlabMaxCols = 512;   // widest slab conv: the decoder's 512-channel convs
 bool conv_takes_slab(const PackedConv& pc, const ConvIO& io, int H, int W, int impl) {
-  static int slab_on = -1, slab_maxn = -1, slab_res = -1;
-  if (slab_on < 0) { const char* e = getenv("HDRVAE_SLAB"); slab_on = (e && atoi(e) == 0) ? 0 : 1; }
-  if (slab_maxn < 0) { const char* e = getenv("HDRVAE_SLAB_MAXN"); slab_maxn = e ? atoi(e) : 512; }
-  if (slab_res < 0) { const char* e = getenv("HDRVAE_SLAB_RES"); slab_res = e ? atoi(e) : 1; }
-  static int slab_up = -1;
-  if (slab_up < 0) { const char* e = getenv("HDRVAE_SLAB_UP"); slab_up = (e && atoi(e) == 0) ? 0 : 1; }
-  const bool res_ok = io.residual == nullptr || pc.cout_pad > 128 || slab_res != 0;
   if (pc.upsample)    // the decoder's upsample convs (256-column tiles, statistics [+ scaled operand copy] epilogues)
-    return slab_on && slab_up && pc.ks == 3 && pc.w_dtype != DT_F32 && pc.kmul == 1 && impl == HDRVAE_CONV_TCGEN05 && H * W >= 128 &&
-           pc.cout_pad >= 256 && pc.cout_pad <= slab_maxn && io.residual == nullptr && io.stats != nullptr &&
+    return pc.ks == 3 && pc.w_dtype != DT_F32 && pc.kmul == 1 && impl == HDRVAE_CONV_TCGEN05 && H * W >= 128 &&
+           pc.cout_pad >= 256 && pc.cout_pad <= kSlabMaxCols && io.residual == nullptr && io.stats != nullptr &&
            (io.y_dtype == DT_F32 || io.y2 == nullptr) && io.lrelu == 0.f && io.residual2 == nullptr;
-  return slab_on && pc.ks == 3 && pc.w_dtype != DT_F32 && impl != HDRVAE_CONV_DIRECT && H * W >= 128 &&
-         (pc.cout_pad <= 64 || (pc.cout_pad <= slab_maxn && res_ok));
+  return pc.ks == 3 && pc.w_dtype != DT_F32 && impl != HDRVAE_CONV_DIRECT && H * W >= 128 && pc.cout_pad <= kSlabMaxCols;
 }
 
 // Plain K-major GEMM: out[M][n_cols] = row_scale[m] * alpha * A[M][K] * Bm[n_cols][K]^T (+ bias) on the same kernel.
@@ -308,11 +320,11 @@ static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = f
   pl.off_vt = take((size_t)B * 512 * pl.Tp * 2 * km);
   pl.off_o = take((size_t)B * pl.T * 512 * 2 * km);
   pl.off_f32 = take(high ? (size_t)pl.Tp * 1536 * 4 + (size_t)B * 64 * pl.T * 4 : 0);   // high: fp32 q|k, v^T / o of one image; fp32 NHWC latent
-  // score / probability chunks, row partials and split-K partials exist only for the GEMM-level attention (validation
-  // build, HDRVAE_ATTN_FUSED=0, high precision): the fused kernel keeps S and P on the SM (up to 6.1 GiB less at 4096^2)
+  // score / probability chunks, row sums and split-K partials exist only for the GEMM-level attention (validation
+  // build, high precision): the fused kernel keeps S and P on the SM (up to 6.1 GiB less at 4096^2)
   pl.off_s = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 4 : 0);
   pl.off_p = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 2 * km : 0);
-  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 * 2 : 0);      // 1 / row sum, and -row max of the two-pass soft-max
+  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 : 0);          // 1 / row sum
   pl.off_part = take(attn_scratch ? (size_t)kSplitRowsBudget * 512 * 4 : 0);   // split-K partials of the PV GEMM
   // key splits of the fused kernel (fp32 O partials + (m, l) per row and split): the decoder lends its idle fp32 buffer
   // (off_h: nothing of a ResnetBlock is live across mid.attn_1); the stand-alone attention entry has no such buffer
@@ -336,18 +348,14 @@ static constexpr float kRawOperandScale = 1.0f / 16.0f;
 // type (2 B instead of 4 written by conv1, 2 instead of 4 read by norm2; its GroupNorm statistics still come from the
 // fp32 accumulators).  HDRVAE_H16=0 keeps it fp32.  Not used by the high-precision mode or the validation kernels.
 static bool h_is_16bit(hdrvae_ctx* ctx) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("HDRVAE_H16"); on = (e && atoi(e) == 0) ? 0 : 1; }
-  return on && !ctx->high && ctx->conv_impl == HDRVAE_CONV_TCGEN05;
+  return switches().h16 && !ctx->high && ctx->conv_impl == HDRVAE_CONV_TCGEN05;
 }
 
 // nin_shortcut fused into conv2 (extra K blocks of the slab conv kernel: K = 9 * Cout + Cin) instead of a separate 1x1 conv
 // whose fp32 output conv2 then reads back as its residual.  HDRVAE_FUSE_NIN=0 keeps the two launches.
 static bool nin_is_fused(hdrvae_ctx* ctx, const ResW& rw, int H, int W) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("HDRVAE_FUSE_NIN"); on = (e && atoi(e) == 0) ? 0 : 1; }
   ConvIO probe;
-  return on && rw.has_nin && !ctx->high && rw.nin_x16.w[0] != nullptr && conv_takes_slab(rw.c2, probe, H, W, ctx->conv_impl);
+  return switches().fuse_nin && rw.has_nin && !ctx->high && rw.nin_x16.w[0] != nullptr && conv_takes_slab(rw.c2, probe, H, W, ctx->conv_impl);
 }
 
 // The residual stream x itself is stored as fp16 scaled by 2^-4 (what the raw-stream convs read anyway): conv2 / proj_out
@@ -357,41 +365,23 @@ static bool nin_is_fused(hdrvae_ctx* ctx, const ResW& rw, int H, int W) {
 // the fp32 oracle; every parity test keeps its 1e-2 bound).  HDRVAE_X16=0 keeps the fp32 stream.  Needs the fused
 // shortcut and fp16 operands; not used by the bf16 and high-precision modes or the validation kernels.
 static bool x_is_16bit(hdrvae_ctx* ctx) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("HDRVAE_X16"); on = (e && atoi(e) == 0) ? 0 : 1; }
-  static int nin_on = -1;
-  if (nin_on < 0) { const char* e = getenv("HDRVAE_FUSE_NIN"); nin_on = (e && atoi(e) == 0) ? 0 : 1; }
-  return on && nin_on && !ctx->high && ctx->op_dtype == DT_F16 && ctx->conv_impl == HDRVAE_CONV_TCGEN05 && h_is_16bit(ctx);
+  return switches().x16 && switches().fuse_nin && !ctx->high && ctx->op_dtype == DT_F16 && ctx->conv_impl == HDRVAE_CONV_TCGEN05 && h_is_16bit(ctx);
 }
 
 // GroupNorm + SiLU applied inside the consuming conv (GemmParams::xf_*) instead of by the streaming kernel: for the 3x3
 // slab convs whose input is a scaled fp16 tensor (x and h in the default mode).  HDRVAE_FUSE_GN=0 keeps the streaming kernel.
 static bool gn_is_fused(hdrvae_ctx* ctx, const PackedConv& pc, const ConvIO& io, int x_dtype, int H, int W) {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("HDRVAE_FUSE_GN");
-    const char* g = getenv("HDRVAE_CTA_GROUP");
-    on = ((e && atoi(e) == 0) || (g && atoi(g) == 1)) ? 0 : 1;      // the fused builds are CTA-pair builds
-  }
-  // (256-column tiles only: a 128-column slab's MMAs are too short to hide the transform behind, gemm_tc.cu)
-  return on && x_is_16bit(ctx) && x_dtype == DT_F16 && pc.w_dtype == DT_F16 && pc.kmul == 1 && !pc.upsample && pc.ks == 3 &&
+  // (256-column tiles only: a 128-column slab's MMAs are too short to hide the transform behind, gemm_tc.cu; the fused
+  // builds are CTA-pair builds)
+  return switches().fuse_gn && x_is_16bit(ctx) && x_dtype == DT_F16 && pc.w_dtype == DT_F16 && pc.kmul == 1 && !pc.upsample && pc.ks == 3 &&
          pc.cout_pad >= 256 && pc.cin_pad % 64 == 0 && ctx->cta_group != 1 && io.x2 == nullptr && io.y_dtype == DT_F16 &&
          io.stats != nullptr && conv_takes_slab(pc, io, H, W, ctx->conv_impl);
 }
 
-// HDRVAE_ATTN_FUSED=0 selects the GEMM-level form (QK^T twice with the soft-max fused into the GEMM epilogues, P through
-// HBM, split-K PV + reduce) that the fused kernel replaced; the CUDA-core validation build always takes it.
-static bool attention_fused_enabled(hdrvae_ctx* ctx) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("HDRVAE_ATTN_FUSED"); on = (e && atoi(e) == 0) ? 0 : 1; }
-  return on && ctx->conv_impl == HDRVAE_CONV_TCGEN05;
-}
-static int attention_cta_group(hdrvae_ctx* ctx) {
-  static int cg = -1;
-  if (cg < 0) { const char* e = getenv("HDRVAE_ATTN_CG"); cg = e ? atoi(e) : 0; }
-  if (cg == 1 || cg == 2) return cg;
-  return ctx->cta_group == 1 ? 1 : 2;
-}
+// The fused attention kernel runs with the tensor-core convs; the CUDA-core validation build takes the GEMM-level form
+// (fp32 S, row soft-max kernel, P through HBM, split-K PV + reduce) that the fused kernel replaced.
+static bool attention_fused_enabled(hdrvae_ctx* ctx) { return ctx->conv_impl == HDRVAE_CONV_TCGEN05; }
+static int attention_cta_group(hdrvae_ctx* ctx) { return ctx->cta_group == 1 ? 1 : 2; }
 
 // Attention of n_q query rows (q: 16-bit, row stride 1024) against T keys (k: row stride 1024, rows >= T zero up to
 // Tp) and v^T [512][Tp]; o: 16-bit [n_q][512].  Scratch (S, P, 1/sum, split-K partials) comes from the plan.
@@ -413,43 +403,14 @@ static int attention_rows(hdrvae_ctx* ctx, uint8_t* ws, size_t off_s, size_t off
   float* S = reinterpret_cast<float*>(ws + off_s);
   uint16_t* P = reinterpret_cast<uint16_t*>(ws + off_p);
   float* inv = reinterpret_cast<float*>(ws + off_inv);
-  float* negmax = inv + s_rows;                        // the plan reserves 2 * s_rows floats at off_inv
-  static int two_pass_on = -1;
-  if (two_pass_on < 0) { const char* e = getenv("HDRVAE_ATTN_TWO_PASS"); two_pass_on = (e && atoi(e) == 0) ? 0 : 1; }
-  // the fused form needs the 256-column CTA-pair build and whole 256-column tiles of keys
-  const bool two_pass = two_pass_on && impl == HDRVAE_CONV_TCGEN05 && ctx->cta_group != 1 && Tp % 256 == 0 && Tp >= 256;
   for (int r0 = 0; r0 < n_q; r0 += s_rows) {
     const int rows = std::min(s_rows, n_q - r0);
-    if (two_pass) {
-      // Soft-max fused into the QK^T GEMM, two passes (no fp32 score matrix in HBM: 4 bytes per score instead of 12).
-      // Pass 1: row max of alpha q k^T from the epilogue's row-per-thread layout; pass 2 recomputes q k^T and writes
-      // P = exp(s - rowmax) as the 16-bit operand of the PV GEMM plus the row sums.  S doubles as the partial buffer.
-      GemmParams g;
-      memset(&g, 0, sizeof g);
-      g.a = q + (size_t)r0 * 1024; g.ab_dtype = dt;
-      g.a_px_stride = 1024; g.a_row_stride = (long long)rows * 1024; g.a_img_stride = (long long)rows * 1024;
-      g.n_img = 1; g.H = 1; g.W = rows;
-      g.k_per_tap = 512; g.ntaps = 1;
-      g.b = k; g.b_row_stride = 1024; g.b_rows = Tp; g.n_cols = Tp; g.n_valid_cols = T;
-      g.out = P; g.out_dtype = dt; g.out_px_stride = Tp;
-      g.sy = g.sx = 1; g.alpha = qk_alpha;
-      g.tw_log2 = 7; g.TW = 128; g.TH = 1; g.tiles_x = (rows + 127) / 128; g.tiles_y = 1;
-      g.cta_group = ctx->cta_group;
-      g.row_part = S; g.row_parts = (Tp / 256) * 2;
-      g.row_mode = 1;
-      HDRVAE_TRY(launch_gemm_tc(g, ctx->num_sms, s));
-      HDRVAE_TRY(launch_attn_row_parts(S, rows, g.row_parts, 1, negmax, s));
-      g.row_mode = 2; g.bias = negmax; g.bias_per_row = 1;
-      HDRVAE_TRY(launch_gemm_tc(g, ctx->num_sms, s));
-      HDRVAE_TRY(launch_attn_row_parts(S, rows, g.row_parts, 2, inv, s));
-    } else {
-      // S = alpha q k^T, fp32 (the decoder folds 1/sqrt(d) into the q weights: alpha = 1); padded key
-      // columns give 0 and are masked by the softmax
-      HDRVAE_TRY(run_gemm(ctx, dt, q + (size_t)r0 * 1024, 1024, rows, 512, k, 1024, Tp, Tp, S, Tp, DT_F32, nullptr, false,
-                          qk_alpha, nullptr, impl, s));
-      // P = exp(S - rowmax) (16-bit), inv = 1 / rowsum; O = inv * (P V)
-      HDRVAE_TRY(launch_softmax_rows(S, P, dt, inv, rows, T, Tp, Tp, Tp, s));
-    }
+    // S = alpha q k^T, fp32 (the decoder folds 1/sqrt(d) into the q weights: alpha = 1); padded key
+    // columns give 0 and are masked by the softmax
+    HDRVAE_TRY(run_gemm(ctx, dt, q + (size_t)r0 * 1024, 1024, rows, 512, k, 1024, Tp, Tp, S, Tp, DT_F32, nullptr, false,
+                        qk_alpha, nullptr, impl, s));
+    // P = exp(S - rowmax) (16-bit), inv = 1 / rowsum; O = inv * (P V)
+    HDRVAE_TRY(launch_softmax_rows(S, P, dt, inv, rows, T, Tp, Tp, Tp, s));
     // A row chunk gives only rows/128 x 2 tiles: when that cannot fill the GPU the K (key) dimension is split
     // across `splits` images of one GEMM (fp32 partials) and reduced afterwards.
     const int tiles = ((rows + 127) / 128) * 2;
@@ -485,16 +446,13 @@ static int attention_rows(hdrvae_ctx* ctx, uint8_t* ws, size_t off_s, size_t off
 
 // Epilogue phase A on the decoder's features (slab start `feat`, `pad` halo rows above / below each image's H rows).
 // fp16 operands: conv_out runs on the tensor cores into `conv8` (dense [B][H][W][8] fp32 scratch), then one streaming
-// pass does the MAX-pool and the statistics; otherwise (bf16 operands, validation kernel, HDRVAE_TC_CONVOUT=0) the
-// all-in-one CUDA-core kernel.
+// pass does the MAX-pool and the statistics; otherwise (bf16 operands, validation kernel) the all-in-one CUDA-core kernel.
 static int run_phase_a(hdrvae_ctx* ctx, const void* feat, int B, int H, int W, int pad, float* conv8, void* epi, cudaStream_t s) {
-  static int tc_on = -1;
-  if (tc_on < 0) { const char* e = getenv("HDRVAE_TC_CONVOUT"); tc_on = (e && atoi(e) == 0) ? 0 : 1; }
   const long long img_stride = (long long)(H + 2 * pad) * W * 128;
   if (ctx->high)     // fp32 features: conv_out in fp32 on the CUDA cores (the 1e-5 parity kernel)
     return launch_epilogue_phase_a(feat, DT_F32, B, H, W, ctx->conv_out_w, ctx->conv_out_b, nullptr, epi, s, 0, img_stride);
   const uint16_t* interior = reinterpret_cast<const uint16_t*>(feat) + (size_t)pad * W * 128;
-  if (tc_on && ctx->op_dtype == DT_F16 && ctx->conv_impl == HDRVAE_CONV_TCGEN05 && ctx->conv_out_tc.w[0] != nullptr) {
+  if (ctx->op_dtype == DT_F16 && ctx->conv_impl == HDRVAE_CONV_TCGEN05 && ctx->conv_out_tc.w[0] != nullptr) {
     ConvIO io; io.x = feat; io.x_pad = pad; io.y = conv8; io.y_dtype = DT_F32; io.y_channels = 8; io.n_store = 8;
     HDRVAE_TRY(run_conv(ctx, ctx->conv_out_tc, io, B, H, W, HDRVAE_CONV_TCGEN05, s));
     return launch_epilogue_phase_a_pre(interior, ctx->op_dtype, B, H, W, conv8, ctx->conv_out_b, nullptr, epi, s, img_stride);
@@ -605,7 +563,7 @@ static RowsPlan make_rows_plan(int h, int w, int world, bool attn_scratch = true
   pl.off_o = take((size_t)pl.Tl * 512 * 2);
   pl.off_s = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 4 : 0);      // GEMM-level attention only (see make_plan)
   pl.off_p = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 2 : 0);
-  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 * 2 : 0);
+  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 : 0);
   pl.off_part = take(attn_scratch ? (size_t)kSplitRowsBudget * 512 * 4 : 0);
   pl.off_epi = take(epilogue_scratch_bytes(1, 8 * pl.hl, 8 * w));
   pl.off_mail = take(sizeof(RowsMailbox));              // flags / tables of the device-driven exchanges (rows_p2p.cu)
@@ -1046,8 +1004,7 @@ int hdrvae_create(hdrvae_ctx** out, int device) {
   hdrvae_ctx* ctx = new hdrvae_ctx();
   ctx->device = device;
   ctx->num_sms = prop.multiProcessorCount;
-  const char* impl = getenv("HDRVAE_CONV_IMPL");
-  if (impl != nullptr && strcmp(impl, "direct") == 0) ctx->conv_impl = HDRVAE_CONV_DIRECT;
+  if (switches().conv_direct) ctx->conv_impl = HDRVAE_CONV_DIRECT;
   *out = ctx;
   return 0;
 }
@@ -1269,9 +1226,7 @@ int hdrvae_workspace_bytes(hdrvae_ctx* ctx, int B, int h, int w, size_t* bytes) 
 // sharded path replays the same graphs as the single-GPU one.  The latent is staged into / the image out of fixed
 // workspace buffers so the graphs do not depend on the caller's tensor addresses.  HDRVAE_NO_GRAPH=1 disables it.
 static bool graphs_enabled(hdrvae_ctx* ctx, cudaStream_t s) {
-  static int no_graph = -1;
-  if (no_graph < 0) { const char* e = getenv("HDRVAE_NO_GRAPH"); no_graph = (e && atoi(e) != 0) ? 1 : 0; }
-  return ctx->use_graphs && !no_graph && !g_prof_on && s != nullptr;     // capture needs a non-default stream
+  return ctx->use_graphs && switches().graphs && !g_prof_on && s != nullptr;     // capture needs a non-default stream
 }
 
 static int run_segment(hdrvae_ctx* ctx, hdrvae_ctx::GraphEntry key, cudaStream_t s, const std::function<int()>& body) {

@@ -480,15 +480,11 @@ int map3d(CUtensorMap* m, const void* base, int dt, long long d0, long long d1, 
 // 2048^2, 2 at 4096^2.  It exists for wave quantisation: one rank's 32 768 query rows of a 4096^2 image row-tiled over 8
 // GPUs are 256 pair units = 3.46 waves of the 74 concurrent pairs (86 %); with 2 splits 6.9 waves (99 %).  More splits
 // than needed cost: every unit loads its Q tile and ramps its pipeline again (measured at T = 65 536: 4 splits 9.20 ms
-// against 8.57 ms unsplit), so the rule is as coarse as the C4 case allows.  HDRVAE_ATTN_SPLITS forces a count.
+// against 8.57 ms unsplit), so the rule is as coarse as the C4 case allows.
 int attention_key_splits(int n_keys) {
-  static int forced = -1;
-  if (forced < 0) { const char* e = getenv("HDRVAE_ATTN_SPLITS"); forced = e ? atoi(e) : 0; }
   const int n_blocks = (n_keys + kABlockKeys - 1) / kABlockKeys;
   int splits = 1;
   while (splits < 8 && n_blocks / (splits * 2) >= 1024) splits *= 2;
-  if (forced >= 1) splits = forced;
-  while (splits > 1 && n_blocks / splits < 8) splits /= 2;
   return splits;
 }
 

@@ -38,6 +38,19 @@ extern long long g_launch_count;   // kernels launched by this library (bench.py
     if (_r != 0) return _r;   \
   } while (0)
 
+// The library's environment switches (DESIGN.md §6), read once per process by switches() (api.cu).  Defaults are the
+// product path; each field says what setting the variable changes.
+struct Switches {
+  bool h16 = true;           // HDRVAE_H16=0: the block-internal tensor h in fp32
+  bool x16 = true;           // HDRVAE_X16=0: the residual stream in fp32
+  bool fuse_nin = true;      // HDRVAE_FUSE_NIN=0: nin_shortcut as its own launch
+  bool fuse_gn = true;       // HDRVAE_FUSE_GN=0: GroupNorm + SiLU by the streaming kernel everywhere
+  bool graphs = true;        // HDRVAE_NO_GRAPH=1: no CUDA-graph capture
+  bool conv_direct = false;  // HDRVAE_CONV_IMPL=direct: new contexts start on the CUDA-core validation conv
+  int gemm_dbg = 0;          // HDRVAE_GEMM_DBG: GemmParams::dbg of every tensor-core GEMM launch
+};
+const Switches& switches();
+
 inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -99,14 +112,6 @@ struct GemmParams {
   const float* residual2;  // second fp32 residual, same addressing as out, added unscaled; or null
   float lrelu;       // LeakyReLU negative slope applied last (0: none)
   int n_store;       // columns actually stored (multiple of 4; 0: n_cols) — a Cout padded up to 32 stores less
-  // attention soft-max fused into the QK^T GEMM, two passes (row_mode 1 and 2): the epilogue works on whole rows in
-  // the TMEM row-per-thread layout.  1: per-row max of alpha * acc over this tile's valid columns -> row_part, nothing
-  // else is stored.  2: e = exp(alpha * acc + bias[row]) (bias = -row max), stored as the 16-bit output (0 in the
-  // padding columns), per-row sum of e -> row_part.  row_part[row * row_parts + n_tile * 2 + column half].
-  int row_mode;
-  float* row_part;
-  int row_parts;
-  int n_valid_cols;        // columns >= this are padding (0: n_cols)
   const float* row_scale;  // per M row (x coordinate) multiplier of the accumulator, or null
   float alpha;       // accumulator scale applied before bias (1.0 for convs)
   void* out2;        // optional second output: out * out2_scale as a 16-bit tensor (same addressing), or null
@@ -128,28 +133,12 @@ struct GemmParams {
   float xf_in_scale;
   int xf_y_lo, xf_y_hi;
   int cta_group;     // 0 = library default (CTA pairs), 1 = single CTA, 2 = CTA pair (tcgen05 cta_group::2)
-  int dbg;           // diagnostics (env HDRVAE_GEMM_DBG): bit0 = producer skips the TMA loads, bit1 = issuer skips the MMAs
+  int dbg;           // diagnostics (Switches::gemm_dbg): bit0 = producer skips the TMA loads, bit1 = issuer skips the MMAs,
+                     // bit5 (32) = CTA 0 prints its wait cycles
 };
 
 #ifdef __CUDACC__
-// SiLU variants of the GroupNorm + SiLU kernel (HDRVAE_SILU_MUFU).  silu_f: exp(-v) on the FMA pipe — round-to-nearest
-// split t = n + f by the 1.5 * 2^23 trick, 2^f as a degree-6 polynomial on [-0.5, 0.5] (relative error < 3e-8), exponent
-// inserted with integer arithmetic — the special-function unit is left with the one reciprocal.
-__device__ __forceinline__ float silu_f(float v) {
-  float t = fminf(fmaxf(-v * 1.4426950408889634f, -125.f), 125.f);
-  const float tm = t + 12582912.f;                       // n = round(t) sits in the low mantissa bits
-  const float f = t - (tm - 12582912.f);
-  float p = 1.54035304e-4f;
-  p = fmaf(p, f, 1.33335581e-3f);
-  p = fmaf(p, f, 9.61812911e-3f);
-  p = fmaf(p, f, 5.55041087e-2f);
-  p = fmaf(p, f, 2.40226507e-1f);
-  p = fmaf(p, f, 6.93147181e-1f);
-  p = fmaf(p, f, 1.0f);
-  const float e = __int_as_float(__float_as_int(p) + (__float_as_int(tm) << 23));     // 2^t = exp(-v)
-  return __fdividef(v, 1.f + e);
-}
-// the same with exp on the special-function unit (ex2 + rcp): fewer instructions, two XU operations per element
+// SiLU with exp on the special-function unit (ex2 + rcp): two XU operations per element
 __device__ __forceinline__ float silu_mufu(float v) { return __fdividef(v, 1.f + __expf(-v)); }
 // Packed fp32 pairs (sm_100 FFMA2 / FADD2 / FMUL2): one issue slot per two lanes of arithmetic.
 __device__ __forceinline__ float2 f2_fma(float2 a, float2 b, float2 c) {

@@ -27,7 +27,6 @@ int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, 
                                const float* pq_b, int h, int w, int y0, int rows, int cpad, cudaStream_t s);
 int launch_softmax_rows(const float* s, void* p, int p_dtype, float* inv_sum, int n_rows, int n_valid, int n_pad,
                         long long s_ld, long long p_ld, cudaStream_t st);
-int launch_attn_row_parts(const float* part, int rows, int parts, int mode, float* out, cudaStream_t st);
 int launch_transpose_pad(const void* in, void* out, int rows, int cols, int out_ld, cudaStream_t s);
 int launch_attn_reduce_splits(const float* part, const float* inv_sum, void* out, int out_dtype, int rows, int cols,
                               int splits, cudaStream_t st);

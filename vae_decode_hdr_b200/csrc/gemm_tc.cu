@@ -20,10 +20,6 @@
 #pragma nv_diag_suppress 128   // "loop is not reachable": the tap-reload loops after the slab branch of an if-constexpr
 #include "ptx.cuh"
 
-#ifndef HDRVAE_SLAB_PITCH
-#define HDRVAE_SLAB_PITCH 10
-#endif
-
 namespace hdrvae {
 
 constexpr int kBlockM = 128;
@@ -51,7 +47,7 @@ constexpr int kSmemFixed = 8 * 4096 /*epilogue transpose patches*/ + 256 /*barri
 // Pitch: the 10 pixels a tile row needs (8 + halo), not a power of two: the 128-byte swizzle is a function of the shared
 // memory address bits, which TMA (writing) and the UMMA descriptors (reading, 8-row groups 10 lines apart) both honour,
 // so row groups need not start on 1024-byte boundaries — only the buffers do.
-constexpr int kSlabRows = 18, kSlabPitch = HDRVAE_SLAB_PITCH;
+constexpr int kSlabRows = 18, kSlabPitch = 10;
 constexpr int kSlabBytes = kSlabRows * kSlabPitch * kRowBytes;   // 22.5 KB of TMA traffic per slab
 constexpr int kSlabBufBytes = (kSlabBytes + 1023) / 1024 * 1024;
 template <int BLOCK_N, int CG, int KSUB, int SLAB = 0>
@@ -118,8 +114,6 @@ enum : int {
   EPI_ROWOPS = 32,   // per-row bias / per-row scale (attention GEMMs)
   EPI_LRELU = 64,    // LeakyReLU applied last (upscaler convs)
   EPI_RES2 = 128,    // + second fp32 residual (end of an RRDB: 0.04 acc + 0.2 x2 + x0)
-  EPI_ROWMAX = 256,  // attention pass 1: per-row max of the scores, nothing stored (GemmParams::row_mode 1)
-  EPI_EXPSUM = 512,  // attention pass 2: exp(score - row max) as the 16-bit output + per-row sums (row_mode 2)
   EPI_RES16 = 1024,  // + residual stored as a (scaled) 16-bit tensor of type res_dtype: t += res_scale * r
 };
 
@@ -613,7 +607,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // Fast path (specialised builds, tiles that lie wholly inside the image): the element offset of this lane's 4 columns
     // of pixel `it` relative to the tile origin is the same for every tile, so it is computed once per kernel; a tile
     // then costs one (warp-uniform) origin and no per-pixel address arithmetic or bounds masks.
-    constexpr bool kFastBuild = !kGen && (EPI & (EPI_ROWOPS | EPI_ROWMAX | EPI_EXPSUM)) == 0;
+    constexpr bool kFastBuild = !kGen && (EPI & EPI_ROWOPS) == 0;
     uint32_t lo[8], lo2[8];
 #pragma unroll
     for (int it = 0; it < 8; ++it) {
@@ -810,69 +804,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
 
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BLOCK_N;
-      if constexpr ((EPI & (EPI_ROWMAX | EPI_EXPSUM)) != 0) {
-        // ---- soft-max passes of the attention (rows = queries, H = 1, 128-pixel row tiles): TMEM hands every thread
-        // one whole query row of the tile, so the row max / the row sum of exp are plain per-thread reductions
-        constexpr bool kExp = (EPI & EPI_EXPSUM) != 0;
-        const int xrow = tx * p.TW + q * 32 + lane;
-        const bool row_live = tile_live && xrow < p.W;
-        const int n_valid = p.n_valid_cols > 0 ? p.n_valid_cols : p.n_cols;
-        const float negm = (kExp && row_live) ? __ldg(p.bias + xrow) : 0.f;
-        float racc = kExp ? 0.f : -INFINITY;
-        ptx::mbar_wait(&tmem_full_bar[acc], acc_phase);
-        ptx::tc_fence_after_sync();
-        uint32_t v[32];
-        ptx::tmem_ld_32x32(t_row + cbase, v);
-#pragma unroll 1
-        for (int ci = 0; ci < kChunksPerWarp; ++ci) {
-          const int c0 = cbase + ci * 32;
-          const int col = c0 + slot * 4;
-          ptx::tmem_ld_wait(v);
-          float e[32];
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const bool valid = (n0 + c0 + j) < n_valid;
-            const float sv = __uint_as_float(v[j]);
-            if (kExp) {
-              e[j] = valid ? __expf(fmaf(sv, alpha, negm)) : 0.f;
-              racc += e[j];
-            } else if (valid) {
-              racc = fmaxf(racc, sv * alpha);
-            }
-          }
-          if (kExp) {
-            __syncwarp();                                   // previous chunk's readers are done with the patch
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-              patch[lane * 8 + (j ^ (lane & 7))] = make_float4(e[4 * j], e[4 * j + 1], e[4 * j + 2], e[4 * j + 3]);
-          }
-          if (ci + 1 < kChunksPerWarp) ptx::tmem_ld_32x32(t_row + c0 + 32, v);
-          if (kExp) {
-            __syncwarp();
-            const uint32_t cmask = (n0 + col) < p.n_cols ? pmask : 0u;
-#pragma unroll
-            for (int it = 0; it < 8; ++it) {
-              const int rr = it * 4 + sr;
-              const float4 a = patch[rr * 8 + (slot ^ (rr & 7))];
-              if (cmask >> it & 1) {
-                uint2 o;
-                if (out16_bf) { o.x = pack_bf16x2(a.x, a.y); o.y = pack_bf16x2(a.z, a.w); }
-                else { o.x = pack_f16x2(a.x, a.y); o.y = pack_f16x2(a.z, a.w); }
-                *reinterpret_cast<uint2*>(outh + poff[it] + col) = o;
-              }
-            }
-          }
-        }
-        if (row_live) p.row_part[(long long)xrow * p.row_parts + nt * 2 + half] = racc;
-        ptx::tc_fence_before_sync();
-        __syncwarp();
-        if (lane == 0) {
-          if (CG == 2) ptx::mbar_arrive_cluster(&tmem_empty_bar[acc], 0);
-          else ptx::mbar_arrive(&tmem_empty_bar[acc]);
-        }
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        continue;
-      }
       // Software pipeline over the warp's chunks: the TMEM load of chunk ci+1 is issued as soon as the registers of
       // chunk ci have gone to the transpose patch, so it overlaps the store phase.  ncu on the in-place-residual
       // 128 -> 128 conv (profiles/r02_ncu_conv128_residual_summary.txt): tensor pipe 50 %, DRAM 48 %, the epilogue warps
@@ -906,7 +837,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const uint32_t cmask = (n0 + col) < n_store ? pmask : 0u;   // n_cols % 32 == 0 and n_store % 4 == 0 on every call site
         float4 (&rres)[8] = rres_buf[kPre == 2 ? ci : 0];
         if (ci > 0 && kPre == 1) load_res(ci, rres);      // residual: issued first, overlaps the TMEM wait / transpose
-        if (ci > 0 && (p.dbg & 4)) ptx::tmem_ld_32x32(t_row + c0, v);   // diagnostics: un-pipelined TMEM load
         float4 rres2[8];
         if (has_res2) {
 #pragma unroll
@@ -921,7 +851,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         for (int j = 0; j < 8; ++j)
           patch[lane * 8 + (j ^ (lane & 7))] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
                                                            __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-        if (ci + 1 < kChunksPerWarp && !(p.dbg & 4)) {    // v has been consumed: start the next chunk's loads now
+        if (ci + 1 < kChunksPerWarp) {                    // v has been consumed: start the next chunk's loads now
           ptx::tmem_ld_32x32(t_row + c0 + 32, v);
         }
         __syncwarp();
@@ -1153,10 +1083,7 @@ static int launch_tc(const GemmParams& p_in, int num_sms, cudaStream_t stream) {
   GemmParams p = p_in;
   if (p.res_scale == 0.f) p.res_scale = 1.f;
   using Cfg = TcConfig<BLOCK_N, CG, KSUB, SLAB>;
-  {
-    const char* d = getenv("HDRVAE_GEMM_DBG");
-    p.dbg = d ? atoi(d) : 0;
-  }
+  p.dbg = switches().gemm_dbg;
   p.n_tiles_n = (p.n_cols + BLOCK_N - 1) / BLOCK_N;
   TensorMapPair maps;
   HDRVAE_TRY(make_maps(p, BLOCK_N / CG, &maps, SLAB));  // a CTA of a pair stages half of the B rows
@@ -1202,10 +1129,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
                  "gemm_tc: GroupNorm statistics need 128/256/512 output channels");
   HDRVAE_REQUIRE(p.stats == nullptr || (p.n_cols & (p.n_cols - 1)) == 0, "gemm_tc: GroupNorm statistics need 128/256/512 output channels");
   const bool tf32 = p.ab_dtype == DT_F32;
-  HDRVAE_REQUIRE(p.row_mode == 0 || (!tf32 && p.cta_group != 1), "gemm_tc: the soft-max passes exist for 16-bit CTA-pair builds");
-  static int cg = -1;                                       // CTA pairs by default; HDRVAE_CTA_GROUP=1 selects single CTAs
-  if (cg < 0) { const char* e = getenv("HDRVAE_CTA_GROUP"); cg = (e && atoi(e) == 1) ? 1 : 2; }
-  int use_cg = p.cta_group > 0 ? p.cta_group : cg;
+  int use_cg = p.cta_group > 0 ? p.cta_group : 2;           // CTA pairs by default
   // A CTA pair shares one B tile, so with a per-image K offset into B (split-K) both m-tiles of a pair must
   // belong to the same image: an odd number of tiles per image runs as single CTAs.
   if (p.b_img_k_stride != 0 && (p.tiles_x * p.tiles_y) % 2 != 0) use_cg = 1;
@@ -1272,13 +1196,6 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
     } else {
       epi = -1;
     }
-    if (p.row_mode != 0) {
-      HDRVAE_REQUIRE(!n128 && p.tw_log2 == 7 && p.H == 1 && p.row_part != nullptr && p.ntaps == 1 && p.b_img_k_stride == 0,
-                     "gemm_tc: the soft-max passes are row-major GEMMs with >= 256 columns");
-      if (p.row_mode == 1) return launch_tc<256, false, 2, EPI_ROWMAX>(p, num_sms, stream);
-      HDRVAE_REQUIRE(p.out_dtype != DT_F32 && p.bias != nullptr, "gemm_tc: soft-max pass 2 writes a 16-bit output and needs -max per row");
-      return launch_tc<256, false, 2, EPI_OUT16 | EPI_EXPSUM>(p, num_sms, stream);
-    }
     if (p.slab && n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0) {
       // the decoder's 128-channel 3x3 convs: slab variant, weights in groups of 3 taps
       if (epi == EPI_STATS) return launch_tc<128, false, 2, EPI_STATS, 3>(p, num_sms, stream);
@@ -1305,7 +1222,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
       HDRVAE_REQUIRE(false, "gemm_tc: no fused-GroupNorm build for this epilogue (%d)", epi);
     }
     if (p.slab && !n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0) {
-      // 256-column tiles: slab variant with one tap of weights per stage (experiment switch HDRVAE_SLAB_MAXN)
+      // 256-column tiles: slab variant with one tap of weights per stage
       if (epi == EPI_STATS) return launch_tc<256, false, 2, EPI_STATS, 1>(p, num_sms, stream);
       if (epi == (EPI_OUT16 | EPI_STATS)) return launch_tc<256, false, 2, EPI_OUT16 | EPI_STATS, 1>(p, num_sms, stream);
       if (epi == (EPI_RES | EPI_STATS)) return launch_tc<256, false, 2, EPI_RES | EPI_STATS, 1>(p, num_sms, stream);

@@ -204,30 +204,26 @@ static int gn_slices(int n_chunks) {
 }
 
 
-// kExp: how the SiLU's exp / reciprocal are evaluated — 0 polynomial (FMA pipe only), 1 ex2 + rcp (two XU ops), 2 ex2 +
-// Newton reciprocal (one XU op)
-template <int kExp> __device__ __forceinline__ float silu_sel(float v) {
-  return kExp == 1 ? silu_mufu(v) : kExp == 2 ? silu_nr(v) : silu_f(v);
-}
-
 // v[j] = [silu](v[j] * a[j] + b[j]) for 8 channels of one pixel, in packed fp32 pairs (FFMA2 / FMUL2 / FADD2): the same
 // operations in the same order as the scalar form, bit for bit, and the SAME helper (silu_nr2) the conv kernel's in-place
 // slab transform uses, which is what keeps the two roads identical.  A third fewer instructions; measured neutral on the
 // kernel's time (0.484 vs 0.488 ms for the 128-channel layers at 4 x 1024^2): it waits on its latency chain, not on issue.
-template <bool kSilu, int kExp>
+// kNewton: how the SiLU's exp / reciprocal are evaluated — ex2 + Newton reciprocal (one XU op, 16-bit outputs) or ex2 +
+// rcp (two XU ops, fp32 / hi|lo|hi outputs)
+template <bool kSilu, bool kNewton>
 __device__ __forceinline__ void norm_act8(float (&v)[8], const float (&a)[8], const float (&b)[8]) {
 #pragma unroll
   for (int j = 0; j < 8; j += 2) {
     float2 t = f2_fma(make_float2(v[j], v[j + 1]), make_float2(a[j], a[j + 1]), make_float2(b[j], b[j + 1]));
     if (kSilu) {
-      if (kExp == 2) t = silu_nr2(t);
-      else t = make_float2(silu_sel<kExp>(t.x), silu_sel<kExp>(t.y));
+      if (kNewton) t = silu_nr2(t);
+      else t = make_float2(silu_mufu(t.x), silu_mufu(t.y));
     }
     v[j] = t.x; v[j + 1] = t.y;
   }
 }
 
-template <typename TIn, typename TOut, bool kSilu, int kMufu = 0>
+template <typename TIn, typename TOut, bool kSilu, bool kNewton>
 __global__ void __launch_bounds__(kGnThreads)
 gn_apply_kernel(const TIn* __restrict__ x, TOut* __restrict__ y, const float* __restrict__ scale,
                 const float* __restrict__ shift, int HW, int C, int px_per_block, long long x_img_stride,
@@ -261,14 +257,14 @@ gn_apply_kernel(const TIn* __restrict__ x, TOut* __restrict__ y, const float* __
     for (int u = 0; u < U; ++u) Ld8<TIn>::ld(xin + ((long long)(p + u * p_step) * vpp + vi) * 8, v[u]);
 #pragma unroll
     for (int u = 0; u < U; ++u) {
-      norm_act8<kSilu, kMufu>(v[u], a, b);
+      norm_act8<kSilu, kNewton>(v[u], a, b);
       store8<TOut>(yout, (long long)(p + u * p_step), vpp, vi, v[u]);
     }
   }
   for (; p < p1; p += p_step) {
     float v[8];
     Ld8<TIn>::ld(xin + ((long long)p * vpp + vi) * 8, v);
-    norm_act8<kSilu, kMufu>(v, a, b);
+    norm_act8<kSilu, kNewton>(v, a, b);
     store8<TOut>(yout, (long long)p, vpp, vi, v);
   }
 }
@@ -324,27 +320,18 @@ static void launch_apply(const void* x, void* y, const float* scale, const float
                          int /*ppb*/, bool silu, long long xs, long long ys, cudaStream_t s, float in_scale = 1.f) {
   const size_t sm = 2 * C * sizeof(float);
   // This kernel is not purely HBM bound: same-box A/B of the C2 step 44.3 ms (polynomial exp) vs 43.4 ms (ex2 + rcp).
-  // HDRVAE_SILU_MUFU: 0 polynomial exp on the FMA pipe, 1 ex2 + rcp on the special-function unit, 2 (default for 16-bit
-  // outputs) ex2 + Newton reciprocal.  fp32 / hi|lo|hi outputs (high-precision mode) always take ex2 + rcp.
-  static int mufu = -1;
-  if (mufu < 0) { const char* e = getenv("HDRVAE_SILU_MUFU"); mufu = e ? atoi(e) : 2; }
-  const int how = sizeof(TOut) == 2 && !std::is_same<TOut, HalfSplit3>::value ? mufu : 1;
-  static int occ[4] = {0, 0, 0, 0};
+  // 16-bit outputs take ex2 + Newton reciprocal (silu_nr2); fp32 / hi|lo|hi outputs (high-precision mode) ex2 + rcp.
+  constexpr bool kNewton = sizeof(TOut) == 2 && !std::is_same<TOut, HalfSplit3>::value;
+  static int occ[2] = {0, 0};
   int chunks = 1, ppb = HW;
   const TIn* xi = reinterpret_cast<const TIn*>(x);
   TOut* yo = reinterpret_cast<TOut*>(y);
-  if (silu && how == 2) {
-    apply_chunking(gn_apply_kernel<TIn, TOut, true, 2>, &occ[0], sm, B, HW, C, &chunks, &ppb);
-    gn_apply_kernel<TIn, TOut, true, 2><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
-  } else if (silu && how == 1) {
-    apply_chunking(gn_apply_kernel<TIn, TOut, true, 1>, &occ[1], sm, B, HW, C, &chunks, &ppb);
-    gn_apply_kernel<TIn, TOut, true, 1><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
-  } else if (silu) {
-    apply_chunking(gn_apply_kernel<TIn, TOut, true, 0>, &occ[2], sm, B, HW, C, &chunks, &ppb);
-    gn_apply_kernel<TIn, TOut, true, 0><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
+  if (silu) {
+    apply_chunking(gn_apply_kernel<TIn, TOut, true, kNewton>, &occ[0], sm, B, HW, C, &chunks, &ppb);
+    gn_apply_kernel<TIn, TOut, true, kNewton><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
   } else {
-    apply_chunking(gn_apply_kernel<TIn, TOut, false, 0>, &occ[3], sm, B, HW, C, &chunks, &ppb);
-    gn_apply_kernel<TIn, TOut, false, 0><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
+    apply_chunking(gn_apply_kernel<TIn, TOut, false, false>, &occ[1], sm, B, HW, C, &chunks, &ppb);
+    gn_apply_kernel<TIn, TOut, false, false><<<dim3(chunks, B), kGnThreads, sm, s>>>(xi, yo, scale, shift, HW, C, ppb, xs, ys, in_scale);
   }
 }
 

@@ -375,28 +375,6 @@ int launch_softmax_rows(const float* s, void* p, int p_dtype, float* inv_sum, in
   return 0;
 }
 
-// ------------------------------------------------------------------ soft-max passes: fold the per-tile row partials
-// mode 1: out[row] = -max over the parts (the bias of pass 2); mode 2: out[row] = 1 / sum over the parts
-__global__ void attn_row_parts_kernel(const float* __restrict__ part, int rows, int parts, int mode, float* __restrict__ out) {
-  const int row = blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5);
-  if (row >= rows) return;
-  const int lane = threadIdx.x & 31;
-  const float* p = part + (long long)row * parts;
-  float a = mode == 1 ? -INFINITY : 0.f;
-  for (int i = lane; i < parts; i += 32) a = mode == 1 ? fmaxf(a, p[i]) : a + p[i];
-  for (int o = 16; o; o >>= 1) {
-    const float b = __shfl_xor_sync(0xffffffffu, a, o);
-    a = mode == 1 ? fmaxf(a, b) : a + b;
-  }
-  if (lane == 0) out[row] = mode == 1 ? -a : 1.f / a;
-}
-int launch_attn_row_parts(const float* part, int rows, int parts, int mode, float* out, cudaStream_t st) {
-  attn_row_parts_kernel<<<ceil_div(rows, 8), 256, 0, st>>>(part, rows, parts, mode, out);
-  HDRVAE_LAUNCHED();
-  HDRVAE_CUDA_OK(cudaGetLastError());
-  return 0;
-}
-
 // ------------------------------------------------------------------ split-K reduction of the PV GEMM
 // out[r][c] = inv_sum[r] * sum_s part[s][r][c]  (fp32 partials -> 16-bit attention output), fixed summation order
 __global__ void attn_reduce_splits_kernel(const float* __restrict__ part, const float* __restrict__ inv_sum,
