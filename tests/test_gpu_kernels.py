@@ -180,14 +180,21 @@ def test_groupnorm_is_run_to_run_deterministic(engine):
     assert torch.equal(a, b)
 
 
+@pytest.mark.parametrize("impl", ["tcgen05", "direct"])
 @pytest.mark.parametrize("dt", [torch.float16, torch.bfloat16])
 @pytest.mark.parametrize("B,T", [(1, 64), (2, 256), (1, 24), (1, 1000), (1, 4096)])
-def test_attention(engine, B, T, dt):
+def test_attention(engine, B, T, dt, impl):
+    """The fused kernel (tensor-core build) and the GEMM-level form (CUDA-core validation build)."""
+    from vae_decode_hdr_b200 import _native as N
     g = torch.Generator().manual_seed(T)
     q = torch.randn(B, T, 512, generator=g).to(dt).to(DEV)
     k = torch.randn(B, T, 512, generator=g).to(dt).to(DEV)
     v = torch.randn(B, T, 512, generator=g).to(dt).to(DEV)
-    o = engine.attention(q, k, v).float()
+    engine.set_conv_impl(N.CONV_DIRECT if impl == "direct" else N.CONV_TCGEN05)
+    try:
+        o = engine.attention(q, k, v).float()
+    finally:
+        engine.set_conv_impl(N.CONV_TCGEN05)
     p = torch.softmax(q.float() @ k.float().transpose(1, 2) / math.sqrt(512.0), dim=-1)
     ref = p @ v.float()
     # exp(s - max) is rounded to the operand type before PV, the output once more: ~half an ulp each

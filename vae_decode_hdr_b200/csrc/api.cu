@@ -276,64 +276,68 @@ static int run_gemm(hdrvae_ctx* ctx, int ab_dtype, const void* A, long long lda,
   return launch_gemm_tc(p, ctx->num_sms, s);
 }
 
+// The fused attention kernel runs with the tensor-core convs; the CUDA-core validation build takes the GEMM-level form
+// (fp32 S, row soft-max kernel, P through HBM, PV GEMM) that the fused kernel replaced.
+static bool attention_fused_enabled(hdrvae_ctx* ctx) { return ctx->conv_impl == HDRVAE_CONV_TCGEN05; }
+static int attention_cta_group(hdrvae_ctx* ctx) { return ctx->cta_group == 1 ? 1 : 2; }
+
 // ---- workspace plan -----------------------------------------------------------------------------
 struct Plan {
   int B, h, w, T, Tp, s_rows, gn_chunks;
-  size_t off_lat, off_x, off_h, off_t, off_x16, off_x16b, off_gn, off_qk, off_vt, off_o, off_f32, off_s, off_p, off_inv, off_part, off_kpart, kpart_bytes, off_epi, off_lat_in, off_img, total;
+  size_t off_lat, off_x, off_h, off_t, off_x16, off_x16b, off_gn, off_qk, off_vt, off_o, off_f32, off_s, off_p, off_inv, off_epi, off_lat_in, off_img, total;
 };
 static constexpr long long kScoreBudgetElems = 1024ll << 20;  // fp32 score chunk <= 4 GiB (K and V^T are re-read once per chunk)
-static constexpr int kSplitRowsBudget = 65536;                // rows x splits of fp32 PV partials (128 MiB)
 
-// Rows of one score / probability chunk of the GEMM-level attention (n_q query rows against Tp keys), and the GroupNorm
-// partial chunks per image that the decoder's convs can write for an h x w latent (convs == false: no convs).
-static void chunk_sizes(int n_q, int Tp, int h, int w, bool convs, int* s_rows, int* gn_chunks) {
+// Rows of one score / probability chunk of the GEMM-level attention (n_q query rows against Tp keys).
+static int score_chunk_rows(int n_q, int Tp) {
   long long rows = kScoreBudgetElems / Tp;
   rows = rows / 128 * 128;
   if (rows < 128) rows = 128;
   const long long q128 = (n_q + 127) / 128 * 128;
-  if (rows > q128) rows = q128;
-  *s_rows = (int)rows;
-  *gn_chunks = 1184;
-  if (convs)
-    for (int l = 1; l <= 8; l *= 2) *gn_chunks = std::max(*gn_chunks, 4 * tiles_for(l * h, l * w));
+  return (int)std::min(rows, q128);
 }
 
-// c_lat: channels of the caller's latent (sizes the graph-input copy)
-static Plan make_plan(int B, int h, int w, bool attn_only = false, bool high = false, bool attn_scratch = true, int c_lat = 16) {
+// GroupNorm partial chunks per image that the decoder's convs can write for an h x w latent.
+static int gn_chunk_capacity(int h, int w) {
+  int chunks = 1184;
+  for (int l = 1; l <= 8; l *= 2) chunks = std::max(chunks, 4 * tiles_for(l * h, l * w));
+  return chunks;
+}
+
+// Workspace of a decode of B latents of h x w on this context.
+static Plan decode_plan(hdrvae_ctx* ctx, int B, int h, int w) {
   Plan pl;
+  const bool high = ctx->high;
   const size_t km = high ? 3 : 1;                              // hi|lo|hi operands are 3x as wide
   pl.B = B; pl.h = h; pl.w = w;
   pl.T = h * w;
   pl.Tp = (pl.T + 63) / 64 * 64;
-  chunk_sizes(pl.T, pl.Tp, h, w, !attn_only, &pl.s_rows, &pl.gn_chunks);
+  pl.s_rows = score_chunk_rows(pl.T, pl.Tp);
+  pl.gn_chunks = gn_chunk_capacity(h, w);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes, 1024); return o; };
-  const size_t widest = attn_only ? 0 : (size_t)B * pl.T * 64 * 256;   // elements of [B, 8h, 8w, 256]
-  pl.off_lat = take(attn_only ? 0 : (size_t)B * pl.T * 64 * 2 * km);
+  const size_t widest = (size_t)B * pl.T * 64 * 256;   // elements of [B, 8h, 8w, 256]
+  pl.off_lat = take((size_t)B * pl.T * 64 * 2 * km);
   pl.off_x = take(widest * 4);       // residual stream, fp32
   pl.off_h = take(widest * 4);       // conv1 / shortcut / upsample outputs, fp32
   pl.off_t = take(widest * 2 * km);  // GroupNorm outputs: 16-bit tensor-core operands
   pl.off_x16 = take(widest / 2 * km);  // scaled 16-bit copy of x feeding an upsample conv (<= [B,4h,4w,256] elements)
   pl.off_x16b = take(widest * 2 * km); // scaled 16-bit copy of an upsample output feeding a nin_shortcut (<= [B,8h,8w,256])
-  pl.off_gn = take(attn_only ? 0 : gn_scratch_bytes(B, 512, pl.gn_chunks));
+  pl.off_gn = take(gn_scratch_bytes(B, 512, pl.gn_chunks));
   pl.off_qk = take((size_t)B * pl.Tp * 1024 * 2 * km);
   pl.off_vt = take((size_t)B * 512 * pl.Tp * 2 * km);
   pl.off_o = take((size_t)B * pl.T * 512 * 2 * km);
   pl.off_f32 = take(high ? (size_t)pl.Tp * 1536 * 4 + (size_t)B * 64 * pl.T * 4 : 0);   // high: fp32 q|k, v^T / o of one image; fp32 NHWC latent
-  // score / probability chunks, row sums and split-K partials exist only for the GEMM-level attention (validation
-  // build, high precision): the fused kernel keeps S and P on the SM (up to 6.1 GiB less at 4096^2)
-  pl.off_s = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 4 : 0);
-  pl.off_p = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 2 * km : 0);
-  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 : 0);          // 1 / row sum
-  pl.off_part = take(attn_scratch ? (size_t)kSplitRowsBudget * 512 * 4 : 0);   // split-K partials of the PV GEMM
-  // key splits of the fused kernel (fp32 O partials + (m, l) per row and split): the decoder lends its idle fp32 buffer
-  // (off_h: nothing of a ResnetBlock is live across mid.attn_1); the stand-alone attention entry has no such buffer
-  const size_t ksp = (size_t)attention_key_splits(pl.T);
-  pl.kpart_bytes = attn_only && ksp > 1 ? (size_t)B * pl.T * (512 + 2) * 4 * ksp : 0;
-  pl.off_kpart = take(pl.kpart_bytes);
-  pl.off_epi = take(attn_only ? 0 : epilogue_scratch_bytes(B, 8 * h, 8 * w));
-  pl.off_lat_in = take(attn_only ? 0 : (size_t)B * c_lat * pl.T * 4);       // graph input: fp32 latent copy
-  pl.off_img = take(attn_only ? 0 : (size_t)B * 64 * pl.T * 3 * 4);        // graph output: fp32 BHWC image
+  // score / probability chunks and row sums exist only for the GEMM-level attention (validation build, high precision):
+  // the fused kernel keeps S and P on the SM (up to 6.1 GiB less at 4096^2).  Its key-split partials borrow off_h
+  // (attend_dense).
+  const bool gemm_attention = high || !attention_fused_enabled(ctx);
+  pl.off_s = take(gemm_attention ? (size_t)pl.s_rows * pl.Tp * 4 : 0);
+  pl.off_p = take(gemm_attention ? (size_t)pl.s_rows * pl.Tp * 2 * km : 0);
+  pl.off_inv = take(gemm_attention ? (size_t)pl.s_rows * 4 : 0);          // 1 / row sum
+  pl.off_epi = take(epilogue_scratch_bytes(B, 8 * h, 8 * w));
+  pl.off_lat_in = take((size_t)B * ctx->c_lat * pl.T * 4);       // graph input: fp32 latent copy
+  pl.off_img = take((size_t)B * 64 * pl.T * 3 * 4);        // graph output: fp32 BHWC image
   pl.total = off;
   return pl;
 }
@@ -378,68 +382,46 @@ static bool gn_is_fused(hdrvae_ctx* ctx, const PackedConv& pc, const ConvIO& io,
          io.stats != nullptr && conv_takes_slab(pc, io, H, W, ctx->conv_impl);
 }
 
-// The fused attention kernel runs with the tensor-core convs; the CUDA-core validation build takes the GEMM-level form
-// (fp32 S, row soft-max kernel, P through HBM, split-K PV + reduce) that the fused kernel replaced.
-static bool attention_fused_enabled(hdrvae_ctx* ctx) { return ctx->conv_impl == HDRVAE_CONV_TCGEN05; }
-static int attention_cta_group(hdrvae_ctx* ctx) { return ctx->cta_group == 1 ? 1 : 2; }
+// One chunk of the GEMM-level attention's scratch: `rows` query rows against Tp keys, fp32 scores S [rows][Tp], probabilities
+// P [rows][km Tp] (km = 3 for the [hi|lo|hi] operand of the high-precision mode) and 1 / row sum [rows].
+struct AttnChunk { float* S; void* P; float* inv; int rows; };
+static AttnChunk plan_chunk(const Plan& pl, uint8_t* ws) {
+  return {reinterpret_cast<float*>(ws + pl.off_s), ws + pl.off_p, reinterpret_cast<float*>(ws + pl.off_inv), pl.s_rows};
+}
 
-// Attention of n_q query rows (q: 16-bit, row stride 1024) against T keys (k: row stride 1024, rows >= T zero up to
-// Tp) and v^T [512][Tp]; o: 16-bit [n_q][512].  Scratch (S, P, 1/sum, split-K partials) comes from the plan.
-static int attention_rows(hdrvae_ctx* ctx, uint8_t* ws, size_t off_s, size_t off_p, size_t off_inv, size_t off_part,
-                          void* ksplit_scratch, size_t ksplit_bytes, int s_rows, const uint16_t* q, int n_q, const uint16_t* k, const uint16_t* v, int T, int Tp,
-                          uint16_t* o, float qk_alpha, cudaStream_t s) {
-  const int impl = ctx->conv_impl, dt = ctx->op_dtype;
-  if (attention_fused_enabled(ctx)) {
-    // ONE launch: flash-style kernel, scores and probabilities never leave the SM (attention.cu)
-    // key-split scratch: [splits][n_q][512] fp32 partials, then [splits][n_q][2] (m, l)
-    const int ksp = attention_key_splits(T);
-    const size_t need = (size_t)ksp * n_q * (512 + 2) * 4;
-    float* part = (ksp > 1 && ksplit_scratch != nullptr && ksplit_bytes >= need) ? reinterpret_cast<float*>(ksplit_scratch) : nullptr;
-    HDRVAE_REQUIRE(ksp == 1 || part != nullptr, "attention: key-split scratch too small (%zu < %zu bytes)", ksplit_bytes, need);
-    return launch_attention_fused(q, 1024, 0, n_q, k, 1024, 0, Tp, v, Tp, 0, T, o, (long long)n_q * 512, 1, dt, qk_alpha,
-                                  attention_cta_group(ctx), ctx->num_sms, part, part ? part + (size_t)ksp * n_q * 512 : nullptr,
-                                  (long long)ksp * n_q, s);
-  }
-  float* S = reinterpret_cast<float*>(ws + off_s);
-  uint16_t* P = reinterpret_cast<uint16_t*>(ws + off_p);
-  float* inv = reinterpret_cast<float*>(ws + off_inv);
-  for (int r0 = 0; r0 < n_q; r0 += s_rows) {
-    const int rows = std::min(s_rows, n_q - r0);
-    // S = alpha q k^T, fp32 (the decoder folds 1/sqrt(d) into the q weights: alpha = 1); padded key
-    // columns give 0 and are masked by the softmax
-    HDRVAE_TRY(run_gemm(ctx, dt, q + (size_t)r0 * 1024, 1024, rows, 512, k, 1024, Tp, Tp, S, Tp, DT_F32, nullptr, false,
-                        qk_alpha, nullptr, impl, s));
-    // P = exp(S - rowmax) (16-bit), inv = 1 / rowsum; O = inv * (P V)
-    HDRVAE_TRY(launch_softmax_rows(S, P, dt, inv, rows, T, Tp, Tp, Tp, s));
-    // A row chunk gives only rows/128 x 2 tiles: when that cannot fill the GPU the K (key) dimension is split
-    // across `splits` images of one GEMM (fp32 partials) and reduced afterwards.
-    const int tiles = ((rows + 127) / 128) * 2;
-    int splits = 1;
-    while (tiles * splits < ctx->num_sms && splits < 32 && (Tp / (splits * 2)) % 128 == 0 &&
-           (long long)rows * splits * 2 <= kSplitRowsBudget)
-      splits *= 2;
-    uint16_t* o_rows = o + (size_t)r0 * 512;
-    if (splits == 1) {
-      HDRVAE_TRY(run_gemm(ctx, dt, P, Tp, rows, Tp, v, Tp, 512, 512, o_rows, 512, dt, nullptr, false, 1.0f, inv, impl, s));
-    } else {
-      float* part = reinterpret_cast<float*>(ws + off_part);
-      const int ks = Tp / splits;
-      GemmParams p;
-      memset(&p, 0, sizeof p);
-      p.a = P; p.ab_dtype = dt;
-      p.a_px_stride = Tp; p.a_row_stride = (long long)rows * Tp; p.a_img_stride = ks;   // image s = K range s
-      p.n_img = splits; p.H = 1; p.W = rows;
-      p.k_per_tap = ks; p.ntaps = 1;
-      p.b = v; p.b_row_stride = Tp; p.b_rows = 512; p.n_cols = 512; p.b_img_k_stride = ks;
-      p.out = part; p.out_dtype = DT_F32;
-      p.out_px_stride = 512; p.out_row_stride = 0; p.out_img_stride = (long long)rows * 512;
-      p.sy = p.sx = 1; p.alpha = 1.0f;
-      p.tw_log2 = 7; p.TW = 128; p.TH = 1; p.tiles_x = (rows + 127) / 128; p.tiles_y = 1;
-      p.cta_group = ctx->cta_group;
-      if (impl == HDRVAE_CONV_DIRECT) HDRVAE_TRY(launch_gemm_direct(p, s));
-      else HDRVAE_TRY(launch_gemm_tc(p, ctx->num_sms, s));
-      HDRVAE_TRY(launch_attn_reduce_splits(part, inv, o_rows, dt, rows, 512, splits, s));
-    }
+// The fused kernel (attention.cu: ONE launch, scores and probabilities never leave the SM) over n_img images: q and k
+// 16-bit with row stride 1024 in a [n_img][Tp][1024] buffer (key rows >= T zero up to Tp), v^T [n_img][512][Tp], n_q query
+// rows per image, o 16-bit [n_img][n_q][512].  ksplit: memory for the key-split partials ([splits][n_img n_q][512] fp32,
+// then [splits][n_img n_q][2] (m, l)), needed only when T takes more than one split.
+static int attention_fused(hdrvae_ctx* ctx, const uint16_t* q, const uint16_t* k, const uint16_t* vt, int n_img, int n_q,
+                           int T, int Tp, void* o, float alpha, void* ksplit, size_t ksplit_bytes, cudaStream_t s) {
+  const int ksp = attention_key_splits(T);
+  const size_t rows = (size_t)n_img * n_q, need = (size_t)ksp * rows * (512 + 2) * 4;
+  HDRVAE_REQUIRE(ksp == 1 || (ksplit != nullptr && ksplit_bytes >= need), "attention: key-split scratch too small (%zu < %zu bytes)",
+                 ksplit_bytes, need);
+  float* part = ksp > 1 ? reinterpret_cast<float*>(ksplit) : nullptr;
+  return launch_attention_fused(q, 1024, (long long)Tp * 1024, n_q, k, 1024, (long long)Tp * 1024, Tp, vt, Tp, (long long)512 * Tp,
+                                T, o, (long long)n_q * 512, n_img, ctx->op_dtype, alpha, attention_cta_group(ctx), ctx->num_sms,
+                                part, part ? part + (size_t)ksp * rows * 512 : nullptr, (long long)ksp * rows, s);
+}
+
+// GEMM-level attention of n_q query rows (q, row stride ldq) against T keys (k, row stride ldk, rows >= T zero up to Tp) and
+// v^T [512][ldv], in chunks of c.rows query rows: S = alpha q k^T in fp32 (the padded key columns give 0 and are masked by
+// the soft-max), P = exp(S - rowmax) and inv = 1 / rowsum (launch_softmax_rows), o = inv * (P V) (o_dtype, row stride ldo).
+// p_dtype is P's type: the 16-bit operand type, or DT_F16X3 for the high-precision mode, whose fp16 hi|lo operands q, k, v^T
+// and P are three times as wide.
+static int attention_gemm(hdrvae_ctx* ctx, const uint16_t* q, long long ldq, const uint16_t* k, long long ldk, const uint16_t* vt,
+                          long long ldv, int n_q, int T, int Tp, int p_dtype, void* o, int o_dtype, long long ldo, float alpha,
+                          const AttnChunk& c, cudaStream_t s) {
+  const int km = p_dtype == DT_F16X3 ? 3 : 1, ab = p_dtype == DT_F16X3 ? DT_F16 : p_dtype, impl = ctx->conv_impl;
+  for (int r0 = 0; r0 < n_q; r0 += c.rows) {
+    const int rows = std::min(c.rows, n_q - r0);
+    HDRVAE_TRY(run_gemm(ctx, ab, q + (size_t)r0 * ldq, ldq, rows, 512 * km, k, ldk, Tp, Tp, c.S, Tp, DT_F32, nullptr, false,
+                        alpha, nullptr, impl, s));
+    HDRVAE_TRY(launch_softmax_rows(c.S, c.P, p_dtype, c.inv, rows, T, Tp, Tp, (long long)km * Tp, s));
+    HDRVAE_TRY(run_gemm(ctx, ab, c.P, (long long)km * Tp, rows, km * Tp, vt, ldv, 512, 512,
+                        reinterpret_cast<uint8_t*>(o) + (size_t)r0 * ldo * dt_bytes(o_dtype), ldo, o_dtype, nullptr, false, 1.0f,
+                        c.inv, impl, s));
   }
   return 0;
 }
@@ -462,16 +444,14 @@ static int run_phase_a(hdrvae_ctx* ctx, const void* feat, int B, int H, int W, i
 
 // "precision high" attention of ONE image: every GEMM on K-concatenated fp16 hi / lo operands (activations [hi|lo|hi],
 // weight-like operands [hi|hi|lo]), fp32 scores and outputs.  t3: GroupNorm output [T][1536]; o3: [T][1536] operand of
-// proj_out.  GEMM-level form (the fused kernel keeps a 16-bit Q tile resident and has no room for a second copy).
+// proj_out.  The projections run in fp32 and are split into the operands of the GEMM-level form (the fused kernel keeps a
+// 16-bit Q tile resident and has no room for a second copy), whose fp32 output is split once more for proj_out.
 static int run_attention_high(hdrvae_ctx* ctx, const Plan& pl, uint8_t* ws, const uint16_t* t3, uint16_t* o3, cudaStream_t s) {
   const int impl = ctx->conv_impl, T = pl.T, Tp = pl.Tp;
   float* f32 = reinterpret_cast<float*>(ws + pl.off_f32);                 // [Tp][1024] q|k, then [512][Tp] v^T, then [T][512] o
   uint16_t* q3 = reinterpret_cast<uint16_t*>(ws + pl.off_qk);            // [Tp][1536] hi|lo|hi
   uint16_t* k3 = q3 + (size_t)Tp * 1536;                                 // [Tp][1536] hi|hi|lo
   uint16_t* vt3 = reinterpret_cast<uint16_t*>(ws + pl.off_vt);           // [512][3 Tp] hi|hi|lo along the keys
-  float* S = reinterpret_cast<float*>(ws + pl.off_s);
-  uint16_t* P3 = reinterpret_cast<uint16_t*>(ws + pl.off_p);             // [rows][3 Tp] hi|lo|hi
-  float* inv = reinterpret_cast<float*>(ws + pl.off_inv);
   if (Tp != T) HDRVAE_CUDA_OK(cudaMemsetAsync(f32, 0, (size_t)Tp * 1024 * 4, s));
   HDRVAE_TRY(run_gemm(ctx, DT_F16, t3, 1536, T, 1536, ctx->qk.w[0], 1536, 1024, 1024, f32, 1024, DT_F32, ctx->qk.bias, false, 1.0f,
                       nullptr, impl, s));
@@ -482,40 +462,25 @@ static int run_attention_high(hdrvae_ctx* ctx, const Plan& pl, uint8_t* ws, cons
                       nullptr, impl, s));
   HDRVAE_TRY(launch_split3(f32, Tp, vt3, 3ll * Tp, 512, Tp, 1.f, 1, s));
   float* of = f32;                                                       // [T][512], v^T fp32 is dead after the split
-  for (int r0 = 0; r0 < T; r0 += pl.s_rows) {
-    const int rows = std::min(pl.s_rows, T - r0);
-    HDRVAE_TRY(run_gemm(ctx, DT_F16, q3 + (size_t)r0 * 1536, 1536, rows, 1536, k3, 1536, Tp, Tp, S, Tp, DT_F32, nullptr, false, 1.0f,
-                        nullptr, impl, s));
-    HDRVAE_TRY(launch_softmax_rows(S, P3, DT_F16X3, inv, rows, T, Tp, Tp, 3ll * Tp, s));
-    HDRVAE_TRY(run_gemm(ctx, DT_F16, P3, 3ll * Tp, rows, 3 * Tp, vt3, 3ll * Tp, 512, 512, of + (size_t)r0 * 512, 512, DT_F32, nullptr,
-                        false, 1.0f, inv, impl, s));
-  }
+  HDRVAE_TRY(attention_gemm(ctx, q3, 1536, k3, 1536, vt3, 3ll * Tp, T, T, Tp, DT_F16X3, of, DT_F32, 512, 1.0f, plan_chunk(pl, ws), s));
   return launch_split3(of, 512, o3, 1536, T, 512, 1.f, 0, s);
 }
 
-// ksplit_scratch: idle memory for the fused kernel's key-split partials ([splits][B*T][512] fp32 + [splits][B*T][2])
-static int run_attention_core(hdrvae_ctx* ctx, const Plan& pl, uint8_t* ws, const void* qk /*[B][Tp][1024]*/,
-                              const void* vt /*[B][512][Tp]*/, void* o /*[B][T][512]*/, float qk_alpha,
-                              void* ksplit_scratch, size_t ksplit_bytes, cudaStream_t s) {
+// Attention core of B images: q|k [B][Tp][1024], v^T [B][512][Tp] -> o 16-bit [B][T][512].  The fused kernel takes all
+// images in one launch (ksplit: idle memory for its key-split partials); the validation build runs the GEMM-level form one
+// image at a time in the scratch chunk c.
+static int run_attention_core(hdrvae_ctx* ctx, int B, int T, int Tp, const void* qk, const void* vt, void* o, float qk_alpha,
+                              void* ksplit, size_t ksplit_bytes, const AttnChunk& c, cudaStream_t s) {
+  const uint16_t* q = reinterpret_cast<const uint16_t*>(qk);
+  const uint16_t* v = reinterpret_cast<const uint16_t*>(vt);
   if (attention_fused_enabled(ctx)) {
-    // all images in one launch
-    ProfScope prof("attention fused kernel", 4.0 * pl.B * (double)pl.T * pl.T * 512, 0.0, s);
-    const uint16_t* q = reinterpret_cast<const uint16_t*>(qk);
-    const int ksp = attention_key_splits(pl.T);
-    const size_t rows = (size_t)pl.B * pl.T, need = (size_t)ksp * rows * (512 + 2) * 4;
-    HDRVAE_REQUIRE(ksp == 1 || (ksplit_scratch != nullptr && ksplit_bytes >= need),
-                   "attention: key-split scratch too small (%zu < %zu bytes)", ksplit_bytes, need);
-    float* part = ksp > 1 ? reinterpret_cast<float*>(ksplit_scratch) : nullptr;
-    return launch_attention_fused(q, 1024, (long long)pl.Tp * 1024, pl.T, q + 512, 1024, (long long)pl.Tp * 1024, pl.Tp, vt, pl.Tp,
-                                  (long long)512 * pl.Tp, pl.T, o, (long long)pl.T * 512, pl.B, ctx->op_dtype, qk_alpha,
-                                  attention_cta_group(ctx), ctx->num_sms, part, part ? part + (size_t)ksp * rows * 512 : nullptr,
-                                  (long long)ksp * rows, s);
+    ProfScope prof("attention fused kernel", 4.0 * B * (double)T * T * 512, 0.0, s);
+    return attention_fused(ctx, q, q + 512, v, B, T, T, Tp, o, qk_alpha, ksplit, ksplit_bytes, s);
   }
-  for (int b = 0; b < pl.B; ++b) {
-    const uint16_t* q = reinterpret_cast<const uint16_t*>(qk) + (size_t)b * pl.Tp * 1024;
-    HDRVAE_TRY(attention_rows(ctx, ws, pl.off_s, pl.off_p, pl.off_inv, pl.off_part, nullptr, 0, pl.s_rows, q, pl.T, q + 512,
-                              reinterpret_cast<const uint16_t*>(vt) + (size_t)b * 512 * pl.Tp, pl.T, pl.Tp,
-                              reinterpret_cast<uint16_t*>(o) + (size_t)b * pl.T * 512, qk_alpha, s));
+  for (int b = 0; b < B; ++b) {
+    const uint16_t* qb = q + (size_t)b * Tp * 1024;
+    HDRVAE_TRY(attention_gemm(ctx, qb, 1024, qb + 512, 1024, v + (size_t)b * 512 * Tp, Tp, T, T, Tp, ctx->op_dtype,
+                              reinterpret_cast<uint16_t*>(o) + (size_t)b * T * 512, ctx->op_dtype, 512, qk_alpha, c, s));
   }
   return 0;
 }
@@ -534,17 +499,16 @@ static int check_ws(const Plan& pl, void* ws, size_t bytes) {
 // lives in a slab with one halo row above and below; conv outputs get their halo rows from the neighbours
 // (HALO exchange), GroupNorm sums are all-reduced, attention K/V are all-gathered.  See include/hdrvae.h.
 struct RowsPlan {
-  int h, w, hl, world, T, Tl, Tp, s_rows, gn_chunks;
-  size_t off_lat, off_x, off_h, off_t, off_xa, off_xb, off_gn, off_qk, off_v, off_vt, off_o, off_s, off_p, off_inv,
-      off_part, off_epi, off_mail, total;
+  int h, w, hl, world, T, Tl, Tp, gn_chunks;
+  size_t off_lat, off_x, off_h, off_t, off_xa, off_xb, off_gn, off_qk, off_v, off_vt, off_o, off_epi, off_mail, total;
 };
 
-static RowsPlan make_rows_plan(int h, int w, int world, bool attn_scratch = true) {
+static RowsPlan make_rows_plan(int h, int w, int world) {
   RowsPlan pl;
   pl.h = h; pl.w = w; pl.world = world; pl.hl = h / world;
   pl.T = h * w; pl.Tl = pl.hl * w;
   pl.Tp = (pl.T + 63) / 64 * 64;
-  chunk_sizes(pl.Tl, pl.Tp, pl.hl, w, true, &pl.s_rows, &pl.gn_chunks);
+  pl.gn_chunks = gn_chunk_capacity(pl.hl, w);
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += align_up(bytes, 1024); return o; };
   const size_t widest = (size_t)(8 * pl.hl + 2) * 8 * w * 256;           // slab elements incl. halo rows
@@ -561,10 +525,6 @@ static RowsPlan make_rows_plan(int h, int w, int world, bool attn_scratch = true
   pl.off_v = take((size_t)pl.Tp * 512 * 2);            // gathered v [T][512]
   pl.off_vt = take((size_t)512 * pl.Tp * 2);
   pl.off_o = take((size_t)pl.Tl * 512 * 2);
-  pl.off_s = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 4 : 0);      // GEMM-level attention only (see make_plan)
-  pl.off_p = take(attn_scratch ? (size_t)pl.s_rows * pl.Tp * 2 : 0);
-  pl.off_inv = take(attn_scratch ? (size_t)pl.s_rows * 4 : 0);
-  pl.off_part = take(attn_scratch ? (size_t)kSplitRowsBudget * 512 * 4 : 0);
   pl.off_epi = take(epilogue_scratch_bytes(1, 8 * pl.hl, 8 * w));
   pl.off_mail = take(sizeof(RowsMailbox));              // flags / tables of the device-driven exchanges (rows_p2p.cu)
   pl.total = off;
@@ -871,7 +831,7 @@ static int attend_dense(Decoder& d, const Plan& pl, uint8_t* ws, const void** o_
   }
   ProfScope prof("attention core (QK^T, softmax, PV)", 4.0 * B * (double)pl.T * pl.T * 512, 10.0 * B * (double)pl.T * pl.Tp, s);
   // key-split partials borrow the block-internal fp32 buffer: nothing of a ResnetBlock is live across mid.attn_1
-  return run_attention_core(ctx, pl, ws, qk, vt, o, 1.0f, d.hbuf, (size_t)B * pl.T * 64 * 256 * 4, s);
+  return run_attention_core(ctx, B, pl.T, pl.Tp, qk, vt, o, 1.0f, d.hbuf, (size_t)B * pl.T * 64 * 256 * 4, plan_chunk(pl, ws), s);
 }
 
 static int run_decoder(hdrvae_ctx* ctx, const float* latent, const Plan& pl, uint8_t* ws, void** features,
@@ -939,8 +899,7 @@ static void attend_rows(Decoder& d, int W, const void** o_out) {
   rows_exchange(st, ex);
   step(d, [=](cudaStream_t s) {
     HDRVAE_TRY(launch_transpose_pad(vb, vt, pl.T, 512, pl.Tp, s));
-    return attention_rows(ctx, ws, pl.off_s, pl.off_p, pl.off_inv, pl.off_part, hscr, hscr_bytes, pl.s_rows,
-                          qk + (size_t)rank * pl.Tl * 1024, pl.Tl, qk + 512, vt, pl.T, pl.Tp, o, 1.0f, s);
+    return attention_fused(ctx, qk + (size_t)rank * pl.Tl * 1024, qk + 512, vt, 1, pl.Tl, pl.T, pl.Tp, o, 1.0f, hscr, hscr_bytes, s);
   });
 }
 
@@ -1215,7 +1174,7 @@ int hdrvae_load_weights(hdrvae_ctx* ctx, const hdrvae_weight_desc* descs, int n,
 int hdrvae_workspace_bytes(hdrvae_ctx* ctx, int B, int h, int w, size_t* bytes) {
   HDRVAE_REQUIRE(ctx != nullptr && bytes != nullptr, "hdrvae_workspace_bytes: null argument");
   HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_workspace_bytes: empty latent batch [%d,%d,%d,%d]", B, ctx->c_lat, h, w);
-  *bytes = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat).total;
+  *bytes = decode_plan(ctx, B, h, w).total;
   return 0;
 }
 
@@ -1272,7 +1231,7 @@ int hdrvae_decode_begin(hdrvae_ctx* ctx, const float* latent, int B, int h, int 
   HDRVAE_REQUIRE(ctx != nullptr && latent != nullptr, "hdrvae_decode: null argument");
   HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode: empty latent batch [%d,%d,%d,%d]", B, ctx->c_lat, h, w);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
+  const Plan pl = decode_plan(ctx, B, h, w);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
@@ -1299,7 +1258,7 @@ int hdrvae_decode_finish(hdrvae_ctx* ctx, int B, int h, int w, int mode, float e
   HDRVAE_REQUIRE(ctx != nullptr && out_bhwc != nullptr, "hdrvae_decode: null argument");
   HDRVAE_REQUIRE(mode >= 0 && mode <= 3, "hdrvae_decode: bad mode %d", mode);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
+  const Plan pl = decode_plan(ctx, B, h, w);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
@@ -1343,7 +1302,7 @@ int hdrvae_raw_stats_merge(const void* blocks, int n, void* dst, void* stream) {
 int hdrvae_rows_workspace_bytes(hdrvae_ctx* ctx, int h, int w, int world, size_t* bytes) {
   HDRVAE_REQUIRE(ctx && bytes && h >= 1 && w >= 1 && world >= 1, "hdrvae_rows_workspace_bytes: bad argument");
   HDRVAE_REQUIRE(h % world == 0, "row tiling needs the latent height (%d) to be a multiple of the rank count (%d)", h, world);
-  *bytes = make_rows_plan(h, w, world, !attention_fused_enabled(ctx)).total;
+  *bytes = make_rows_plan(h, w, world).total;
   return 0;
 }
 
@@ -1359,7 +1318,7 @@ int hdrvae_rows_begin(hdrvae_ctx* ctx, const float* latent_full, int h, int w, i
   HDRVAE_REQUIRE(!ctx->high, "row tiling is not available in the high-precision mode");
   hdrvae_rows* st = new hdrvae_rows();
   st->ctx = ctx;
-  st->pl = make_rows_plan(h, w, world, !attention_fused_enabled(ctx));
+  st->pl = make_rows_plan(h, w, world);
   if (ws_bytes < st->pl.total || (reinterpret_cast<uintptr_t>(workspace) & 1023) != 0) {
     set_error("hdrvae_rows_begin: workspace too small or misaligned (%zu < %zu bytes)", ws_bytes, st->pl.total);
     delete st;
@@ -1510,7 +1469,7 @@ int hdrvae_decode_features(hdrvae_ctx* ctx, const float* latent, int B, int h, i
   HDRVAE_REQUIRE(ctx != nullptr && latent != nullptr && features != nullptr, "hdrvae_decode_features: null argument");
   HDRVAE_REQUIRE(B >= 1 && h >= 1 && w >= 1, "hdrvae_decode_features: empty latent batch");
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
-  const Plan pl = make_plan(B, h, w, false, ctx->high, ctx->high || !attention_fused_enabled(ctx), ctx->c_lat);
+  const Plan pl = decode_plan(ctx, B, h, w);
   HDRVAE_TRY(check_ws(pl, workspace, ws_bytes));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   void* feat = nullptr;
@@ -1596,27 +1555,38 @@ int hdrvae_attention(hdrvae_ctx* ctx, const void* q, const void* k, const void* 
   HDRVAE_REQUIRE(dtype == HDRVAE_BF16 || dtype == HDRVAE_F16, "hdrvae_attention: q/k/v must be bf16 or fp16");
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  Plan pl = make_plan(B, 1, T, true, false, !attention_fused_enabled(ctx));
+  // the q|k and v^T operands, then the fused kernel's key-split partials or one GEMM-level scratch chunk
+  const int Tp = (T + 63) / 64 * 64;
+  size_t total = 0;
+  auto take = [&](size_t bytes) { size_t o = total; total += align_up(bytes, 1024); return o; };
+  const size_t off_qk = take((size_t)B * Tp * 1024 * 2), off_vt = take((size_t)B * 512 * Tp * 2);
+  const bool fused = attention_fused_enabled(ctx);
+  const size_t ksp = attention_key_splits(T), ksplit_bytes = fused && ksp > 1 ? (size_t)B * T * (512 + 2) * 4 * ksp : 0;
+  const size_t off_ksplit = take(ksplit_bytes);
+  const int s_rows = score_chunk_rows(T, Tp);
+  const size_t off_s = take(fused ? 0 : (size_t)s_rows * Tp * 4), off_p = take(fused ? 0 : (size_t)s_rows * Tp * 2),
+               off_inv = take(fused ? 0 : (size_t)s_rows * 4);
   uint8_t* ws = nullptr;
-  HDRVAE_CUDA_OK(cudaMalloc((void**)&ws, pl.total));
-  uint16_t* qk = reinterpret_cast<uint16_t*>(ws + pl.off_qk);
-  uint16_t* vt = reinterpret_cast<uint16_t*>(ws + pl.off_vt);
+  HDRVAE_CUDA_OK(cudaMalloc((void**)&ws, total));
+  uint16_t* qk = reinterpret_cast<uint16_t*>(ws + off_qk);
+  uint16_t* vt = reinterpret_cast<uint16_t*>(ws + off_vt);
+  const AttnChunk chunk{reinterpret_cast<float*>(ws + off_s), ws + off_p, reinterpret_cast<float*>(ws + off_inv), s_rows};
   int r = 0;
   const float scale = 1.0f / sqrtf(512.0f);
-  cudaMemsetAsync(qk, 0, (size_t)B * pl.Tp * 1024 * 2, s);
-  cudaMemsetAsync(vt, 0, (size_t)B * 512 * pl.Tp * 2, s);
+  cudaMemsetAsync(qk, 0, (size_t)B * Tp * 1024 * 2, s);
+  cudaMemsetAsync(vt, 0, (size_t)B * 512 * Tp * 2, s);
   const uint16_t* q16 = reinterpret_cast<const uint16_t*>(q);
   const uint16_t* k16 = reinterpret_cast<const uint16_t*>(k);
   const uint16_t* v16 = reinterpret_cast<const uint16_t*>(v);
   for (int b = 0; b < B && r == 0; ++b) {
     // interleave q and k rows into the [Tp][1024] operand, transpose v
-    r = launch_transpose_pad(v16 + (size_t)b * T * 512, vt + (size_t)b * 512 * pl.Tp, T, 512, pl.Tp, s);
-    if (r == 0) HDRVAE_CUDA_OK(cudaMemcpy2DAsync(qk + (size_t)b * pl.Tp * 1024, 2048, q16 + (size_t)b * T * 512, 1024, 1024, T, cudaMemcpyDeviceToDevice, s));
-    if (r == 0) HDRVAE_CUDA_OK(cudaMemcpy2DAsync(qk + (size_t)b * pl.Tp * 1024 + 512, 2048, k16 + (size_t)b * T * 512, 1024, 1024, T, cudaMemcpyDeviceToDevice, s));
+    r = launch_transpose_pad(v16 + (size_t)b * T * 512, vt + (size_t)b * 512 * Tp, T, 512, Tp, s);
+    if (r == 0) HDRVAE_CUDA_OK(cudaMemcpy2DAsync(qk + (size_t)b * Tp * 1024, 2048, q16 + (size_t)b * T * 512, 1024, 1024, T, cudaMemcpyDeviceToDevice, s));
+    if (r == 0) HDRVAE_CUDA_OK(cudaMemcpy2DAsync(qk + (size_t)b * Tp * 1024 + 512, 2048, k16 + (size_t)b * T * 512, 1024, 1024, T, cudaMemcpyDeviceToDevice, s));
   }
   const int saved = ctx->op_dtype;
   ctx->op_dtype = dtype;
-  if (r == 0) r = run_attention_core(ctx, pl, ws, qk, vt, o, scale, ws + pl.off_kpart, pl.kpart_bytes, s);
+  if (r == 0) r = run_attention_core(ctx, B, T, Tp, qk, vt, o, scale, ws + off_ksplit, ksplit_bytes, chunk, s);
   ctx->op_dtype = saved;
   cudaStreamSynchronize(s);
   cudaFree(ws);

@@ -73,7 +73,6 @@ struct GemmParams {
   // B operand (weights / keys), [cols][ktot] K-major, same element type as A
   const void* b;
   long long b_row_stride;
-  long long b_img_k_stride;  // B's K coordinate of image i starts at i * b_img_k_stride (split-K GEMMs), else 0
   int b_rows;       // rows of B that exist in memory (0: same as n_cols); rows beyond are zero-filled by TMA
   int ab_dtype;
   int n_img, H, W;  // source grid of the M dimension

@@ -28,8 +28,6 @@ int launch_latent_rows_to_nhwc(const float* z, void* out, int out_dtype, int C, 
 int launch_softmax_rows(const float* s, void* p, int p_dtype, float* inv_sum, int n_rows, int n_valid, int n_pad,
                         long long s_ld, long long p_ld, cudaStream_t st);
 int launch_transpose_pad(const void* in, void* out, int rows, int cols, int out_ld, cudaStream_t s);
-int launch_attn_reduce_splits(const float* part, const float* inv_sum, void* out, int out_dtype, int rows, int cols,
-                              int splits, cudaStream_t st);
 int launch_pack_half(const float* img, uint16_t* out, int B, int H, int W, int layout, cudaStream_t s);
 size_t quantile_scratch_bytes();
 int launch_quantiles(const float* x, long long n, const unsigned long long* ranks_host, int nq, float* out, void* scratch,

@@ -249,7 +249,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int ty = rem / p.tiles_x;
       const int tx = rem - ty * p.tiles_x;
       const int x0 = tx * p.TW, y0 = ty * p.TH, n0 = nt * BLOCK_N + (int)rank * (BLOCK_N / CG);
-      const int bk0 = (int)(img * p.b_img_k_stride);       // split-K: this image's K range of B
       if constexpr (SLAB > 0) {
         if (tile == w_first) issue_next_slab();             // the very first slab; afterwards always one K block ahead
         for (int kb = 0; kb < kb_per_tap; ++kb) {
@@ -326,10 +325,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const int xs = x0 + p.tap_dx[t], ys = y0 + p.tap_dy[t] + p.y_pad;
               if (CG == 2) {
                 ptx::tma_load_4d_pair(sa, &tmA, &full_bar[stage], kb * kElemsPerRow, xs, ys, img);
-                ptx::tma_load_2d_pair(sb, &tmB, &full_bar[stage], bk0 + kbl * kElemsPerRow, n0);
+                ptx::tma_load_2d_pair(sb, &tmB, &full_bar[stage], kbl * kElemsPerRow, n0);
               } else {
                 ptx::tma_load_4d(sa, &tmA, &full_bar[stage], kb * kElemsPerRow, xs, ys, img);
-                ptx::tma_load_2d(sb, &tmB, &full_bar[stage], bk0 + kbl * kElemsPerRow, n0);
+                ptx::tma_load_2d(sb, &tmB, &full_bar[stage], kbl * kElemsPerRow, n0);
               }
             }
           }
@@ -1025,8 +1024,7 @@ static int make_maps(const GemmParams& p, int block_n, TensorMapPair* maps, int 
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     HDRVAE_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(B, slab) failed: %d (K=%d cols=%d)", (int)r, p.k_per_tap, p.n_cols);
   } else {
-    cuuint64_t dims[2] = {(cuuint64_t)(p.b_img_k_stride > 0 ? p.b_img_k_stride * p.n_img : (long long)p.k_per_tap * p.ntaps),
-                          (cuuint64_t)(p.b_rows > 0 ? p.b_rows : p.n_cols)};
+    cuuint64_t dims[2] = {(cuuint64_t)p.k_per_tap * p.ntaps, (cuuint64_t)(p.b_rows > 0 ? p.b_rows : p.n_cols)};
     cuuint64_t strides[1] = {(cuuint64_t)p.b_row_stride * eb};
     cuuint32_t box[2] = {(cuuint32_t)row_elems, (cuuint32_t)block_n};
     cuuint32_t estr[2] = {1, 1};
@@ -1129,10 +1127,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
                  "gemm_tc: GroupNorm statistics need 128/256/512 output channels");
   HDRVAE_REQUIRE(p.stats == nullptr || (p.n_cols & (p.n_cols - 1)) == 0, "gemm_tc: GroupNorm statistics need 128/256/512 output channels");
   const bool tf32 = p.ab_dtype == DT_F32;
-  int use_cg = p.cta_group > 0 ? p.cta_group : 2;           // CTA pairs by default
-  // A CTA pair shares one B tile, so with a per-image K offset into B (split-K) both m-tiles of a pair must
-  // belong to the same image: an odd number of tiles per image runs as single CTAs.
-  if (p.b_img_k_stride != 0 && (p.tiles_x * p.tiles_y) % 2 != 0) use_cg = 1;
+  const int use_cg = p.cta_group > 0 ? p.cta_group : 2;     // CTA pairs by default
   const bool n128 = p.n_cols <= 128;
   if (p.n_cols <= 64 && !tf32) {
     // narrow tiles (the upscaler's 32- and 64-channel convs): 32 / 64 accumulator columns instead of 128, so the
@@ -1145,7 +1140,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
             (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0);
     }
     if (p.slab) {
-      HDRVAE_REQUIRE(p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0,
+      HDRVAE_REQUIRE(p.ntaps == 9 && p.TW == 8 && p.TH == 16,
                      "gemm_tc: the slab variant is a 3x3 conv on 8x16-pixel tiles");
       if (use_cg == 2) {
         if (n32) {
@@ -1196,7 +1191,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
     } else {
       epi = -1;
     }
-    if (p.slab && n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0) {
+    if (p.slab && n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16) {
       // the decoder's 128-channel 3x3 convs: slab variant, weights in groups of 3 taps
       if (epi == EPI_STATS) return launch_tc<128, false, 2, EPI_STATS, 3>(p, num_sms, stream);
       if (epi == (EPI_OUT16 | EPI_STATS)) return launch_tc<128, false, 2, EPI_OUT16 | EPI_STATS, 3>(p, num_sms, stream);
@@ -1206,7 +1201,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
       if (epi == 0) return launch_tc<128, false, 2, 0, 3>(p, num_sms, stream);
       if (epi == EPI_RES) return launch_tc<128, false, 2, EPI_RES, 3>(p, num_sms, stream);
     }
-    if (p.slab && !n128 && p.ntaps == 4 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0) {
+    if (p.slab && !n128 && p.ntaps == 4 && p.TW == 8 && p.TH == 16) {
       // one output phase of an upsample conv: 4 taps of the same halo slab (tap-reload form: L2 -> SM bound, the issuer
       // waited for operands 60 % of the time)
       if (epi == (EPI_OUT2 | EPI_STATS)) return launch_tc<256, false, 2, EPI_OUT2 | EPI_STATS, 1>(p, num_sms, stream);
@@ -1215,13 +1210,13 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
       HDRVAE_REQUIRE(false, "gemm_tc: no slab build for this upsample epilogue (%d)", epi);
     }
     if (p.xf_scale != nullptr) {
-      HDRVAE_REQUIRE(p.slab && !n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0 && p.k2 == 0,
+      HDRVAE_REQUIRE(p.slab && !n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.k2 == 0,
                      "gemm_tc: the fused GroupNorm exists for the 256-column 3x3 slab convs");
       if (epi == (EPI_OUT16 | EPI_STATS)) return launch_tc<256, false, 2, EPI_OUT16 | EPI_STATS, 1, true>(p, num_sms, stream);
       if (epi == (EPI_OUT16 | EPI_RES16 | EPI_STATS)) return launch_tc<256, false, 2, EPI_OUT16 | EPI_RES16 | EPI_STATS, 1, true>(p, num_sms, stream);
       HDRVAE_REQUIRE(false, "gemm_tc: no fused-GroupNorm build for this epilogue (%d)", epi);
     }
-    if (p.slab && !n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16 && p.b_img_k_stride == 0) {
+    if (p.slab && !n128 && p.ntaps == 9 && p.TW == 8 && p.TH == 16) {
       // 256-column tiles: slab variant with one tap of weights per stage
       if (epi == EPI_STATS) return launch_tc<256, false, 2, EPI_STATS, 1>(p, num_sms, stream);
       if (epi == (EPI_OUT16 | EPI_STATS)) return launch_tc<256, false, 2, EPI_OUT16 | EPI_STATS, 1>(p, num_sms, stream);

@@ -191,7 +191,7 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
         const int ys = y + p.tap_dy[t] + p.y_pad, xs = x + p.tap_dx[t];
         if (ys < 0 || ys >= p.H + 2 * p.y_pad || xs < 0 || xs >= p.W) continue;
         const long long ao = img * p.a_img_stride + ys * p.a_row_stride + xs * p.a_px_stride;
-        const long long bo = col * p.b_row_stride + (long long)t * p.k_per_tap + img * p.b_img_k_stride;
+        const long long bo = col * p.b_row_stride + (long long)t * p.k_per_tap;
         const int kv = p.a_k_valid > 0 ? p.a_k_valid : p.k_per_tap;
         for (int c = 0; c < kv; ++c) {
           float av = load_as(p.a, ao + c, p.ab_dtype), bv = load_as(p.b, bo + c, p.ab_dtype);
@@ -370,35 +370,6 @@ int launch_softmax_rows(const float* s, void* p, int p_dtype, float* inv_sum, in
                         long long s_ld, long long p_ld, cudaStream_t st) {
   HDRVAE_REQUIRE(s_ld % 4 == 0 && p_ld % 4 == 0 && n_pad >= n_valid, "softmax: bad leading dimensions");
   softmax_rows_kernel<<<n_rows, 256, 0, st>>>(s, p, p_dtype, inv_sum, n_valid, n_pad, s_ld, p_ld);
-  HDRVAE_LAUNCHED();
-  HDRVAE_CUDA_OK(cudaGetLastError());
-  return 0;
-}
-
-// ------------------------------------------------------------------ split-K reduction of the PV GEMM
-// out[r][c] = inv_sum[r] * sum_s part[s][r][c]  (fp32 partials -> 16-bit attention output), fixed summation order
-__global__ void attn_reduce_splits_kernel(const float* __restrict__ part, const float* __restrict__ inv_sum,
-                                          void* __restrict__ out, int out_dtype, int rows, int cols, int splits) {
-  const long long n4 = (long long)rows * cols / 4;
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
-    float4 a = reinterpret_cast<const float4*>(part)[i];
-    for (int s2 = 1; s2 < splits; ++s2) {
-      const float4 b = reinterpret_cast<const float4*>(part)[(long long)s2 * n4 + i];
-      a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
-    }
-    const float sc = inv_sum[(i * 4) / cols];
-    uint2 o;
-    o.x = pack2(a.x * sc, a.y * sc, out_dtype);
-    o.y = pack2(a.z * sc, a.w * sc, out_dtype);
-    reinterpret_cast<uint2*>(out)[i] = o;
-  }
-}
-int launch_attn_reduce_splits(const float* part, const float* inv_sum, void* out, int out_dtype, int rows, int cols,
-                              int splits, cudaStream_t st) {
-  const long long n4 = (long long)rows * cols / 4;
-  int grid = ceil_div(n4, 256);
-  if (grid > 148 * 8) grid = 148 * 8;
-  attn_reduce_splits_kernel<<<grid, 256, 0, st>>>(part, inv_sum, out, out_dtype, rows, cols, splits);
   HDRVAE_LAUNCHED();
   HDRVAE_CUDA_OK(cudaGetLastError());
   return 0;
