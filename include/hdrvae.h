@@ -241,14 +241,23 @@ int hdrvae_rows_run_direct(hdrvae_rows* state, void* stream);
 /* After HDRVAE_EX_END: copy the statistics (global: pre/post/conv/pre3; local slab: out_*, pixel counts) and free. */
 int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
 
-/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for ESRGAN /
- * RRDBNet 4x models (nf 64, gc 32, any block count; what spandrel loads for "ESRGAN" checkpoints, :73-77).
- * The model object is created against a decode context (device, SM count, conv implementation).
- *   load_weights : the model's state dict in either key layout (Real-ESRGAN "conv_first / body.N.rdbK.convJ / ..."
- *                  or BasicSR-spandrel "model.0 / model.1.sub.N.RDBK.convJ.0 / ..."), host or device pointers;
- *   forward      : the network (+ reversal hook) on n equal tiles, x [n,h,w,3] -> y [n,4h,4w,3], float32 device
- *                  (kernel-level parity entry: what `upscale_model(a)` with the forward hook returns, :92-105);
- *   upscale      : the whole node: image [B,H,W,3] float32 -> out [B,4H,4W,3]; two passes (input as is / clamped to
+/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for two of the
+ * architectures spandrel loads from models/upscale_models (:73-77):
+ *   - ESRGAN / RRDBNet 4x (nf 64, gc 32, any block count);
+ *   - Real-ESRGAN Compact (SRVGGNetCompact with PReLU: realesr-general-x4v3, realesr-animevideov3, the 2x / 1x
+ *     "compact" models): 3 input channels, nf a multiple of 8 in 8..64, any body depth, scale s = 1, 2 or 4.
+ * The layout is recognised by its keys (Compact: body.0.weight and no conv_first); anything else is rejected with a
+ * message naming the tensor and its shape.  The model object is created against a decode context (device, SM count,
+ * conv implementation).  s below is the model's scale (hdrvae_upscaler_scale).
+ *   load_weights : the model's state dict, host or device pointers.  RRDBNet in either key layout (Real-ESRGAN
+ *                  "conv_first / body.N.rdbK.convJ / ..." or BasicSR-spandrel "model.0 / model.1.sub.N.RDBK.convJ.0 /
+ *                  ..."); Compact as "body.0 / body.1 (PReLU) / ... / body.{2nc+2}";
+ *   blocks       : RRDB blocks, or the Compact's body convs nc (0 allowed); < 0 without a model;
+ *   scale        : 4 for RRDBNet, s for Compact; < 0 before the weights are loaded;
+ *   forward      : the network (+ reversal hook) on n equal tiles, x [n,h,w,3] -> y [n,s*h,s*w,3], float32 device
+ *                  (kernel-level parity entry: what `upscale_model(a)` with the forward hook returns, :92-105; for
+ *                  Compact that includes the nearest-upsampled input the network adds);
+ *   upscale      : the whole node: image [B,H,W,3] float32 -> out [B,s*H,s*W,3]; two passes (input as is / clamped to
  *                  [-1,1], :181-186) through 512-pixel tiles with 64 overlap and feather blending (:110-146,
  *                  comfy.utils.tiled_scale), Y from the first and Cb/Cr from the second pass, clamp(Y,0,8), 3x3 median
  *                  (:189-218), optional output median (small_blur, :219-224) and local hot-spot fix (:229-258). */
@@ -257,6 +266,7 @@ int hdrvae_upscaler_create(hdrvae_ctx* ctx, hdrvae_upscaler** out);
 int hdrvae_upscaler_destroy(hdrvae_upscaler* up);
 int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* descs, int n);
 int hdrvae_upscaler_blocks(hdrvae_upscaler* up);
+int hdrvae_upscaler_scale(hdrvae_upscaler* up);
 int hdrvae_upscaler_forward_bytes(hdrvae_upscaler* up, int n, int h, int w, size_t* bytes);
 int hdrvae_upscaler_forward(hdrvae_upscaler* up, const float* x_bhwc, int n, int h, int w, int reversal,
                             float* y_bhwc, void* workspace, size_t workspace_bytes, void* stream);

@@ -107,6 +107,7 @@ SIGNATURES = {
     "hdrvae_upscaler_destroy": (_i, [_vp]),
     "hdrvae_upscaler_load_weights": (_i, [_vp, C.POINTER(HdrvaeWeightDesc), _i]),
     "hdrvae_upscaler_blocks": (_i, [_vp]),
+    "hdrvae_upscaler_scale": (_i, [_vp]),
     "hdrvae_upscaler_forward_bytes": (_i, [_vp, _i, _i, _i, C.POINTER(_sz)]),
     "hdrvae_upscaler_forward": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
     "hdrvae_upscale_workspace_bytes": (_i, [_vp, _i, _i, _i, C.POINTER(_sz)]),

@@ -110,6 +110,7 @@ struct GemmParams {
   float res_scale;   // multiplier of `residual` (0 is read as 1)
   const float* residual2;  // second fp32 residual, same addressing as out, added unscaled; or null
   float lrelu;       // LeakyReLU negative slope applied last (0: none)
+  const float* act_slope;  // per-column PReLU negative slope, zero-padded to the GEMM's columns, applied last; or null
   int n_store;       // columns actually stored (multiple of 4; 0: n_cols) — a Cout padded up to 32 stores less
   const float* row_scale;  // per M row (x coordinate) multiplier of the accumulator, or null
   float alpha;       // accumulator scale applied before bias (1.0 for convs)

@@ -114,6 +114,7 @@ enum : int {
   EPI_ROWOPS = 32,   // per-row bias / per-row scale (attention GEMMs)
   EPI_LRELU = 64,    // LeakyReLU applied last (upscaler convs)
   EPI_RES2 = 128,    // + second fp32 residual (end of an RRDB: 0.04 acc + 0.2 x2 + x0)
+  EPI_PRELU = 256,   // per-column PReLU applied last (Real-ESRGAN Compact convs)
   EPI_RES16 = 1024,  // + residual stored as a (scaled) 16-bit tensor of type res_dtype: t += res_scale * r
 };
 
@@ -576,6 +577,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const bool do_round = kGen && p.round_tf32 != 0;
     const bool has_lrelu = kGen ? (p.lrelu != 0.f) : ((EPI & EPI_LRELU) != 0);
     const bool has_res2 = kGen ? (p.residual2 != nullptr) : ((EPI & EPI_RES2) != 0);
+    const bool has_prelu = kGen ? (p.act_slope != nullptr) : ((EPI & EPI_PRELU) != 0);
     const float lrelu = p.lrelu, res_scale = p.res_scale;
     const int n_store = p.n_store > 0 ? p.n_store : p.n_cols;
     const int q = warp & 3;                 // TMEM lane quarter this warp may access
@@ -673,6 +675,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             float4 bias4 = make_float4(0.f, 0.f, 0.f, 0.f);
             if (p.bias != nullptr) bias4 = __ldg(reinterpret_cast<const float4*>(p.bias + n0 + cbase + ci * 32 + slot * 4));
             const float2 b01 = make_float2(bias4.x, bias4.y), b23 = make_float2(bias4.z, bias4.w);
+            float4 slope4 = make_float4(0.f, 0.f, 0.f, 0.f);
+            if constexpr ((EPI & EPI_PRELU) != 0) slope4 = __ldg(reinterpret_cast<const float4*>(p.act_slope + n0 + cbase + ci * 32 + slot * 4));
             ptx::tmem_ld_wait(v);
             __syncwarp();                                 // previous chunk's readers are done with the patch
 #pragma unroll
@@ -724,6 +728,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               if constexpr ((EPI & EPI_LRELU) != 0) {
                 t01.x = t01.x < 0.f ? t01.x * lrelu : t01.x; t01.y = t01.y < 0.f ? t01.y * lrelu : t01.y;
                 t23.x = t23.x < 0.f ? t23.x * lrelu : t23.x; t23.y = t23.y < 0.f ? t23.y * lrelu : t23.y;
+              }
+              if constexpr ((EPI & EPI_PRELU) != 0) {
+                t01.x = t01.x < 0.f ? t01.x * slope4.x : t01.x; t01.y = t01.y < 0.f ? t01.y * slope4.y : t01.y;
+                t23.x = t23.x < 0.f ? t23.x * slope4.z : t23.x; t23.y = t23.y < 0.f ? t23.y * slope4.w : t23.y;
               }
               if constexpr ((EPI & EPI_OUT2) != 0) {
                 const float2 u01 = f2_mul(t01, s2_2), u23 = f2_mul(t23, s2_2);
@@ -844,6 +852,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         float4 bias4 = make_float4(0.f, 0.f, 0.f, 0.f);
         if (!(row_ops && p.bias_per_row) && p.bias != nullptr && cmask != 0u) bias4 = __ldg(reinterpret_cast<const float4*>(p.bias + n0 + col));
+        float4 slope4 = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (has_prelu && cmask != 0u) slope4 = __ldg(reinterpret_cast<const float4*>(p.act_slope + n0 + col));
         ptx::tmem_ld_wait(v);
         __syncwarp();                                     // previous chunk's readers are done with the patch
 #pragma unroll
@@ -903,6 +913,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (has_lrelu) {
             t.x = t.x < 0.f ? t.x * lrelu : t.x; t.y = t.y < 0.f ? t.y * lrelu : t.y;
             t.z = t.z < 0.f ? t.z * lrelu : t.z; t.w = t.w < 0.f ? t.w * lrelu : t.w;
+          }
+          if (has_prelu) {
+            t.x = t.x < 0.f ? t.x * slope4.x : t.x; t.y = t.y < 0.f ? t.y * slope4.y : t.y;
+            t.z = t.z < 0.f ? t.z * slope4.z : t.z; t.w = t.w < 0.f ? t.w * slope4.w : t.w;
           }
           if (has_out2) {
             // second, scaled 16-bit copy of the output: the tensor-core operand of a conv that consumes this
@@ -1137,7 +1151,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
     if (use_cg == 2 && !p.round_tf32 && p.stats == nullptr && !p.bias_per_row && p.row_scale == nullptr &&
         (p.residual == nullptr || p.res_dtype == DT_F32)) {
       epi = (p.out_dtype != DT_F32 ? EPI_OUT16 : 0) | (p.residual ? EPI_RES : 0) | (p.residual2 ? EPI_RES2 : 0) |
-            (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0);
+            (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0) | (p.act_slope ? EPI_PRELU : 0);
     }
     if (p.slab) {
       HDRVAE_REQUIRE(p.ntaps == 9 && p.TW == 8 && p.TH == 16,
@@ -1149,6 +1163,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
           return launch_tc<32, false, 2, EPI_GENERIC, 9>(p, num_sms, stream);
         }
         if (epi == (EPI_OUT16 | EPI_LRELU)) return launch_tc<64, false, 2, EPI_OUT16 | EPI_LRELU, 9>(p, num_sms, stream);
+        if (epi == (EPI_OUT16 | EPI_PRELU)) return launch_tc<64, false, 2, EPI_OUT16 | EPI_PRELU, 9>(p, num_sms, stream);
         if (epi == (EPI_RES | EPI_OUT2)) return launch_tc<64, false, 2, EPI_RES | EPI_OUT2, 9>(p, num_sms, stream);
         if (epi == (EPI_RES | EPI_RES2 | EPI_OUT2)) return launch_tc<64, false, 2, EPI_RES | EPI_RES2 | EPI_OUT2, 9>(p, num_sms, stream);
         if (epi == EPI_OUT2) return launch_tc<64, false, 2, EPI_OUT2, 9>(p, num_sms, stream);
@@ -1172,7 +1187,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
                        : launch_tc<64, false, 1, EPI_GENERIC>(p, num_sms, stream);
   }
   const bool res16 = p.residual != nullptr && p.res_dtype != DT_F32;
-  if (use_cg == 2 && !tf32 && p.lrelu == 0.f && p.residual2 == nullptr && (p.res_scale == 0.f || p.res_scale == 1.f || res16)) {
+  if (use_cg == 2 && !tf32 && p.lrelu == 0.f && p.act_slope == nullptr && p.residual2 == nullptr && (p.res_scale == 0.f || p.res_scale == 1.f || res16)) {
     // specialised epilogues for what the decoder launches; anything else takes the generic build
     int epi = 0;
     const bool simple_res = p.residual == nullptr || p.res_dtype == DT_F32;

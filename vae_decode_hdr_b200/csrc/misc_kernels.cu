@@ -207,6 +207,7 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
     if (p.residual != nullptr) v += (p.res_scale != 0.f ? p.res_scale : 1.f) * load_as(p.residual, off, p.res_dtype);
     if (p.residual2 != nullptr) v += p.residual2[off];
     if (p.lrelu != 0.f && v < 0.f) v *= p.lrelu;
+    if (p.act_slope != nullptr && v < 0.f) v *= p.act_slope[col];
     if (p.n_store > 0 && col >= p.n_store) continue;
     if (p.out2 != nullptr) {
       const long long off2 = p.out2_px_stride == 0 ? off

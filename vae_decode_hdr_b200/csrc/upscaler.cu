@@ -1,8 +1,9 @@
 // HDR upscaler path: replaces HDRUpscaleWithModel.upscale of the reference
-// (/root/reference/hdr_upscale_with_model.py:148-263): two passes of an ESRGAN / RRDBNet 4x model through
-// overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output (:79-107, :110-146),
-// feather blending (restated comfy.utils.tiled_scale), then the luma / chroma recombination in YCbCr with a 3x3
-// median on Y (:187-224) and the optional local hot-spot fix (:229-258).
+// (/root/reference/hdr_upscale_with_model.py:148-263): two passes of the model (ESRGAN / RRDBNet 4x, or Real-ESRGAN
+// Compact at 1x, 2x or 4x) through overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output
+// (:79-107, :110-146), feather blending (restated comfy.utils.tiled_scale), then the luma / chroma recombination in YCbCr
+// with a 3x3 median on Y (:187-224) and the optional local hot-spot fix (:229-258).  Everything after the model reads
+// the float4 tile-output layout [n][s h][s w] that both forwards leave, with the model's scale s.
 //
 // The RRDB convs run on the tcgen05 implicit-GEMM kernel of gemm_tc.cu with narrow (32 / 64 column) tiles:
 //   * a dense block keeps one 192-channel fp16 buffer per pixel [x | g1 | g2 | g3 | g4]; conv k reads the channel
@@ -13,6 +14,9 @@
 //     residual operands) and writes, besides the fp32 stream, the fp16 operand copy into the next block's buffer;
 //   * the two nearest-2x upsamples are folded into the loads of conv_up1 / conv_up2 (4 phase convs each);
 //   * conv_last (64 -> 3) computes 32 columns and stores 4.
+// The Compact convs (SRVGGNetCompact: conv, PReLU, ..., conv to 3 s^2 channels) run on the same kernel with the
+// per-channel PReLU in the epilogue; up_shuffle_base_kernel then applies the pixel shuffle and adds the nearest-upsampled
+// fp32 input (the network's base).
 // Everything after the model (hook, feather blend, YCbCr, median, local fix) is elementwise / stencil work in
 // fp32 with the reference's operation order (no FMA contraction) so that it is bit-comparable to the oracle.
 #include <string.h>
@@ -64,7 +68,29 @@ __device__ __forceinline__ float up_reversal(float v, int kind) {
   return v;
 }
 
-// model output [n][4h][4w][4] fp32 -> reversal hook -> [n][4h][4w][3] (kernel-level parity entry)
+// Compact tail: y = pixel_shuffle(conv, s) + nearest_upsample(x, s).  conv is the last conv's fp32 output [n][h][w][cl]
+// (channel c s^2 + i s + j of input pixel (y, x) -> channel c of output pixel (y s + i, x s + j)); the base is the tile's
+// fp32 input pixel, clamped to [-1, 1] for the second pass's tiles (tile table .w) like the network's own input.  Writes
+// the float4 [n][s h][s w] tile-output layout of the RRDBNet forward (.w = 0).
+__global__ void up_shuffle_base_kernel(const float* __restrict__ conv, int cl, const float* __restrict__ img, int H, int W,
+                                       const int4* __restrict__ tiles, int n, int h, int w, int s, float4* __restrict__ out) {
+  const int OH = h * s, OW = w * s, s2 = s * s;
+  const long long total = (long long)n * OH * OW;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int X = (int)(i % OW);
+    const int Y = (int)((i / OW) % OH);
+    const int t = (int)(i / ((long long)OW * OH));
+    const int y = Y / s, x = X / s;
+    const int4 tl = tiles[t];                     // image, y0, x0, clamp flag
+    const float* src = img + (((long long)tl.x * H + tl.y + y) * W + tl.z + x) * 3;
+    float r = src[0], g = src[1], b = src[2];
+    if (tl.w) { r = fminf(fmaxf(r, -1.f), 1.f); g = fminf(fmaxf(g, -1.f), 1.f); b = fminf(fmaxf(b, -1.f), 1.f); }
+    const float* c = conv + (((long long)t * h + y) * w + x) * cl + (Y - y * s) * s + (X - x * s);
+    out[i] = make_float4(__fadd_rn(c[0], r), __fadd_rn(c[s2], g), __fadd_rn(c[2 * s2], b), 0.f);
+  }
+}
+
+// model output [n][s h][s w][4] fp32 -> reversal hook -> [n][s h][s w][3] (kernel-level parity entry)
 __global__ void up_finish_tiles_kernel(const float4* __restrict__ in, long long n_px, int kind, float* __restrict__ out) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_px; i += (long long)gridDim.x * blockDim.x) {
     const float4 v = in[i];
@@ -214,9 +240,9 @@ __global__ void up_local_fix_kernel(const float* __restrict__ img, int B, int H,
     if (method == HDRVAE_UPSCALE_BISLERP) {
       // comfy.utils.bislerp on the 1-channel luma (restated in oracle/upscaler_oracle.py): separable, width pass first.
       // Per axis: the two source pixels bilinear interpolation (align_corners = False) would blend, c1 = floor(src),
-      // c2 = min(c1 + 1, last), ratio r = frac(src) with src = max((dst + 0.5) / scale - 0.5, 0) — exact in fp32 for the
-      // 4x scale — then a SPHERICAL interpolation of the channel vectors; for scalars: same sign -> the first pixel,
-      // opposite signs -> linear, a zero -> sine weights times the linearly interpolated magnitude.
+      // c2 = min(c1 + 1, last), ratio r = frac(src) with src = max((dst + 0.5) / scale - 0.5, 0) — exact in fp32 for
+      // power-of-two scales — then a SPHERICAL interpolation of the channel vectors; for scalars: same sign -> the first
+      // pixel, opposite signs -> linear, a zero -> sine weights times the linearly interpolated magnitude.
       auto slerp1 = [](float b1, float b2, float r) {
         const float n1 = fabsf(b1), n2 = fabsf(b2);
         const float u1 = n1 == 0.f ? 0.f : b1 / n1, u2 = n2 == 0.f ? 0.f : b2 / n2;
@@ -288,22 +314,40 @@ struct hdrvae_upscaler {
   hdrvae_ctx* ctx = nullptr;      // device / SM count / conv implementation come from the decode context
   hdrvae_ctx store;               // owns this model's device allocations
   bool loaded = false;
-  int nb = 0;
+  bool compact = false;           // Real-ESRGAN SRVGGNetCompact; else ESRGAN / RRDBNet
+  int scale = 4;                  // output pixels per input pixel along each axis
+  int nb = 0;                     // RRDB blocks (RRDBNet) or body convs (Compact)
   PackedConv conv_first, conv_body, up1, up2, hr, last;
   std::vector<UpRdb> rdb;         // 3 per RRDB
+  std::vector<PackedConv> body;   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2)
+  std::vector<float*> slopes;     // Compact: PReLU slopes applied after body[k], k <= nb (cout_pad floats, zero-padded)
 };
 
 namespace hdrvae {
 
+// channels per pixel of the Compact last conv's fp32 output: 3 s^2 rounded up to the epilogue's 4-column stores
+static int up_last_channels(const hdrvae_upscaler* up) { return (3 * up->scale * up->scale + 3) / 4 * 4; }
+
 struct UpPlan {                   // workspace of one forward over n tiles of h x w
-  size_t img8, cat0, cat1, f_feat, f_a, f_b, f_c, u0, u1, u2, u3, total;
+  size_t img8, cat0, cat1, f_feat, f_a, f_b, f_c, u0, u1, u2, u3;   // RRDBNet
+  size_t act0, act1, last;                                          // Compact
+  size_t total;
 };
-static UpPlan up_make_plan(int n, int h, int w) {
+static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
   UpPlan pl;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 1023) / 1024 * 1024; return o; };
   const size_t P = (size_t)n * h * w;
   pl.img8 = take(P * 8 * 2);
+  if (up->compact) {
+    // fp16 activations at a pixel stride of cout_pad (the convs read the first nf channels), ping-pong
+    const size_t cp = (size_t)up->body[0].cout_pad;
+    pl.act0 = take(P * cp * 2);
+    pl.act1 = take(P * cp * 2);
+    pl.last = take(P * up_last_channels(up) * 4);
+    pl.total = off;
+    return pl;
+  }
   pl.cat0 = take(P * 192 * 2);
   pl.cat1 = take(P * 192 * 2);
   pl.f_feat = take(P * 64 * 4);
@@ -384,12 +428,53 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
   return 0;
 }
 
+// Compact forward on n tiles (fp16 [n][h][w][8] in pl.img8) -> the last conv's fp32 [n][h][w][up_last_channels] in pl.last
+static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, cudaStream_t s) {
+  hdrvae_ctx* ctx = up->ctx;
+  const int cp = up->body[0].cout_pad;
+  uint8_t* act[2] = {ws + pl.act0, ws + pl.act1};
+  const size_t nconv = up->body.size();
+  for (size_t k = 0; k < nconv; ++k) {
+    ConvIO io;
+    io.x = k == 0 ? ws + pl.img8 : act[(k - 1) & 1];
+    io.x_channels = k == 0 ? 8 : cp;
+    if (k + 1 < nconv) {
+      io.y = act[k & 1]; io.y_dtype = DT_F16; io.y_channels = cp; io.act_slope = up->slopes[k];
+    } else {
+      io.y = ws + pl.last; io.y_dtype = DT_F32; io.y_channels = up_last_channels(up);
+    }
+    HDRVAE_TRY(run_conv(ctx, up->body[k], io, n, h, w, ctx->conv_impl, s));
+  }
+  return 0;
+}
+
+// The network on n tiles of h x w cut from img [.][H][W][3] at the origins of `tiles` (image, y0, x0, clamp to [-1, 1])
+// -> fp32 [n][s h][s w][4] at out4
+static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, const int4* tiles, int n, int h, int w,
+                        uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
+  {
+    ProfScope prof("upscaler extract tiles", 0.0, (double)n * h * w * (12 + 16), s);
+    up_extract_tiles_kernel<<<up_grid((long long)n * h * w), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0,
+                                                                         reinterpret_cast<uint4*>(ws + pl.img8));
+    HDRVAE_LAUNCHED();
+  }
+  if (!up->compact) return up_forward(up, n, h, w, ws, pl, out4, s);
+  HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s));
+  const int sc = up->scale, cl = up_last_channels(up);
+  const long long opx = (long long)n * sc * sc * h * w;
+  ProfScope prof("upscaler pixel shuffle + base", 0.0, (double)n * h * w * (cl * 4 + 12) + opx * 16, s);
+  up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float*>(ws + pl.last), cl, img, H, W, tiles, n, h, w,
+                                                      sc, reinterpret_cast<float4*>(out4));
+  HDRVAE_LAUNCHED();
+  return 0;
+}
+
 }  // namespace hdrvae
 
 // ------------------------------------------------------------------------------------------------ tiling plan
 namespace hdrvae {
 
-static const int kUpTile = 512, kUpOverlap = 64, kUpScale = 4;     // hdr_upscale_with_model.py:115-116, 4x ESRGAN
+static const int kUpTile = 512, kUpOverlap = 64;                   // hdr_upscale_with_model.py:115-116
 static const long long kUpMaxChunkPx = 8LL * 512 * 512;            // pixels of one forward batch (bounds the workspace: ~14 GB)
 
 struct UpHostTile { int b, y0, x0, h, w; long long off, off2; };
@@ -414,7 +499,7 @@ struct UpTiling {
   long long out_px = 0;               // float4 elements of all tile outputs (both passes)
 };
 
-static UpTiling up_make_tiling(int B, int H, int W) {
+static UpTiling up_make_tiling(int B, int H, int W, int scale) {
   UpTiling t;
   t.single = H <= kUpTile && W <= kUpTile;
   const std::vector<int> py = up_positions(H), px = up_positions(W);
@@ -439,7 +524,7 @@ static UpTiling up_make_tiling(int B, int H, int W) {
   }
   long long off = 0;
   for (UpGroup& g : t.groups) {
-    const long long per = (long long)g.h * g.w, sz = 16 * per;
+    const long long per = (long long)g.h * g.w, sz = (long long)scale * scale * per;
     const int cap = (int)std::max<long long>(1, std::min<long long>((long long)g.tiles.size(), kUpMaxChunkPx / (2 * per)));
     for (size_t i0 = 0; i0 < g.tiles.size(); i0 += cap) {
       UpChunk c;
@@ -459,17 +544,18 @@ static UpTiling up_make_tiling(int B, int H, int W) {
 }
 
 struct UpWs { size_t descs, origins, out, ycc, tmp, fwd, total; };
-static UpWs up_make_ws(const UpTiling& t, int B, int H, int W) {
+static UpWs up_make_ws(const hdrvae_upscaler* up, const UpTiling& t, int B, int H, int W) {
   UpWs w;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 1023) / 1024 * 1024; return o; };
+  const size_t s2 = (size_t)up->scale * up->scale;
   w.descs = take(t.tiles.size() * sizeof(UpTile));
   w.origins = take(2 * t.tiles.size() * sizeof(int4));
   w.out = take((size_t)t.out_px * 16);
-  w.ycc = take((size_t)B * 16 * H * W * 3 * 4);
-  w.tmp = take((size_t)B * 16 * H * W * 3 * 4);
+  w.ycc = take((size_t)B * s2 * H * W * 3 * 4);
+  w.tmp = take((size_t)B * s2 * H * W * 3 * 4);
   size_t fwd = 0;
-  for (const UpChunk& c : t.chunks) fwd = std::max(fwd, up_make_plan(2 * c.n, c.h, c.w).total);
+  for (const UpChunk& c : t.chunks) fwd = std::max(fwd, up_make_plan(up, 2 * c.n, c.h, c.w).total);
   w.fwd = take(fwd);
   w.total = off;
   return w;
@@ -517,6 +603,96 @@ static std::string up_canonical(const std::string& k, int nb_hint) {
   return "";
 }
 
+static std::string up_shape_str(const std::vector<int64_t>& sh) {
+  std::string r = "[";
+  for (size_t i = 0; i < sh.size(); ++i) r += (i ? "," : "") + std::to_string(sh[i]);
+  return r + "]";
+}
+
+// Real-ESRGAN SRVGGNetCompact as spandrel loads it with act_type "prelu": body.0 = conv 3 -> nf, body.{2k+1} = PReLU
+// slopes [nf] (k = 0..nc), body.{2+2m} = conv nf -> nf (m < nc), body.{2nc+2} = conv nf -> 3 s^2.  The scale s is
+// limited to powers of two (1, 2, 4): only there do the local fix's resampling coordinates (dst + 0.5) / s equal torch's.
+static int up_pack_compact(hdrvae_upscaler* up, cudaStream_t s) {
+  hdrvae_ctx* st = &up->store;
+  auto shape_of = [&](const std::string& k) -> const std::vector<int64_t>* {
+    auto it = st->shapes.find(k);
+    return it == st->shapes.end() ? nullptr : &it->second;
+  };
+  int last = -1;
+  for (const auto& kv : st->shapes) {
+    int bi = -1;
+    if (sscanf(kv.first.c_str(), "body.%d.", &bi) == 1) last = std::max(last, bi);
+  }
+  HDRVAE_REQUIRE(last >= 2 && last % 2 == 0,
+                 "Compact upscaler: the highest body index is %d; the last conv must sit at an even index >= 2", last);
+  const int nc = (last - 2) / 2;
+  const std::vector<int64_t>& w0 = *shape_of("body.0.weight");
+  HDRVAE_REQUIRE(w0.size() == 4 && w0[1] == 3 && w0[2] == 3 && w0[3] == 3,
+                 "Compact upscaler: body.0.weight has shape %s; want [nf,3,3,3] (3 input channels)", up_shape_str(w0).c_str());
+  const int nf = (int)w0[0];
+  HDRVAE_REQUIRE(nf >= 8 && nf <= 64 && nf % 8 == 0,
+                 "Compact upscaler: body.0.weight has shape %s; nf must be a multiple of 8 in 8..64", up_shape_str(w0).c_str());
+  const std::string last_key = "body." + std::to_string(last) + ".weight";
+  const std::vector<int64_t>* wl = shape_of(last_key);
+  HDRVAE_REQUIRE(wl != nullptr && wl->size() == 4 && (*wl)[1] == nf && (*wl)[2] == 3 && (*wl)[3] == 3 &&
+                 ((*wl)[0] == 3 || (*wl)[0] == 12 || (*wl)[0] == 48),
+                 "Compact upscaler: %s has shape %s; want [3*scale^2,%d,3,3] with scale 1, 2 or 4", last_key.c_str(),
+                 wl ? up_shape_str(*wl).c_str() : "(missing)", nf);
+  up->scale = (*wl)[0] == 3 ? 1 : (*wl)[0] == 12 ? 2 : 4;
+  up->nb = nc;
+  auto conv = [&](int idx, int cout, int cin, PackedConv* pc) -> int {
+    const std::string k = "body." + std::to_string(idx);
+    const std::vector<int64_t>* w = shape_of(k + ".weight");
+    const std::vector<int64_t>* b = shape_of(k + ".bias");
+    HDRVAE_REQUIRE(w != nullptr && b != nullptr, "Compact upscaler state dict lacks %s.{weight,bias}", k.c_str());
+    HDRVAE_REQUIRE(w->size() == 4 && (*w)[0] == cout && (*w)[1] == cin && (*w)[2] == 3 && (*w)[3] == 3,
+                   "Compact upscaler: %s.weight has shape %s; want [%d,%d,3,3]", k.c_str(), up_shape_str(*w).c_str(), cout, cin);
+    HDRVAE_REQUIRE(b->size() == 1 && (*b)[0] == cout, "Compact upscaler: %s.bias has shape %s; want [%d]", k.c_str(),
+                   up_shape_str(*b).c_str(), cout);
+    return pack_conv(st, st->raw[k + ".weight"], st->raw[k + ".bias"], cout, cin, 3, false, 1.f, DT_F16, pc, s);
+  };
+  up->body.resize((size_t)nc + 2);
+  HDRVAE_TRY(conv(0, nf, 3, &up->body[0]));
+  for (int m = 0; m < nc; ++m) HDRVAE_TRY(conv(2 + 2 * m, nf, nf, &up->body[1 + m]));
+  HDRVAE_TRY(conv(last, 3 * up->scale * up->scale, nf, &up->body[nc + 1]));
+  const int cp = up->body[0].cout_pad;
+  for (int k = 0; k <= nc; ++k) {
+    const std::string key = "body." + std::to_string(2 * k + 1) + ".weight";
+    const std::vector<int64_t>* sh = shape_of(key);
+    HDRVAE_REQUIRE(sh != nullptr, "Compact upscaler state dict lacks the PReLU slopes %s (only act_type \"prelu\" is supported)",
+                   key.c_str());
+    HDRVAE_REQUIRE(sh->size() == 1 && (*sh)[0] == nf, "Compact upscaler: %s has shape %s; want [%d] (one PReLU slope per channel)",
+                   key.c_str(), up_shape_str(*sh).c_str(), nf);
+    float* slope = nullptr;
+    HDRVAE_TRY(dev_alloc(st, cp * sizeof(float), (void**)&slope));
+    HDRVAE_CUDA_OK(cudaMemsetAsync(slope, 0, cp * sizeof(float), s));
+    HDRVAE_CUDA_OK(cudaMemcpyAsync(slope, st->raw[key], nf * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    up->slopes.push_back(slope);
+  }
+  up->compact = true;
+  return 0;
+}
+
+// After packing: waits for the copies, frees the staging buffers and the fp32 copies of the state dict.
+static int up_finish_load(hdrvae_upscaler* up, std::vector<void*>& staging, cudaStream_t s) {
+  hdrvae_ctx* st = &up->store;
+  HDRVAE_CUDA_OK(cudaStreamSynchronize(s));
+  for (void* p : staging) cudaFree(p);
+  for (auto& kv : st->raw) cudaFree(kv.second);        // fp32 copies are no longer needed
+  {
+    std::vector<void*> keep;
+    for (void* p : st->owned) {
+      bool raw = false;
+      for (auto& kv : st->raw) if (kv.second == p) { raw = true; break; }
+      if (!raw) keep.push_back(p);
+    }
+    st->owned.swap(keep);
+    st->raw.clear();
+  }
+  up->loaded = true;
+  return 0;
+}
+
 int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* descs, int n) {
   HDRVAE_REQUIRE(up != nullptr && descs != nullptr && n > 0, "hdrvae_upscaler_load_weights: null argument");
   HDRVAE_REQUIRE(!up->loaded, "hdrvae_upscaler_load_weights: model already loaded (create a new one)");
@@ -525,6 +701,7 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
   cudaStream_t s = nullptr;
   std::vector<void*> staging;
   int nb = 0;
+  bool has_body0 = false, has_conv_first = false;      // Compact: body.0.weight and no conv_first (in either layout)
   for (int i = 0; i < n; ++i) {
     const hdrvae_weight_desc& d = descs[i];
     HDRVAE_REQUIRE(d.name && d.data && d.ndim >= 1 && d.ndim <= 4, "hdrvae_upscaler_load_weights: bad descriptor %d", i);
@@ -543,10 +720,18 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
     HDRVAE_TRY(launch_to_f32(stage, d.dtype, f, cnt, s));
     st->raw[name] = f;
     st->shapes[name] = shp;
+    has_body0 = has_body0 || name == "body.0.weight";
+    has_conv_first = has_conv_first || name.compare(0, 11, "conv_first.") == 0;
     int bi = -1;
     if (sscanf(name.c_str(), "body.%d.", &bi) == 1) nb = std::max(nb, bi + 1);
   }
-  HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0)");
+  // (checked first: the RRDB block scan below also counts the Compact's body.N keys)
+  if (has_body0 && !has_conv_first) {
+    HDRVAE_TRY(up_pack_compact(up, s));
+    return up_finish_load(up, staging, s);
+  }
+  HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
+                 "no Real-ESRGAN Compact model (body.0.weight without conv_first)");
   up->nb = nb;
   auto conv = [&](const std::string& k, int cout, int cin, bool upsample, float scale, PackedConv* pc) -> int {
     auto it = st->shapes.find(k + ".weight");
@@ -576,29 +761,20 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
   HDRVAE_TRY(conv("conv_up2", 64, 64, true, 1.f, &up->up2));
   HDRVAE_TRY(conv("conv_hr", 64, 64, false, 1.f, &up->hr));
   HDRVAE_TRY(conv("conv_last", 3, 64, false, 1.f, &up->last));
-  HDRVAE_CUDA_OK(cudaStreamSynchronize(s));
-  for (void* p : staging) cudaFree(p);
-  for (auto& kv : st->raw) cudaFree(kv.second);        // fp32 copies are no longer needed
-  {
-    std::vector<void*> keep;
-    for (void* p : st->owned) {
-      bool raw = false;
-      for (auto& kv : st->raw) if (kv.second == p) { raw = true; break; }
-      if (!raw) keep.push_back(p);
-    }
-    st->owned.swap(keep);
-    st->raw.clear();
-  }
-  up->loaded = true;
-  return 0;
+  return up_finish_load(up, staging, s);
 }
 
 int hdrvae_upscaler_blocks(hdrvae_upscaler* up) { return up ? up->nb : -1; }
 
+int hdrvae_upscaler_scale(hdrvae_upscaler* up) {
+  HDRVAE_REQUIRE(up != nullptr && up->loaded, "hdrvae_upscaler_scale: weights not loaded");
+  return up->scale;
+}
+
 int hdrvae_upscaler_forward_bytes(hdrvae_upscaler* up, int n, int h, int w, size_t* bytes) {
   HDRVAE_REQUIRE(up && bytes && n >= 1 && h >= 1 && w >= 1, "hdrvae_upscaler_forward_bytes: bad argument");
-  const UpPlan pl = up_make_plan(n, h, w);
-  *bytes = pl.total + (size_t)n * 16 * h * w * 16 + (size_t)n * sizeof(int4) + 4096;
+  const UpPlan pl = up_make_plan(up, n, h, w);
+  *bytes = pl.total + (size_t)n * up->scale * up->scale * h * w * 16 + (size_t)n * sizeof(int4) + 4096;
   return 0;
 }
 
@@ -612,17 +788,14 @@ int hdrvae_upscaler_forward(hdrvae_upscaler* up, const float* x_bhwc, int n, int
   HDRVAE_CUDA_OK(cudaSetDevice(up->store.device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
-  const UpPlan pl = up_make_plan(n, h, w);
+  const UpPlan pl = up_make_plan(up, n, h, w);
+  const long long npx = (long long)n * up->scale * up->scale * h * w;
   float* out4 = reinterpret_cast<float*>(ws + pl.total);
-  int4* origins = reinterpret_cast<int4*>(ws + pl.total + (size_t)n * 16 * h * w * 16);
+  int4* origins = reinterpret_cast<int4*>(ws + pl.total + (size_t)npx * 16);
   std::vector<int4> host(n);
   for (int i = 0; i < n; ++i) host[i] = make_int4(i, 0, 0, 0);
   HDRVAE_CUDA_OK(cudaMemcpyAsync(origins, host.data(), n * sizeof(int4), cudaMemcpyHostToDevice, s));
-  up_extract_tiles_kernel<<<up_grid((long long)n * h * w), 256, 0, s>>>(x_bhwc, h, w, origins, n, h, w, 0,
-                                                                       reinterpret_cast<uint4*>(ws + pl.img8));
-  HDRVAE_LAUNCHED();
-  HDRVAE_TRY(up_forward(up, n, h, w, ws, pl, out4, s));
-  const long long npx = (long long)n * 16 * h * w;
+  HDRVAE_TRY(up_run_model(up, x_bhwc, h, w, origins, n, h, w, ws, pl, out4, s));
   up_finish_tiles_kernel<<<up_grid(npx), 256, 0, s>>>(reinterpret_cast<const float4*>(out4), npx, reversal, y_bhwc);
   HDRVAE_LAUNCHED();
   HDRVAE_CUDA_OK(cudaGetLastError());
@@ -631,8 +804,8 @@ int hdrvae_upscaler_forward(hdrvae_upscaler* up, const float* x_bhwc, int n, int
 
 int hdrvae_upscale_workspace_bytes(hdrvae_upscaler* up, int B, int H, int W, size_t* bytes) {
   HDRVAE_REQUIRE(up && bytes && B >= 1 && H >= 1 && W >= 1, "hdrvae_upscale_workspace_bytes: bad argument");
-  const UpTiling t = up_make_tiling(B, H, W);
-  *bytes = up_make_ws(t, B, H, W).total;
+  const UpTiling t = up_make_tiling(B, H, W, up->scale);
+  *bytes = up_make_ws(up, t, B, H, W).total;
   return 0;
 }
 
@@ -645,17 +818,18 @@ int hdrvae_upscale(hdrvae_upscaler* up, const float* image_bhwc, int B, int H, i
                  "hdrvae_upscale: local_fix supports upscale_method nearest-exact, bilinear, area, bicubic and bislerp (got %d)", upscale_method);
   HDRVAE_CUDA_OK(cudaSetDevice(up->store.device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  const UpTiling t = up_make_tiling(B, H, W);
-  const UpWs wsl = up_make_ws(t, B, H, W);
+  const int sc = up->scale;
+  const UpTiling t = up_make_tiling(B, H, W, sc);
+  const UpWs wsl = up_make_ws(up, t, B, H, W);
   HDRVAE_REQUIRE(workspace_bytes >= wsl.total, "hdrvae_upscale: workspace too small (%zu < %zu)", workspace_bytes, wsl.total);
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
-  const int OH = H * kUpScale, OW = W * kUpScale;
+  const int OH = H * sc, OW = W * sc;
   // tile descriptors (output coordinates) in the reference's accumulation order
   std::vector<UpTile> descs(t.tiles.size());
   for (size_t i = 0; i < t.tiles.size(); ++i) {
     const UpHostTile& u = t.tiles[i];
-    descs[i].b = u.b; descs[i].oy = u.y0 * kUpScale; descs[i].ox = u.x0 * kUpScale;
-    descs[i].oh = u.h * kUpScale; descs[i].ow = u.w * kUpScale; descs[i].off = u.off; descs[i].off2 = u.off2;
+    descs[i].b = u.b; descs[i].oy = u.y0 * sc; descs[i].ox = u.x0 * sc;
+    descs[i].oh = u.h * sc; descs[i].ow = u.w * sc; descs[i].off = u.off; descs[i].off2 = u.off2;
   }
   HDRVAE_CUDA_OK(cudaMemcpyAsync(ws + wsl.descs, descs.data(), descs.size() * sizeof(UpTile), cudaMemcpyHostToDevice, s));
   // small_blur's input filter (:176-178) is torchvision gaussian_blur(kernel 3, sigma 0.1): taps exp(-50) = 1.9e-22
@@ -671,30 +845,33 @@ int hdrvae_upscale(hdrvae_upscaler* up, const float* image_bhwc, int B, int H, i
   HDRVAE_CUDA_OK(cudaMemcpyAsync(origins, host_or.data(), host_or.size() * sizeof(int4), cudaMemcpyHostToDevice, s));
   float* out_all = reinterpret_cast<float*>(ws + wsl.out);
   for (const UpChunk& c : t.chunks) {
-    const int n2 = 2 * c.n;
-    const long long per = (long long)c.h * c.w;
-    const UpPlan pl = up_make_plan(n2, c.h, c.w);
-    uint8_t* fws = ws + wsl.fwd;
-    up_extract_tiles_kernel<<<up_grid((long long)n2 * per), 256, 0, s>>>(image_bhwc, H, W, origins + c.origin0, n2, c.h, c.w, 0,
-                                                                        reinterpret_cast<uint4*>(fws + pl.img8));
-    HDRVAE_LAUNCHED();
-    HDRVAE_TRY(up_forward(up, n2, c.h, c.w, fws, pl, out_all + c.out_base * 4, s));
+    const UpPlan pl = up_make_plan(up, 2 * c.n, c.h, c.w);
+    HDRVAE_TRY(up_run_model(up, image_bhwc, H, W, origins + c.origin0, 2 * c.n, c.h, c.w, ws + wsl.fwd, pl,
+                            out_all + c.out_base * 4, s));
   }
   const long long opx = (long long)B * OH * OW;
   float* ycc = reinterpret_cast<float*>(ws + wsl.ycc);
   float* tmp = reinterpret_cast<float*>(ws + wsl.tmp);
-  up_blend_ycc_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float4*>(ws + wsl.out),
-                                                    reinterpret_cast<const UpTile*>(ws + wsl.descs), (int)t.tiles.size(),
-                                                    t.single ? 1 : 0, B, OH, OW, kUpOverlap * kUpScale, reversal, ycc);
-  HDRVAE_LAUNCHED();
-  up_recombine_kernel<<<up_grid(opx), 256, 0, s>>>(ycc, B, OH, OW, small_blur ? tmp : out_bhwc);
-  HDRVAE_LAUNCHED();
+  {
+    ProfScope prof("upscaler blend + YCbCr", 0.0, (double)t.out_px * 16 + opx * 12, s);
+    up_blend_ycc_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float4*>(ws + wsl.out),
+                                                      reinterpret_cast<const UpTile*>(ws + wsl.descs), (int)t.tiles.size(),
+                                                      t.single ? 1 : 0, B, OH, OW, kUpOverlap * sc, reversal, ycc);
+    HDRVAE_LAUNCHED();
+  }
+  {
+    ProfScope prof("upscaler median Y + recombine", 0.0, opx * 24.0, s);
+    up_recombine_kernel<<<up_grid(opx), 256, 0, s>>>(ycc, B, OH, OW, small_blur ? tmp : out_bhwc);
+    HDRVAE_LAUNCHED();
+  }
   if (small_blur) {
+    ProfScope prof("upscaler median RGB (small_blur)", 0.0, opx * 24.0, s);
     up_median_rgb_kernel<<<up_grid(opx * 3), 256, 0, s>>>(tmp, B, OH, OW, out_bhwc);
     HDRVAE_LAUNCHED();
   }
   if (local_fix) {
-    up_local_fix_kernel<<<up_grid(opx), 256, 0, s>>>(image_bhwc, B, H, W, kUpScale, upscale_method, out_bhwc);
+    ProfScope prof("upscaler local fix", 0.0, opx * 24.0 + (double)B * H * W * 12, s);
+    up_local_fix_kernel<<<up_grid(opx), 256, 0, s>>>(image_bhwc, B, H, W, sc, upscale_method, out_bhwc);
     HDRVAE_LAUNCHED();
   }
   HDRVAE_CUDA_OK(cudaGetLastError());

@@ -1,14 +1,16 @@
 """`HDRUpscaleWithModel` — drop-in for the reference node of the same name
 (/root/reference/hdr_upscale_with_model.py:50-279): same INPUT_TYPES / RETURN_TYPES / FUNCTION / CATEGORY, same
-argument meaning, IMAGE in ([B,H,W,3] float32) -> IMAGE out ([B,4H,4W,3] float32).
+argument meaning, IMAGE in ([B,H,W,3] float32) -> IMAGE out ([B,sH,sW,3] float32, s = the model's scale).
 
-What changes is where the work happens: the ESRGAN / RRDBNet model, the reversal hook, the tiled feather blend and
-the YCbCr recombination all run in libhdrvae.so on the GPU (vae_decode_hdr_b200/csrc/upscaler.cu).  There is no CPU
-path: without a CUDA device or without the library the node raises.
+What changes is where the work happens: the model, the reversal hook, the tiled feather blend and the YCbCr
+recombination all run in libhdrvae.so on the GPU (vae_decode_hdr_b200/csrc/upscaler.cu).  There is no CPU path: without
+a CUDA device or without the library the node raises.
 
 Model loading stays what it is in ComfyUI (folder_paths + spandrel, :73-77); the node only reads
-`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Architectures other than
-the 4x RRDBNet (nf 64, gc 32) are rejected by the library with an error naming the tensor that does not fit.
+`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Two architectures run: the 4x
+RRDBNet (ESRGAN: nf 64, gc 32) and Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x.  An RRDBNet of
+another scale fails before any GPU work; any other architecture is rejected by the library with an error naming the
+tensor that does not fit; a `descriptor.scale` that disagrees with the weights is an error too.
 """
 from __future__ import annotations
 
@@ -19,7 +21,7 @@ from typing import Any, Tuple
 
 import torch
 
-from .upscaler import UPSCALE_METHODS, HdrUpscalerEngine, reversal_for_architecture
+from .upscaler import UPSCALE_METHODS, HdrUpscalerEngine, is_compact_state_dict, reversal_for_architecture
 
 
 def _model_filenames():
@@ -78,6 +80,22 @@ class HDRUpscaleWithModel:
         except (OSError, TypeError):
             return (str(path), 0, 0, str(device))
 
+    @staticmethod
+    def _new_engine(descriptor, device: torch.device) -> HdrUpscalerEngine:
+        """Packs the descriptor's weights; the engine's scale (read from the weights) must be `descriptor.scale`."""
+        scale = getattr(descriptor, "scale", 4)
+        sd = descriptor.model.state_dict()
+        if scale != 4 and not is_compact_state_dict(sd):
+            # the only RRDBNet form implemented is the 4x one: fail before any weights reach the GPU
+            raise RuntimeError(f"HDRUpscaleWithModel (B200) implements RRDBNet / ESRGAN at scale 4 only; this model has "
+                               f"scale {scale}")
+        engine = HdrUpscalerEngine(sd, device)
+        if engine.scale != scale:
+            engine.close()
+            raise RuntimeError(f"HDRUpscaleWithModel (B200): the model descriptor gives scale {scale}, its weights are a "
+                               f"{engine.scale}x network")
+        return engine
+
     @classmethod
     def _engine_for(cls, key, load_descriptor, device: torch.device):
         """-> (engine, scale, architecture name).  `load_descriptor()` is only called on a cache miss."""
@@ -86,10 +104,8 @@ class HDRUpscaleWithModel:
             cls._engines.move_to_end(key)
             return hit
         descriptor = load_descriptor()
-        scale = getattr(descriptor, "scale", 4)
-        if scale != 4:
-            raise RuntimeError(f"HDRUpscaleWithModel (B200) implements 4x RRDBNet models; this model has scale {scale}")
-        entry = (HdrUpscalerEngine(descriptor.model.state_dict(), device), scale, descriptor.architecture.name)
+        engine = cls._new_engine(descriptor, device)
+        entry = (engine, engine.scale, descriptor.architecture.name)
         cls._engines[key] = entry
         while len(cls._engines) > cls.MAX_ENGINES:
             _, (old, _, _) = cls._engines.popitem(last=False)
@@ -110,9 +126,7 @@ class HDRUpscaleWithModel:
             key = None
         if key is None:
             descriptor = self._load_model_internal(model_name)
-            if getattr(descriptor, "scale", 4) != 4:
-                raise RuntimeError(f"HDRUpscaleWithModel (B200) implements 4x RRDBNet models; {model_name!r} has scale {descriptor.scale}")
-            engine = HdrUpscalerEngine(descriptor.model.state_dict(), device)
+            engine = self._new_engine(descriptor, device)
             try:
                 out = engine.upscale(image, reversal_for_architecture(descriptor.architecture.name), bool(small_blur),
                                      bool(local_fix), upscale_method)

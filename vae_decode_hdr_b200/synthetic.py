@@ -135,3 +135,30 @@ def random_upscaler_state_dict(seed: int = 0, nb: int = 23) -> Dict[str, torch.T
             bound = 1.0 / math.sqrt(shape[1] * shape[2] * shape[3])
         sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * bound
     return sd
+
+
+def compact_param_shapes(nf: int = 64, nc: int = 32, s: int = 4) -> List[Tuple[str, Tuple[int, ...]]]:
+    """Real-ESRGAN Compact (SRVGGNetCompact, PReLU) parameters: body.0 conv 3 -> nf, body.{2k+1} PReLU slopes,
+    body.{2+2m} convs nf -> nf, body.{2nc+2} conv nf -> 3 s^2."""
+    out: List[Tuple[str, Tuple[int, ...]]] = []
+    for i in range(2 * nc + 3):
+        if i % 2:
+            out.append((f"body.{i}.weight", (nf,)))
+            continue
+        cout, cin = (3 * s * s if i == 2 * nc + 2 else nf), (3 if i == 0 else nf)
+        out.append((f"body.{i}.weight", (cout, cin, 3, 3)))
+        out.append((f"body.{i}.bias", (cout,)))
+    return out
+
+
+def random_compact_state_dict(seed: int = 0, nf: int = 64, nc: int = 32, s: int = 4) -> Dict[str, torch.Tensor]:
+    """PyTorch-default-style conv init of a Compact model, PReLU slopes ~ U(-0.5, 0.5) per channel, fp32, CPU."""
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    sd: Dict[str, torch.Tensor] = {}
+    bound = 1.0
+    for name, shape in compact_param_shapes(nf, nc, s):
+        if len(shape) == 4:
+            bound = 1.0 / math.sqrt(shape[1] * shape[2] * shape[3])
+        scale = 0.5 if len(shape) == 1 and name.endswith(".weight") else bound
+        sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * scale
+    return sd

@@ -1,4 +1,4 @@
-"""Host side of the HDR upscaler path (libhdrvae.so `hdrvae_upscale*`): owns one model object per (ESRGAN weights,
+"""Host side of the HDR upscaler path (libhdrvae.so `hdrvae_upscale*`): owns one model object per (upscaler weights,
 device).  PyTorch is plumbing only (device memory, current stream); all arithmetic happens in the library."""
 from __future__ import annotations
 
@@ -23,10 +23,15 @@ def reversal_for_architecture(name: str) -> str:
     return "logit"
 
 
-class HdrUpscalerEngine:
-    """One RRDBNet (ESRGAN 4x: nf 64, gc 32) packed for the tcgen05 conv kernel on one GPU."""
+def is_compact_state_dict(state_dict) -> bool:
+    """The Real-ESRGAN Compact (SRVGGNetCompact) key layout, as the library recognises it: `body.0.weight` and no
+    `conv_first.*`.  Every other model the library runs is a 4x RRDBNet."""
+    return "body.0.weight" in state_dict and not any(k.startswith("conv_first.") for k in state_dict)
 
-    scale = 4
+
+class HdrUpscalerEngine:
+    """One upscaler model packed for the tcgen05 conv kernel on one GPU: an RRDBNet (ESRGAN 4x: nf 64, gc 32) or a
+    Real-ESRGAN Compact (SRVGGNetCompact, PReLU, 1x / 2x / 4x).  `scale` is the model's, read from the library."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda"):
         self.lib = N.load_library()
@@ -54,6 +59,7 @@ class HdrUpscalerEngine:
             torch.cuda.synchronize(self.device)
             N.check(self.lib.hdrvae_upscaler_load_weights(self._up, arr, len(descs)), "hdrvae_upscaler_load_weights")
         self.blocks = int(self.lib.hdrvae_upscaler_blocks(self._up))
+        self.scale = int(self.lib.hdrvae_upscaler_scale(self._up))
 
     def set_conv_impl(self, impl: int) -> None:
         N.check(self.lib.hdrvae_set_conv_impl(self._ctx, impl), "hdrvae_set_conv_impl")
@@ -68,13 +74,13 @@ class HdrUpscalerEngine:
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def forward(self, x_bhwc: torch.Tensor, reversal: str = "atanh") -> torch.Tensor:
-        """The network + reversal hook on a batch of equal tiles: [n,h,w,3] -> [n,4h,4w,3] (fp32)."""
+        """The network + reversal hook on a batch of equal tiles: [n,h,w,3] -> [n,s*h,s*w,3] (fp32, s = self.scale)."""
         if x_bhwc.dim() != 4 or x_bhwc.shape[-1] != 3:
             raise ValueError(f"expected [n,h,w,3], got {tuple(x_bhwc.shape)}")
         n, h, w, _ = x_bhwc.shape
         with torch.cuda.device(self.device):
             x = x_bhwc.to(self.device, torch.float32).contiguous()
-            y = torch.empty((n, 4 * h, 4 * w, 3), dtype=torch.float32, device=self.device)
+            y = torch.empty((n, self.scale * h, self.scale * w, 3), dtype=torch.float32, device=self.device)
             need = C.c_size_t()
             N.check(self.lib.hdrvae_upscaler_forward_bytes(self._up, n, h, w, C.byref(need)), "hdrvae_upscaler_forward_bytes")
             ws = self._ws(int(need.value))
@@ -84,7 +90,7 @@ class HdrUpscalerEngine:
 
     def upscale(self, image_bhwc: torch.Tensor, reversal: str = "atanh", small_blur: bool = False, local_fix: bool = False,
                 upscale_method: str = "bilinear", out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """The whole node path on the GPU: [B,H,W,3] fp32 -> [B,4H,4W,3] fp32."""
+        """The whole node path on the GPU: [B,H,W,3] fp32 -> [B,s*H,s*W,3] fp32 (s = self.scale)."""
         if image_bhwc.dim() != 4 or image_bhwc.shape[-1] != 3:
             raise ValueError(f"expected an IMAGE tensor [B,H,W,3], got {tuple(image_bhwc.shape)}")
         if reversal not in ("atanh", "logit"):
@@ -95,7 +101,7 @@ class HdrUpscalerEngine:
         with torch.cuda.device(self.device):
             x = image_bhwc.to(self.device, torch.float32).contiguous()
             if out is None:
-                out = torch.empty((B, 4 * H, 4 * W, 3), dtype=torch.float32, device=self.device)
+                out = torch.empty((B, self.scale * H, self.scale * W, 3), dtype=torch.float32, device=self.device)
             need = C.c_size_t()
             N.check(self.lib.hdrvae_upscale_workspace_bytes(self._up, B, H, W, C.byref(need)), "hdrvae_upscale_workspace_bytes")
             ws = self._ws(int(need.value))
