@@ -1,6 +1,6 @@
 // HDR upscaler path: replaces HDRUpscaleWithModel.upscale of the reference
-// (/root/reference/hdr_upscale_with_model.py:148-263): two passes of the model (ESRGAN / RRDBNet 4x, or Real-ESRGAN
-// Compact at 1x, 2x or 4x) through overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output
+// (/root/reference/hdr_upscale_with_model.py:148-263): two passes of the model (ESRGAN / RRDBNet at 1x, 2x or 4x, or
+// Real-ESRGAN Compact at 1x, 2x or 4x) through overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output
 // (:79-107, :110-146), feather blending (restated comfy.utils.tiled_scale), then the luma / chroma recombination in YCbCr
 // with a 3x3 median on Y (:187-224) and the optional local hot-spot fix (:229-258).  Everything after the model reads
 // the float4 tile-output layout [n][s h][s w] that both forwards leave, with the model's scale s.
@@ -12,8 +12,10 @@
 //     channels into the next slice: the concat never exists as a copy;
 //   * conv5 adds the fp32 residual stream (0.2 conv + x; at the end of an RRDB 0.04 conv + 0.2 x2 + x0 with two
 //     residual operands) and writes, besides the fp32 stream, the fp16 operand copy into the next block's buffer;
-//   * the two nearest-2x upsamples are folded into the loads of conv_up1 / conv_up2 (4 phase convs each);
-//   * conv_last (64 -> 3) computes 32 columns and stores 4.
+//   * the u (0, 1 or 2) nearest-2x upsamples are folded into the loads of conv_up1 / conv_up2 (4 phase convs each);
+//   * conv_last (64 -> 3) computes 32 columns and stores 4;
+//   * a pixel-unshuffle RRDBNet (RealESRGAN_x2plus: f = 2) reads its tile reflect-padded to a multiple of f and unshuffled
+//     into 3 f^2 channels (up_extract_tiles_kernel<f>); the scale is 2^u / f, and a padded tile's output is cropped.
 // The Compact convs (SRVGGNetCompact: conv, PReLU, ..., conv to 3 s^2 channels) run on the same kernel with the
 // per-channel PReLU in the epilogue; up_shuffle_base_kernel then applies the pixel shuffle and adds the nearest-upsampled
 // fp32 input (the network's base).
@@ -30,24 +32,58 @@
 namespace hdrvae {
 
 // ------------------------------------------------------------------------------------------------ kernels
-// image fp32 BHWC (3 channels) -> fp16 tile batch [n][h][w][8] (channels 3..7 zero), optional clamp to [-1, 1]
+// fp16 channels per pixel of the network input for pixel-unshuffle factor f: 3 f^2 rounded up to a 16-byte pixel stride
+// (the TMA row stride); the conv reads the first 3 f^2 of them (ConvIO::x_channels)
+__host__ __device__ constexpr int up_in_channels(int f) { return f == 1 ? 8 : f == 2 ? 16 : 48; }
+
+// image fp32 BHWC (3 channels) -> fp16 network input [n][h'][w'][up_in_channels(F)] of tiles of h x w at the origins of
+// `tiles`, h' = ceil(h / F): clamp to [-1, 1] (flag or tile table .w), reflect pad of the tile's bottom / right edge to
+// F h' x F w' (torch "reflect": row h + k reads row h - 2 - k), pixel unshuffle by F (channel c F^2 + i F + j = channel c
+// at pixel (y F + i, x F + j)), channels beyond 3 F^2 zero.  The clamp is elementwise, so it commutes with pad and
+// unshuffle.  F = 1 is the plain [n][h][w][8] copy.
+template <int F>
 __global__ void up_extract_tiles_kernel(const float* __restrict__ img, int H, int W, const int4* __restrict__ tiles /*b,y0,x0,_*/,
                                         int n, int h, int w, int clamp1, uint4* __restrict__ out) {
-  const long long total = (long long)n * h * w;
+  constexpr int CX = up_in_channels(F), F2 = F * F;
+  const int hq = (h + F - 1) / F, wq = (w + F - 1) / F;
+  const long long total = (long long)n * hq * wq;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int x = (int)(i % w);
-    const int y = (int)((i / w) % h);
-    const int t = (int)(i / ((long long)w * h));
+    const int x = (int)(i % wq);
+    const int y = (int)((i / wq) % hq);
+    const int t = (int)(i / ((long long)wq * hq));
     const int4 tl = tiles[t];                     // image, y0, x0, clamp flag
-    const float* src = img + (((long long)tl.x * H + tl.y + y) * W + tl.z + x) * 3;
-    float r = src[0], g = src[1], b = src[2];
-    if (clamp1 || tl.w) { r = fminf(fmaxf(r, -1.f), 1.f); g = fminf(fmaxf(g, -1.f), 1.f); b = fminf(fmaxf(b, -1.f), 1.f); }
-    const __half2 rg = __floats2half2_rn(r, g), b0 = __floats2half2_rn(b, 0.f);
-    uint4 o;
-    o.x = *reinterpret_cast<const uint32_t*>(&rg);
-    o.y = *reinterpret_cast<const uint32_t*>(&b0);
-    o.z = 0u; o.w = 0u;
-    out[i] = o;
+    __align__(16) __half v[CX];
+#pragma unroll
+    for (int c = 0; c < CX; ++c) v[c] = __float2half_rn(0.f);
+#pragma unroll
+    for (int a = 0; a < F; ++a) {
+      int yy = y * F + a;
+      if (yy >= h) yy = 2 * (h - 1) - yy;
+#pragma unroll
+      for (int b = 0; b < F; ++b) {
+        int xx = x * F + b;
+        if (xx >= w) xx = 2 * (w - 1) - xx;
+        const float* src = img + (((long long)tl.x * H + tl.y + yy) * W + tl.z + xx) * 3;
+        float r = src[0], g = src[1], bl = src[2];
+        if (clamp1 || tl.w) { r = fminf(fmaxf(r, -1.f), 1.f); g = fminf(fmaxf(g, -1.f), 1.f); bl = fminf(fmaxf(bl, -1.f), 1.f); }
+        v[a * F + b] = __float2half_rn(r);
+        v[F2 + a * F + b] = __float2half_rn(g);
+        v[2 * F2 + a * F + b] = __float2half_rn(bl);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < CX / 8; ++k) out[i * (CX / 8) + k] = reinterpret_cast<const uint4*>(v)[k];
+  }
+}
+
+// top-left [oh][ow] window of each of n float4 images [ih][iw]: the output of a reflect-padded tile cut to s h x s w
+__global__ void up_crop_kernel(const float4* __restrict__ in, int ih, int iw, int n, int oh, int ow, float4* __restrict__ out) {
+  const long long total = (long long)n * oh * ow;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int x = (int)(i % ow);
+    const int y = (int)((i / ow) % oh);
+    const int t = (int)(i / ((long long)ow * oh));
+    out[i] = in[((long long)t * ih + y) * iw + x];
   }
 }
 
@@ -315,8 +351,10 @@ struct hdrvae_upscaler {
   hdrvae_ctx store;               // owns this model's device allocations
   bool loaded = false;
   bool compact = false;           // Real-ESRGAN SRVGGNetCompact; else ESRGAN / RRDBNet
-  int scale = 4;                  // output pixels per input pixel along each axis
+  int scale = 4;                  // output pixels per input pixel along each axis (RRDBNet: 2^n_up / shuffle)
   int nb = 0;                     // RRDB blocks (RRDBNet) or body convs (Compact)
+  int n_up = 2;                   // RRDBNet: nearest-2x + conv upsampling stages (0, 1 or 2)
+  int shuffle = 1;                // RRDBNet: pixel-unshuffle factor of the input (1, 2 or 4; conv_first reads 3 f^2 channels)
   PackedConv conv_first, conv_body, up1, up2, hr, last;
   std::vector<UpRdb> rdb;         // 3 per RRDB
   std::vector<PackedConv> body;   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2)
@@ -328,6 +366,20 @@ namespace hdrvae {
 // channels per pixel of the Compact last conv's fp32 output: 3 s^2 rounded up to the epilogue's 4-column stores
 static int up_last_channels(const hdrvae_upscaler* up) { return (3 * up->scale * up->scale + 3) / 4 * 4; }
 
+// network grid of a tile of h x w: the reflect-padded tile pixel-unshuffled by the model's factor f
+static int up_net_side(const hdrvae_upscaler* up, int side) { return (side + up->shuffle - 1) / up->shuffle; }
+
+// torch's reflect pad needs pad < side; a tile side for which the pad to a multiple of f fails is refused
+static int up_check_sides(const hdrvae_upscaler* up, int h, int w) {
+  const int f = up->shuffle;
+  for (int side : {h, w}) {
+    const int pad = (f - side % f) % f;
+    HDRVAE_REQUIRE(pad < side, "upscaler: a tile side of %d pixels is too short for the reflect pad of %d pixels that the "
+                   "model's %dx pixel unshuffle needs (the pad must be shorter than the side)", side, pad, f);
+  }
+  return 0;
+}
+
 struct UpPlan {                   // workspace of one forward over n tiles of h x w
   size_t img8, cat0, cat1, f_feat, f_a, f_b, f_c, u0, u1, u2, u3;   // RRDBNet
   size_t act0, act1, last;                                          // Compact
@@ -337,8 +389,8 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
   UpPlan pl;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 1023) / 1024 * 1024; return o; };
-  const size_t P = (size_t)n * h * w;
-  pl.img8 = take(P * 8 * 2);
+  const size_t P = (size_t)n * up_net_side(up, h) * up_net_side(up, w);   // pixels of the network's input grid
+  pl.img8 = take(P * up_in_channels(up->shuffle) * 2);
   if (up->compact) {
     // fp16 activations at a pixel stride of cout_pad (the convs read the first nf channels), ping-pong
     const size_t cp = (size_t)up->body[0].cout_pad;
@@ -354,26 +406,34 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
   pl.f_a = take(P * 64 * 4);
   pl.f_b = take(P * 64 * 4);
   pl.f_c = take(P * 64 * 4);
+  // fp16 operands of the upsampling stages: conv_body's copy (h' w'), conv_up1's (4 h' w'), conv_up2's (16 h' w'), conv_hr's
+  const size_t Pu = P << (2 * up->n_up);
   pl.u0 = take(P * 64 * 2);
-  pl.u1 = take(P * 4 * 64 * 2);
-  pl.u2 = take(P * 16 * 64 * 2);
-  pl.u3 = take(P * 16 * 64 * 2);
+  pl.u1 = take(up->n_up >= 1 ? P * 4 * 64 * 2 : 0);
+  pl.u2 = take(up->n_up >= 2 ? P * 16 * 64 * 2 : 0);
+  pl.u3 = take(Pu * 64 * 2);
   pl.total = off;
   return pl;
 }
 
-// RRDBNet forward on n tiles (fp16 [n][h][w][8] in pl.img8) -> fp32 [n][4h][4w][4] at `out4`
+// RRDBNet forward on n tiles of h x w (fp16 network input [n][h'][w'][cx] in pl.img8, h' = ceil(h / f)) -> fp32
+// [n][s h][s w][4] at `out4`.  The network runs at h' x w' and conv_last at 2^u h' x 2^u w' = f s h' x f s w'; when the
+// tile was padded (f h' > h) conv_last writes into the dense-block buffer cat0 (dead by then) and the top-left window is
+// copied to out4.
 static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
   hdrvae_ctx* ctx = up->ctx;
   const int impl = ctx->conv_impl;
+  const int hq = up_net_side(up, h), wq = up_net_side(up, w);
+  const int u = up->n_up, hu = hq << u, wu = wq << u;
+  const bool crop = up->shuffle * hq != h || up->shuffle * wq != w;
   uint16_t* cat[2] = {reinterpret_cast<uint16_t*>(ws + pl.cat0), reinterpret_cast<uint16_t*>(ws + pl.cat1)};
   float* feat = reinterpret_cast<float*>(ws + pl.f_feat);
   float* fb[3] = {reinterpret_cast<float*>(ws + pl.f_a), reinterpret_cast<float*>(ws + pl.f_b), reinterpret_cast<float*>(ws + pl.f_c)};
   int cur = 0;                                        // cat[cur] holds the fp16 copy of the current stream in channels 0..63
   {
-    ConvIO io; io.x = ws + pl.img8; io.x_channels = 8; io.y = feat; io.y_dtype = DT_F32;
+    ConvIO io; io.x = ws + pl.img8; io.x_channels = up_in_channels(up->shuffle); io.y = feat; io.y_dtype = DT_F32;
     io.y2 = cat[cur]; io.y2_channels = 192; io.y2_chan_off = 0;
-    HDRVAE_TRY(run_conv(ctx, up->conv_first, io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->conv_first, io, n, hq, wq, impl, s));
   }
   // fp32 stream buffers: x0 (the RRDB input) lives in feat (first block) or fb[xi]; x1 -> fb[P], x2 -> fb[Q] and the
   // block output overwrites x1's buffer (dead by then), which makes it the next block's x0
@@ -388,7 +448,7 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
       for (int j = 0; j < 4; ++j) {
         ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y = cat[cur]; io.y_dtype = DT_F16; io.y_channels = 192;
         io.y_chan_off = 64 + 32 * j; io.lrelu = 0.2f;
-        HDRVAE_TRY(run_conv(ctx, R.c[j], io, n, h, w, impl, s));
+        HDRVAE_TRY(run_conv(ctx, R.c[j], io, n, hq, wq, impl, s));
       }
       ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y_dtype = DT_F32; io.y = outs[k];
       io.y2 = cat[cur ^ 1]; io.y2_channels = 192; io.y2_chan_off = 0;
@@ -396,34 +456,47 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
       // k < 2: x_{k+1} = 0.2 conv5 + x_k (weights and bias packed x 0.2); end of the RRDB:
       // (0.2 conv5 + x2) 0.2 + x0 = 0.04 conv5 + 0.2 x2 + x0 (weights and bias packed x 0.04)
       if (k == 2) { io.res_scale = 0.2f; io.residual2 = x0; }
-      HDRVAE_TRY(run_conv(ctx, R.c[4], io, n, h, w, impl, s));
+      HDRVAE_TRY(run_conv(ctx, R.c[4], io, n, hq, wq, impl, s));
       xin = outs[k];
       cur ^= 1;
     }
     x0 = outs[2];
     xi = P;
   }
-  // trunk conv + long skip: t = conv_body(x) + feat; only its fp16 copy is needed (operand of conv_up1)
+  // trunk conv + long skip: t = conv_body(x) + feat; only its fp16 copy is needed (operand of the first upsampling conv,
+  // or of conv_hr when there is none)
   {
     ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y = fb[(xi + 2) % 3]; io.y_dtype = DT_F32;
     io.residual = feat; io.res_dtype = DT_F32; io.y2 = ws + pl.u0;
-    HDRVAE_TRY(run_conv(ctx, up->conv_body, io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->conv_body, io, n, hq, wq, impl, s));
   }
-  {
+  uint8_t* hr_in = ws + pl.u0;
+  if (u >= 1) {
     ConvIO io; io.x = ws + pl.u0; io.y = ws + pl.u1; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->up1, io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->up1, io, n, hq, wq, impl, s));
+    hr_in = ws + pl.u1;
   }
-  {
+  if (u >= 2) {
     ConvIO io; io.x = ws + pl.u1; io.y = ws + pl.u2; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->up2, io, n, 2 * h, 2 * w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->up2, io, n, 2 * hq, 2 * wq, impl, s));
+    hr_in = ws + pl.u2;
   }
   {
-    ConvIO io; io.x = ws + pl.u2; io.y = ws + pl.u3; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->hr, io, n, 4 * h, 4 * w, impl, s));
+    ConvIO io; io.x = hr_in; io.y = ws + pl.u3; io.y_dtype = DT_F16; io.lrelu = 0.2f;
+    HDRVAE_TRY(run_conv(ctx, up->hr, io, n, hu, wu, impl, s));
   }
+  float* last_out = crop ? reinterpret_cast<float*>(ws + pl.cat0) : out4;     // cat0: 384 bytes per h' w' pixel >= 16 4^u
   {
-    ConvIO io; io.x = ws + pl.u3; io.y = out4; io.y_dtype = DT_F32; io.y_channels = 4; io.n_store = 4;
-    HDRVAE_TRY(run_conv(ctx, up->last, io, n, 4 * h, 4 * w, impl, s));
+    ConvIO io; io.x = ws + pl.u3; io.y = last_out; io.y_dtype = DT_F32; io.y_channels = 4; io.n_store = 4;
+    HDRVAE_TRY(run_conv(ctx, up->last, io, n, hu, wu, impl, s));
+  }
+  if (crop) {
+    const int oh = up->scale * h, ow = up->scale * w;
+    const long long opx = (long long)n * oh * ow;
+    ProfScope prof("upscaler crop padded tiles", 0.0, opx * 32.0, s);
+    up_crop_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float4*>(last_out), hu, wu, n, oh, ow,
+                                                reinterpret_cast<float4*>(out4));
+    HDRVAE_LAUNCHED();
   }
   return 0;
 }
@@ -453,9 +526,13 @@ static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t*
 static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, const int4* tiles, int n, int h, int w,
                         uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
   {
-    ProfScope prof("upscaler extract tiles", 0.0, (double)n * h * w * (12 + 16), s);
-    up_extract_tiles_kernel<<<up_grid((long long)n * h * w), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0,
-                                                                         reinterpret_cast<uint4*>(ws + pl.img8));
+    const int f = up->shuffle;
+    const long long npx = (long long)n * up_net_side(up, h) * up_net_side(up, w);
+    ProfScope prof("upscaler extract tiles", 0.0, (double)npx * (f * f * 12 + up_in_channels(f) * 2), s);
+    uint4* x = reinterpret_cast<uint4*>(ws + pl.img8);
+    if (f == 1) up_extract_tiles_kernel<1><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
+    else if (f == 2) up_extract_tiles_kernel<2><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
+    else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
     HDRVAE_LAUNCHED();
   }
   if (!up->compact) return up_forward(up, n, h, w, ws, pl, out4, s);
@@ -583,24 +660,52 @@ int hdrvae_upscaler_destroy(hdrvae_upscaler* up) {
   return 0;
 }
 
+// Top-level conv index K of an old-arch key "model.K.weight" / "model.K.bias" (K != 1, the trunk), else -1.
+static int up_old_top_index(const std::string& k) {
+  int K = -1, len = 0;
+  if (sscanf(k.c_str(), "model.%d.%n", &K, &len) != 1 || len == 0 || K == 1) return -1;
+  const std::string leaf = k.substr(len);
+  return leaf == "weight" || leaf == "bias" ? K : -1;
+}
+
 // Canonical (Real-ESRGAN) name of a state-dict key given in either layout; "" if it is not an RRDBNet tensor.
-static std::string up_canonical(const std::string& k, int nb_hint) {
+// BasicSR's sequential() flattens each upsampling stage into (Upsample, conv, LeakyReLU) and conv_hr into (conv,
+// LeakyReLU), so with u upsampling convs the old-arch top-level convs sit at 0 (conv_first), 3 + 3k (conv_up{k+1}),
+// 3u + 2 (conv_hr) and 3u + 4 (conv_last).
+static std::string up_canonical(const std::string& k, int n_up) {
   if (k.compare(0, 6, "model.") != 0) return k;
   auto leaf = k.substr(k.rfind('.') + 1);
   const std::string head = k.substr(0, k.rfind('.'));
-  if (head == "model.0") return "conv_first." + leaf;
-  if (head == "model.3") return "conv_up1." + leaf;
-  if (head == "model.6") return "conv_up2." + leaf;
-  if (head == "model.8") return "conv_hr." + leaf;
-  if (head == "model.10") return "conv_last." + leaf;
+  const int K = up_old_top_index(k);
+  if (K >= 0) {
+    if (K == 0) return "conv_first." + leaf;
+    if (K >= 3 && K < 3 + 3 * n_up && K % 3 == 0) return "conv_up" + std::to_string(K / 3) + "." + leaf;
+    if (K == 3 * n_up + 2) return "conv_hr." + leaf;
+    if (K == 3 * n_up + 4) return "conv_last." + leaf;
+    return "";
+  }
   int i = -1, r = -1, c = -1;
   if (sscanf(head.c_str(), "model.1.sub.%d.RDB%d.conv%d.0", &i, &r, &c) == 3)
     return "body." + std::to_string(i) + ".rdb" + std::to_string(r) + ".conv" + std::to_string(c) + "." + leaf;
-  if (sscanf(head.c_str(), "model.1.sub.%d", &i) == 1 && head == "model.1.sub." + std::to_string(i)) {
-    (void)nb_hint;
-    return "conv_body." + leaf;
-  }
+  if (sscanf(head.c_str(), "model.1.sub.%d", &i) == 1 && head == "model.1.sub." + std::to_string(i)) return "conv_body." + leaf;
   return "";
+}
+
+// Upsampling convs of an RRDBNet state dict, found before any key is mapped: from the highest old-arch top-level conv
+// index (conv_last sits at 3u + 4), else from the Real-ESRGAN conv_up1 / conv_up2 / conv_up3 names.  -1: an old-arch
+// layout whose conv_last index fits no u.
+static int up_count_upconvs(const hdrvae_weight_desc* descs, int n, std::string* last_key) {
+  int top = -1, named = 0;
+  for (int i = 0; i < n; ++i) {
+    if (descs[i].name == nullptr) continue;           // refused by the load loop
+    const std::string k = descs[i].name;
+    const int K = up_old_top_index(k);
+    if (K > top) { top = K; *last_key = "model." + std::to_string(K) + ".weight"; }
+    for (int j = 1; j <= 3; ++j)
+      if (k == "conv_up" + std::to_string(j) + ".weight") named = std::max(named, j);
+  }
+  if (top < 0) return named;
+  return top >= 4 && (top - 4) % 3 == 0 ? (top - 4) / 3 : -1;
 }
 
 static std::string up_shape_str(const std::vector<int64_t>& sh) {
@@ -702,10 +807,17 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
   std::vector<void*> staging;
   int nb = 0;
   bool has_body0 = false, has_conv_first = false;      // Compact: body.0.weight and no conv_first (in either layout)
+  std::string top_key;
+  const int n_up = up_count_upconvs(descs, n, &top_key);
+  auto desc_shape = [&](const std::string& k) {
+    for (int i = 0; i < n; ++i)
+      if (descs[i].name && k == descs[i].name) return up_shape_str(std::vector<int64_t>(descs[i].shape, descs[i].shape + descs[i].ndim));
+    return std::string("(missing)");
+  };
   for (int i = 0; i < n; ++i) {
     const hdrvae_weight_desc& d = descs[i];
     HDRVAE_REQUIRE(d.name && d.data && d.ndim >= 1 && d.ndim <= 4, "hdrvae_upscaler_load_weights: bad descriptor %d", i);
-    const std::string name = up_canonical(d.name, 0);
+    const std::string name = up_canonical(d.name, n_up);
     if (name.empty()) continue;
     long long cnt = 1;
     std::vector<int64_t> shp;
@@ -733,12 +845,35 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
   HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
                  "no Real-ESRGAN Compact model (body.0.weight without conv_first)");
   up->nb = nb;
+  // the layout: u upsampling convs (found above) and the pixel-unshuffle factor f from conv_first's 3 f^2 input channels
+  HDRVAE_REQUIRE(n_up >= 0, "RRDBNet: %s has shape %s; an old-arch RRDBNet's last top-level conv sits at index 3u + 4 "
+                 "(4, 7 or 10 for u = 0, 1 or 2 upsampling convs)", top_key.c_str(), desc_shape(top_key).c_str());
+  {
+    const std::string k3 = top_key.empty() ? "conv_up3.weight" : "model.9.weight";
+    HDRVAE_REQUIRE(n_up <= 2, "RRDBNet: %s has shape %s: a third upsampling conv (an 8x RRDBNet) is not supported; RRDBNet "
+                   "runs with 0, 1 or 2 upsampling convs", k3.c_str(), desc_shape(k3).c_str());
+  }
+  {
+    auto it = st->shapes.find("conv_first.weight");
+    HDRVAE_REQUIRE(it != st->shapes.end(), "upscaler state dict lacks conv_first.{weight,bias}");
+    const std::vector<int64_t>& w0 = it->second;
+    const int64_t cin = w0.size() == 4 ? w0[1] : 0;
+    HDRVAE_REQUIRE(cin == 3 || cin == 12 || cin == 48, "RRDBNet: conv_first.weight has shape %s; want [64,3 f^2,3,3] with "
+                   "pixel-unshuffle factor f = 1, 2 or 4 (3, 12 or 48 input channels)", up_shape_str(w0).c_str());
+    const int f = cin == 3 ? 1 : cin == 12 ? 2 : 4;
+    HDRVAE_REQUIRE((1 << n_up) >= f, "RRDBNet: conv_first.weight has shape %s (pixel-unshuffle factor %d) and the model has "
+                   "%d upsampling conv(s): its scale 2^%d / %d would be below 1", up_shape_str(w0).c_str(), f, n_up, n_up, f);
+    up->n_up = n_up;
+    up->shuffle = f;
+    up->scale = (1 << n_up) / f;
+  }
   auto conv = [&](const std::string& k, int cout, int cin, bool upsample, float scale, PackedConv* pc) -> int {
     auto it = st->shapes.find(k + ".weight");
     HDRVAE_REQUIRE(it != st->shapes.end() && st->raw.count(k + ".bias"), "upscaler state dict lacks %s.{weight,bias}", k.c_str());
     const auto& sh = it->second;
     HDRVAE_REQUIRE(sh.size() == 4 && sh[0] == cout && sh[1] == cin && sh[2] == 3 && sh[3] == 3,
-                   "%s.weight has the wrong shape (want [%d,%d,3,3]: RRDBNet nf 64, gc 32)", k.c_str(), cout, cin);
+                   "%s.weight has the wrong shape %s (want [%d,%d,3,3]: RRDBNet nf 64, gc 32)", k.c_str(),
+                   up_shape_str(sh).c_str(), cout, cin);
     HDRVAE_TRY(pack_conv(st, st->raw[k + ".weight"], st->raw[k + ".bias"], cout, cin, 3, upsample, scale, DT_F16, pc, s));
     if (scale != 1.f) {
       up_scale_f32_kernel<<<1, 64, 0, s>>>(pc->bias, cout, scale);
@@ -746,7 +881,7 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
     }
     return 0;
   };
-  HDRVAE_TRY(conv("conv_first", 64, 3, false, 1.f, &up->conv_first));
+  HDRVAE_TRY(conv("conv_first", 64, 3 * up->shuffle * up->shuffle, false, 1.f, &up->conv_first));
   up->rdb.resize((size_t)nb * 3);
   for (int i = 0; i < nb; ++i)
     for (int r = 0; r < 3; ++r) {
@@ -757,8 +892,8 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
       HDRVAE_TRY(conv(base + "5", 64, 192, false, r == 2 ? 0.2f * 0.2f : 0.2f, &R.c[4]));
     }
   HDRVAE_TRY(conv("conv_body", 64, 64, false, 1.f, &up->conv_body));
-  HDRVAE_TRY(conv("conv_up1", 64, 64, true, 1.f, &up->up1));
-  HDRVAE_TRY(conv("conv_up2", 64, 64, true, 1.f, &up->up2));
+  if (n_up >= 1) HDRVAE_TRY(conv("conv_up1", 64, 64, true, 1.f, &up->up1));
+  if (n_up >= 2) HDRVAE_TRY(conv("conv_up2", 64, 64, true, 1.f, &up->up2));
   HDRVAE_TRY(conv("conv_hr", 64, 64, false, 1.f, &up->hr));
   HDRVAE_TRY(conv("conv_last", 3, 64, false, 1.f, &up->last));
   return up_finish_load(up, staging, s);
@@ -773,6 +908,7 @@ int hdrvae_upscaler_scale(hdrvae_upscaler* up) {
 
 int hdrvae_upscaler_forward_bytes(hdrvae_upscaler* up, int n, int h, int w, size_t* bytes) {
   HDRVAE_REQUIRE(up && bytes && n >= 1 && h >= 1 && w >= 1, "hdrvae_upscaler_forward_bytes: bad argument");
+  HDRVAE_TRY(up_check_sides(up, h, w));
   const UpPlan pl = up_make_plan(up, n, h, w);
   *bytes = pl.total + (size_t)n * up->scale * up->scale * h * w * 16 + (size_t)n * sizeof(int4) + 4096;
   return 0;
@@ -805,6 +941,7 @@ int hdrvae_upscaler_forward(hdrvae_upscaler* up, const float* x_bhwc, int n, int
 int hdrvae_upscale_workspace_bytes(hdrvae_upscaler* up, int B, int H, int W, size_t* bytes) {
   HDRVAE_REQUIRE(up && bytes && B >= 1 && H >= 1 && W >= 1, "hdrvae_upscale_workspace_bytes: bad argument");
   const UpTiling t = up_make_tiling(B, H, W, up->scale);
+  for (const UpGroup& g : t.groups) HDRVAE_TRY(up_check_sides(up, g.h, g.w));
   *bytes = up_make_ws(up, t, B, H, W).total;
   return 0;
 }
@@ -820,6 +957,7 @@ int hdrvae_upscale(hdrvae_upscaler* up, const float* image_bhwc, int B, int H, i
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int sc = up->scale;
   const UpTiling t = up_make_tiling(B, H, W, sc);
+  for (const UpGroup& g : t.groups) HDRVAE_TRY(up_check_sides(up, g.h, g.w));
   const UpWs wsl = up_make_ws(up, t, B, H, W);
   HDRVAE_REQUIRE(workspace_bytes >= wsl.total, "hdrvae_upscale: workspace too small (%zu < %zu)", workspace_bytes, wsl.total);
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);

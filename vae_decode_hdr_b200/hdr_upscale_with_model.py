@@ -7,10 +7,12 @@ recombination all run in libhdrvae.so on the GPU (vae_decode_hdr_b200/csrc/upsca
 a CUDA device or without the library the node raises.
 
 Model loading stays what it is in ComfyUI (folder_paths + spandrel, :73-77); the node only reads
-`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Two architectures run: the 4x
-RRDBNet (ESRGAN: nf 64, gc 32) and Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x.  An RRDBNet of
-another scale fails before any GPU work; any other architecture is rejected by the library with an error naming the
-tensor that does not fit; a `descriptor.scale` that disagrees with the weights is an error too.
+`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Two architectures run: RRDBNet
+(ESRGAN: nf 64, gc 32) at 1x, 2x and 4x -- the plain form with 0, 1 or 2 upsampling convs and the pixel-unshuffle form
+(RealESRGAN_x2plus) -- and Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x.  An RRDBNet of another
+scale (8x), or one whose `descriptor.scale` disagrees with its weights, fails before any GPU work; any other architecture
+is rejected by the library with an error naming the tensor that does not fit; a Compact model whose `descriptor.scale`
+disagrees with its weights is an error too.
 """
 from __future__ import annotations
 
@@ -21,7 +23,7 @@ from typing import Any, Tuple
 
 import torch
 
-from .upscaler import UPSCALE_METHODS, HdrUpscalerEngine, is_compact_state_dict, reversal_for_architecture
+from .upscaler import UPSCALE_METHODS, HdrUpscalerEngine, is_compact_state_dict, reversal_for_architecture, rrdbnet_scale
 
 
 def _model_filenames():
@@ -85,10 +87,16 @@ class HDRUpscaleWithModel:
         """Packs the descriptor's weights; the engine's scale (read from the weights) must be `descriptor.scale`."""
         scale = getattr(descriptor, "scale", 4)
         sd = descriptor.model.state_dict()
-        if scale != 4 and not is_compact_state_dict(sd):
-            # the only RRDBNet form implemented is the 4x one: fail before any weights reach the GPU
-            raise RuntimeError(f"HDRUpscaleWithModel (B200) implements RRDBNet / ESRGAN at scale 4 only; this model has "
-                               f"scale {scale}")
+        if not is_compact_state_dict(sd):
+            # RRDBNet: the scale follows from the key layout, so both checks fail before any weights reach the GPU (an
+            # unrecognised layout goes on to the library, whose error names the tensor that does not fit)
+            weights = rrdbnet_scale(sd)
+            if weights is not None and weights not in (1, 2, 4):
+                raise RuntimeError(f"HDRUpscaleWithModel (B200) implements RRDBNet / ESRGAN at scales 1, 2 and 4; these "
+                                   f"weights upscale {weights}x (descriptor scale {scale})")
+            if weights is not None and weights != scale:
+                raise RuntimeError(f"HDRUpscaleWithModel (B200): the model descriptor gives scale {scale}, its weights "
+                                   f"are a {weights}x network")
         engine = HdrUpscalerEngine(sd, device)
         if engine.scale != scale:
             engine.close()

@@ -106,31 +106,33 @@ def synthetic_latent(b: int, h: int, w: int, seed: int = 1234) -> torch.Tensor:
     return torch.randn(b, Z, h, w, generator=g, dtype=torch.float32)
 
 
-def upscaler_param_shapes(nb: int = 23) -> List[Tuple[str, Tuple[int, ...]]]:
-    """RRDBNet (ESRGAN 4x: nf 64, gc 32) parameters in Real-ESRGAN key order."""
+def upscaler_param_shapes(nb: int = 23, n_up: int = 2, shuffle: int = 1) -> List[Tuple[str, Tuple[int, ...]]]:
+    """RRDBNet (ESRGAN: nf 64, gc 32) parameters in Real-ESRGAN key order: `n_up` upsampling convs, conv_first reading
+    3 shuffle^2 channels (the pixel-unshuffle form); the defaults are the 4x model."""
     out: List[Tuple[str, Tuple[int, ...]]] = []
 
     def conv(name, cout, cin):
         out.append((name + ".weight", (cout, cin, 3, 3)))
         out.append((name + ".bias", (cout,)))
-    conv("conv_first", 64, 3)
+    conv("conv_first", 64, 3 * shuffle * shuffle)
     for i in range(nb):
         for r in (1, 2, 3):
             for j in range(4):
                 conv(f"body.{i}.rdb{r}.conv{j + 1}", 32, 64 + 32 * j)
             conv(f"body.{i}.rdb{r}.conv5", 64, 192)
-    for name in ("conv_body", "conv_up1", "conv_up2", "conv_hr"):
+    for name in ["conv_body"] + [f"conv_up{k + 1}" for k in range(n_up)] + ["conv_hr"]:
         conv(name, 64, 64)
     conv("conv_last", 3, 64)
     return out
 
 
-def random_upscaler_state_dict(seed: int = 0, nb: int = 23) -> Dict[str, torch.Tensor]:
-    """PyTorch-default-style init of an RRDBNet (config C5: random-init ESRGAN), fp32, CPU."""
+def random_upscaler_state_dict(seed: int = 0, nb: int = 23, n_up: int = 2, shuffle: int = 1) -> Dict[str, torch.Tensor]:
+    """PyTorch-default-style init of an RRDBNet (config C5: random-init ESRGAN; `n_up` / `shuffle` as in
+    `upscaler_param_shapes`), fp32, CPU."""
     g = torch.Generator(device="cpu").manual_seed(seed)
     sd: Dict[str, torch.Tensor] = {}
     bound = 1.0
-    for name, shape in upscaler_param_shapes(nb):
+    for name, shape in upscaler_param_shapes(nb, n_up, shuffle):
         if len(shape) == 4:
             bound = 1.0 / math.sqrt(shape[1] * shape[2] * shape[3])
         sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * bound

@@ -3,6 +3,7 @@ device).  PyTorch is plumbing only (device memory, current stream); all arithmet
 from __future__ import annotations
 
 import ctypes as C
+import re
 from typing import Dict, Optional
 
 import torch
@@ -25,13 +26,39 @@ def reversal_for_architecture(name: str) -> str:
 
 def is_compact_state_dict(state_dict) -> bool:
     """The Real-ESRGAN Compact (SRVGGNetCompact) key layout, as the library recognises it: `body.0.weight` and no
-    `conv_first.*`.  Every other model the library runs is a 4x RRDBNet."""
+    `conv_first.*`.  Every other model the library runs is an RRDBNet (see `rrdbnet_scale`)."""
     return "body.0.weight" in state_dict and not any(k.startswith("conv_first.") for k in state_dict)
 
 
+_OLD_TOP = re.compile(r"model\.(\d+)\.(weight|bias)$")
+
+
+def rrdbnet_scale(state_dict) -> Optional[int]:
+    """Scale of an RRDBNet state dict by the library's rules, without a device: s = 2^u / f for u upsampling convs (old
+    arch: conv_last at top-level index 3u + 4; Real-ESRGAN names: conv_up1 / conv_up2 / conv_up3) and pixel-unshuffle
+    factor f (conv_first reads 3 f^2 channels).  8 for three upsampling convs; None for a layout the library does not
+    recognise (no conv_first, f not 1 / 2 / 4, s below 1, an old-arch conv_last index that fits no u)."""
+    tops = [int(m.group(1)) for m in (_OLD_TOP.match(k) for k in state_dict) if m and m.group(1) != "1"]
+    if tops:
+        top = max(tops)
+        if top < 4 or (top - 4) % 3:
+            return None
+        n_up, first = (top - 4) // 3, state_dict.get("model.0.weight")
+    else:
+        n_up = max([j for j in (1, 2, 3) if f"conv_up{j}.weight" in state_dict], default=0)
+        first = state_dict.get("conv_first.weight")
+    if n_up >= 3:
+        return 8
+    if first is None or len(first.shape) != 4 or first.shape[1] not in (3, 12, 48):
+        return None
+    f = {3: 1, 12: 2, 48: 4}[int(first.shape[1])]
+    return (1 << n_up) // f if (1 << n_up) >= f else None
+
+
 class HdrUpscalerEngine:
-    """One upscaler model packed for the tcgen05 conv kernel on one GPU: an RRDBNet (ESRGAN 4x: nf 64, gc 32) or a
-    Real-ESRGAN Compact (SRVGGNetCompact, PReLU, 1x / 2x / 4x).  `scale` is the model's, read from the library."""
+    """One upscaler model packed for the tcgen05 conv kernel on one GPU: an RRDBNet (ESRGAN: nf 64, gc 32; 0, 1 or 2
+    upsampling convs, pixel-unshuffle factor 1, 2 or 4, scale 1, 2 or 4) or a Real-ESRGAN Compact (SRVGGNetCompact,
+    PReLU, 1x / 2x / 4x).  `scale` is the model's, read from the library."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda"):
         self.lib = N.load_library()
