@@ -241,7 +241,7 @@ int hdrvae_rows_run_direct(hdrvae_rows* state, void* stream);
 /* After HDRVAE_EX_END: copy the statistics (global: pre/post/conv/pre3; local slab: out_*, pixel counts) and free. */
 int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
 
-/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for two of the
+/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for three of the
  * architectures spandrel loads from models/upscale_models (:73-77):
  *   - ESRGAN / RRDBNet (nf 64, gc 32, any block count) with u = 0, 1 or 2 upsampling convs (nearest 2x + conv) and
  *     pixel-unshuffle factor f = 1, 2 or 4 (conv_first reads 3 f^2 channels: RealESRGAN_x2plus has u 2, f 2), scale
@@ -249,17 +249,21 @@ int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
  *     tile side that is not a multiple of f is reflect-padded (the pad must be shorter than the side) and the output
  *     cropped, as spandrel does;
  *   - Real-ESRGAN Compact (SRVGGNetCompact with PReLU: realesr-general-x4v3, realesr-animevideov3, the 2x / 1x
- *     "compact" models): 3 input channels, nf a multiple of 8 in 8..64, any body depth, scale s = 1, 2 or 4.
- * The layout is recognised by its keys (Compact: body.0.weight and no conv_first); anything else is rejected with a
+ *     "compact" models): 3 input channels, nf a multiple of 8 in 8..64, any body depth, scale s = 1, 2 or 4;
+ *   - SPAN (spandrel's "SPAN"): 3 input channels, nf a multiple of 8 in 8..64, blocks block_1 .. block_6, any Conv3XC
+ *     hidden width, scale s = 1, 2 or 4, with or without the input normalisation (buffer no_norm).  Every Conv3XC is
+ *     fused from conv.0 / conv.1 / conv.2 and sk at load time, as its eval-mode forward does; eval_conv.* is ignored.
+ * The layout is recognised by its keys (Compact: body.0.weight and no conv_first; SPAN: conv_1.sk.weight); anything else is rejected with a
  * message naming the tensor and its shape.  The model object is created against a decode context (device, SM count,
  * conv implementation).  s below is the model's scale (hdrvae_upscaler_scale).
  *   load_weights : the model's state dict, host or device pointers.  RRDBNet in either key layout (Real-ESRGAN
  *                  "conv_first / body.N.rdbK.convJ / conv_body / conv_up1 / conv_up2 / conv_hr / conv_last" or
  *                  BasicSR-spandrel "model.0 / model.1.sub.N.RDBK.convJ.0 / ...", whose top-level convs sit at 0,
  *                  3 + 3k (upsampling conv k + 1), 3u + 2 (conv_hr) and 3u + 4 (conv_last)); Compact as
- *                  "body.0 / body.1 (PReLU) / ... / body.{2nc+2}";
- *   blocks       : RRDB blocks, or the Compact's body convs nc (0 allowed); < 0 without a model;
- *   scale        : 2^u / f for RRDBNet, s for Compact; < 0 before the weights are loaded;
+ *                  "body.0 / body.1 (PReLU) / ... / body.{2nc+2}"; SPAN as "conv_1 / block_K.cJ_r / conv_2" (each
+ *                  ".sk / .conv.0 / .conv.1 / .conv.2 / .eval_conv") / "conv_cat" / "upsampler.0" [/ "no_norm"];
+ *   blocks       : RRDB blocks, the Compact's body convs nc (0 allowed), or 6 (SPAN); < 0 without a model;
+ *   scale        : 2^u / f for RRDBNet, s for Compact and SPAN; < 0 before the weights are loaded;
  *   forward      : the network (+ reversal hook) on n equal tiles, x [n,h,w,3] -> y [n,s*h,s*w,3], float32 device
  *                  (kernel-level parity entry: what `upscale_model(a)` with the forward hook returns, :92-105; for
  *                  Compact that includes the nearest-upsampled input the network adds);

@@ -167,7 +167,7 @@ int run_conv(hdrvae_ctx* ctx, const PackedConv& pc, const ConvIO& io, int B, int
   p.k_per_tap = kpad;
   p.n_cols = pc.cout_pad;
   p.n_store = io.n_store > 0 ? io.n_store : (pc.cout_pad != pc.cout ? (pc.cout + 3) / 4 * 4 : 0);
-  p.res_scale = io.res_scale; p.lrelu = io.lrelu; p.act_slope = io.act_slope;
+  p.res_scale = io.res_scale; p.lrelu = io.lrelu; p.act_slope = io.act_slope; p.act = io.act;
   p.out_dtype = io.y_dtype;
   p.out_scale = io.y_scale;
   p.bias = io.bias != nullptr ? io.bias : pc.bias; p.bias_per_row = 0; p.res_dtype = io.res_dtype; p.alpha = io.alpha;

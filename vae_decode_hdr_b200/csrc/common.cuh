@@ -59,6 +59,7 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 enum { DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2,
        DT_F16X3 = 3 /* internal: fp16 [hi | lo | hi] K-concatenated operand of the "high" precision mode (groupnorm output) */ };
 __host__ __device__ inline int dt_bytes(int dt) { return dt == DT_F32 ? 4 : 2; }
+enum { ACT_NONE = 0, ACT_SILU = 1, ACT_GATE = 2 };   // GemmParams::act
 
 // out[n, y*sy+py, x*sx+px, col] = row_scale[x] * alpha * sum_{t<ntaps} sum_{c<K_per_tap}
 //        A[n, y+dy[t], x+dx[t], c] * Bw[col][t*K_per_tap + c]  + bias[col]  (+ residual[...])
@@ -111,6 +112,8 @@ struct GemmParams {
   const float* residual2;  // second fp32 residual, same addressing as out, added unscaled; or null
   float lrelu;       // LeakyReLU negative slope applied last (0: none)
   const float* act_slope;  // per-column PReLU negative slope, zero-padded to the GEMM's columns, applied last; or null
+  int act;           // ACT_SILU: y = t sigmoid(t), applied last; ACT_GATE: y = (t + r)(sigmoid(t) - 1/2) for t = alpha acc +
+                     // bias and r = res_scale * residual, in place of the residual add (SPAN); ACT_NONE: neither
   int n_store;       // columns actually stored (multiple of 4; 0: n_cols) — a Cout padded up to 32 stores less
   const float* row_scale;  // per M row (x coordinate) multiplier of the accumulator, or null
   float alpha;       // accumulator scale applied before bias (1.0 for convs)
@@ -186,6 +189,15 @@ __device__ __forceinline__ float silu_nr(float v) {
   r = r * fmaf(-d, r, 2.f);
   r = r * fmaf(-d, r, 2.f);
   return v * r;
+}
+// sigmoid(v) by silu_nr's steps (one XU operation): the conv epilogue's SiLU and SPAN gate
+__device__ __forceinline__ float sigmoid_nr(float v) {
+  float e;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(fminf(-v * 1.4426950408889634f, 80.f)));
+  const float d = 1.f + e;
+  float r = __int_as_float(0x7EF311C7 - __float_as_int(d));
+  r = r * fmaf(-d, r, 2.f);
+  return r * fmaf(-d, r, 2.f);
 }
 #endif
 

@@ -201,6 +201,7 @@ struct ConvIO {
   const float* residual2 = nullptr;
   float lrelu = 0.f;              // LeakyReLU slope (0: none)
   const float* act_slope = nullptr;       // per-channel PReLU slopes (cout_pad floats, zero-padded), or null
+  int act = ACT_NONE;             // ACT_SILU, or ACT_GATE: y = (t + residual)(sigmoid(t) - 1/2) (GemmParams::act)
   int n_store = 0;                // channels of y stored (multiple of 4; 0: all)
   // fused 1x1 conv of a second tensor (slab form): y += conv1x1(x2, *pc2); x2 has x's spatial shape / halo rows and
   // pc2->cin_pad channels per pixel (dense); `bias` replaces the conv's own bias when set

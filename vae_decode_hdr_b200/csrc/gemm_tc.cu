@@ -116,6 +116,8 @@ enum : int {
   EPI_RES2 = 128,    // + second fp32 residual (end of an RRDB: 0.04 acc + 0.2 x2 + x0)
   EPI_PRELU = 256,   // per-column PReLU applied last (Real-ESRGAN Compact convs)
   EPI_RES16 = 1024,  // + residual stored as a (scaled) 16-bit tensor of type res_dtype: t += res_scale * r
+  EPI_SILU = 2048,   // SiLU applied last (SPAN convs)
+  EPI_GATE = 4096,   // SPAN's attention gate in place of the residual add: (t + r) (sigmoid(t) - 1/2)
 };
 
 // XF builds (GroupNorm + SiLU applied to the activation slabs in place) carry two more warpgroups: 8 transform warps per
@@ -578,6 +580,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const bool has_lrelu = kGen ? (p.lrelu != 0.f) : ((EPI & EPI_LRELU) != 0);
     const bool has_res2 = kGen ? (p.residual2 != nullptr) : ((EPI & EPI_RES2) != 0);
     const bool has_prelu = kGen ? (p.act_slope != nullptr) : ((EPI & EPI_PRELU) != 0);
+    const bool has_silu = kGen ? (p.act == ACT_SILU) : ((EPI & EPI_SILU) != 0);
+    const bool has_gate = kGen ? (p.act == ACT_GATE) : ((EPI & EPI_GATE) != 0);
     const float lrelu = p.lrelu, res_scale = p.res_scale;
     const int n_store = p.n_store > 0 ? p.n_store : p.n_cols;
     const int q = warp & 3;                 // TMEM lane quarter this warp may access
@@ -705,6 +709,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             for (int it = 0; it < 8; ++it) {
               float2 t01 = f2_fma(make_float2(a[it].x, a[it].y), alpha2, b01);
               float2 t23 = f2_fma(make_float2(a[it].z, a[it].w), alpha2, b23);
+              float2 g01, g23;                           // the gate's factor, from t before the residual
+              if constexpr ((EPI & EPI_GATE) != 0) {
+                g01 = make_float2(sigmoid_nr(t01.x) - 0.5f, sigmoid_nr(t01.y) - 0.5f);
+                g23 = make_float2(sigmoid_nr(t23.x) - 0.5f, sigmoid_nr(t23.y) - 0.5f);
+              }
               if constexpr ((EPI & EPI_RES) != 0) {
                 t01 = f2_fma(make_float2(rr[it].x, rr[it].y), rs2, t01);
                 t23 = f2_fma(make_float2(rr[it].z, rr[it].w), rs2, t23);
@@ -732,6 +741,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               if constexpr ((EPI & EPI_PRELU) != 0) {
                 t01.x = t01.x < 0.f ? t01.x * slope4.x : t01.x; t01.y = t01.y < 0.f ? t01.y * slope4.y : t01.y;
                 t23.x = t23.x < 0.f ? t23.x * slope4.z : t23.x; t23.y = t23.y < 0.f ? t23.y * slope4.w : t23.y;
+              }
+              if constexpr ((EPI & EPI_SILU) != 0) {
+                t01 = f2_mul(t01, make_float2(sigmoid_nr(t01.x), sigmoid_nr(t01.y)));
+                t23 = f2_mul(t23, make_float2(sigmoid_nr(t23.x), sigmoid_nr(t23.y)));
+              }
+              if constexpr ((EPI & EPI_GATE) != 0) {
+                t01 = f2_mul(t01, g01);
+                t23 = f2_mul(t23, g23);
               }
               if constexpr ((EPI & EPI_OUT2) != 0) {
                 const float2 u01 = f2_mul(t01, s2_2), u23 = f2_mul(t23, s2_2);
@@ -891,6 +908,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           }
           t.x = fmaf(t.x, scale, bias4.x); t.y = fmaf(t.y, scale, bias4.y);
           t.z = fmaf(t.z, scale, bias4.z); t.w = fmaf(t.w, scale, bias4.w);
+          float4 g;                                       // the gate's factor, from t before the residual
+          if (has_gate) g = make_float4(sigmoid_nr(t.x) - 0.5f, sigmoid_nr(t.y) - 0.5f, sigmoid_nr(t.z) - 0.5f, sigmoid_nr(t.w) - 0.5f);
           if (has_res_f32) {
             t.x = fmaf(rres[it].x, res_scale, t.x); t.y = fmaf(rres[it].y, res_scale, t.y);
             t.z = fmaf(rres[it].z, res_scale, t.z); t.w = fmaf(rres[it].w, res_scale, t.w);
@@ -918,6 +937,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             t.x = t.x < 0.f ? t.x * slope4.x : t.x; t.y = t.y < 0.f ? t.y * slope4.y : t.y;
             t.z = t.z < 0.f ? t.z * slope4.z : t.z; t.w = t.w < 0.f ? t.w * slope4.w : t.w;
           }
+          if (has_silu) {
+            t.x *= sigmoid_nr(t.x); t.y *= sigmoid_nr(t.y); t.z *= sigmoid_nr(t.z); t.w *= sigmoid_nr(t.w);
+          }
+          if (has_gate) { t.x *= g.x; t.y *= g.y; t.z *= g.z; t.w *= g.w; }
           if (has_out2) {
             // second, scaled 16-bit copy of the output: the tensor-core operand of a conv that consumes this
             // (un-normalised) tensor directly; the power-of-two scale keeps fp16 far from overflow
@@ -1151,7 +1174,8 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
     if (use_cg == 2 && !p.round_tf32 && p.stats == nullptr && !p.bias_per_row && p.row_scale == nullptr &&
         (p.residual == nullptr || p.res_dtype == DT_F32)) {
       epi = (p.out_dtype != DT_F32 ? EPI_OUT16 : 0) | (p.residual ? EPI_RES : 0) | (p.residual2 ? EPI_RES2 : 0) |
-            (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0) | (p.act_slope ? EPI_PRELU : 0);
+            (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0) | (p.act_slope ? EPI_PRELU : 0) |
+            (p.act == ACT_SILU ? EPI_SILU : 0) | (p.act == ACT_GATE ? EPI_GATE : 0);
     }
     if (p.slab) {
       HDRVAE_REQUIRE(p.ntaps == 9 && p.TW == 8 && p.TH == 16,
@@ -1164,6 +1188,10 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
         }
         if (epi == (EPI_OUT16 | EPI_LRELU)) return launch_tc<64, false, 2, EPI_OUT16 | EPI_LRELU, 9>(p, num_sms, stream);
         if (epi == (EPI_OUT16 | EPI_PRELU)) return launch_tc<64, false, 2, EPI_OUT16 | EPI_PRELU, 9>(p, num_sms, stream);
+        // SPAN's 48 / 64-channel convs: c1_r / c2_r with SiLU; c3_r with the gate on the fp32 block stream, which also
+        // writes the fp16 operand copy of the block output
+        if (epi == (EPI_OUT16 | EPI_SILU)) return launch_tc<64, false, 2, EPI_OUT16 | EPI_SILU, 9>(p, num_sms, stream);
+        if (epi == (EPI_RES | EPI_GATE | EPI_OUT2)) return launch_tc<64, false, 2, EPI_RES | EPI_GATE | EPI_OUT2, 9>(p, num_sms, stream);
         if (epi == (EPI_RES | EPI_OUT2)) return launch_tc<64, false, 2, EPI_RES | EPI_OUT2, 9>(p, num_sms, stream);
         if (epi == (EPI_RES | EPI_RES2 | EPI_OUT2)) return launch_tc<64, false, 2, EPI_RES | EPI_RES2 | EPI_OUT2, 9>(p, num_sms, stream);
         if (epi == EPI_OUT2) return launch_tc<64, false, 2, EPI_OUT2, 9>(p, num_sms, stream);
@@ -1187,7 +1215,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
                        : launch_tc<64, false, 1, EPI_GENERIC>(p, num_sms, stream);
   }
   const bool res16 = p.residual != nullptr && p.res_dtype != DT_F32;
-  if (use_cg == 2 && !tf32 && p.lrelu == 0.f && p.act_slope == nullptr && p.residual2 == nullptr && (p.res_scale == 0.f || p.res_scale == 1.f || res16)) {
+  if (use_cg == 2 && !tf32 && p.lrelu == 0.f && p.act_slope == nullptr && p.act == ACT_NONE && p.residual2 == nullptr && (p.res_scale == 0.f || p.res_scale == 1.f || res16)) {
     // specialised epilogues for what the decoder launches; anything else takes the generic build
     int epi = 0;
     const bool simple_res = p.residual == nullptr || p.res_dtype == DT_F32;

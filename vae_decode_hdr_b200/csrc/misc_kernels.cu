@@ -202,12 +202,15 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
     }
     float v = acc * p.alpha * (p.row_scale != nullptr ? p.row_scale[x] : 1.f);
     if (p.bias != nullptr) v += p.bias_per_row ? p.bias[x] : p.bias[col];
+    const float gate = p.act == ACT_GATE ? 1.f / (1.f + expf(-v)) - 0.5f : 0.f;    // from t before the residual
     const long long off = (long long)img * p.out_img_stride + (long long)(y * p.sy + p.py) * p.out_row_stride +
                           (long long)(x * p.sx + p.px) * p.out_px_stride + col;
     if (p.residual != nullptr) v += (p.res_scale != 0.f ? p.res_scale : 1.f) * load_as(p.residual, off, p.res_dtype);
     if (p.residual2 != nullptr) v += p.residual2[off];
     if (p.lrelu != 0.f && v < 0.f) v *= p.lrelu;
     if (p.act_slope != nullptr && v < 0.f) v *= p.act_slope[col];
+    if (p.act == ACT_SILU) v *= 1.f / (1.f + expf(-v));
+    if (p.act == ACT_GATE) v *= gate;
     if (p.n_store > 0 && col >= p.n_store) continue;
     if (p.out2 != nullptr) {
       const long long off2 = p.out2_px_stride == 0 ? off

@@ -1,6 +1,6 @@
 // HDR upscaler path: replaces HDRUpscaleWithModel.upscale of the reference
 // (/root/reference/hdr_upscale_with_model.py:148-263): two passes of the model (ESRGAN / RRDBNet at 1x, 2x or 4x, or
-// Real-ESRGAN Compact at 1x, 2x or 4x) through overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output
+// Real-ESRGAN Compact or SPAN at 1x, 2x or 4x) through overlapping 512-pixel tiles with the atanh / logit reversal hook on every tile output
 // (:79-107, :110-146), feather blending (restated comfy.utils.tiled_scale), then the luma / chroma recombination in YCbCr
 // with a 3x3 median on Y (:187-224) and the optional local hot-spot fix (:229-258).  Everything after the model reads
 // the float4 tile-output layout [n][s h][s w] that both forwards leave, with the model's scale s.
@@ -19,6 +19,9 @@
 // The Compact convs (SRVGGNetCompact: conv, PReLU, ..., conv to 3 s^2 channels) run on the same kernel with the
 // per-channel PReLU in the epilogue; up_shuffle_base_kernel then applies the pixel shuffle and adds the nearest-upsampled
 // fp32 input (the network's base).
+// SPAN (conv_1, six SPAB blocks, conv_2, conv_cat, upsampler.0) runs on the same kernel too: every Conv3XC is fused into
+// one 3x3 conv at load time, SiLU and SPAN's attention gate are epilogue operations, and the four tensors conv_cat reads
+// are channel slices of one fp16 buffer, so that conv_cat is a plain 1x1 conv (up_forward_span).
 // Everything after the model (hook, feather blend, YCbCr, median, local fix) is elementwise / stencil work in
 // fp32 with the reference's operation order (no FMA contraction) so that it is bit-comparable to the oracle.
 #include <string.h>
@@ -37,13 +40,14 @@ namespace hdrvae {
 __host__ __device__ constexpr int up_in_channels(int f) { return f == 1 ? 8 : f == 2 ? 16 : 48; }
 
 // image fp32 BHWC (3 channels) -> fp16 network input [n][h'][w'][up_in_channels(F)] of tiles of h x w at the origins of
-// `tiles`, h' = ceil(h / F): clamp to [-1, 1] (flag or tile table .w), reflect pad of the tile's bottom / right edge to
+// `tiles`, h' = ceil(h / F): clamp to [-1, 1] (flag or tile table .w), minus `mean` (SPAN's normalisation; zero for the
+// other models, where it leaves every value as it is), reflect pad of the tile's bottom / right edge to
 // F h' x F w' (torch "reflect": row h + k reads row h - 2 - k), pixel unshuffle by F (channel c F^2 + i F + j = channel c
 // at pixel (y F + i, x F + j)), channels beyond 3 F^2 zero.  The clamp is elementwise, so it commutes with pad and
 // unshuffle.  F = 1 is the plain [n][h][w][8] copy.
 template <int F>
 __global__ void up_extract_tiles_kernel(const float* __restrict__ img, int H, int W, const int4* __restrict__ tiles /*b,y0,x0,_*/,
-                                        int n, int h, int w, int clamp1, uint4* __restrict__ out) {
+                                        int n, int h, int w, int clamp1, float3 mean, uint4* __restrict__ out) {
   constexpr int CX = up_in_channels(F), F2 = F * F;
   const int hq = (h + F - 1) / F, wq = (w + F - 1) / F;
   const long long total = (long long)n * hq * wq;
@@ -66,6 +70,7 @@ __global__ void up_extract_tiles_kernel(const float* __restrict__ img, int H, in
         const float* src = img + (((long long)tl.x * H + tl.y + yy) * W + tl.z + xx) * 3;
         float r = src[0], g = src[1], bl = src[2];
         if (clamp1 || tl.w) { r = fminf(fmaxf(r, -1.f), 1.f); g = fminf(fmaxf(g, -1.f), 1.f); bl = fminf(fmaxf(bl, -1.f), 1.f); }
+        r = __fsub_rn(r, mean.x); g = __fsub_rn(g, mean.y); bl = __fsub_rn(bl, mean.z);
         v[a * F + b] = __float2half_rn(r);
         v[F2 + a * F + b] = __float2half_rn(g);
         v[2 * F2 + a * F + b] = __float2half_rn(bl);
@@ -107,7 +112,8 @@ __device__ __forceinline__ float up_reversal(float v, int kind) {
 // Compact tail: y = pixel_shuffle(conv, s) + nearest_upsample(x, s).  conv is the last conv's fp32 output [n][h][w][cl]
 // (channel c s^2 + i s + j of input pixel (y, x) -> channel c of output pixel (y s + i, x s + j)); the base is the tile's
 // fp32 input pixel, clamped to [-1, 1] for the second pass's tiles (tile table .w) like the network's own input.  Writes
-// the float4 [n][s h][s w] tile-output layout of the RRDBNet forward (.w = 0).
+// the float4 [n][s h][s w] tile-output layout of the RRDBNet forward (.w = 0).  img == null: the plain pixel shuffle
+// (SPAN, which adds no base).
 __global__ void up_shuffle_base_kernel(const float* __restrict__ conv, int cl, const float* __restrict__ img, int H, int W,
                                        const int4* __restrict__ tiles, int n, int h, int w, int s, float4* __restrict__ out) {
   const int OH = h * s, OW = w * s, s2 = s * s;
@@ -117,11 +123,15 @@ __global__ void up_shuffle_base_kernel(const float* __restrict__ conv, int cl, c
     const int Y = (int)((i / OW) % OH);
     const int t = (int)(i / ((long long)OW * OH));
     const int y = Y / s, x = X / s;
+    const float* c = conv + (((long long)t * h + y) * w + x) * cl + (Y - y * s) * s + (X - x * s);
+    if (img == nullptr) {
+      out[i] = make_float4(c[0], c[s2], c[2 * s2], 0.f);
+      continue;
+    }
     const int4 tl = tiles[t];                     // image, y0, x0, clamp flag
     const float* src = img + (((long long)tl.x * H + tl.y + y) * W + tl.z + x) * 3;
     float r = src[0], g = src[1], b = src[2];
     if (tl.w) { r = fminf(fmaxf(r, -1.f), 1.f); g = fminf(fmaxf(g, -1.f), 1.f); b = fminf(fmaxf(b, -1.f), 1.f); }
-    const float* c = conv + (((long long)t * h + y) * w + x) * cl + (Y - y * s) * s + (X - x * s);
     out[i] = make_float4(__fadd_rn(c[0], r), __fadd_rn(c[s2], g), __fadd_rn(c[2 * s2], b), 0.f);
   }
 }
@@ -350,14 +360,17 @@ struct hdrvae_upscaler {
   hdrvae_ctx* ctx = nullptr;      // device / SM count / conv implementation come from the decode context
   hdrvae_ctx store;               // owns this model's device allocations
   bool loaded = false;
-  bool compact = false;           // Real-ESRGAN SRVGGNetCompact; else ESRGAN / RRDBNet
+  bool compact = false;           // Real-ESRGAN SRVGGNetCompact
+  bool span = false;              // SPAN; neither: ESRGAN / RRDBNet
+  float3 mean = {0.f, 0.f, 0.f};  // subtracted from the network input (SPAN's normalisation; its 255 is in conv_1's weights)
   int scale = 4;                  // output pixels per input pixel along each axis (RRDBNet: 2^n_up / shuffle)
-  int nb = 0;                     // RRDB blocks (RRDBNet) or body convs (Compact)
+  int nb = 0;                     // RRDB blocks (RRDBNet), body convs (Compact) or SPAB blocks (SPAN: 6)
   int n_up = 2;                   // RRDBNet: nearest-2x + conv upsampling stages (0, 1 or 2)
   int shuffle = 1;                // RRDBNet: pixel-unshuffle factor of the input (1, 2 or 4; conv_first reads 3 f^2 channels)
   PackedConv conv_first, conv_body, up1, up2, hr, last;
   std::vector<UpRdb> rdb;         // 3 per RRDB
-  std::vector<PackedConv> body;   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2)
+  std::vector<PackedConv> body;   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2); SPAN: the fused conv_1,
+                                  // block_k.c{1,2,3}_r (k = 1..6), conv_2, then conv_cat (1x1, 4 nf -> nf) and upsampler.0
   std::vector<float*> slopes;     // Compact: PReLU slopes applied after body[k], k <= nb (cout_pad floats, zero-padded)
 };
 
@@ -382,7 +395,8 @@ static int up_check_sides(const hdrvae_upscaler* up, int h, int w) {
 
 struct UpPlan {                   // workspace of one forward over n tiles of h x w
   size_t img8, cat0, cat1, f_feat, f_a, f_b, f_c, u0, u1, u2, u3;   // RRDBNet
-  size_t act0, act1, last;                                          // Compact
+  size_t act0, act1, last;                                          // Compact (SPAN: last)
+  size_t sp_r0, sp_r1, sp_d, sp_t0, sp_t1, sp_cat;                  // SPAN
   size_t total;
 };
 static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
@@ -396,6 +410,18 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
     const size_t cp = (size_t)up->body[0].cout_pad;
     pl.act0 = take(P * cp * 2);
     pl.act1 = take(P * cp * 2);
+    pl.last = take(P * up_last_channels(up) * 4);
+    pl.total = off;
+    return pl;
+  }
+  if (up->span) {
+    const size_t nf = (size_t)up->body[0].cout;
+    pl.sp_r0 = take(P * nf * 4);      // fp32 block stream (the gate's residual), ping-pong
+    pl.sp_r1 = take(P * nf * 4);
+    pl.sp_d = take(P * nf * 2);       // fp16 operand copy of a block output
+    pl.sp_t0 = take(P * nf * 2);      // SiLU'd c1_r / c2_r outputs
+    pl.sp_t1 = take(P * nf * 2);
+    pl.sp_cat = take(P * 4 * nf * 2); // [f | b6 | b1 | b5_2]: conv_cat's input, the channel order of torch.cat
     pl.last = take(P * up_last_channels(up) * 4);
     pl.total = off;
     return pl;
@@ -521,6 +547,62 @@ static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t*
   return 0;
 }
 
+// SPAN forward on n tiles (fp16 [n][h][w][8] x - mean in pl.img8) -> upsampler.0's fp32 [n][h][w][up_last_channels] in
+// pl.last.  Every conv is one launch of the conv kernel; conv_1 carries the normalisation's 255 in its weights.  The
+// four tensors conv_cat reads are written straight into their channel slices of one fp16 buffer (conv_1 and block_1's
+// c3_r as their fp16 operand copy, block_6's c1_r and conv_2 as their output), and the convs that read a slice (block_1,
+// block_2, block_6's c2_r) address it through the A operand's base pointer at the slice's first channel with the
+// buffer's pixel stride.  The block stream x, which the gate adds, stays fp32.
+static int up_forward_span(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, cudaStream_t s) {
+  hdrvae_ctx* ctx = up->ctx;
+  const int impl = ctx->conv_impl;
+  const int nf = up->body[0].cout, c4 = 4 * nf;
+  uint16_t* cat = reinterpret_cast<uint16_t*>(ws + pl.sp_cat);
+  float* r[2] = {reinterpret_cast<float*>(ws + pl.sp_r0), reinterpret_cast<float*>(ws + pl.sp_r1)};
+  uint8_t* d = ws + pl.sp_d;
+  uint8_t* t[2] = {ws + pl.sp_t0, ws + pl.sp_t1};
+  {
+    ConvIO io; io.x = ws + pl.img8; io.x_channels = 8; io.y = r[0]; io.y_dtype = DT_F32; io.y_channels = nf;
+    io.y2 = cat; io.y2_channels = c4; io.y2_chan_off = 0;                                   // f
+    HDRVAE_TRY(run_conv(ctx, up->body[0], io, n, h, w, impl, s));
+  }
+  const void* xin = cat;                  // the block input's fp16 operand and its pixel stride
+  int xch = c4, cur = 0;
+  for (int b = 0; b < 6; ++b) {
+    const PackedConv* c = &up->body[1 + 3 * b];
+    {
+      ConvIO io; io.x = xin; io.x_channels = xch; io.y_dtype = DT_F16; io.act = ACT_SILU;
+      if (b == 5) { io.y = cat; io.y_channels = c4; io.y_chan_off = 3 * nf; }           // b5_2: block_6's SiLU'd out1
+      else { io.y = t[0]; io.y_channels = nf; }
+      HDRVAE_TRY(run_conv(ctx, c[0], io, n, h, w, impl, s));
+    }
+    {
+      ConvIO io; io.x = b == 5 ? static_cast<const void*>(cat + 3 * nf) : t[0]; io.x_channels = b == 5 ? c4 : nf;
+      io.y = t[1]; io.y_dtype = DT_F16; io.y_channels = nf; io.act = ACT_SILU;
+      HDRVAE_TRY(run_conv(ctx, c[1], io, n, h, w, impl, s));
+    }
+    {
+      // out = (c3_r + x)(sigmoid(c3_r) - 1/2) into the other fp32 stream buffer, its fp16 copy for the next conv
+      ConvIO io; io.x = t[1]; io.x_channels = nf; io.y = r[cur ^ 1]; io.y_dtype = DT_F32; io.y_channels = nf;
+      io.residual = r[cur]; io.res_dtype = DT_F32; io.act = ACT_GATE;
+      if (b == 0) { io.y2 = cat; io.y2_channels = c4; io.y2_chan_off = 2 * nf; xin = cat + 2 * nf; xch = c4; }   // b1
+      else { io.y2 = d; io.y2_channels = nf; xin = d; xch = nf; }
+      HDRVAE_TRY(run_conv(ctx, c[2], io, n, h, w, impl, s));
+      cur ^= 1;
+    }
+  }
+  {
+    ConvIO io; io.x = d; io.x_channels = nf; io.y = cat; io.y_dtype = DT_F16; io.y_channels = c4; io.y_chan_off = nf;   // b6
+    HDRVAE_TRY(run_conv(ctx, up->body[19], io, n, h, w, impl, s));
+  }
+  {
+    ConvIO io; io.x = cat; io.x_channels = c4; io.y = t[0]; io.y_dtype = DT_F16; io.y_channels = nf;
+    HDRVAE_TRY(run_conv(ctx, up->body[20], io, n, h, w, impl, s));
+  }
+  ConvIO io; io.x = t[0]; io.x_channels = nf; io.y = ws + pl.last; io.y_dtype = DT_F32; io.y_channels = up_last_channels(up);
+  return run_conv(ctx, up->body[21], io, n, h, w, impl, s);
+}
+
 // The network on n tiles of h x w cut from img [.][H][W][3] at the origins of `tiles` (image, y0, x0, clamp to [-1, 1])
 // -> fp32 [n][s h][s w][4] at out4
 static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, const int4* tiles, int n, int h, int w,
@@ -530,18 +612,23 @@ static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, con
     const long long npx = (long long)n * up_net_side(up, h) * up_net_side(up, w);
     ProfScope prof("upscaler extract tiles", 0.0, (double)npx * (f * f * 12 + up_in_channels(f) * 2), s);
     uint4* x = reinterpret_cast<uint4*>(ws + pl.img8);
-    if (f == 1) up_extract_tiles_kernel<1><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
-    else if (f == 2) up_extract_tiles_kernel<2><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
-    else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, x);
+    const float3 m = up->mean;
+    if (f == 1) up_extract_tiles_kernel<1><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
+    else if (f == 2) up_extract_tiles_kernel<2><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
+    else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
     HDRVAE_LAUNCHED();
   }
-  if (!up->compact) return up_forward(up, n, h, w, ws, pl, out4, s);
-  HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s));
+  if (!up->compact && !up->span) return up_forward(up, n, h, w, ws, pl, out4, s);
+  if (up->compact) HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s));
+  else HDRVAE_TRY(up_forward_span(up, n, h, w, ws, pl, s));
   const int sc = up->scale, cl = up_last_channels(up);
   const long long opx = (long long)n * sc * sc * h * w;
-  ProfScope prof("upscaler pixel shuffle + base", 0.0, (double)n * h * w * (cl * 4 + 12) + opx * 16, s);
-  up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float*>(ws + pl.last), cl, img, H, W, tiles, n, h, w,
-                                                      sc, reinterpret_cast<float4*>(out4));
+  // SPAN adds no base: the plain shuffle
+  ProfScope prof(up->compact ? "upscaler pixel shuffle + base" : "upscaler pixel shuffle",
+                 0.0, (double)n * h * w * (cl * 4 + (up->compact ? 12 : 0)) + opx * 16, s);
+  up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float*>(ws + pl.last), cl,
+                                                      up->compact ? img : nullptr, H, W, tiles, n, h, w, sc,
+                                                      reinterpret_cast<float4*>(out4));
   HDRVAE_LAUNCHED();
   return 0;
 }
@@ -778,6 +865,131 @@ static int up_pack_compact(hdrvae_upscaler* up, cudaStream_t s) {
   return 0;
 }
 
+// SPAN (spandrel's "SPAN"; hongyuanyu/SPAN) as spandrel loads it: conv_1, block_1 .. block_6 (c1_r, c2_r, c3_r), conv_2 —
+// each a Conv3XC — then conv_cat (1x1, 4 nf -> nf) and upsampler.0 (3x3, nf -> 3 s^2, then the pixel shuffle); the
+// buffer no_norm switches the input normalisation (x - mean) 255 off.  A Conv3XC in eval mode rebuilds eval_conv from
+// sk (1x1, cin -> cout), conv.0 (1x1, cin -> m1), conv.1 (3x3, m1 -> m2) and conv.2 (1x1, m2 -> cout) on every forward
+// and runs eval_conv with zero padding 1; the stored eval_conv.* may be stale, so the same fusion happens here, in fp64:
+//   W = w3 . w2 . w1 (+ sk at the centre tap),  b = w3 (sum_{m1,taps} w2 b1 + b2) + b3 + b_sk.
+static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
+  hdrvae_ctx* st = &up->store;
+  auto shape_str = [&](const std::string& k) {
+    auto it = st->shapes.find(k);
+    return it == st->shapes.end() ? std::string("(missing)") : up_shape_str(it->second);
+  };
+  // the tensor k with shape `want` (its shape and the wanted one in the error)
+  auto need = [&](const std::string& k, const std::vector<int64_t>& want) -> int {
+    auto it = st->shapes.find(k);
+    HDRVAE_REQUIRE(it != st->shapes.end(), "SPAN upscaler state dict lacks %s (want shape %s)", k.c_str(), up_shape_str(want).c_str());
+    HDRVAE_REQUIRE(it->second == want, "SPAN upscaler: %s has shape %s; want %s", k.c_str(), up_shape_str(it->second).c_str(),
+                   up_shape_str(want).c_str());
+    return 0;
+  };
+  auto host = [&](const std::string& k, std::vector<double>* out) -> int {
+    size_t cnt = 1;
+    for (int64_t d : st->shapes[k]) cnt *= (size_t)d;
+    std::vector<float> f(cnt);
+    HDRVAE_CUDA_OK(cudaMemcpy(f.data(), st->raw[k], cnt * sizeof(float), cudaMemcpyDeviceToHost));
+    out->assign(f.begin(), f.end());
+    return 0;
+  };
+  const std::vector<int64_t>& w0 = st->shapes["conv_1.sk.weight"];
+  HDRVAE_REQUIRE(w0.size() == 4 && w0[1] == 3 && w0[2] == 1 && w0[3] == 1,
+                 "SPAN upscaler: conv_1.sk.weight has shape %s; want [nf,3,1,1] (3 input channels)", up_shape_str(w0).c_str());
+  const int nf = (int)w0[0];
+  HDRVAE_REQUIRE(nf >= 8 && nf <= 64 && nf % 8 == 0,
+                 "SPAN upscaler: conv_1.sk.weight has shape %s; nf must be a multiple of 8 in 8..64", up_shape_str(w0).c_str());
+  for (const auto& kv : st->shapes) {
+    int bi = -1;
+    HDRVAE_REQUIRE(sscanf(kv.first.c_str(), "block_%d.", &bi) != 1 || (bi >= 1 && bi <= 6),
+                   "SPAN upscaler: %s has shape %s; SPAN has exactly the blocks block_1 .. block_6", kv.first.c_str(),
+                   up_shape_str(kv.second).c_str());
+  }
+  {
+    const std::vector<int64_t>* wu = st->shapes.count("upsampler.0.weight") ? &st->shapes["upsampler.0.weight"] : nullptr;
+    HDRVAE_REQUIRE(wu != nullptr && wu->size() == 4 && (*wu)[1] == nf && (*wu)[2] == 3 && (*wu)[3] == 3 &&
+                   ((*wu)[0] == 3 || (*wu)[0] == 12 || (*wu)[0] == 48),
+                   "SPAN upscaler: upsampler.0.weight has shape %s; want [3*scale^2,%d,3,3] with scale 1, 2 or 4",
+                   shape_str("upsampler.0.weight").c_str(), nf);
+    up->scale = (*wu)[0] == 3 ? 1 : (*wu)[0] == 12 ? 2 : 4;
+  }
+  const bool norm = st->shapes.count("no_norm") == 0;
+  // Conv3XC `pre` (cin -> cout) fused into one 3x3 conv, packed with its weights scaled by wscale
+  auto conv3xc = [&](const std::string& pre, int cin, int cout, float wscale, PackedConv* pc) -> int {
+    auto it = st->shapes.find(pre + ".conv.0.weight");
+    const int m1 = it != st->shapes.end() && it->second.size() == 4 ? (int)it->second[0] : 0;
+    it = st->shapes.find(pre + ".conv.1.weight");
+    const int m2 = it != st->shapes.end() && it->second.size() == 4 ? (int)it->second[0] : 0;
+    HDRVAE_REQUIRE(m1 >= 1 && m2 >= 1, "SPAN upscaler: %s.conv.0.weight has shape %s and %s.conv.1.weight %s; want [m1,%d,1,1] "
+                   "and [m2,m1,3,3]", pre.c_str(), shape_str(pre + ".conv.0.weight").c_str(), pre.c_str(),
+                   shape_str(pre + ".conv.1.weight").c_str(), cin);
+    HDRVAE_TRY(need(pre + ".sk.weight", {cout, cin, 1, 1}));
+    HDRVAE_TRY(need(pre + ".sk.bias", {cout}));
+    HDRVAE_TRY(need(pre + ".conv.0.weight", {m1, cin, 1, 1}));
+    HDRVAE_TRY(need(pre + ".conv.0.bias", {m1}));
+    HDRVAE_TRY(need(pre + ".conv.1.weight", {m2, m1, 3, 3}));
+    HDRVAE_TRY(need(pre + ".conv.1.bias", {m2}));
+    HDRVAE_TRY(need(pre + ".conv.2.weight", {cout, m2, 1, 1}));
+    HDRVAE_TRY(need(pre + ".conv.2.bias", {cout}));
+    std::vector<double> sk, skb, w1, b1, w2, b2, w3, b3;
+    HDRVAE_TRY(host(pre + ".sk.weight", &sk)); HDRVAE_TRY(host(pre + ".sk.bias", &skb));
+    HDRVAE_TRY(host(pre + ".conv.0.weight", &w1)); HDRVAE_TRY(host(pre + ".conv.0.bias", &b1));
+    HDRVAE_TRY(host(pre + ".conv.1.weight", &w2)); HDRVAE_TRY(host(pre + ".conv.1.bias", &b2));
+    HDRVAE_TRY(host(pre + ".conv.2.weight", &w3)); HDRVAE_TRY(host(pre + ".conv.2.bias", &b3));
+    // a[m2][i][tap] = sum_m1 w2[m2][m1][tap] w1[m1][i];  bm[m2] = sum_{m1,tap} w2[m2][m1][tap] b1[m1] + b2[m2]
+    std::vector<double> a((size_t)m2 * cin * 9, 0.0), bm(m2);
+    for (int o = 0; o < m2; ++o) {
+      double acc = b2[o];
+      for (int j = 0; j < m1; ++j)
+        for (int k = 0; k < 9; ++k) {
+          const double v = w2[((size_t)o * m1 + j) * 9 + k];
+          acc += v * b1[j];
+          for (int i = 0; i < cin; ++i) a[((size_t)o * cin + i) * 9 + k] += v * w1[(size_t)j * cin + i];
+        }
+      bm[o] = acc;
+    }
+    std::vector<float> wf((size_t)cout * cin * 9), bf(cout);
+    for (int o = 0; o < cout; ++o) {
+      double acc = b3[o] + skb[o];
+      for (int m = 0; m < m2; ++m) acc += w3[(size_t)o * m2 + m] * bm[m];
+      bf[o] = (float)acc;
+      for (int i = 0; i < cin; ++i)
+        for (int k = 0; k < 9; ++k) {
+          double v = k == 4 ? sk[(size_t)o * cin + i] : 0.0;
+          for (int m = 0; m < m2; ++m) v += w3[(size_t)o * m2 + m] * a[((size_t)m * cin + i) * 9 + k];
+          wf[((size_t)o * cin + i) * 9 + k] = (float)v;
+        }
+    }
+    // device copies under the fp32 state-dict map, so that up_finish_load frees them with the rest
+    float *dw = nullptr, *db = nullptr;
+    HDRVAE_TRY(dev_alloc(st, wf.size() * sizeof(float), (void**)&dw));
+    HDRVAE_TRY(dev_alloc(st, bf.size() * sizeof(float), (void**)&db));
+    st->raw[pre + ".fused.weight"] = dw;
+    st->raw[pre + ".fused.bias"] = db;
+    HDRVAE_CUDA_OK(cudaMemcpy(dw, wf.data(), wf.size() * sizeof(float), cudaMemcpyHostToDevice));
+    HDRVAE_CUDA_OK(cudaMemcpy(db, bf.data(), bf.size() * sizeof(float), cudaMemcpyHostToDevice));
+    return pack_conv(st, dw, db, cout, cin, 3, false, wscale, DT_F16, pc, s);
+  };
+  up->body.resize(22);
+  // (x - mean) 255: the input stage subtracts the mean, conv_1's weights carry the 255 (its bias is not scaled)
+  HDRVAE_TRY(conv3xc("conv_1", 3, nf, norm ? 255.f : 1.f, &up->body[0]));
+  for (int b = 0; b < 6; ++b)
+    for (int c = 0; c < 3; ++c)
+      HDRVAE_TRY(conv3xc("block_" + std::to_string(b + 1) + ".c" + std::to_string(c + 1) + "_r", nf, nf, 1.f,
+                         &up->body[1 + 3 * b + c]));
+  HDRVAE_TRY(conv3xc("conv_2", nf, nf, 1.f, &up->body[19]));
+  HDRVAE_TRY(need("conv_cat.weight", {nf, 4 * nf, 1, 1}));
+  HDRVAE_TRY(need("conv_cat.bias", {nf}));
+  HDRVAE_TRY(pack_conv(st, st->raw["conv_cat.weight"], st->raw["conv_cat.bias"], nf, 4 * nf, 1, false, 1.f, DT_F16, &up->body[20], s));
+  HDRVAE_TRY(need("upsampler.0.bias", {3 * up->scale * up->scale}));
+  HDRVAE_TRY(pack_conv(st, st->raw["upsampler.0.weight"], st->raw["upsampler.0.bias"], 3 * up->scale * up->scale, nf, 3, false,
+                       1.f, DT_F16, &up->body[21], s));
+  if (norm) up->mean = make_float3(0.4488f, 0.4371f, 0.4040f);
+  up->nb = 6;
+  up->span = true;
+  return 0;
+}
+
 // After packing: waits for the copies, frees the staging buffers and the fp32 copies of the state dict.
 static int up_finish_load(hdrvae_upscaler* up, std::vector<void*>& staging, cudaStream_t s) {
   hdrvae_ctx* st = &up->store;
@@ -842,8 +1054,12 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
     HDRVAE_TRY(up_pack_compact(up, s));
     return up_finish_load(up, staging, s);
   }
+  if (st->shapes.count("conv_1.sk.weight")) {
+    HDRVAE_TRY(up_pack_span(up, s));
+    return up_finish_load(up, staging, s);
+  }
   HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
-                 "no Real-ESRGAN Compact model (body.0.weight without conv_first)");
+                 "no Real-ESRGAN Compact model (body.0.weight without conv_first) or SPAN model (conv_1.sk.weight)");
   up->nb = nb;
   // the layout: u upsampling convs (found above) and the pixel-unshuffle factor f from conv_first's 3 f^2 input channels
   HDRVAE_REQUIRE(n_up >= 0, "RRDBNet: %s has shape %s; an old-arch RRDBNet's last top-level conv sits at index 3u + 4 "

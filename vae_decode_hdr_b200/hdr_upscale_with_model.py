@@ -7,12 +7,13 @@ recombination all run in libhdrvae.so on the GPU (vae_decode_hdr_b200/csrc/upsca
 a CUDA device or without the library the node raises.
 
 Model loading stays what it is in ComfyUI (folder_paths + spandrel, :73-77); the node only reads
-`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Two architectures run: RRDBNet
-(ESRGAN: nf 64, gc 32) at 1x, 2x and 4x -- the plain form with 0, 1 or 2 upsampling convs and the pixel-unshuffle form
-(RealESRGAN_x2plus) -- and Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x.  An RRDBNet of another
-scale (8x), or one whose `descriptor.scale` disagrees with its weights, fails before any GPU work; any other architecture
-is rejected by the library with an error naming the tensor that does not fit; a Compact model whose `descriptor.scale`
-disagrees with its weights is an error too.
+`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Three architectures run:
+RRDBNet (ESRGAN: nf 64, gc 32) at 1x, 2x and 4x -- the plain form with 0, 1 or 2 upsampling convs and the pixel-unshuffle
+form (RealESRGAN_x2plus) --, Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x, and SPAN (nf <= 64) at
+1x, 2x and 4x, which gets the logit reversal like every architecture outside the reference's atanh list.  An RRDBNet of
+another scale (8x), or one whose `descriptor.scale` disagrees with its weights, fails before any GPU work; any other
+architecture is rejected by the library with an error naming the tensor that does not fit; a Compact or SPAN model whose
+`descriptor.scale` disagrees with its weights is an error too.
 """
 from __future__ import annotations
 

@@ -164,3 +164,53 @@ def random_compact_state_dict(seed: int = 0, nf: int = 64, nc: int = 32, s: int 
         scale = 0.5 if len(shape) == 1 and name.endswith(".weight") else bound
         sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * scale
     return sd
+
+
+def span_param_shapes(nf: int = 48, s: int = 4, norm: bool = True) -> List[Tuple[str, Tuple[int, ...]]]:
+    """SPAN (spandrel's "SPAN") state-dict keys in module order: Conv3XC conv_1 (3 -> nf), block_1 .. block_6 (c1_r, c2_r,
+    c3_r: nf -> nf), conv_cat (1x1, 4 nf -> nf), Conv3XC conv_2, upsampler.0 (nf -> 3 s^2), and the buffer no_norm when
+    the input normalisation is off.  Each Conv3XC holds sk, conv.0 / conv.1 / conv.2 (hidden width 2 cin / 2 cout) and
+    eval_conv."""
+    out: List[Tuple[str, Tuple[int, ...]]] = []
+
+    def conv(name, cout, cin, k):
+        out.append((f"{name}.weight", (cout, cin, k, k)))
+        out.append((f"{name}.bias", (cout,)))
+
+    def conv3xc(name, cin, cout):
+        conv(f"{name}.sk", cout, cin, 1)
+        conv(f"{name}.conv.0", 2 * cin, cin, 1)
+        conv(f"{name}.conv.1", 2 * cout, 2 * cin, 3)
+        conv(f"{name}.conv.2", cout, 2 * cout, 1)
+        conv(f"{name}.eval_conv", cout, cin, 3)
+    if not norm:
+        out.append(("no_norm", (1,)))
+    conv3xc("conv_1", 3, nf)
+    for b in range(1, 7):
+        for c in (1, 2, 3):
+            conv3xc(f"block_{b}.c{c}_r", nf, nf)
+    conv("conv_cat", nf, 4 * nf, 1)
+    conv3xc("conv_2", nf, nf)
+    conv("upsampler.0", 3 * s * s, nf, 3)
+    return out
+
+
+def random_span_state_dict(seed: int = 0, nf: int = 48, s: int = 4, norm: bool = True) -> Dict[str, torch.Tensor]:
+    """Random SPAN weights with unit-gain convs (U(+-sqrt(3 / fan_in)), biases U(+-0.05)), fp32, CPU; with `norm`,
+    conv_1's sk and conv.0 are scaled by 1/255 against the x 255 input.  eval_conv.* are random too: the library
+    rebuilds them from conv.* and sk, as SPAN's own eval-mode forward does."""
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    sd: Dict[str, torch.Tensor] = {}
+    bound = 1.0
+    for name, shape in span_param_shapes(nf, s, norm):
+        if name == "no_norm":
+            sd[name] = torch.zeros(shape)
+            continue
+        if len(shape) == 4:
+            bound = math.sqrt(3.0 / (shape[1] * shape[2] * shape[3]))
+            if norm and name in ("conv_1.sk.weight", "conv_1.conv.0.weight"):
+                bound /= 255.0
+            sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * bound
+        else:
+            sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * 0.05
+    return sd

@@ -26,7 +26,8 @@ def reversal_for_architecture(name: str) -> str:
 
 def is_compact_state_dict(state_dict) -> bool:
     """The Real-ESRGAN Compact (SRVGGNetCompact) key layout, as the library recognises it: `body.0.weight` and no
-    `conv_first.*`.  Every other model the library runs is an RRDBNet (see `rrdbnet_scale`)."""
+    `conv_first.*`.  The library then checks for SPAN (`conv_1.sk.weight`); every other model it runs is an RRDBNet (see
+    `rrdbnet_scale`)."""
     return "body.0.weight" in state_dict and not any(k.startswith("conv_first.") for k in state_dict)
 
 
@@ -57,8 +58,10 @@ def rrdbnet_scale(state_dict) -> Optional[int]:
 
 class HdrUpscalerEngine:
     """One upscaler model packed for the tcgen05 conv kernel on one GPU: an RRDBNet (ESRGAN: nf 64, gc 32; 0, 1 or 2
-    upsampling convs, pixel-unshuffle factor 1, 2 or 4, scale 1, 2 or 4) or a Real-ESRGAN Compact (SRVGGNetCompact,
-    PReLU, 1x / 2x / 4x).  `scale` is the model's, read from the library."""
+    upsampling convs, pixel-unshuffle factor 1, 2 or 4, scale 1, 2 or 4), a Real-ESRGAN Compact (SRVGGNetCompact,
+    PReLU, 1x / 2x / 4x) or a SPAN (nf <= 64, 1x / 2x / 4x; the library fuses every Conv3XC from its conv.* and sk
+    tensors and ignores eval_conv.*).  `scale` is the model's, read from the library; `blocks` is the RRDB count, the
+    Compact's body-conv count or SPAN's 6."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda"):
         self.lib = N.load_library()
