@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define HDRVAE_ABI_VERSION 1
+#define HDRVAE_ABI_VERSION 2
 
 typedef struct hdrvae_ctx hdrvae_ctx;
 
@@ -316,11 +316,32 @@ int hdrvae_epilogue(hdrvae_ctx* ctx, const void* pre_nhwc, int dtype, int B, int
  *   residual [B,OH,OW,Cout] of res_dtype or NULL; upsample2x != 0: nearest-2x upsample folded into the load
  *   (OH=2H, OW=2W); y [B,OH,OW,Cout] of y_dtype; round_tf32: round a float32 y to tf32 (RN);
  *   gn_partials: optional device float32 [B][chunks][32][2] receiving the GroupNorm (sum, sum of squares)
- *   partials of y, chunks = hdrvae_conv2d_stats_chunks(H, W, upsample2x) (also stored to *gn_chunks). */
+ *   partials of y, chunks = hdrvae_conv2d_stats_chunks(H, W, upsample2x) (also stored to *gn_chunks).
+ *   extra: NULL, or the channel slices, second output and epilogue of the upscalers' convs (hdrvae_conv_extra).
+ * Without extra (or with its x_channels / y_channels 0) Cin must be a multiple of 64 and Cout of 32 and the tensors are
+ * dense.  With x_channels, Cin is free (x_channels % 8 == 0, x_channels >= Cin); with y_channels, Cout is free
+ * (y_chan_off % 4 == 0, y_channels % 4 == 0, y_chan_off + round_up(Cout, 4) <= y_channels) and the residuals share
+ * y's addressing. */
+enum { HDRVAE_ACT_NONE = 0, HDRVAE_ACT_SILU = 1, HDRVAE_ACT_GATE = 2 };
+typedef struct hdrvae_conv_extra {
+  int32_t x_channels;        /* pixel stride of x in elements (0: Cin); the conv reads the first Cin channels */
+  int32_t y_channels;        /* pixel stride of y (0: Cout) ... */
+  int32_t y_chan_off;        /* ... and the first channel of y written; round_up(Cout, 4) channels are stored */
+  int32_t y2_dtype;          /* HDRVAE_F16 / HDRVAE_BF16 */
+  void* y2;                  /* optional second output y * y2_scale (0: 1), 16-bit, [B,OH,OW,y2_channels] ... */
+  float y2_scale;
+  int32_t y2_channels;       /* ... (0: y's pixel stride and channel offset) */
+  int32_t y2_chan_off;
+  float res_scale;           /* t = conv + bias + res_scale * residual + residual2 (0: 1) */
+  const float* residual2;    /* optional float32 in y's layout */
+  const float* act_slope;    /* optional per-channel PReLU slopes, Cout floats */
+  float lrelu;               /* LeakyReLU slope (0: none) */
+  int32_t act;               /* HDRVAE_ACT_*: SiLU, or the gate y = (t + residual terms)(sigmoid(t) - 1/2) of SPAN */
+} hdrvae_conv_extra;
 int hdrvae_conv2d(hdrvae_ctx* ctx, const void* x, int x_dtype, int B, int H, int W, int Cin, const float* w,
                   const float* bias, int Cout, int ksize, int upsample2x, const void* residual, int res_dtype,
                   void* y, int y_dtype, int round_tf32, float* gn_partials, int* gn_chunks, int impl,
-                  void* stream);
+                  void* stream, const hdrvae_conv_extra* extra);
 int hdrvae_conv2d_stats_chunks(int H, int W, int upsample2x);
 
 /* GroupNorm(32 groups, eps 1e-6, affine) [+ SiLU] on NHWC: replaces norm1/norm2/norm_out + swish of

@@ -38,7 +38,21 @@ def test_library_exports_every_declared_symbol(lib):
         assert hasattr(lib, n), f"libhdrvae.so lacks {n} declared in include/hdrvae.h"
         assert n in _native.SIGNATURES, f"{n} has no ctypes signature in _native.py"
     assert sorted(_native.SIGNATURES) == names
-    assert lib.hdrvae_abi_version() == 1
+
+
+def test_abi_version_and_argument_counts_match_header(lib):
+    """The library, the ctypes binding and include/hdrvae.h agree on HDRVAE_ABI_VERSION, and every ctypes signature takes
+    as many arguments as the header's prototype (a stale binding would pass garbage for a new trailing argument)."""
+    from vae_decode_hdr_b200 import _native
+    src = open(os.path.join(ROOT, "include", "hdrvae.h")).read()
+    version = int(re.search(r"#define HDRVAE_ABI_VERSION (\d+)", src).group(1))
+    assert lib.hdrvae_abi_version() == _native.ABI_VERSION == version
+    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+    protos = dict(re.findall(r"\b(hdrvae_[a-z0-9_]+)\s*\(([^()]*)\)\s*;", src))
+    assert sorted(protos) == sorted(_native.SIGNATURES)
+    for name, params in protos.items():
+        n = 0 if params.strip() in ("", "void") else params.count(",") + 1
+        assert len(_native.SIGNATURES[name][1]) == n, f"{name}: header declares {n} arguments"
 
 
 def test_struct_layouts_match_header():
@@ -46,6 +60,7 @@ def test_struct_layouts_match_header():
     assert C.sizeof(N.HdrvaeStats) == 200           # static_assert'ed in csrc/api.cu
     assert C.sizeof(N.HdrvaeRawStats) == 96
     assert C.sizeof(N.HdrvaeWeightDesc) == 56
+    assert C.sizeof(N.HdrvaeConvExtra) == 64 and N.HdrvaeConvExtra.y2.offset == 16 and N.HdrvaeConvExtra.act.offset == 60
     assert N.HdrvaeStats.norm_function.offset == 184 and N.HdrvaeStats.hdr_pixels.offset == 144
 
 

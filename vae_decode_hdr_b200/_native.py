@@ -21,6 +21,8 @@ F32, BF16, F16 = range(3)
 PRECISION_BF16, PRECISION_F16, PRECISION_HIGH = 0, 1, 2
 CONV_TCGEN05, CONV_DIRECT = 0, 1
 RAW_NMIN, RAW_NMAX, RAW_NSUM = 4, 4, 8
+ACT_NONE, ACT_SILU, ACT_GATE = range(3)
+ABI_VERSION = 2
 
 
 class HdrvaeStats(C.Structure):
@@ -61,6 +63,13 @@ class HdrvaeRawStats(C.Structure):
     _fields_ = [("vmin", C.c_float * RAW_NMIN), ("vmax", C.c_float * RAW_NMAX), ("vsum", C.c_double * RAW_NSUM)]
 
 
+class HdrvaeConvExtra(C.Structure):
+    _fields_ = [("x_channels", C.c_int32), ("y_channels", C.c_int32), ("y_chan_off", C.c_int32), ("y2_dtype", C.c_int32),
+                ("y2", C.c_void_p), ("y2_scale", C.c_float), ("y2_channels", C.c_int32), ("y2_chan_off", C.c_int32),
+                ("res_scale", C.c_float), ("residual2", C.c_void_p), ("act_slope", C.c_void_p), ("lrelu", C.c_float),
+                ("act", C.c_int32)]
+
+
 # every symbol include/hdrvae.h declares: name -> (restype, argtypes)
 _vp, _i, _f, _sz = C.c_void_p, C.c_int, C.c_float, C.c_size_t
 SIGNATURES = {
@@ -97,7 +106,7 @@ SIGNATURES = {
     "hdrvae_features_dtype": (_i, [_vp]),
     "hdrvae_set_cta_group": (_i, [_vp, _i]),
     "hdrvae_conv2d": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _i, _vp, _i, _i, _vp,
-                           C.POINTER(_i), _i, _vp]),
+                           C.POINTER(_i), _i, _vp, C.POINTER(HdrvaeConvExtra)]),
     "hdrvae_conv2d_stats_chunks": (_i, [_i, _i, _i]),
     "hdrvae_groupnorm_silu": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp, _i, _vp]),
     "hdrvae_attention": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
@@ -143,7 +152,7 @@ def load_library() -> C.CDLL:
         fn = getattr(lib, name)       # AttributeError if the .so lacks a declared symbol
         fn.restype = res
         fn.argtypes = args
-    if lib.hdrvae_abi_version() != 1:
+    if lib.hdrvae_abi_version() != ABI_VERSION:
         raise RuntimeError("libhdrvae.so ABI version mismatch")
     _lib = lib
     return lib

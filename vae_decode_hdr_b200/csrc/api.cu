@@ -977,8 +977,11 @@ int hdrvae_destroy(hdrvae_ctx* ctx) {
   return 0;
 }
 
-static_assert(sizeof(hdrvae_stats) == 200 && sizeof(hdrvae_raw_stats) == 96 && sizeof(hdrvae_exchange) == 152,
-              "ABI struct layout changed");
+static_assert(sizeof(hdrvae_stats) == 200 && sizeof(hdrvae_raw_stats) == 96 && sizeof(hdrvae_exchange) == 152 &&
+              sizeof(hdrvae_conv_extra) == 64, "ABI struct layout changed");
+static_assert((int)HDRVAE_ACT_NONE == (int)ACT_NONE && (int)HDRVAE_ACT_SILU == (int)ACT_SILU &&
+              (int)HDRVAE_ACT_GATE == (int)ACT_GATE,
+              "hdrvae_conv_extra::act is GemmParams::act");
 
 long long hdrvae_launch_count(void) { return g_launch_count; }
 
@@ -1504,21 +1507,61 @@ int hdrvae_epilogue(hdrvae_ctx* ctx, const void* pre, int dtype, int B, int H, i
 // ---- kernel-level entry points -------------------------------------------------------------------
 int hdrvae_conv2d(hdrvae_ctx* ctx, const void* x, int x_dtype, int B, int H, int W, int Cin, const float* w,
                   const float* bias, int Cout, int ksize, int upsample2x, const void* residual, int res_dtype, void* y,
-                  int y_dtype, int round_tf32, float* gn_partials, int* gn_chunks, int impl, void* stream) {
+                  int y_dtype, int round_tf32, float* gn_partials, int* gn_chunks, int impl, void* stream,
+                  const hdrvae_conv_extra* extra) {
   HDRVAE_REQUIRE(ctx && x && w && y, "hdrvae_conv2d: null argument");
-  HDRVAE_REQUIRE(Cin % 64 == 0, "hdrvae_conv2d: Cin must be a multiple of 64 (pad the activation channels)");
-  HDRVAE_REQUIRE(Cout % 32 == 0 && (ksize == 1 || ksize == 3), "hdrvae_conv2d: Cout %% 32 == 0 and ksize in {1,3}");
+  HDRVAE_REQUIRE(ksize == 1 || ksize == 3, "hdrvae_conv2d: ksize must be 1 or 3");
   HDRVAE_REQUIRE(x_dtype >= 0 && x_dtype <= 2 && y_dtype >= 0 && y_dtype <= 2 && res_dtype >= 0 && res_dtype <= 2,
                  "hdrvae_conv2d: bad dtype");
+  hdrvae_conv_extra e;
+  memset(&e, 0, sizeof e);
+  if (extra != nullptr) e = *extra;
+  if (e.x_channels > 0)
+    HDRVAE_REQUIRE(e.x_channels % 8 == 0 && e.x_channels >= Cin, "hdrvae_conv2d: x_channels (%d) must be a multiple of 8 "
+                   "(16-byte pixel strides for the TMA) and at least Cin (%d)", e.x_channels, Cin);
+  else
+    HDRVAE_REQUIRE(Cin % 64 == 0, "hdrvae_conv2d: Cin (%d) must be a multiple of 64 unless x_channels gives x's pixel stride", Cin);
+  const int cout4 = (Cout + 3) / 4 * 4;     // the columns a conv with Cout % 32 != 0 stores
+  if (e.y_channels > 0)
+    HDRVAE_REQUIRE(e.y_chan_off >= 0 && e.y_chan_off % 4 == 0 && e.y_channels % 4 == 0 && e.y_chan_off + cout4 <= e.y_channels,
+                   "hdrvae_conv2d: the output slice [%d, %d + round_up(Cout, 4) = %d) must lie in y_channels (%d), "
+                   "with the offset and the stride multiples of 4", e.y_chan_off, e.y_chan_off, e.y_chan_off + cout4, e.y_channels);
+  else
+    HDRVAE_REQUIRE(Cout % 32 == 0 && e.y_chan_off == 0,
+                   "hdrvae_conv2d: Cout (%d) must be a multiple of 32 and y_chan_off 0 unless y_channels gives y's pixel stride", Cout);
+  if (e.y2 != nullptr) {
+    HDRVAE_REQUIRE(e.y2_dtype == HDRVAE_F16 || e.y2_dtype == HDRVAE_BF16, "hdrvae_conv2d: y2 must be fp16 or bf16");
+    if (e.y2_channels > 0)
+      HDRVAE_REQUIRE(e.y2_chan_off >= 0 && e.y2_chan_off % 4 == 0 && e.y2_channels % 4 == 0 && e.y2_chan_off + cout4 <= e.y2_channels,
+                     "hdrvae_conv2d: the y2 slice [%d, %d) must lie in y2_channels (%d), with the offset and the stride "
+                     "multiples of 4", e.y2_chan_off, e.y2_chan_off + cout4, e.y2_channels);
+    else
+      HDRVAE_REQUIRE(e.y2_chan_off == 0, "hdrvae_conv2d: y2_chan_off needs y2_channels");
+  }
+  HDRVAE_REQUIRE(e.act >= HDRVAE_ACT_NONE && e.act <= HDRVAE_ACT_GATE, "hdrvae_conv2d: bad act (%d)", e.act);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   hdrvae_ctx tmp;                     // owns the temporary packed operands
   tmp.device = ctx->device; tmp.num_sms = ctx->num_sms; tmp.cta_group = ctx->cta_group;
   PackedConv pc;
   int r = pack_conv(&tmp, w, bias, Cout, Cin, ksize, upsample2x != 0, 1.f, x_dtype, &pc, s);
+  float* slopes = nullptr;            // the kernels read cout_pad slopes, zero-padded (as the upscaler packs them)
+  if (r == 0 && e.act_slope != nullptr) {
+    r = dev_alloc(&tmp, pc.cout_pad * sizeof(float), (void**)&slopes);
+    if (r == 0 && (cudaMemsetAsync(slopes, 0, pc.cout_pad * sizeof(float), s) != cudaSuccess ||
+                   cudaMemcpyAsync(slopes, e.act_slope, Cout * sizeof(float), cudaMemcpyDeviceToDevice, s) != cudaSuccess)) {
+      set_error("hdrvae_conv2d: copying the PReLU slopes failed");
+      r = -1;
+    }
+  }
   if (r == 0) {
     ConvIO io; io.x = x; io.y = y; io.y_dtype = y_dtype; io.residual = residual; io.res_dtype = res_dtype;
     io.round_tf32 = round_tf32 != 0; io.stats = gn_partials; io.stats_chunks = gn_chunks;
+    io.x_channels = e.x_channels; io.y_channels = e.y_channels; io.y_chan_off = e.y_chan_off;
+    io.y2 = e.y2; io.y2_dtype = e.y2 != nullptr ? e.y2_dtype : DT_F16; io.y2_scale = e.y2_scale != 0.f ? e.y2_scale : 1.f;
+    io.y2_channels = e.y2_channels; io.y2_chan_off = e.y2_chan_off;
+    io.res_scale = e.res_scale != 0.f ? e.res_scale : 1.f; io.residual2 = e.residual2;
+    io.lrelu = e.lrelu; io.act_slope = slopes; io.act = e.act;
     r = run_conv(&tmp, pc, io, B, H, W, impl, s);
   }
   cudaStreamSynchronize(s);

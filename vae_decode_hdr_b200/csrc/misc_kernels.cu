@@ -181,6 +181,7 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
   const bool tf32 = p.ab_dtype == DT_F32;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int col = (int)(i % p.n_cols);
+    if (p.n_store > 0 && col >= p.n_store) continue;   // a column that is not stored reads no residual / slope either
     long long r = i / p.n_cols;
     const int x = (int)(r % p.W); r /= p.W;
     const int y = (int)(r % p.H);
@@ -211,7 +212,6 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
     if (p.act_slope != nullptr && v < 0.f) v *= p.act_slope[col];
     if (p.act == ACT_SILU) v *= 1.f / (1.f + expf(-v));
     if (p.act == ACT_GATE) v *= gate;
-    if (p.n_store > 0 && col >= p.n_store) continue;
     if (p.out2 != nullptr) {
       const long long off2 = p.out2_px_stride == 0 ? off
           : (long long)img * p.out2_img_stride + (long long)(y * p.sy + p.py) * p.out2_row_stride +

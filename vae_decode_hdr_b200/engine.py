@@ -276,26 +276,73 @@ class HdrVaeEngine:
     # -- kernel-level entry points (unit parity tests) ------------------------------------------------
     def conv2d(self, x_nhwc: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], ksize: int,
                upsample2x: bool = False, residual: Optional[torch.Tensor] = None, out_dtype=torch.float32,
-               round_tf32: bool = False, want_stats: bool = False, impl: int = N.CONV_TCGEN05):
-        """x_nhwc dtype selects the MMA kind: float16/bfloat16 -> kind::f16, float32 -> kind::tf32."""
-        B, H, W, cin = x_nhwc.shape
+               round_tf32: bool = False, want_stats: bool = False, impl: int = N.CONV_TCGEN05, *,
+               cin: Optional[int] = None, x_chan_off: int = 0, out: Optional[torch.Tensor] = None, out_chan_off: int = 0,
+               out2: Optional[torch.Tensor] = None, out2_chan_off: Optional[int] = None, out2_scale: float = 1.0,
+               residual2: Optional[torch.Tensor] = None, res_scale: float = 1.0, lrelu: float = 0.0,
+               prelu: Optional[torch.Tensor] = None, act: int = N.ACT_NONE):
+        """x_nhwc dtype selects the MMA kind: float16/bfloat16 -> kind::f16, float32 -> kind::tf32.
+
+        The keyword arguments are the upscalers' conv features (include/hdrvae.h, hdrvae_conv_extra):
+          cin / x_chan_off: the conv reads channels [x_chan_off, x_chan_off + cin) of x_nhwc [B,H,W,X] (X is the pixel
+                           stride); without cin it reads all of them, densely;
+          out / out_chan_off: write round_up(Cout, 4) channels from out_chan_off on into this device tensor
+                           [B,OH,OW,Y] (its dtype is the output's) and return it; residual / residual2 share its layout;
+          out2 / out2_chan_off / out2_scale: second, 16-bit output y * out2_scale into a slice of out2 [B,OH,OW,Y2]
+                           (without out2_chan_off, out2 has y's pixel stride and channel offset);
+          residual2 (float32), res_scale: t = conv + bias + res_scale * residual + residual2;
+          lrelu, prelu (Cout slopes), act (N.ACT_SILU / N.ACT_GATE): the activation of t.
+        The device tensors given here are used in place (no copies), so they may alias one another as in the upscalers."""
+        B, H, W, xc = x_nhwc.shape
         cout = weight.shape[0]
         OH, OW = (2 * H, 2 * W) if upsample2x else (H, W)
+        sliced = cin is not None
+        cin = xc if cin is None else cin
+        if not 0 <= x_chan_off <= xc - cin:
+            raise ValueError(f"channels [{x_chan_off}, {x_chan_off + cin}) lie outside x's {xc}")
+        for name, t in (("x_nhwc", x_nhwc if sliced else None), ("out", out), ("out2", out2), ("residual2", residual2),
+                        ("residual", residual if out is not None else None), ("prelu", prelu)):
+            if t is not None and (t.device != self.device or not t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous tensor on {self.device} when used in place")
+        ext = N.HdrvaeConvExtra()
+        if sliced:
+            ext.x_channels = xc
+        if out is not None:
+            if tuple(out.shape[:3]) != (B, OH, OW):
+                raise ValueError(f"out {tuple(out.shape)} does not match the output grid {(B, OH, OW)}")
+            ext.y_channels, ext.y_chan_off = out.shape[3], out_chan_off
+        if out2 is not None:
+            if tuple(out2.shape[:3]) != (B, OH, OW):
+                raise ValueError(f"out2 {tuple(out2.shape)} does not match the output grid {(B, OH, OW)}")
+            ext.y2, ext.y2_dtype, ext.y2_scale = out2.data_ptr(), _DTYPE_ID[out2.dtype], out2_scale
+            if out2_chan_off is not None:
+                ext.y2_channels, ext.y2_chan_off = out2.shape[3], out2_chan_off
+            elif out2.shape[3] != (out.shape[3] if out is not None else cout):
+                raise ValueError("out2 without out2_chan_off must have y's pixel stride")
+        if residual2 is not None:
+            if residual2.dtype != torch.float32:
+                raise ValueError("residual2 must be float32")
+            ext.residual2 = residual2.data_ptr()
+        if prelu is not None:
+            if prelu.dtype != torch.float32 or prelu.numel() != cout:
+                raise ValueError(f"prelu must hold {cout} float32 slopes")
+            ext.act_slope = prelu.data_ptr()
+        ext.res_scale, ext.lrelu, ext.act = res_scale, lrelu, act
         with torch.cuda.device(self.device):
-            x = x_nhwc.to(self.device).contiguous()
+            x = x_nhwc if sliced else x_nhwc.to(self.device).contiguous()
             wt = weight.to(self.device, torch.float32).contiguous()
             bs = bias.to(self.device, torch.float32).contiguous() if bias is not None else None
-            rs = residual.to(self.device).contiguous() if residual is not None else None
-            y = torch.empty((B, OH, OW, cout), dtype=out_dtype, device=self.device)
+            rs = residual if out is not None or residual is None else residual.to(self.device).contiguous()
+            y = out if out is not None else torch.empty((B, OH, OW, cout), dtype=out_dtype, device=self.device)
             chunks = self.lib.hdrvae_conv2d_stats_chunks(H, W, int(upsample2x))
             part = torch.zeros((B, chunks, 32, 2), dtype=torch.float32, device=self.device) if want_stats else None
             nch = C.c_int(0)
             N.check(self.lib.hdrvae_conv2d(
-                self._ctx, x.data_ptr(), _DTYPE_ID[x.dtype], B, H, W, cin, wt.data_ptr(),
+                self._ctx, x.data_ptr() + x_chan_off * x.element_size(), _DTYPE_ID[x.dtype], B, H, W, cin, wt.data_ptr(),
                 bs.data_ptr() if bs is not None else None, cout, ksize, int(upsample2x),
                 rs.data_ptr() if rs is not None else None, _DTYPE_ID[rs.dtype] if rs is not None else 0, y.data_ptr(),
-                _DTYPE_ID[out_dtype], int(round_tf32), part.data_ptr() if want_stats else None, C.byref(nch), impl,
-                self._stream()), "hdrvae_conv2d")
+                _DTYPE_ID[y.dtype], int(round_tf32), part.data_ptr() if want_stats else None, C.byref(nch), impl,
+                self._stream(), C.byref(ext)), "hdrvae_conv2d")
         if want_stats:      # the library packs the partials with the chunk count it actually used (<= the capacity asked for)
             part = part.flatten()[:B * nch.value * 64].view(B, nch.value, 32, 2)
         return (y, part) if want_stats else y
