@@ -1,4 +1,4 @@
-"""Comparison metrics shared by the GPU parity tests."""
+"""Comparison metrics and helpers shared by the GPU parity tests."""
 import torch
 import torch.nn.functional as F
 
@@ -7,6 +7,23 @@ SAT_BAND = 1e-3
 
 def rel_l2(a: torch.Tensor, b: torch.Tensor) -> float:
     return float((a.double() - b.double()).norm() / b.double().norm())
+
+
+def rel_trimmed(a, b, frac):
+    e = ((a - b).double() ** 2).sum(dim=-1).flatten()
+    k = e.numel() - int(frac * e.numel())
+    return float(e.sort().values[:k].sum().sqrt() / b.double().norm())
+
+
+class GpuModel(torch.nn.Module):
+    """The oracle's tiling / recombination driven by the GPU network: isolates everything after the model."""
+
+    def __init__(self, eng):
+        super().__init__()
+        self.eng = eng
+
+    def forward(self, a):
+        return self.eng.forward(a.movedim(1, -1).contiguous().to("cuda:0"), "none").cpu().movedim(-1, 1)
 
 
 def saturation_band_mask(dec, pre_nchw: torch.Tensor, band: float = SAT_BAND) -> torch.Tensor:

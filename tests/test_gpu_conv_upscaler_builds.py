@@ -1,6 +1,6 @@
 """Every tensor-core conv build the upscalers launch, one launch at a time against a plain fp64 evaluation of that launch.
 
-The rows below restate the call sites of csrc/upscaler.cu (up_forward: RRDBNet, up_forward_compact, up_forward_span) through
+The rows below restate the call sites of csrc/upscaler.cu (up_forward_rrdb, up_forward_compact, up_forward_span) through
 hdrvae_conv2d with the same ConvIO fields: channel slices of wider buffers on input and output, the second 16-bit output,
 the residual pair with res_scale, and LeakyReLU / PReLU / SiLU / SPAN's gate.  Each row runs
   - on four shapes: whole 8 x 16 slab tiles (every tile takes the epilogue's fast path), a ragged slab shape with an odd
@@ -53,7 +53,7 @@ def row(name, build, cin, cout, *, ks=3, up=False, xc=None, xoff=0, alias=False,
 # With set_cta_group(1) every narrow conv takes launch_tc<32,false,1,EPI_GENERIC,9> / <32,false,1,EPI_GENERIC> (32 columns,
 # slab / non-slab) or launch_tc<64,false,1,EPI_GENERIC> (64 columns, both forms).
 ROWS = [
-    # ---- RRDBNet (up_forward): nf 64, gc 32
+    # ---- RRDBNet (up_forward_rrdb): nf 64, gc 32
     *[row(f"rrdb.conv_first.f{f}", "launch_tc<64,false,2,EPI_OUT2,9> / <64,false,2,EPI_OUT2>",
           3 * f * f, 64, xc={1: 8, 2: 16, 4: 48}[f], yc=64, y2=(192, 0)) for f in (1, 2, 4)],
     *[row(f"rrdb.rdb.conv{j + 1}", "launch_tc<32,false,2,EPI_OUT16|EPI_LRELU,9> / <32,false,2,EPI_OUT16|EPI_LRELU>",

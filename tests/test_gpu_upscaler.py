@@ -11,21 +11,12 @@ import numpy as np
 import pytest
 import torch
 
+from _metrics import GpuModel, rel_l2, rel_trimmed
 from oracle import upscaler_oracle as uo
 from oracle.make_golden_upscale import CASES, make_image
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-
-
-def _rel(a, b):
-    return float((a.double() - b.double()).norm() / b.double().norm())
-
-
-def _rel_trimmed(a, b, frac):
-    e = ((a - b).double() ** 2).sum(dim=-1).flatten()
-    k = e.numel() - int(frac * e.numel())
-    return float(e.sort().values[:k].sum().sqrt() / b.double().norm())
 
 
 @pytest.fixture(scope="module")
@@ -50,7 +41,7 @@ def test_rrdbnet_forward_vs_oracle(nets, n, h, w, reversal):
             ref = uo.reversal(ref, "atanh")
     got = eng.forward(x.to(DEV), reversal)
     assert got.shape == (n, 4 * h, 4 * w, 3)
-    assert _rel(got.cpu(), ref.movedim(1, -1)) < 1e-2
+    assert rel_l2(got.cpu(), ref.movedim(1, -1)) < 1e-2
 
 
 def test_rrdbnet_tcgen05_vs_cuda_core_kernel(nets):
@@ -65,7 +56,7 @@ def test_rrdbnet_tcgen05_vs_cuda_core_kernel(nets):
         b = eng.forward(x, "none")
     finally:
         eng.set_conv_impl(N.CONV_TCGEN05)
-    assert _rel(a, b) < 3e-3
+    assert rel_l2(a, b) < 3e-3
 
 
 def test_old_arch_state_dict_gives_identical_model(nets):
@@ -82,21 +73,10 @@ def test_wrong_architecture_fails_loudly():
     net = uo.build_upscaler(0, nb=1)
     sd = dict(net.state_dict())
     sd["body.0.rdb1.conv1.weight"] = torch.zeros(16, 64, 3, 3)
-    with pytest.raises(RuntimeError, match="wrong shape"):
+    with pytest.raises(RuntimeError, match=r"body\.0\.rdb1\.conv1\.weight has shape \[16,64,3,3\]; want \[32,64,3,3\]"):
         HdrUpscalerEngine(sd, DEV)
     with pytest.raises(RuntimeError, match="no RRDB blocks"):
         HdrUpscalerEngine({"foo.weight": torch.zeros(4, 4, 3, 3)}, DEV)
-
-
-class _GpuModel(torch.nn.Module):
-    """The oracle's tiling / recombination driven by the GPU network: isolates everything after the model."""
-
-    def __init__(self, eng):
-        super().__init__()
-        self.eng = eng
-
-    def forward(self, a):
-        return self.eng.forward(a.movedim(1, -1).contiguous().to(DEV), "none").cpu().movedim(-1, 1)
 
 
 @pytest.mark.parametrize("B,H,W,blur,fix,method", [(1, 24, 20, False, False, "bilinear"), (1, 530, 24, False, False, "bilinear"),
@@ -107,7 +87,7 @@ class _GpuModel(torch.nn.Module):
 def test_tiling_blend_and_recombination_are_exact_given_the_model(nets, B, H, W, blur, fix, method):
     net, eng = nets[(1, 1.0)] if max(H, W) > 512 else nets[(2, 40.0)]
     img = make_image(B, H, W, 31, 3.0)
-    want = uo.upscale(img, uo.FakeDescriptor(_GpuModel(eng)), blur, fix, method)
+    want = uo.upscale(img, uo.FakeDescriptor(GpuModel(eng)), blur, fix, method)
     got = eng.upscale(img.to(DEV), "atanh", blur, fix, method).cpu()
     assert got.shape == want.shape
     err = (got - want).abs()
@@ -127,9 +107,9 @@ def test_upscale_vs_reference_golden(nets, golden_dir, case):
     if last_gain > 1.0:
         # conv_last x 40 drives the model output into the +-1 saturation of atanh(clamp(.)): ill-conditioned like the
         # decoder's logit modes, so the 0.5 % worst pixels are set aside
-        assert _rel_trimmed(got, ref, 0.005) < 1e-2, _rel_trimmed(got, ref, 0.005)
+        assert rel_trimmed(got, ref, 0.005) < 1e-2, rel_trimmed(got, ref, 0.005)
     else:
-        assert _rel(got, ref) < 1e-2, _rel(got, ref)
+        assert rel_l2(got, ref) < 1e-2, rel_l2(got, ref)
 
 
 def test_node_surface_and_call(nets, golden_dir, monkeypatch):
@@ -148,11 +128,11 @@ def test_node_surface_and_call(nets, golden_dir, monkeypatch):
     g = dict(np.load(os.path.join(golden_dir, "up_a_single_tile.npz"), allow_pickle=False))
     (out,) = node.upscale(torch.from_numpy(g["image"]), "fake.pth", False, False, "bislerp")
     assert out.device.type == "cpu" and out.dtype == torch.float32 and out.shape == g["output"].shape
-    assert _rel(out, torch.from_numpy(g["output"])) < 1e-2
+    assert rel_l2(out, torch.from_numpy(g["output"])) < 1e-2
     # the node's own defaults with local_fix ticked (ADVICE r1): bislerp is implemented, an unknown method is a ValueError
     (fixed,) = node.upscale(torch.from_numpy(g["image"]), "fake.pth", False, True, "bislerp")
     ref_fixed = uo.upscale(torch.from_numpy(g["image"]), uo.FakeDescriptor(net, 4, "ESRGAN"), False, True, "bislerp")
-    assert _rel(fixed, ref_fixed) < 1e-2, _rel(fixed, ref_fixed)
+    assert rel_l2(fixed, ref_fixed) < 1e-2, rel_l2(fixed, ref_fixed)
     with pytest.raises(ValueError):
         node.upscale(torch.from_numpy(g["image"]), "fake.pth", False, True, "lanczos")
 
@@ -175,7 +155,7 @@ def test_c5_pipeline_decode_upscale_pack(nets):
     ref_img, _, _ = ho.simple_hdr_decode(dec, z, "moderate", 1.0)
     ref_big = uo.upscale(ref_img, uo.FakeDescriptor(net))
     ref_half = torch.from_numpy(ref_big.numpy().astype(np.float16)).float()
-    assert _rel(half.float().cpu(), ref_half) < 1e-2, _rel(half.float().cpu(), ref_half)
+    assert rel_l2(half.float().cpu(), ref_half) < 1e-2, rel_l2(half.float().cpu(), ref_half)
     eng.close()
 
 
@@ -190,5 +170,5 @@ def test_rrdbnet_full_depth_nb23_vs_oracle():
     with torch.no_grad():
         ref = net(x.movedim(-1, 1)).movedim(1, -1)
     got = eng.forward(x.to(DEV), "none").cpu()
-    assert _rel(got, ref) < 1e-2, _rel(got, ref)
+    assert rel_l2(got, ref) < 1e-2, rel_l2(got, ref)
     eng.close()

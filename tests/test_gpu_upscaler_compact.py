@@ -9,21 +9,12 @@ import pytest
 import torch
 
 from _compact_oracle import build_compact
+from _metrics import GpuModel, rel_l2, rel_trimmed
 from oracle import upscaler_oracle as uo
 from oracle.make_golden_upscale import make_image
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-
-
-def _rel(a, b):
-    return float((a.double() - b.double()).norm() / b.double().norm())
-
-
-def _rel_trimmed(a, b, frac):
-    e = ((a - b).double() ** 2).sum(dim=-1).flatten()
-    k = e.numel() - int(frac * e.numel())
-    return float(e.sort().values[:k].sum().sqrt() / b.double().norm())
 
 
 @pytest.fixture(scope="module")
@@ -60,7 +51,7 @@ def test_compact_forward_vs_oracle(compact, s, nf, nc, n, h, w):
     x = make_image(n, h, w, 5 + n, 3.0)
     got = eng.forward(x.to(DEV), "none").cpu()
     assert got.shape == (n, s * h, s * w, 3)
-    assert _rel(got, _oracle(net, x, "none")) < 1e-2
+    assert rel_l2(got, _oracle(net, x, "none")) < 1e-2
 
 
 @pytest.mark.parametrize("reversal", ["atanh", "logit"])
@@ -71,7 +62,7 @@ def test_compact_forward_with_reversal_vs_oracle(compact, s, reversal):
     x = make_image(2, 40, 56, 8, 3.0)
     got = eng.forward(x.to(DEV), reversal).cpu()
     ref = _oracle(net, x, reversal)
-    assert _rel_trimmed(got, ref, 0.005) < 1e-2, _rel_trimmed(got, ref, 0.005)
+    assert rel_trimmed(got, ref, 0.005) < 1e-2, rel_trimmed(got, ref, 0.005)
 
 
 def test_compact_full_depth_vs_oracle():
@@ -83,7 +74,7 @@ def test_compact_full_depth_vs_oracle():
         assert (eng.scale, eng.blocks) == (4, 32)
         x = make_image(1, 48, 40, 17, 3.0)
         got = eng.forward(x.to(DEV), "none").cpu()
-        assert _rel(got, _oracle(net, x, "none")) < 1e-2, _rel(got, _oracle(net, x, "none"))
+        assert rel_l2(got, _oracle(net, x, "none")) < 1e-2, rel_l2(got, _oracle(net, x, "none"))
     finally:
         eng.close()
 
@@ -101,18 +92,7 @@ def test_compact_tcgen05_vs_cuda_core_kernel(compact, nf, nc, s):
         b = eng.forward(x, "none")
     finally:
         eng.set_conv_impl(N.CONV_TCGEN05)
-    assert _rel(a, b) < 3e-3
-
-
-class _GpuModel(torch.nn.Module):
-    """The oracle's tiling / recombination driven by the GPU network: isolates everything after the model."""
-
-    def __init__(self, eng):
-        super().__init__()
-        self.eng = eng
-
-    def forward(self, a):
-        return self.eng.forward(a.movedim(1, -1).contiguous().to(DEV), "none").cpu().movedim(-1, 1)
+    assert rel_l2(a, b) < 3e-3
 
 
 _AFTER_MODEL_CASES = [(1, 530, 24, False, False, "bilinear", "atanh"), (1, 40, 600, True, True, "nearest-exact", "logit"),
@@ -127,7 +107,7 @@ def test_tiling_blend_and_recombination_are_exact_given_the_model(compact, s, B,
     _, eng = compact(64, 2, s)
     img = make_image(B, H, W, 31, 3.0)
     arch = "ESRGAN" if reversal == "atanh" else "Compact"              # the oracle picks the reversal by name
-    want = uo.upscale(img, uo.FakeDescriptor(_GpuModel(eng), s, arch), blur, fix, method)
+    want = uo.upscale(img, uo.FakeDescriptor(GpuModel(eng), s, arch), blur, fix, method)
     got = eng.upscale(img.to(DEV), reversal, blur, fix, method).cpu()
     assert got.shape == want.shape == (B, s * H, s * W, 3)
     err = (got - want).abs()
@@ -157,7 +137,7 @@ def test_node_runs_a_2x_compact_model(monkeypatch):
     (out,) = node.upscale(img, "compact_2x.pth", False, True, "bislerp")
     assert out.device.type == "cpu" and out.dtype == torch.float32 and out.shape == (1, 48, 40, 3)
     ref = uo.upscale(img, desc, False, True, "bislerp")
-    assert _rel(out, ref) < 1e-2, _rel(out, ref)
+    assert rel_l2(out, ref) < 1e-2, rel_l2(out, ref)
 
 
 def test_node_cached_compact_engine(monkeypatch, tmp_path):
@@ -172,7 +152,7 @@ def test_node_cached_compact_engine(monkeypatch, tmp_path):
         assert len(calls) == 1                                          # the second call hit the engine cache
         assert a.shape == (1, 80, 112, 3) and torch.equal(a, b)
         ref = uo.upscale(img, desc, True, False, "bilinear")
-        assert _rel(a, ref) < 1e-2, _rel(a, ref)
+        assert rel_l2(a, ref) < 1e-2, rel_l2(a, ref)
     finally:
         HDRUpscaleWithModel.release_memory()
 

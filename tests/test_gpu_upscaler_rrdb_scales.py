@@ -8,6 +8,7 @@ output is compared at rel-L2 <= 1e-2; everything after the model is fp32 in the 
 import pytest
 import torch
 
+from _metrics import GpuModel, rel_l2, rel_trimmed
 import _rrdb_oracle as ro
 from oracle import upscaler_oracle as uo
 from oracle.make_golden_upscale import make_image
@@ -17,16 +18,6 @@ DEV = "cuda:0"
 
 # (n_up, shuffle, scale): the forms this file covers (the 4x one, (2, 1, 4), is tests/test_gpu_upscaler.py's)
 NEW_FORMS = [(2, 2, 2), (2, 4, 1), (1, 1, 2), (0, 1, 1), (1, 2, 1)]
-
-
-def _rel(a, b):
-    return float((a.double() - b.double()).norm() / b.double().norm())
-
-
-def _rel_trimmed(a, b, frac):
-    e = ((a - b).double() ** 2).sum(dim=-1).flatten()
-    k = e.numel() - int(frac * e.numel())
-    return float(e.sort().values[:k].sum().sqrt() / b.double().norm())
 
 
 @pytest.fixture(scope="module")
@@ -66,7 +57,7 @@ def test_rrdbnet_forms_forward_vs_oracle(rrdb, n_up, f, s, nb, n, h, w, reversal
     got = eng.forward(x.to(DEV), reversal).cpu()
     assert got.shape == (n, s * h, s * w, 3)
     ref = _oracle(net, x, reversal)
-    err = _rel(got, ref) if reversal == "none" else _rel_trimmed(got, ref, 0.005)
+    err = rel_l2(got, ref) if reversal == "none" else rel_trimmed(got, ref, 0.005)
     assert err < 1e-2, err
 
 
@@ -83,7 +74,7 @@ def test_rrdbnet_forms_tcgen05_vs_cuda_core_kernel(rrdb, n_up, f, s):
     finally:
         eng.set_conv_impl(N.CONV_TCGEN05)
     assert a.shape == (2, 25 * s, 42 * s, 3)
-    assert _rel(a, b) < 3e-3, _rel(a, b)
+    assert rel_l2(a, b) < 3e-3, rel_l2(a, b)
 
 
 @pytest.mark.parametrize("n_up,f,s", NEW_FORMS)
@@ -99,17 +90,6 @@ def test_old_arch_state_dict_gives_identical_model(rrdb, n_up, f, s):
         eng_old.close()
 
 
-class _GpuModel(torch.nn.Module):
-    """The oracle's tiling / recombination driven by the GPU network: isolates everything after the model."""
-
-    def __init__(self, eng):
-        super().__init__()
-        self.eng = eng
-
-    def forward(self, a):
-        return self.eng.forward(a.movedim(1, -1).contiguous().to(DEV), "none").cpu().movedim(-1, 1)
-
-
 # 531 x 37: the edge tiles (83 rows) and the 37 columns are not multiples of 2 or 4, so they pad
 _AFTER_MODEL_CASES = [(1, 530, 24, False, False, "bilinear", "atanh"), (1, 40, 600, True, True, "nearest-exact", "logit"),
                       (1, 520, 520, False, True, "bilinear", "logit"), (1, 531, 37, False, True, "bislerp", "atanh"),
@@ -122,7 +102,7 @@ def test_tiling_blend_and_recombination_are_exact_given_the_model(rrdb, n_up, f,
     _, eng = rrdb(n_up, f, 1)
     img = make_image(B, H, W, 31, 3.0)
     arch = "ESRGAN" if reversal == "atanh" else "Other"                 # the oracle picks the reversal by name
-    want = uo.upscale(img, uo.FakeDescriptor(_GpuModel(eng), s, arch), blur, fix, method)
+    want = uo.upscale(img, uo.FakeDescriptor(GpuModel(eng), s, arch), blur, fix, method)
     got = eng.upscale(img.to(DEV), reversal, blur, fix, method).cpu()
     assert got.shape == want.shape == (B, s * H, s * W, 3)
     err = (got - want).abs()
@@ -156,7 +136,7 @@ def test_node_runs_the_form_and_caches_it(monkeypatch, tmp_path, n_up, f, s, H, 
         assert len(calls) == 1                                          # the second call hit the engine cache
         assert a.device.type == "cpu" and a.shape == (1, s * H, s * W, 3) and torch.equal(a, b)
         ref = uo.upscale(img, desc, False, True, "bislerp")
-        assert _rel(a, ref) < 1e-2, _rel(a, ref)
+        assert rel_l2(a, ref) < 1e-2, rel_l2(a, ref)
     finally:
         HDRUpscaleWithModel.release_memory()
 
@@ -181,7 +161,11 @@ def test_rejections_name_the_tensor_and_its_shape():
         HdrUpscalerEngine(sd, DEV)
     sd = _sd()
     sd["conv_up1.weight"], sd["conv_up1.bias"] = torch.zeros(256, 64, 3, 3), torch.zeros(256)   # pixel-shuffle upsampler
-    with pytest.raises(RuntimeError, match=r"conv_up1\.weight has the wrong shape \[256,64,3,3\]"):
+    with pytest.raises(RuntimeError, match=r"conv_up1\.weight has shape \[256,64,3,3\]; want \[64,64,3,3\]"):
+        HdrUpscalerEngine(sd, DEV)
+    sd = _sd()
+    sd["conv_body.bias"] = torch.zeros(32)                                      # shorter than the 64 channels packed
+    with pytest.raises(RuntimeError, match=r"conv_body\.bias has shape \[32\]; want \[64\]"):
         HdrUpscalerEngine(sd, DEV)
     old = ro.state_dict_old_arch(ro.build_upscaler(0, nb=1, n_up=1))
     old["model.9.weight"], old["model.9.bias"] = torch.zeros(3, 64, 3, 3), torch.zeros(3)      # conv_last at 9: no u fits

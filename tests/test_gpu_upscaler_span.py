@@ -9,22 +9,13 @@ operation order.  Each comparison prints the error it measured."""
 import pytest
 import torch
 
+from _metrics import GpuModel, rel_l2, rel_trimmed
 from _span_oracle import build_span, stale_eval_conv
 from oracle import upscaler_oracle as uo
 from oracle.make_golden_upscale import make_image
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-
-
-def _rel(a, b):
-    return float((a.double() - b.double()).norm() / b.double().norm())
-
-
-def _rel_trimmed(a, b, frac):
-    e = ((a - b).double() ** 2).sum(dim=-1).flatten()
-    k = e.numel() - int(frac * e.numel())
-    return float(e.sort().values[:k].sum().sqrt() / b.double().norm())
 
 
 @pytest.fixture(scope="module")
@@ -61,7 +52,7 @@ def test_span_forward_vs_oracle(span, s, nf, norm, n, h, w):
     x = make_image(n, h, w, 5 + n, 1.0).clamp(0, 1)
     got = eng.forward(x.to(DEV), "none").cpu()
     assert got.shape == (n, s * h, s * w, 3)
-    err = _rel(got, _oracle(net, x, "none"))
+    err = rel_l2(got, _oracle(net, x, "none"))
     print(f"span nf {nf} {s}x norm {norm} {n}x{h}x{w}: rel-L2 {err:.2e}")
     assert err < 1e-2, err
 
@@ -73,7 +64,7 @@ def test_span_forward_with_reversal_vs_oracle(span, s, reversal):
     net, eng = span(48, s)
     x = make_image(2, 40, 56, 8, 1.0).clamp(0, 1)
     got = eng.forward(x.to(DEV), reversal).cpu()
-    err = _rel_trimmed(got, _oracle(net, x, reversal), 0.005)
+    err = rel_trimmed(got, _oracle(net, x, reversal), 0.005)
     print(f"span {s}x {reversal}: trimmed rel-L2 {err:.2e}")
     assert err < 1e-2, err
 
@@ -86,7 +77,7 @@ def test_span_hdr_range_input(span, norm):
     assert float(x.abs().max()) > 8.0
     got = eng.forward(x.to(DEV), "none").cpu()
     assert bool(torch.isfinite(got).all())
-    err = _rel(got, _oracle(net, x, "none"))
+    err = rel_l2(got, _oracle(net, x, "none"))
     print(f"span HDR amplitude 16 norm {norm}: rel-L2 {err:.2e}")
     assert err < 1e-2, err
 
@@ -104,7 +95,7 @@ def test_span_tcgen05_vs_cuda_core_kernel(span, nf, s):
         b = eng.forward(x, "none")
     finally:
         eng.set_conv_impl(N.CONV_TCGEN05)
-    err = _rel(a, b)
+    err = rel_l2(a, b)
     print(f"span nf {nf} {s}x tcgen05 vs CUDA core: rel-L2 {err:.2e}")
     assert err < 3e-3, err
 
@@ -122,17 +113,6 @@ def test_span_ignores_a_stale_eval_conv():
         b_eng.close()
 
 
-class _GpuModel(torch.nn.Module):
-    """The oracle's tiling / recombination driven by the GPU network: isolates everything after the model."""
-
-    def __init__(self, eng):
-        super().__init__()
-        self.eng = eng
-
-    def forward(self, a):
-        return self.eng.forward(a.movedim(1, -1).contiguous().to(DEV), "none").cpu().movedim(-1, 1)
-
-
 _AFTER_MODEL_CASES = [(1, 530, 24, False, False, "bilinear", "atanh"), (1, 40, 600, True, True, "nearest-exact", "logit"),
                       (1, 36, 44, False, True, "bislerp", "logit"), (2, 30, 26, False, True, "bicubic", "logit")]
 
@@ -143,7 +123,7 @@ def test_tiling_blend_and_recombination_are_exact_given_the_model(span, s, B, H,
     _, eng = span(16, s)
     img = make_image(B, H, W, 31, 1.0).clamp(0, 1)
     arch = "ESRGAN" if reversal == "atanh" else "SPAN"                # the oracle picks the reversal by name
-    want = uo.upscale(img, uo.FakeDescriptor(_GpuModel(eng), s, arch), blur, fix, method)
+    want = uo.upscale(img, uo.FakeDescriptor(GpuModel(eng), s, arch), blur, fix, method)
     got = eng.upscale(img.to(DEV), reversal, blur, fix, method).cpu()
     assert got.shape == want.shape == (B, s * H, s * W, 3)
     err = (got - want).abs()
@@ -185,7 +165,7 @@ def test_node_runs_a_span_model_with_logit_and_its_cache(monkeypatch, tmp_path):
         assert len(calls) == 1 and seen == ["logit", "logit"]           # the second call hit the engine cache
         assert a.shape == (1, 40, 56, 3) and torch.equal(a, b)
         ref = uo.upscale(img, desc, True, True, "bislerp")
-        assert _rel(a, ref) < 1e-2, _rel(a, ref)
+        assert rel_l2(a, ref) < 1e-2, rel_l2(a, ref)
     finally:
         HDRUpscaleWithModel.release_memory()
 

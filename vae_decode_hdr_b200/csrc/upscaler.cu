@@ -354,24 +354,23 @@ static inline int up_grid(long long n) { return (int)std::min<long long>((n + 25
 using namespace hdrvae;
 
 // ------------------------------------------------------------------------------------------------ model
-struct UpRdb { PackedConv c[5]; };
+enum UpArch { UP_RRDB, UP_COMPACT, UP_SPAN };   // ESRGAN / RRDBNet, Real-ESRGAN SRVGGNetCompact, SPAN
 
 struct hdrvae_upscaler {
   hdrvae_ctx* ctx = nullptr;      // device / SM count / conv implementation come from the decode context
   hdrvae_ctx store;               // owns this model's device allocations
   bool loaded = false;
-  bool compact = false;           // Real-ESRGAN SRVGGNetCompact
-  bool span = false;              // SPAN; neither: ESRGAN / RRDBNet
+  UpArch arch = UP_RRDB;
   float3 mean = {0.f, 0.f, 0.f};  // subtracted from the network input (SPAN's normalisation; its 255 is in conv_1's weights)
   int scale = 4;                  // output pixels per input pixel along each axis (RRDBNet: 2^n_up / shuffle)
   int nb = 0;                     // RRDB blocks (RRDBNet), body convs (Compact) or SPAB blocks (SPAN: 6)
   int n_up = 2;                   // RRDBNet: nearest-2x + conv upsampling stages (0, 1 or 2)
   int shuffle = 1;                // RRDBNet: pixel-unshuffle factor of the input (1, 2 or 4; conv_first reads 3 f^2 channels)
-  PackedConv conv_first, conv_body, up1, up2, hr, last;
-  std::vector<UpRdb> rdb;         // 3 per RRDB
-  std::vector<PackedConv> body;   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2); SPAN: the fused conv_1,
+  std::vector<PackedConv> convs;  // every conv in launch order.  RRDBNet: conv_first, conv1 .. conv5 of each dense block
+                                  // (3 per RRDB), conv_body, conv_up1 / conv_up2 (n_up of them), conv_hr, conv_last.
+                                  // Compact: first conv, nb body convs, last conv (nf -> 3 s^2).  SPAN: the fused conv_1,
                                   // block_k.c{1,2,3}_r (k = 1..6), conv_2, then conv_cat (1x1, 4 nf -> nf) and upsampler.0
-  std::vector<float*> slopes;     // Compact: PReLU slopes applied after body[k], k <= nb (cout_pad floats, zero-padded)
+  std::vector<float*> slopes;     // Compact: PReLU slopes applied after convs[k], k <= nb (cout_pad floats, zero-padded)
 };
 
 namespace hdrvae {
@@ -405,39 +404,40 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
   auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 1023) / 1024 * 1024; return o; };
   const size_t P = (size_t)n * up_net_side(up, h) * up_net_side(up, w);   // pixels of the network's input grid
   pl.img8 = take(P * up_in_channels(up->shuffle) * 2);
-  if (up->compact) {
-    // fp16 activations at a pixel stride of cout_pad (the convs read the first nf channels), ping-pong
-    const size_t cp = (size_t)up->body[0].cout_pad;
-    pl.act0 = take(P * cp * 2);
-    pl.act1 = take(P * cp * 2);
-    pl.last = take(P * up_last_channels(up) * 4);
-    pl.total = off;
-    return pl;
+  switch (up->arch) {
+    case UP_COMPACT: {
+      // fp16 activations at a pixel stride of cout_pad (the convs read the first nf channels), ping-pong
+      const size_t cp = (size_t)up->convs[0].cout_pad;
+      pl.act0 = take(P * cp * 2);
+      pl.act1 = take(P * cp * 2);
+      pl.last = take(P * up_last_channels(up) * 4);
+      break;
+    }
+    case UP_SPAN: {
+      const size_t nf = (size_t)up->convs[0].cout;
+      pl.sp_r0 = take(P * nf * 4);      // fp32 block stream (the gate's residual), ping-pong
+      pl.sp_r1 = take(P * nf * 4);
+      pl.sp_d = take(P * nf * 2);       // fp16 operand copy of a block output
+      pl.sp_t0 = take(P * nf * 2);      // SiLU'd c1_r / c2_r outputs
+      pl.sp_t1 = take(P * nf * 2);
+      pl.sp_cat = take(P * 4 * nf * 2); // [f | b6 | b1 | b5_2]: conv_cat's input, the channel order of torch.cat
+      pl.last = take(P * up_last_channels(up) * 4);
+      break;
+    }
+    case UP_RRDB:
+      pl.cat0 = take(P * 192 * 2);
+      pl.cat1 = take(P * 192 * 2);
+      pl.f_feat = take(P * 64 * 4);
+      pl.f_a = take(P * 64 * 4);
+      pl.f_b = take(P * 64 * 4);
+      pl.f_c = take(P * 64 * 4);
+      // fp16 operands of the upsampling stages: conv_body's copy (h' w'), conv_up1's (4 h' w'), conv_up2's (16 h' w'), conv_hr's
+      pl.u0 = take(P * 64 * 2);
+      pl.u1 = take(up->n_up >= 1 ? P * 4 * 64 * 2 : 0);
+      pl.u2 = take(up->n_up >= 2 ? P * 16 * 64 * 2 : 0);
+      pl.u3 = take((P << (2 * up->n_up)) * 64 * 2);
+      break;
   }
-  if (up->span) {
-    const size_t nf = (size_t)up->body[0].cout;
-    pl.sp_r0 = take(P * nf * 4);      // fp32 block stream (the gate's residual), ping-pong
-    pl.sp_r1 = take(P * nf * 4);
-    pl.sp_d = take(P * nf * 2);       // fp16 operand copy of a block output
-    pl.sp_t0 = take(P * nf * 2);      // SiLU'd c1_r / c2_r outputs
-    pl.sp_t1 = take(P * nf * 2);
-    pl.sp_cat = take(P * 4 * nf * 2); // [f | b6 | b1 | b5_2]: conv_cat's input, the channel order of torch.cat
-    pl.last = take(P * up_last_channels(up) * 4);
-    pl.total = off;
-    return pl;
-  }
-  pl.cat0 = take(P * 192 * 2);
-  pl.cat1 = take(P * 192 * 2);
-  pl.f_feat = take(P * 64 * 4);
-  pl.f_a = take(P * 64 * 4);
-  pl.f_b = take(P * 64 * 4);
-  pl.f_c = take(P * 64 * 4);
-  // fp16 operands of the upsampling stages: conv_body's copy (h' w'), conv_up1's (4 h' w'), conv_up2's (16 h' w'), conv_hr's
-  const size_t Pu = P << (2 * up->n_up);
-  pl.u0 = take(P * 64 * 2);
-  pl.u1 = take(up->n_up >= 1 ? P * 4 * 64 * 2 : 0);
-  pl.u2 = take(up->n_up >= 2 ? P * 16 * 64 * 2 : 0);
-  pl.u3 = take(Pu * 64 * 2);
   pl.total = off;
   return pl;
 }
@@ -446,7 +446,7 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
 // [n][s h][s w][4] at `out4`.  The network runs at h' x w' and conv_last at 2^u h' x 2^u w' = f s h' x f s w'; when the
 // tile was padded (f h' > h) conv_last writes into the dense-block buffer cat0 (dead by then) and the top-left window is
 // copied to out4.
-static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
+static int up_forward_rrdb(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
   hdrvae_ctx* ctx = up->ctx;
   const int impl = ctx->conv_impl;
   const int hq = up_net_side(up, h), wq = up_net_side(up, w);
@@ -455,11 +455,12 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
   uint16_t* cat[2] = {reinterpret_cast<uint16_t*>(ws + pl.cat0), reinterpret_cast<uint16_t*>(ws + pl.cat1)};
   float* feat = reinterpret_cast<float*>(ws + pl.f_feat);
   float* fb[3] = {reinterpret_cast<float*>(ws + pl.f_a), reinterpret_cast<float*>(ws + pl.f_b), reinterpret_cast<float*>(ws + pl.f_c)};
+  const PackedConv* conv = up->convs.data();          // walked in the order up_pack_rrdb packed them
   int cur = 0;                                        // cat[cur] holds the fp16 copy of the current stream in channels 0..63
   {
     ConvIO io; io.x = ws + pl.img8; io.x_channels = up_in_channels(up->shuffle); io.y = feat; io.y_dtype = DT_F32;
     io.y2 = cat[cur]; io.y2_channels = 192; io.y2_chan_off = 0;
-    HDRVAE_TRY(run_conv(ctx, up->conv_first, io, n, hq, wq, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hq, wq, impl, s));
   }
   // fp32 stream buffers: x0 (the RRDB input) lives in feat (first block) or fb[xi]; x1 -> fb[P], x2 -> fb[Q] and the
   // block output overwrites x1's buffer (dead by then), which makes it the next block's x0
@@ -470,11 +471,10 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
     float* outs[3] = {fb[P], fb[Q], fb[P]};
     const float* xin = x0;
     for (int k = 0; k < 3; ++k) {
-      const UpRdb& R = up->rdb[r * 3 + k];
       for (int j = 0; j < 4; ++j) {
         ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y = cat[cur]; io.y_dtype = DT_F16; io.y_channels = 192;
         io.y_chan_off = 64 + 32 * j; io.lrelu = 0.2f;
-        HDRVAE_TRY(run_conv(ctx, R.c[j], io, n, hq, wq, impl, s));
+        HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hq, wq, impl, s));
       }
       ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y_dtype = DT_F32; io.y = outs[k];
       io.y2 = cat[cur ^ 1]; io.y2_channels = 192; io.y2_chan_off = 0;
@@ -482,7 +482,7 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
       // k < 2: x_{k+1} = 0.2 conv5 + x_k (weights and bias packed x 0.2); end of the RRDB:
       // (0.2 conv5 + x2) 0.2 + x0 = 0.04 conv5 + 0.2 x2 + x0 (weights and bias packed x 0.04)
       if (k == 2) { io.res_scale = 0.2f; io.residual2 = x0; }
-      HDRVAE_TRY(run_conv(ctx, R.c[4], io, n, hq, wq, impl, s));
+      HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hq, wq, impl, s));
       xin = outs[k];
       cur ^= 1;
     }
@@ -494,27 +494,27 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
   {
     ConvIO io; io.x = cat[cur]; io.x_channels = 192; io.y = fb[(xi + 2) % 3]; io.y_dtype = DT_F32;
     io.residual = feat; io.res_dtype = DT_F32; io.y2 = ws + pl.u0;
-    HDRVAE_TRY(run_conv(ctx, up->conv_body, io, n, hq, wq, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hq, wq, impl, s));
   }
   uint8_t* hr_in = ws + pl.u0;
   if (u >= 1) {
     ConvIO io; io.x = ws + pl.u0; io.y = ws + pl.u1; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->up1, io, n, hq, wq, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hq, wq, impl, s));
     hr_in = ws + pl.u1;
   }
   if (u >= 2) {
     ConvIO io; io.x = ws + pl.u1; io.y = ws + pl.u2; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->up2, io, n, 2 * hq, 2 * wq, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, 2 * hq, 2 * wq, impl, s));
     hr_in = ws + pl.u2;
   }
   {
     ConvIO io; io.x = hr_in; io.y = ws + pl.u3; io.y_dtype = DT_F16; io.lrelu = 0.2f;
-    HDRVAE_TRY(run_conv(ctx, up->hr, io, n, hu, wu, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hu, wu, impl, s));
   }
   float* last_out = crop ? reinterpret_cast<float*>(ws + pl.cat0) : out4;     // cat0: 384 bytes per h' w' pixel >= 16 4^u
   {
     ConvIO io; io.x = ws + pl.u3; io.y = last_out; io.y_dtype = DT_F32; io.y_channels = 4; io.n_store = 4;
-    HDRVAE_TRY(run_conv(ctx, up->last, io, n, hu, wu, impl, s));
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hu, wu, impl, s));
   }
   if (crop) {
     const int oh = up->scale * h, ow = up->scale * w;
@@ -530,9 +530,9 @@ static int up_forward(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, con
 // Compact forward on n tiles (fp16 [n][h][w][8] in pl.img8) -> the last conv's fp32 [n][h][w][up_last_channels] in pl.last
 static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, cudaStream_t s) {
   hdrvae_ctx* ctx = up->ctx;
-  const int cp = up->body[0].cout_pad;
+  const int cp = up->convs[0].cout_pad;
   uint8_t* act[2] = {ws + pl.act0, ws + pl.act1};
-  const size_t nconv = up->body.size();
+  const size_t nconv = up->convs.size();
   for (size_t k = 0; k < nconv; ++k) {
     ConvIO io;
     io.x = k == 0 ? ws + pl.img8 : act[(k - 1) & 1];
@@ -542,7 +542,7 @@ static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t*
     } else {
       io.y = ws + pl.last; io.y_dtype = DT_F32; io.y_channels = up_last_channels(up);
     }
-    HDRVAE_TRY(run_conv(ctx, up->body[k], io, n, h, w, ctx->conv_impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->convs[k], io, n, h, w, ctx->conv_impl, s));
   }
   return 0;
 }
@@ -556,7 +556,7 @@ static int up_forward_compact(hdrvae_upscaler* up, int n, int h, int w, uint8_t*
 static int up_forward_span(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws, const UpPlan& pl, cudaStream_t s) {
   hdrvae_ctx* ctx = up->ctx;
   const int impl = ctx->conv_impl;
-  const int nf = up->body[0].cout, c4 = 4 * nf;
+  const int nf = up->convs[0].cout, c4 = 4 * nf;
   uint16_t* cat = reinterpret_cast<uint16_t*>(ws + pl.sp_cat);
   float* r[2] = {reinterpret_cast<float*>(ws + pl.sp_r0), reinterpret_cast<float*>(ws + pl.sp_r1)};
   uint8_t* d = ws + pl.sp_d;
@@ -564,12 +564,12 @@ static int up_forward_span(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws
   {
     ConvIO io; io.x = ws + pl.img8; io.x_channels = 8; io.y = r[0]; io.y_dtype = DT_F32; io.y_channels = nf;
     io.y2 = cat; io.y2_channels = c4; io.y2_chan_off = 0;                                   // f
-    HDRVAE_TRY(run_conv(ctx, up->body[0], io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->convs[0], io, n, h, w, impl, s));
   }
   const void* xin = cat;                  // the block input's fp16 operand and its pixel stride
   int xch = c4, cur = 0;
   for (int b = 0; b < 6; ++b) {
-    const PackedConv* c = &up->body[1 + 3 * b];
+    const PackedConv* c = &up->convs[1 + 3 * b];
     {
       ConvIO io; io.x = xin; io.x_channels = xch; io.y_dtype = DT_F16; io.act = ACT_SILU;
       if (b == 5) { io.y = cat; io.y_channels = c4; io.y_chan_off = 3 * nf; }           // b5_2: block_6's SiLU'd out1
@@ -593,14 +593,14 @@ static int up_forward_span(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws
   }
   {
     ConvIO io; io.x = d; io.x_channels = nf; io.y = cat; io.y_dtype = DT_F16; io.y_channels = c4; io.y_chan_off = nf;   // b6
-    HDRVAE_TRY(run_conv(ctx, up->body[19], io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->convs[19], io, n, h, w, impl, s));
   }
   {
     ConvIO io; io.x = cat; io.x_channels = c4; io.y = t[0]; io.y_dtype = DT_F16; io.y_channels = nf;
-    HDRVAE_TRY(run_conv(ctx, up->body[20], io, n, h, w, impl, s));
+    HDRVAE_TRY(run_conv(ctx, up->convs[20], io, n, h, w, impl, s));
   }
   ConvIO io; io.x = t[0]; io.x_channels = nf; io.y = ws + pl.last; io.y_dtype = DT_F32; io.y_channels = up_last_channels(up);
-  return run_conv(ctx, up->body[21], io, n, h, w, impl, s);
+  return run_conv(ctx, up->convs[21], io, n, h, w, impl, s);
 }
 
 // The network on n tiles of h x w cut from img [.][H][W][3] at the origins of `tiles` (image, y0, x0, clamp to [-1, 1])
@@ -618,16 +618,19 @@ static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, con
     else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
     HDRVAE_LAUNCHED();
   }
-  if (!up->compact && !up->span) return up_forward(up, n, h, w, ws, pl, out4, s);
-  if (up->compact) HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s));
-  else HDRVAE_TRY(up_forward_span(up, n, h, w, ws, pl, s));
+  switch (up->arch) {
+    case UP_RRDB: return up_forward_rrdb(up, n, h, w, ws, pl, out4, s);
+    case UP_COMPACT: HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s)); break;
+    case UP_SPAN: HDRVAE_TRY(up_forward_span(up, n, h, w, ws, pl, s)); break;
+  }
   const int sc = up->scale, cl = up_last_channels(up);
   const long long opx = (long long)n * sc * sc * h * w;
   // SPAN adds no base: the plain shuffle
-  ProfScope prof(up->compact ? "upscaler pixel shuffle + base" : "upscaler pixel shuffle",
-                 0.0, (double)n * h * w * (cl * 4 + (up->compact ? 12 : 0)) + opx * 16, s);
+  const bool base = up->arch == UP_COMPACT;
+  ProfScope prof(base ? "upscaler pixel shuffle + base" : "upscaler pixel shuffle",
+                 0.0, (double)n * h * w * (cl * 4 + (base ? 12 : 0)) + opx * 16, s);
   up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float*>(ws + pl.last), cl,
-                                                      up->compact ? img : nullptr, H, W, tiles, n, h, w, sc,
+                                                      base ? img : nullptr, H, W, tiles, n, h, w, sc,
                                                       reinterpret_cast<float4*>(out4));
   HDRVAE_LAUNCHED();
   return 0;
@@ -725,6 +728,60 @@ static UpWs up_make_ws(const hdrvae_upscaler* up, const UpTiling& t, int B, int 
   return w;
 }
 
+// ------------------------------------------------------------------------------------------------ weight shapes
+static std::string up_shape_str(const std::vector<int64_t>& sh) {
+  std::string r = "[";
+  for (size_t i = 0; i < sh.size(); ++i) r += (i ? "," : "") + std::to_string(sh[i]);
+  return r + "]";
+}
+
+// shape of the staged tensor `key`
+static std::string up_shape_str(const hdrvae_ctx* st, const std::string& key) {
+  auto it = st->shapes.find(key);
+  return it == st->shapes.end() ? std::string("(missing)") : up_shape_str(it->second);
+}
+
+// the staged tensor `key` with shape `want`, else an error naming both shapes
+static int up_need(const hdrvae_ctx* st, const char* arch, const std::string& key, const std::vector<int64_t>& want) {
+  auto it = st->shapes.find(key);
+  HDRVAE_REQUIRE(it != st->shapes.end(), "%s upscaler state dict lacks %s (want shape %s)", arch, key.c_str(),
+                 up_shape_str(want).c_str());
+  HDRVAE_REQUIRE(it->second == want, "%s upscaler: %s has shape %s; want %s", arch, key.c_str(),
+                 up_shape_str(it->second).c_str(), up_shape_str(want).c_str());
+  return 0;
+}
+
+// <key>.weight [cout,cin,ks,ks] and <key>.bias [cout] packed for the conv kernel, the weights scaled by wscale
+static int up_pack(hdrvae_ctx* st, const char* arch, const std::string& key, int cout, int cin, int ks, bool upsample,
+                   float wscale, PackedConv* pc, cudaStream_t s) {
+  HDRVAE_TRY(up_need(st, arch, key + ".weight", {cout, cin, ks, ks}));
+  HDRVAE_TRY(up_need(st, arch, key + ".bias", {cout}));
+  return pack_conv(st, st->raw[key + ".weight"], st->raw[key + ".bias"], cout, cin, ks, upsample, wscale, DT_F16, pc, s);
+}
+
+// nf of the first conv `key` [nf,3,ks,ks]: a multiple of 8 in 8..64
+static int up_first_nf(const hdrvae_ctx* st, const char* arch, const std::string& key, int ks, int* nf) {
+  auto it = st->shapes.find(key);
+  HDRVAE_REQUIRE(it != st->shapes.end() && it->second.size() == 4 && it->second[1] == 3 && it->second[2] == ks &&
+                 it->second[3] == ks, "%s upscaler: %s has shape %s; want [nf,3,%d,%d] (3 input channels)", arch,
+                 key.c_str(), up_shape_str(st, key).c_str(), ks, ks);
+  *nf = (int)it->second[0];
+  HDRVAE_REQUIRE(*nf >= 8 && *nf <= 64 && *nf % 8 == 0, "%s upscaler: %s has shape %s; nf must be a multiple of 8 in 8..64",
+                 arch, key.c_str(), up_shape_str(it->second).c_str());
+  return 0;
+}
+
+// scale s of the output conv `key` [3 s^2,nf,3,3] (the pixel shuffle's input): 1, 2 or 4
+static int up_out_scale(const hdrvae_ctx* st, const char* arch, const std::string& key, int nf, int* scale) {
+  auto it = st->shapes.find(key);
+  const int64_t c = it != st->shapes.end() && it->second.size() == 4 && it->second[1] == nf && it->second[2] == 3 &&
+                    it->second[3] == 3 ? it->second[0] : 0;
+  HDRVAE_REQUIRE(c == 3 || c == 12 || c == 48, "%s upscaler: %s has shape %s; want [3*scale^2,%d,3,3] with scale 1, 2 or 4",
+                 arch, key.c_str(), up_shape_str(st, key).c_str(), nf);
+  *scale = c == 3 ? 1 : c == 12 ? 2 : 4;
+  return 0;
+}
+
 }  // namespace hdrvae
 
 // ------------------------------------------------------------------------------------------------ C ABI
@@ -779,15 +836,17 @@ static std::string up_canonical(const std::string& k, int n_up) {
 }
 
 // Upsampling convs of an RRDBNet state dict, found before any key is mapped: from the highest old-arch top-level conv
-// index (conv_last sits at 3u + 4), else from the Real-ESRGAN conv_up1 / conv_up2 / conv_up3 names.  -1: an old-arch
-// layout whose conv_last index fits no u.
-static int up_count_upconvs(const hdrvae_weight_desc* descs, int n, std::string* last_key) {
+// index (conv_last sits at 3u + 4; its weight's key and shape in *top_key / *top_shape), else from the Real-ESRGAN
+// conv_up1 / conv_up2 / conv_up3 names.  -1: an old-arch layout whose conv_last index fits no u.
+static int up_count_upconvs(const hdrvae_weight_desc* descs, int n, std::string* top_key, std::string* top_shape) {
   int top = -1, named = 0;
   for (int i = 0; i < n; ++i) {
-    if (descs[i].name == nullptr) continue;           // refused by the load loop
-    const std::string k = descs[i].name;
+    const hdrvae_weight_desc& d = descs[i];
+    if (d.name == nullptr || d.ndim < 1 || d.ndim > 4) continue;      // refused by the load loop
+    const std::string k = d.name;
     const int K = up_old_top_index(k);
-    if (K > top) { top = K; *last_key = "model." + std::to_string(K) + ".weight"; }
+    if (K > top) { top = K; *top_key = "model." + std::to_string(K) + ".weight"; *top_shape = "(missing)"; }
+    if (k == *top_key) *top_shape = up_shape_str(std::vector<int64_t>(d.shape, d.shape + d.ndim));
     for (int j = 1; j <= 3; ++j)
       if (k == "conv_up" + std::to_string(j) + ".weight") named = std::max(named, j);
   }
@@ -795,21 +854,11 @@ static int up_count_upconvs(const hdrvae_weight_desc* descs, int n, std::string*
   return top >= 4 && (top - 4) % 3 == 0 ? (top - 4) / 3 : -1;
 }
 
-static std::string up_shape_str(const std::vector<int64_t>& sh) {
-  std::string r = "[";
-  for (size_t i = 0; i < sh.size(); ++i) r += (i ? "," : "") + std::to_string(sh[i]);
-  return r + "]";
-}
-
 // Real-ESRGAN SRVGGNetCompact as spandrel loads it with act_type "prelu": body.0 = conv 3 -> nf, body.{2k+1} = PReLU
 // slopes [nf] (k = 0..nc), body.{2+2m} = conv nf -> nf (m < nc), body.{2nc+2} = conv nf -> 3 s^2.  The scale s is
 // limited to powers of two (1, 2, 4): only there do the local fix's resampling coordinates (dst + 0.5) / s equal torch's.
 static int up_pack_compact(hdrvae_upscaler* up, cudaStream_t s) {
   hdrvae_ctx* st = &up->store;
-  auto shape_of = [&](const std::string& k) -> const std::vector<int64_t>* {
-    auto it = st->shapes.find(k);
-    return it == st->shapes.end() ? nullptr : &it->second;
-  };
   int last = -1;
   for (const auto& kv : st->shapes) {
     int bi = -1;
@@ -818,50 +867,30 @@ static int up_pack_compact(hdrvae_upscaler* up, cudaStream_t s) {
   HDRVAE_REQUIRE(last >= 2 && last % 2 == 0,
                  "Compact upscaler: the highest body index is %d; the last conv must sit at an even index >= 2", last);
   const int nc = (last - 2) / 2;
-  const std::vector<int64_t>& w0 = *shape_of("body.0.weight");
-  HDRVAE_REQUIRE(w0.size() == 4 && w0[1] == 3 && w0[2] == 3 && w0[3] == 3,
-                 "Compact upscaler: body.0.weight has shape %s; want [nf,3,3,3] (3 input channels)", up_shape_str(w0).c_str());
-  const int nf = (int)w0[0];
-  HDRVAE_REQUIRE(nf >= 8 && nf <= 64 && nf % 8 == 0,
-                 "Compact upscaler: body.0.weight has shape %s; nf must be a multiple of 8 in 8..64", up_shape_str(w0).c_str());
-  const std::string last_key = "body." + std::to_string(last) + ".weight";
-  const std::vector<int64_t>* wl = shape_of(last_key);
-  HDRVAE_REQUIRE(wl != nullptr && wl->size() == 4 && (*wl)[1] == nf && (*wl)[2] == 3 && (*wl)[3] == 3 &&
-                 ((*wl)[0] == 3 || (*wl)[0] == 12 || (*wl)[0] == 48),
-                 "Compact upscaler: %s has shape %s; want [3*scale^2,%d,3,3] with scale 1, 2 or 4", last_key.c_str(),
-                 wl ? up_shape_str(*wl).c_str() : "(missing)", nf);
-  up->scale = (*wl)[0] == 3 ? 1 : (*wl)[0] == 12 ? 2 : 4;
+  int nf = 0;
+  HDRVAE_TRY(up_first_nf(st, "Compact", "body.0.weight", 3, &nf));
+  HDRVAE_TRY(up_out_scale(st, "Compact", "body." + std::to_string(last) + ".weight", nf, &up->scale));
   up->nb = nc;
-  auto conv = [&](int idx, int cout, int cin, PackedConv* pc) -> int {
-    const std::string k = "body." + std::to_string(idx);
-    const std::vector<int64_t>* w = shape_of(k + ".weight");
-    const std::vector<int64_t>* b = shape_of(k + ".bias");
-    HDRVAE_REQUIRE(w != nullptr && b != nullptr, "Compact upscaler state dict lacks %s.{weight,bias}", k.c_str());
-    HDRVAE_REQUIRE(w->size() == 4 && (*w)[0] == cout && (*w)[1] == cin && (*w)[2] == 3 && (*w)[3] == 3,
-                   "Compact upscaler: %s.weight has shape %s; want [%d,%d,3,3]", k.c_str(), up_shape_str(*w).c_str(), cout, cin);
-    HDRVAE_REQUIRE(b->size() == 1 && (*b)[0] == cout, "Compact upscaler: %s.bias has shape %s; want [%d]", k.c_str(),
-                   up_shape_str(*b).c_str(), cout);
-    return pack_conv(st, st->raw[k + ".weight"], st->raw[k + ".bias"], cout, cin, 3, false, 1.f, DT_F16, pc, s);
-  };
-  up->body.resize((size_t)nc + 2);
-  HDRVAE_TRY(conv(0, nf, 3, &up->body[0]));
-  for (int m = 0; m < nc; ++m) HDRVAE_TRY(conv(2 + 2 * m, nf, nf, &up->body[1 + m]));
-  HDRVAE_TRY(conv(last, 3 * up->scale * up->scale, nf, &up->body[nc + 1]));
-  const int cp = up->body[0].cout_pad;
+  up->convs.resize((size_t)nc + 2);
+  HDRVAE_TRY(up_pack(st, "Compact", "body.0", nf, 3, 3, false, 1.f, &up->convs[0], s));
+  for (int m = 0; m < nc; ++m)
+    HDRVAE_TRY(up_pack(st, "Compact", "body." + std::to_string(2 + 2 * m), nf, nf, 3, false, 1.f, &up->convs[1 + m], s));
+  HDRVAE_TRY(up_pack(st, "Compact", "body." + std::to_string(last), 3 * up->scale * up->scale, nf, 3, false, 1.f,
+                     &up->convs[nc + 1], s));
+  const int cp = up->convs[0].cout_pad;
   for (int k = 0; k <= nc; ++k) {
     const std::string key = "body." + std::to_string(2 * k + 1) + ".weight";
-    const std::vector<int64_t>* sh = shape_of(key);
-    HDRVAE_REQUIRE(sh != nullptr, "Compact upscaler state dict lacks the PReLU slopes %s (only act_type \"prelu\" is supported)",
-                   key.c_str());
-    HDRVAE_REQUIRE(sh->size() == 1 && (*sh)[0] == nf, "Compact upscaler: %s has shape %s; want [%d] (one PReLU slope per channel)",
-                   key.c_str(), up_shape_str(*sh).c_str(), nf);
+    auto it = st->shapes.find(key);
+    HDRVAE_REQUIRE(it != st->shapes.end(), "Compact upscaler state dict lacks the PReLU slopes %s (only act_type \"prelu\" is "
+                   "supported)", key.c_str());
+    HDRVAE_REQUIRE(it->second.size() == 1 && it->second[0] == nf, "Compact upscaler: %s has shape %s; want [%d] (one PReLU "
+                   "slope per channel)", key.c_str(), up_shape_str(it->second).c_str(), nf);
     float* slope = nullptr;
     HDRVAE_TRY(dev_alloc(st, cp * sizeof(float), (void**)&slope));
     HDRVAE_CUDA_OK(cudaMemsetAsync(slope, 0, cp * sizeof(float), s));
     HDRVAE_CUDA_OK(cudaMemcpyAsync(slope, st->raw[key], nf * sizeof(float), cudaMemcpyDeviceToDevice, s));
     up->slopes.push_back(slope);
   }
-  up->compact = true;
   return 0;
 }
 
@@ -873,18 +902,6 @@ static int up_pack_compact(hdrvae_upscaler* up, cudaStream_t s) {
 //   W = w3 . w2 . w1 (+ sk at the centre tap),  b = w3 (sum_{m1,taps} w2 b1 + b2) + b3 + b_sk.
 static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
   hdrvae_ctx* st = &up->store;
-  auto shape_str = [&](const std::string& k) {
-    auto it = st->shapes.find(k);
-    return it == st->shapes.end() ? std::string("(missing)") : up_shape_str(it->second);
-  };
-  // the tensor k with shape `want` (its shape and the wanted one in the error)
-  auto need = [&](const std::string& k, const std::vector<int64_t>& want) -> int {
-    auto it = st->shapes.find(k);
-    HDRVAE_REQUIRE(it != st->shapes.end(), "SPAN upscaler state dict lacks %s (want shape %s)", k.c_str(), up_shape_str(want).c_str());
-    HDRVAE_REQUIRE(it->second == want, "SPAN upscaler: %s has shape %s; want %s", k.c_str(), up_shape_str(it->second).c_str(),
-                   up_shape_str(want).c_str());
-    return 0;
-  };
   auto host = [&](const std::string& k, std::vector<double>* out) -> int {
     size_t cnt = 1;
     for (int64_t d : st->shapes[k]) cnt *= (size_t)d;
@@ -893,26 +910,15 @@ static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
     out->assign(f.begin(), f.end());
     return 0;
   };
-  const std::vector<int64_t>& w0 = st->shapes["conv_1.sk.weight"];
-  HDRVAE_REQUIRE(w0.size() == 4 && w0[1] == 3 && w0[2] == 1 && w0[3] == 1,
-                 "SPAN upscaler: conv_1.sk.weight has shape %s; want [nf,3,1,1] (3 input channels)", up_shape_str(w0).c_str());
-  const int nf = (int)w0[0];
-  HDRVAE_REQUIRE(nf >= 8 && nf <= 64 && nf % 8 == 0,
-                 "SPAN upscaler: conv_1.sk.weight has shape %s; nf must be a multiple of 8 in 8..64", up_shape_str(w0).c_str());
+  int nf = 0;
+  HDRVAE_TRY(up_first_nf(st, "SPAN", "conv_1.sk.weight", 1, &nf));
   for (const auto& kv : st->shapes) {
     int bi = -1;
     HDRVAE_REQUIRE(sscanf(kv.first.c_str(), "block_%d.", &bi) != 1 || (bi >= 1 && bi <= 6),
                    "SPAN upscaler: %s has shape %s; SPAN has exactly the blocks block_1 .. block_6", kv.first.c_str(),
                    up_shape_str(kv.second).c_str());
   }
-  {
-    const std::vector<int64_t>* wu = st->shapes.count("upsampler.0.weight") ? &st->shapes["upsampler.0.weight"] : nullptr;
-    HDRVAE_REQUIRE(wu != nullptr && wu->size() == 4 && (*wu)[1] == nf && (*wu)[2] == 3 && (*wu)[3] == 3 &&
-                   ((*wu)[0] == 3 || (*wu)[0] == 12 || (*wu)[0] == 48),
-                   "SPAN upscaler: upsampler.0.weight has shape %s; want [3*scale^2,%d,3,3] with scale 1, 2 or 4",
-                   shape_str("upsampler.0.weight").c_str(), nf);
-    up->scale = (*wu)[0] == 3 ? 1 : (*wu)[0] == 12 ? 2 : 4;
-  }
+  HDRVAE_TRY(up_out_scale(st, "SPAN", "upsampler.0.weight", nf, &up->scale));
   const bool norm = st->shapes.count("no_norm") == 0;
   // Conv3XC `pre` (cin -> cout) fused into one 3x3 conv, packed with its weights scaled by wscale
   auto conv3xc = [&](const std::string& pre, int cin, int cout, float wscale, PackedConv* pc) -> int {
@@ -921,16 +927,16 @@ static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
     it = st->shapes.find(pre + ".conv.1.weight");
     const int m2 = it != st->shapes.end() && it->second.size() == 4 ? (int)it->second[0] : 0;
     HDRVAE_REQUIRE(m1 >= 1 && m2 >= 1, "SPAN upscaler: %s.conv.0.weight has shape %s and %s.conv.1.weight %s; want [m1,%d,1,1] "
-                   "and [m2,m1,3,3]", pre.c_str(), shape_str(pre + ".conv.0.weight").c_str(), pre.c_str(),
-                   shape_str(pre + ".conv.1.weight").c_str(), cin);
-    HDRVAE_TRY(need(pre + ".sk.weight", {cout, cin, 1, 1}));
-    HDRVAE_TRY(need(pre + ".sk.bias", {cout}));
-    HDRVAE_TRY(need(pre + ".conv.0.weight", {m1, cin, 1, 1}));
-    HDRVAE_TRY(need(pre + ".conv.0.bias", {m1}));
-    HDRVAE_TRY(need(pre + ".conv.1.weight", {m2, m1, 3, 3}));
-    HDRVAE_TRY(need(pre + ".conv.1.bias", {m2}));
-    HDRVAE_TRY(need(pre + ".conv.2.weight", {cout, m2, 1, 1}));
-    HDRVAE_TRY(need(pre + ".conv.2.bias", {cout}));
+                   "and [m2,m1,3,3]", pre.c_str(), up_shape_str(st, pre + ".conv.0.weight").c_str(), pre.c_str(),
+                   up_shape_str(st, pre + ".conv.1.weight").c_str(), cin);
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".sk.weight", {cout, cin, 1, 1}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".sk.bias", {cout}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.0.weight", {m1, cin, 1, 1}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.0.bias", {m1}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.1.weight", {m2, m1, 3, 3}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.1.bias", {m2}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.2.weight", {cout, m2, 1, 1}));
+    HDRVAE_TRY(up_need(st, "SPAN", pre + ".conv.2.bias", {cout}));
     std::vector<double> sk, skb, w1, b1, w2, b2, w3, b3;
     HDRVAE_TRY(host(pre + ".sk.weight", &sk)); HDRVAE_TRY(host(pre + ".sk.bias", &skb));
     HDRVAE_TRY(host(pre + ".conv.0.weight", &w1)); HDRVAE_TRY(host(pre + ".conv.0.bias", &b1));
@@ -970,24 +976,72 @@ static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
     HDRVAE_CUDA_OK(cudaMemcpy(db, bf.data(), bf.size() * sizeof(float), cudaMemcpyHostToDevice));
     return pack_conv(st, dw, db, cout, cin, 3, false, wscale, DT_F16, pc, s);
   };
-  up->body.resize(22);
+  up->convs.resize(22);
   // (x - mean) 255: the input stage subtracts the mean, conv_1's weights carry the 255 (its bias is not scaled)
-  HDRVAE_TRY(conv3xc("conv_1", 3, nf, norm ? 255.f : 1.f, &up->body[0]));
+  HDRVAE_TRY(conv3xc("conv_1", 3, nf, norm ? 255.f : 1.f, &up->convs[0]));
   for (int b = 0; b < 6; ++b)
     for (int c = 0; c < 3; ++c)
       HDRVAE_TRY(conv3xc("block_" + std::to_string(b + 1) + ".c" + std::to_string(c + 1) + "_r", nf, nf, 1.f,
-                         &up->body[1 + 3 * b + c]));
-  HDRVAE_TRY(conv3xc("conv_2", nf, nf, 1.f, &up->body[19]));
-  HDRVAE_TRY(need("conv_cat.weight", {nf, 4 * nf, 1, 1}));
-  HDRVAE_TRY(need("conv_cat.bias", {nf}));
-  HDRVAE_TRY(pack_conv(st, st->raw["conv_cat.weight"], st->raw["conv_cat.bias"], nf, 4 * nf, 1, false, 1.f, DT_F16, &up->body[20], s));
-  HDRVAE_TRY(need("upsampler.0.bias", {3 * up->scale * up->scale}));
-  HDRVAE_TRY(pack_conv(st, st->raw["upsampler.0.weight"], st->raw["upsampler.0.bias"], 3 * up->scale * up->scale, nf, 3, false,
-                       1.f, DT_F16, &up->body[21], s));
+                         &up->convs[1 + 3 * b + c]));
+  HDRVAE_TRY(conv3xc("conv_2", nf, nf, 1.f, &up->convs[19]));
+  HDRVAE_TRY(up_pack(st, "SPAN", "conv_cat", nf, 4 * nf, 1, false, 1.f, &up->convs[20], s));
+  HDRVAE_TRY(up_pack(st, "SPAN", "upsampler.0", 3 * up->scale * up->scale, nf, 3, false, 1.f, &up->convs[21], s));
   if (norm) up->mean = make_float3(0.4488f, 0.4371f, 0.4040f);
   up->nb = 6;
-  up->span = true;
   return 0;
+}
+
+// ESRGAN / RRDBNet (nf 64, gc 32) in Real-ESRGAN names (staging mapped the old-arch keys): conv_first, nb RRDBs of three
+// dense blocks (conv1 .. conv5), conv_body, n_up upsampling convs, conv_hr, conv_last.  n_up, top_*: up_count_upconvs.
+static int up_pack_rrdb(hdrvae_upscaler* up, int n_up, const std::string& top_key, const std::string& top_shape,
+                        cudaStream_t s) {
+  hdrvae_ctx* st = &up->store;
+  int nb = 0;
+  for (const auto& kv : st->shapes) {
+    int bi = -1;
+    if (sscanf(kv.first.c_str(), "body.%d.", &bi) == 1) nb = std::max(nb, bi + 1);
+  }
+  HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
+                 "no Real-ESRGAN Compact model (body.0.weight without conv_first) or SPAN model (conv_1.sk.weight)");
+  up->nb = nb;
+  // the layout: u upsampling convs (counted on load) and the pixel-unshuffle factor f from conv_first's 3 f^2 input channels
+  HDRVAE_REQUIRE(n_up >= 0, "RRDBNet: %s has shape %s; an old-arch RRDBNet's last top-level conv sits at index 3u + 4 "
+                 "(4, 7 or 10 for u = 0, 1 or 2 upsampling convs)", top_key.c_str(), top_shape.c_str());
+  HDRVAE_REQUIRE(n_up <= 2, "RRDBNet: %s has shape %s: a third upsampling conv (an 8x RRDBNet) is not supported; RRDBNet "
+                 "runs with 0, 1 or 2 upsampling convs", top_key.empty() ? "conv_up3.weight" : "model.9.weight",
+                 up_shape_str(st, "conv_up3.weight").c_str());
+  auto it = st->shapes.find("conv_first.weight");
+  HDRVAE_REQUIRE(it != st->shapes.end(), "upscaler state dict lacks conv_first.{weight,bias}");
+  const std::vector<int64_t>& w0 = it->second;
+  const int64_t cin = w0.size() == 4 ? w0[1] : 0;
+  HDRVAE_REQUIRE(cin == 3 || cin == 12 || cin == 48, "RRDBNet: conv_first.weight has shape %s; want [64,3 f^2,3,3] with "
+                 "pixel-unshuffle factor f = 1, 2 or 4 (3, 12 or 48 input channels)", up_shape_str(w0).c_str());
+  const int f = cin == 3 ? 1 : cin == 12 ? 2 : 4;
+  HDRVAE_REQUIRE((1 << n_up) >= f, "RRDBNet: conv_first.weight has shape %s (pixel-unshuffle factor %d) and the model has "
+                 "%d upsampling conv(s): its scale 2^%d / %d would be below 1", up_shape_str(w0).c_str(), f, n_up, n_up, f);
+  up->n_up = n_up;
+  up->shuffle = f;
+  up->scale = (1 << n_up) / f;
+  up->convs.resize(1 + 15 * (size_t)nb + n_up + 3);
+  PackedConv* pc = up->convs.data();                  // filled in launch order
+  HDRVAE_TRY(up_pack(st, "RRDBNet", "conv_first", 64, 3 * f * f, 3, false, 1.f, pc++, s));
+  for (int i = 0; i < nb; ++i)
+    for (int r = 0; r < 3; ++r) {
+      const std::string base = "body." + std::to_string(i) + ".rdb" + std::to_string(r + 1) + ".conv";
+      for (int j = 0; j < 4; ++j)
+        HDRVAE_TRY(up_pack(st, "RRDBNet", base + std::to_string(j + 1), 32, 64 + 32 * j, 3, false, 1.f, pc++, s));
+      // residual scaling folded into conv5's weights and bias: 0.2, and 0.2 * 0.2 for the block that ends an RRDB
+      const float rs = r == 2 ? 0.2f * 0.2f : 0.2f;
+      HDRVAE_TRY(up_pack(st, "RRDBNet", base + "5", 64, 192, 3, false, rs, pc, s));
+      up_scale_f32_kernel<<<1, 64, 0, s>>>(pc->bias, 64, rs);
+      HDRVAE_CUDA_OK(cudaGetLastError());
+      ++pc;
+    }
+  HDRVAE_TRY(up_pack(st, "RRDBNet", "conv_body", 64, 64, 3, false, 1.f, pc++, s));
+  for (int k = 1; k <= n_up; ++k)
+    HDRVAE_TRY(up_pack(st, "RRDBNet", "conv_up" + std::to_string(k), 64, 64, 3, true, 1.f, pc++, s));
+  HDRVAE_TRY(up_pack(st, "RRDBNet", "conv_hr", 64, 64, 3, false, 1.f, pc++, s));
+  return up_pack(st, "RRDBNet", "conv_last", 3, 64, 3, false, 1.f, pc, s);
 }
 
 // After packing: waits for the copies, frees the staging buffers and the fp32 copies of the state dict.
@@ -1017,15 +1071,8 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
   HDRVAE_CUDA_OK(cudaSetDevice(st->device));
   cudaStream_t s = nullptr;
   std::vector<void*> staging;
-  int nb = 0;
-  bool has_body0 = false, has_conv_first = false;      // Compact: body.0.weight and no conv_first (in either layout)
-  std::string top_key;
-  const int n_up = up_count_upconvs(descs, n, &top_key);
-  auto desc_shape = [&](const std::string& k) {
-    for (int i = 0; i < n; ++i)
-      if (descs[i].name && k == descs[i].name) return up_shape_str(std::vector<int64_t>(descs[i].shape, descs[i].shape + descs[i].ndim));
-    return std::string("(missing)");
-  };
+  std::string top_key, top_shape;
+  const int n_up = up_count_upconvs(descs, n, &top_key, &top_shape);
   for (int i = 0; i < n; ++i) {
     const hdrvae_weight_desc& d = descs[i];
     HDRVAE_REQUIRE(d.name && d.data && d.ndim >= 1 && d.ndim <= 4, "hdrvae_upscaler_load_weights: bad descriptor %d", i);
@@ -1044,74 +1091,19 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
     HDRVAE_TRY(launch_to_f32(stage, d.dtype, f, cnt, s));
     st->raw[name] = f;
     st->shapes[name] = shp;
-    has_body0 = has_body0 || name == "body.0.weight";
-    has_conv_first = has_conv_first || name.compare(0, 11, "conv_first.") == 0;
-    int bi = -1;
-    if (sscanf(name.c_str(), "body.%d.", &bi) == 1) nb = std::max(nb, bi + 1);
   }
-  // (checked first: the RRDB block scan below also counts the Compact's body.N keys)
-  if (has_body0 && !has_conv_first) {
-    HDRVAE_TRY(up_pack_compact(up, s));
-    return up_finish_load(up, staging, s);
+  // Compact: body.0.weight and no conv_first (in either layout); SPAN: conv_1.sk.weight; anything else is an RRDBNet
+  bool has_conv_first = false;
+  for (const auto& kv : st->shapes) has_conv_first = has_conv_first || kv.first.compare(0, 11, "conv_first.") == 0;
+  UpArch arch = UP_RRDB;
+  if (st->shapes.count("body.0.weight") && !has_conv_first) arch = UP_COMPACT;
+  else if (st->shapes.count("conv_1.sk.weight")) arch = UP_SPAN;
+  switch (arch) {
+    case UP_RRDB: HDRVAE_TRY(up_pack_rrdb(up, n_up, top_key, top_shape, s)); break;
+    case UP_COMPACT: HDRVAE_TRY(up_pack_compact(up, s)); break;
+    case UP_SPAN: HDRVAE_TRY(up_pack_span(up, s)); break;
   }
-  if (st->shapes.count("conv_1.sk.weight")) {
-    HDRVAE_TRY(up_pack_span(up, s));
-    return up_finish_load(up, staging, s);
-  }
-  HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
-                 "no Real-ESRGAN Compact model (body.0.weight without conv_first) or SPAN model (conv_1.sk.weight)");
-  up->nb = nb;
-  // the layout: u upsampling convs (found above) and the pixel-unshuffle factor f from conv_first's 3 f^2 input channels
-  HDRVAE_REQUIRE(n_up >= 0, "RRDBNet: %s has shape %s; an old-arch RRDBNet's last top-level conv sits at index 3u + 4 "
-                 "(4, 7 or 10 for u = 0, 1 or 2 upsampling convs)", top_key.c_str(), desc_shape(top_key).c_str());
-  {
-    const std::string k3 = top_key.empty() ? "conv_up3.weight" : "model.9.weight";
-    HDRVAE_REQUIRE(n_up <= 2, "RRDBNet: %s has shape %s: a third upsampling conv (an 8x RRDBNet) is not supported; RRDBNet "
-                   "runs with 0, 1 or 2 upsampling convs", k3.c_str(), desc_shape(k3).c_str());
-  }
-  {
-    auto it = st->shapes.find("conv_first.weight");
-    HDRVAE_REQUIRE(it != st->shapes.end(), "upscaler state dict lacks conv_first.{weight,bias}");
-    const std::vector<int64_t>& w0 = it->second;
-    const int64_t cin = w0.size() == 4 ? w0[1] : 0;
-    HDRVAE_REQUIRE(cin == 3 || cin == 12 || cin == 48, "RRDBNet: conv_first.weight has shape %s; want [64,3 f^2,3,3] with "
-                   "pixel-unshuffle factor f = 1, 2 or 4 (3, 12 or 48 input channels)", up_shape_str(w0).c_str());
-    const int f = cin == 3 ? 1 : cin == 12 ? 2 : 4;
-    HDRVAE_REQUIRE((1 << n_up) >= f, "RRDBNet: conv_first.weight has shape %s (pixel-unshuffle factor %d) and the model has "
-                   "%d upsampling conv(s): its scale 2^%d / %d would be below 1", up_shape_str(w0).c_str(), f, n_up, n_up, f);
-    up->n_up = n_up;
-    up->shuffle = f;
-    up->scale = (1 << n_up) / f;
-  }
-  auto conv = [&](const std::string& k, int cout, int cin, bool upsample, float scale, PackedConv* pc) -> int {
-    auto it = st->shapes.find(k + ".weight");
-    HDRVAE_REQUIRE(it != st->shapes.end() && st->raw.count(k + ".bias"), "upscaler state dict lacks %s.{weight,bias}", k.c_str());
-    const auto& sh = it->second;
-    HDRVAE_REQUIRE(sh.size() == 4 && sh[0] == cout && sh[1] == cin && sh[2] == 3 && sh[3] == 3,
-                   "%s.weight has the wrong shape %s (want [%d,%d,3,3]: RRDBNet nf 64, gc 32)", k.c_str(),
-                   up_shape_str(sh).c_str(), cout, cin);
-    HDRVAE_TRY(pack_conv(st, st->raw[k + ".weight"], st->raw[k + ".bias"], cout, cin, 3, upsample, scale, DT_F16, pc, s));
-    if (scale != 1.f) {
-      up_scale_f32_kernel<<<1, 64, 0, s>>>(pc->bias, cout, scale);
-      HDRVAE_CUDA_OK(cudaGetLastError());
-    }
-    return 0;
-  };
-  HDRVAE_TRY(conv("conv_first", 64, 3 * up->shuffle * up->shuffle, false, 1.f, &up->conv_first));
-  up->rdb.resize((size_t)nb * 3);
-  for (int i = 0; i < nb; ++i)
-    for (int r = 0; r < 3; ++r) {
-      UpRdb& R = up->rdb[(size_t)i * 3 + r];
-      const std::string base = "body." + std::to_string(i) + ".rdb" + std::to_string(r + 1) + ".conv";
-      for (int j = 0; j < 4; ++j) HDRVAE_TRY(conv(base + std::to_string(j + 1), 32, 64 + 32 * j, false, 1.f, &R.c[j]));
-      // residual scaling folded into conv5: 0.2 inside a dense block, 0.2 * 0.2 for the block that ends an RRDB
-      HDRVAE_TRY(conv(base + "5", 64, 192, false, r == 2 ? 0.2f * 0.2f : 0.2f, &R.c[4]));
-    }
-  HDRVAE_TRY(conv("conv_body", 64, 64, false, 1.f, &up->conv_body));
-  if (n_up >= 1) HDRVAE_TRY(conv("conv_up1", 64, 64, true, 1.f, &up->up1));
-  if (n_up >= 2) HDRVAE_TRY(conv("conv_up2", 64, 64, true, 1.f, &up->up2));
-  HDRVAE_TRY(conv("conv_hr", 64, 64, false, 1.f, &up->hr));
-  HDRVAE_TRY(conv("conv_last", 3, 64, false, 1.f, &up->last));
+  up->arch = arch;
   return up_finish_load(up, staging, s);
 }
 
