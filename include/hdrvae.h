@@ -241,7 +241,7 @@ int hdrvae_rows_run_direct(hdrvae_rows* state, void* stream);
 /* After HDRVAE_EX_END: copy the statistics (global: pre/post/conv/pre3; local slab: out_*, pixel counts) and free. */
 int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
 
-/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for three of the
+/* ---- HDR upscaler: replaces HDRUpscaleWithModel.upscale (hdr_upscale_with_model.py:148-263) for four of the
  * architectures spandrel loads from models/upscale_models (:73-77):
  *   - ESRGAN / RRDBNet (nf 64, gc 32, any block count) with u = 0, 1 or 2 upsampling convs (nearest 2x + conv) and
  *     pixel-unshuffle factor f = 1, 2 or 4 (conv_first reads 3 f^2 channels: RealESRGAN_x2plus has u 2, f 2), scale
@@ -252,8 +252,16 @@ int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
  *     "compact" models): 3 input channels, nf a multiple of 8 in 8..64, any body depth, scale s = 1, 2 or 4;
  *   - SPAN (spandrel's "SPAN"): 3 input channels, nf a multiple of 8 in 8..64, blocks block_1 .. block_6, any Conv3XC
  *     hidden width, scale s = 1, 2 or 4, with or without the input normalisation (buffer no_norm).  Every Conv3XC is
- *     fused from conv.0 / conv.1 / conv.2 and sk at load time, as its eval-mode forward does; eval_conv.* is ignored.
- * The layout is recognised by its keys (Compact: body.0.weight and no conv_first; SPAN: conv_1.sk.weight); anything else is rejected with a
+ *     fused from conv.0 / conv.1 / conv.2 and sk at load time, as its eval-mode forward does; eval_conv.* is ignored;
+ *   - SwinIR (spandrel's "SwinIR"): 3 input channels, embed_dim C <= 256, head dimension C / heads <= 32, window 8 (shift 4
+ *     in odd blocks), any RSTB count and depths, any MLP width, resi_connection "1conv" or "3conv", with or without
+ *     patch_embed.norm, no absolute_pos_embed; upsampler "pixelshuffle", "pixelshuffledirect" or "nearest+conv" at
+ *     s = 2 or 4, or "" at s = 1.  A tile is reflect-padded to a multiple of 8 (the pad must be shorter than the side), the
+ *     shifted-window mask is computed for the padded size, and the output is cropped.  The stored relative_position_index
+ *     and attn_mask buffers are not read.  HAT (conv_block / overlap_attn / relative_position_index_SA keys), 3x and 8x
+ *     are rejected.
+ * The layout is recognised by its keys (Compact: body.0.weight and no conv_first; SPAN: conv_1.sk.weight; SwinIR:
+ * layers.0.residual_group.blocks.0.attn.relative_position_bias_table); anything else is rejected with a
  * message naming the tensor and its shape.  The model object is created against a decode context (device, SM count,
  * conv implementation).  s below is the model's scale (hdrvae_upscaler_scale).
  *   load_weights : the model's state dict, host or device pointers.  RRDBNet in either key layout (Real-ESRGAN
@@ -261,9 +269,12 @@ int hdrvae_rows_end(hdrvae_rows* state, hdrvae_stats* stats, void* stream);
  *                  BasicSR-spandrel "model.0 / model.1.sub.N.RDBK.convJ.0 / ...", whose top-level convs sit at 0,
  *                  3 + 3k (upsampling conv k + 1), 3u + 2 (conv_hr) and 3u + 4 (conv_last)); Compact as
  *                  "body.0 / body.1 (PReLU) / ... / body.{2nc+2}"; SPAN as "conv_1 / block_K.cJ_r / conv_2" (each
- *                  ".sk / .conv.0 / .conv.1 / .conv.2 / .eval_conv") / "conv_cat" / "upsampler.0" [/ "no_norm"];
- *   blocks       : RRDB blocks, the Compact's body convs nc (0 allowed), or 6 (SPAN); < 0 without a model;
- *   scale        : 2^u / f for RRDBNet, s for Compact and SPAN; < 0 before the weights are loaded;
+ *                  ".sk / .conv.0 / .conv.1 / .conv.2 / .eval_conv") / "conv_cat" / "upsampler.0" [/ "no_norm"]; SwinIR
+ *                  in the network_swinir.py names ("conv_first / layers.i.residual_group.blocks.j.* / layers.i.conv /
+ *                  norm / conv_after_body / ...");
+ *   blocks       : RRDB blocks, the Compact's body convs nc (0 allowed), 6 (SPAN) or the RSTB count (SwinIR); < 0
+ *                  without a model;
+ *   scale        : 2^u / f for RRDBNet, s for Compact, SPAN and SwinIR; < 0 before the weights are loaded;
  *   forward      : the network (+ reversal hook) on n equal tiles, x [n,h,w,3] -> y [n,s*h,s*w,3], float32 device
  *                  (kernel-level parity entry: what `upscale_model(a)` with the forward hook returns, :92-105; for
  *                  Compact that includes the nearest-upsampled input the network adds);
@@ -322,7 +333,7 @@ int hdrvae_epilogue(hdrvae_ctx* ctx, const void* pre_nhwc, int dtype, int B, int
  * dense.  With x_channels, Cin is free (x_channels % 8 == 0, x_channels >= Cin); with y_channels, Cout is free
  * (y_chan_off % 4 == 0, y_channels % 4 == 0, y_chan_off + round_up(Cout, 4) <= y_channels) and the residuals share
  * y's addressing. */
-enum { HDRVAE_ACT_NONE = 0, HDRVAE_ACT_SILU = 1, HDRVAE_ACT_GATE = 2 };
+enum { HDRVAE_ACT_NONE = 0, HDRVAE_ACT_SILU = 1, HDRVAE_ACT_GATE = 2, HDRVAE_ACT_GELU = 3 };
 typedef struct hdrvae_conv_extra {
   int32_t x_channels;        /* pixel stride of x in elements (0: Cin); the conv reads the first Cin channels */
   int32_t y_channels;        /* pixel stride of y (0: Cout) ... */
@@ -336,7 +347,8 @@ typedef struct hdrvae_conv_extra {
   const float* residual2;    /* optional float32 in y's layout */
   const float* act_slope;    /* optional per-channel PReLU slopes, Cout floats */
   float lrelu;               /* LeakyReLU slope (0: none) */
-  int32_t act;               /* HDRVAE_ACT_*: SiLU, or the gate y = (t + residual terms)(sigmoid(t) - 1/2) of SPAN */
+  int32_t act;               /* HDRVAE_ACT_*: SiLU, the gate y = (t + residual terms)(sigmoid(t) - 1/2) of SPAN, or
+                                GELU (erf form, nn.GELU()) applied last */
 } hdrvae_conv_extra;
 int hdrvae_conv2d(hdrvae_ctx* ctx, const void* x, int x_dtype, int B, int H, int W, int Cin, const float* w,
                   const float* bias, int Cout, int ksize, int upsample2x, const void* residual, int res_dtype,
@@ -360,6 +372,22 @@ int hdrvae_groupnorm_silu(hdrvae_ctx* ctx, const void* x, int x_dtype, int B, in
  * itself allocates a scratch copy of the operands in the decoder's layout (q|k interleaved, v transposed). */
 int hdrvae_attention(hdrvae_ctx* ctx, const void* q, const void* k, const void* v, int dtype, int B, int T,
                      void* o, void* stream);
+
+/* LayerNorm over the C <= 256 channels of each of n_tokens fp32 tokens x [n_tokens][C] (eps 1e-5, fp32 statistics,
+ * torch.nn.LayerNorm): y = (x - mean) / sqrt(var + eps) * gamma + beta, gamma / beta float32 [C].  y_dtype HDRVAE_F32
+ * (y [n_tokens][C]) or HDRVAE_F16 (y [n_tokens][y_channels], y_channels >= C a multiple of 8; channels C .. y_channels - 1
+ * are written as zero).  The SwinIR upscaler's norm1 / norm2 / norm / patch_embed.norm. */
+int hdrvae_layernorm(hdrvae_ctx* ctx, const float* x, long long n_tokens, int C, const float* gamma, const float* beta,
+                     void* y, int y_dtype, int y_channels, void* stream);
+
+/* SwinIR's (shifted) window attention, window 8, head dim padded to 32: qkv fp16 [B][H][W][3 * heads * 32] holds per pixel
+ * q (pre-scaled by head_dim^-0.5), k and v, each head-major with 32 channels per head (zero beyond the head dim); bias_table
+ * float32 [225][heads] is the relative-position bias table; shift 0 or 4.  H and W are multiples of 8.  The windows tile
+ * the image rolled by (-shift, -shift) (torch.roll, as the Swin transformer layer does); with a shift, keys of another
+ * region of calculate_mask's partition of the H x W image get -100.  o fp16 [B][H][W][heads * 32]: softmax(q k^T + bias
+ * (+ mask)) v written back at the un-shifted pixel of each query, head-major. */
+int hdrvae_window_attention(hdrvae_ctx* ctx, const void* qkv, int B, int H, int W, int heads, const float* bias_table,
+                            int shift, void* o, void* stream);
 
 /* Exact quantiles by radix select over a device float32 array (statistical profiling; BASELINE.json north_star).
  * The reference computes none (SURVEY.md 0.6): defined as torch.quantile(x, q, interpolation="lower") =

@@ -21,7 +21,7 @@ F32, BF16, F16 = range(3)
 PRECISION_BF16, PRECISION_F16, PRECISION_HIGH = 0, 1, 2
 CONV_TCGEN05, CONV_DIRECT = 0, 1
 RAW_NMIN, RAW_NMAX, RAW_NSUM = 4, 4, 8
-ACT_NONE, ACT_SILU, ACT_GATE = range(3)
+ACT_NONE, ACT_SILU, ACT_GATE, ACT_GELU = range(4)
 ABI_VERSION = 2
 
 
@@ -110,6 +110,8 @@ SIGNATURES = {
     "hdrvae_conv2d_stats_chunks": (_i, [_i, _i, _i]),
     "hdrvae_groupnorm_silu": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp, _i, _vp]),
     "hdrvae_attention": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "hdrvae_layernorm": (_i, [_vp, _vp, C.c_longlong, _i, _vp, _vp, _vp, _i, _i, _vp]),
+    "hdrvae_window_attention": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp]),
     "hdrvae_quantiles": (_i, [_vp, C.c_longlong, C.POINTER(C.c_double), _i, C.POINTER(C.c_float), _vp]),
     "hdrvae_pack_half": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
     "hdrvae_upscaler_create": (_i, [_vp, C.POINTER(_vp)]),

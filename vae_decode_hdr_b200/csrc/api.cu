@@ -1538,7 +1538,7 @@ int hdrvae_conv2d(hdrvae_ctx* ctx, const void* x, int x_dtype, int B, int H, int
     else
       HDRVAE_REQUIRE(e.y2_chan_off == 0, "hdrvae_conv2d: y2_chan_off needs y2_channels");
   }
-  HDRVAE_REQUIRE(e.act >= HDRVAE_ACT_NONE && e.act <= HDRVAE_ACT_GATE, "hdrvae_conv2d: bad act (%d)", e.act);
+  HDRVAE_REQUIRE(e.act >= HDRVAE_ACT_NONE && e.act <= HDRVAE_ACT_GELU, "hdrvae_conv2d: bad act (%d)", e.act);
   HDRVAE_CUDA_OK(cudaSetDevice(ctx->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   hdrvae_ctx tmp;                     // owns the temporary packed operands

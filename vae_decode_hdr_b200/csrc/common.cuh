@@ -59,7 +59,7 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 enum { DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2,
        DT_F16X3 = 3 /* internal: fp16 [hi | lo | hi] K-concatenated operand of the "high" precision mode (groupnorm output) */ };
 __host__ __device__ inline int dt_bytes(int dt) { return dt == DT_F32 ? 4 : 2; }
-enum { ACT_NONE = 0, ACT_SILU = 1, ACT_GATE = 2 };   // GemmParams::act
+enum { ACT_NONE = 0, ACT_SILU = 1, ACT_GATE = 2, ACT_GELU = 3 };   // GemmParams::act
 
 // out[n, y*sy+py, x*sx+px, col] = row_scale[x] * alpha * sum_{t<ntaps} sum_{c<K_per_tap}
 //        A[n, y+dy[t], x+dx[t], c] * Bw[col][t*K_per_tap + c]  + bias[col]  (+ residual[...])
@@ -113,7 +113,8 @@ struct GemmParams {
   float lrelu;       // LeakyReLU negative slope applied last (0: none)
   const float* act_slope;  // per-column PReLU negative slope, zero-padded to the GEMM's columns, applied last; or null
   int act;           // ACT_SILU: y = t sigmoid(t), applied last; ACT_GATE: y = (t + r)(sigmoid(t) - 1/2) for t = alpha acc +
-                     // bias and r = res_scale * residual, in place of the residual add (SPAN); ACT_NONE: neither
+                     // bias and r = res_scale * residual, in place of the residual add (SPAN); ACT_GELU: y = gelu_erf(t),
+                     // applied last (SwinIR's MLP; generic builds only); ACT_NONE: none
   int n_store;       // columns actually stored (multiple of 4; 0: n_cols) — a Cout padded up to 32 stores less
   const float* row_scale;  // per M row (x coordinate) multiplier of the accumulator, or null
   float alpha;       // accumulator scale applied before bias (1.0 for convs)
@@ -190,6 +191,8 @@ __device__ __forceinline__ float silu_nr(float v) {
   r = r * fmaf(-d, r, 2.f);
   return v * r;
 }
+// nn.GELU() (the exact erf form, not the tanh approximation): the conv epilogue's ACT_GELU
+__device__ __forceinline__ float gelu_erf(float v) { return 0.5f * v * (1.f + erff(v * 0.70710678118654752f)); }
 // sigmoid(v) by silu_nr's steps (one XU operation): the conv epilogue's SiLU and SPAN gate
 __device__ __forceinline__ float sigmoid_nr(float v) {
   float e;

@@ -1,5 +1,6 @@
 // Internal declarations shared by api.cu (decoder program, C ABI) and upscaler.cu.
 #pragma once
+#include <algorithm>
 #include <string>
 #include <vector>
 #include <map>
@@ -63,6 +64,12 @@ int launch_attention_fused(const void* q, long long q_ld, long long q_img_stride
                            long long k_img_stride, int k_rows, const void* vt, long long vt_ld, long long vt_img_stride,
                            int n_keys, void* o, long long o_img_stride, int n_img, int dt, float alpha, int cta_group,
                            int num_sms, float* part, float* ml, long long part_rows, cudaStream_t s);
+// SwinIR (swin.cu): LayerNorm of fp32 tokens to fp32 [P][C] or fp16 [P][y_ld]; window attention; fp16 pixel shuffle by 2
+int launch_layernorm(const float* x, long long P, int C, const float* gamma, const float* beta, void* y, int y_dtype,
+                     int y_ld, cudaStream_t s);
+int launch_window_attention(const void* qkv, int B, int H, int W, int heads, const float* table, int shift, void* o,
+                            cudaStream_t s);
+int launch_pixel_shuffle2_f16(const void* in, int n, int h, int w, int c, void* out, cudaStream_t s);
 int launch_raw_stats_merge(const hdrvae_raw_stats* blocks, int n, hdrvae_raw_stats* dst, cudaStream_t s);
 
 // ---- device-driven exchanges of the row-tiled decode (rows_p2p.cu) --------------------------------------------

@@ -61,7 +61,8 @@ struct TcConfig {
   static constexpr int kPitch = kSlabPitch;                          // 128-byte lines per slab row
   static constexpr int kStagesFit = (kSmemLimit - kSmemFixed - kSlabStages * kSlabBuf) / kStageBytes;
   static constexpr int kStages = kStagesFit > 8 ? 8 : kStagesFit;
-  static constexpr int kTmemCols = 2 * BLOCK_N;   // two accumulator stages (power of two: 64 ... 512)
+  // two accumulator stages; the allocation is a power of two (64 ... 512), so a 192-column tile takes 512 columns
+  static constexpr int kTmemCols = 2 * BLOCK_N <= 64 ? 64 : 2 * BLOCK_N <= 128 ? 128 : 2 * BLOCK_N <= 256 ? 256 : 512;
   static constexpr int kSmemBytes = kStages * kStageBytes + kSlabStages * kSlabBuf + kSmemFixed;
   static_assert(kStages >= (SLAB ? 2 : 3) && kSmemBytes <= kSmemLimit, "shared memory plan does not fit");
   static_assert(SLAB == 0 || ((SLAB == 9 || SLAB == 3 || SLAB == 1) && KSUB == 1), "the slab variant stages 9, 3 or 1 taps of B per pipeline slot");
@@ -582,6 +583,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const bool has_prelu = kGen ? (p.act_slope != nullptr) : ((EPI & EPI_PRELU) != 0);
     const bool has_silu = kGen ? (p.act == ACT_SILU) : ((EPI & EPI_SILU) != 0);
     const bool has_gate = kGen ? (p.act == ACT_GATE) : ((EPI & EPI_GATE) != 0);
+    const bool has_gelu = kGen && p.act == ACT_GELU;
     const float lrelu = p.lrelu, res_scale = p.res_scale;
     const int n_store = p.n_store > 0 ? p.n_store : p.n_cols;
     const int q = warp & 3;                 // TMEM lane quarter this warp may access
@@ -941,6 +943,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             t.x *= sigmoid_nr(t.x); t.y *= sigmoid_nr(t.y); t.z *= sigmoid_nr(t.z); t.w *= sigmoid_nr(t.w);
           }
           if (has_gate) { t.x *= g.x; t.y *= g.y; t.z *= g.z; t.w *= g.w; }
+          if (has_gelu) { t.x = gelu_erf(t.x); t.y = gelu_erf(t.y); t.z = gelu_erf(t.z); t.w = gelu_erf(t.w); }
           if (has_out2) {
             // second, scaled 16-bit copy of the output: the tensor-core operand of a conv that consumes this
             // (un-normalised) tensor directly; the power-of-two scale keeps fp16 far from overflow
@@ -1172,7 +1175,7 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
     const bool n32 = p.n_cols <= 32;
     int epi = -1;
     if (use_cg == 2 && !p.round_tf32 && p.stats == nullptr && !p.bias_per_row && p.row_scale == nullptr &&
-        (p.residual == nullptr || p.res_dtype == DT_F32)) {
+        (p.residual == nullptr || p.res_dtype == DT_F32) && p.act != ACT_GELU) {
       epi = (p.out_dtype != DT_F32 ? EPI_OUT16 : 0) | (p.residual ? EPI_RES : 0) | (p.residual2 ? EPI_RES2 : 0) |
             (p.out2 ? EPI_OUT2 : 0) | (p.lrelu != 0.f ? EPI_LRELU : 0) | (p.act_slope ? EPI_PRELU : 0) |
             (p.act == ACT_SILU ? EPI_SILU : 0) | (p.act == ACT_GATE ? EPI_GATE : 0);
@@ -1215,6 +1218,20 @@ int launch_gemm_tc(const GemmParams& p, int num_sms, cudaStream_t stream) {
                        : launch_tc<64, false, 1, EPI_GENERIC>(p, num_sms, stream);
   }
   const bool res16 = p.residual != nullptr && p.res_dtype != DT_F32;
+  // 192-column tiles for column counts that are multiples of 192 but not of 256 (SwinIR-M's 576 / 384 / 192-column linears
+  // and 3x3 convs at C = 180): 256-column tiles would run a third more MMA work on zero columns.  No decoder or conv-only
+  // upscaler launch has such a column count.
+  const bool n192 = !tf32 && use_cg == 2 && p.n_cols % 192 == 0 && p.n_cols % 256 != 0 && p.stats == nullptr &&
+                    p.xf_scale == nullptr && p.k2 == 0;
+  if (n192) {
+    const bool plain = !p.round_tf32 && p.lrelu == 0.f && p.act_slope == nullptr && p.act == ACT_NONE &&
+                       p.residual2 == nullptr && p.out2 == nullptr && !p.bias_per_row && p.row_scale == nullptr &&
+                       (p.res_scale == 0.f || p.res_scale == 1.f);
+    if (plain && p.out_dtype != DT_F32 && p.residual == nullptr) return launch_tc<192, false, 2, EPI_OUT16>(p, num_sms, stream);
+    if (plain && p.out_dtype == DT_F32 && p.residual != nullptr && p.res_dtype == DT_F32)
+      return launch_tc<192, false, 2, EPI_RES>(p, num_sms, stream);
+    return launch_tc<192, false, 2, EPI_GENERIC>(p, num_sms, stream);
+  }
   if (use_cg == 2 && !tf32 && p.lrelu == 0.f && p.act_slope == nullptr && p.act == ACT_NONE && p.residual2 == nullptr && (p.res_scale == 0.f || p.res_scale == 1.f || res16)) {
     // specialised epilogues for what the decoder launches; anything else takes the generic build
     int epi = 0;

@@ -212,6 +212,7 @@ __global__ void gemm_direct_kernel(const GemmParams p) {
     if (p.act_slope != nullptr && v < 0.f) v *= p.act_slope[col];
     if (p.act == ACT_SILU) v *= 1.f / (1.f + expf(-v));
     if (p.act == ACT_GATE) v *= gate;
+    if (p.act == ACT_GELU) v = 0.5f * v * (1.f + erff(v * 0.70710678118654752f));
     if (p.out2 != nullptr) {
       const long long off2 = p.out2_px_stride == 0 ? off
           : (long long)img * p.out2_img_stride + (long long)(y * p.sy + p.py) * p.out2_row_stride +

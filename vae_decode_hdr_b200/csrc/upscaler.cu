@@ -22,6 +22,8 @@
 // SPAN (conv_1, six SPAB blocks, conv_2, conv_cat, upsampler.0) runs on the same kernel too: every Conv3XC is fused into
 // one 3x3 conv at load time, SiLU and SPAN's attention gate are epilogue operations, and the four tensors conv_cat reads
 // are channel slices of one fp16 buffer, so that conv_cat is a plain 1x1 conv (up_forward_span).
+// SwinIR (up_forward_swinir) runs its linears and convs on the same kernel (fc1 with the GELU epilogue) and its LayerNorm,
+// shifted-window attention and fp16 pixel shuffle in swin.cu, on the tile reflect-padded to a multiple of the 8-pixel window.
 // Everything after the model (hook, feather blend, YCbCr, median, local fix) is elementwise / stencil work in
 // fp32 with the reference's operation order (no FMA contraction) so that it is bit-comparable to the oracle.
 #include <string.h>
@@ -40,16 +42,16 @@ namespace hdrvae {
 __host__ __device__ constexpr int up_in_channels(int f) { return f == 1 ? 8 : f == 2 ? 16 : 48; }
 
 // image fp32 BHWC (3 channels) -> fp16 network input [n][h'][w'][up_in_channels(F)] of tiles of h x w at the origins of
-// `tiles`, h' = ceil(h / F): clamp to [-1, 1] (flag or tile table .w), minus `mean` (SPAN's normalisation; zero for the
+// `tiles`: clamp to [-1, 1] (flag or tile table .w), minus `mean` (SPAN's and SwinIR's normalisation; zero for the
 // other models, where it leaves every value as it is), reflect pad of the tile's bottom / right edge to
 // F h' x F w' (torch "reflect": row h + k reads row h - 2 - k), pixel unshuffle by F (channel c F^2 + i F + j = channel c
 // at pixel (y F + i, x F + j)), channels beyond 3 F^2 zero.  The clamp is elementwise, so it commutes with pad and
-// unshuffle.  F = 1 is the plain [n][h][w][8] copy.
+// unshuffle.  h' = ceil(h / F) for RRDBNet, and h rounded up to a multiple of 8 (SwinIR's window, F = 1); F = 1 without
+// a pad is the plain [n][h][w][8] copy.
 template <int F>
 __global__ void up_extract_tiles_kernel(const float* __restrict__ img, int H, int W, const int4* __restrict__ tiles /*b,y0,x0,_*/,
-                                        int n, int h, int w, int clamp1, float3 mean, uint4* __restrict__ out) {
+                                        int n, int h, int w, int hq, int wq, int clamp1, float3 mean, uint4* __restrict__ out) {
   constexpr int CX = up_in_channels(F), F2 = F * F;
-  const int hq = (h + F - 1) / F, wq = (w + F - 1) / F;
   const long long total = (long long)n * hq * wq;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int x = (int)(i % wq);
@@ -354,7 +356,25 @@ static inline int up_grid(long long n) { return (int)std::min<long long>((n + 25
 using namespace hdrvae;
 
 // ------------------------------------------------------------------------------------------------ model
-enum UpArch { UP_RRDB, UP_COMPACT, UP_SPAN };   // ESRGAN / RRDBNet, Real-ESRGAN SRVGGNetCompact, SPAN
+enum UpArch { UP_RRDB, UP_COMPACT, UP_SPAN, UP_SWINIR };   // ESRGAN / RRDBNet, Real-ESRGAN SRVGGNetCompact, SPAN, SwinIR
+enum UpSwinTail { SW_NONE, SW_PIXELSHUFFLE, SW_DIRECT, SW_NEAREST };   // SwinIR upsampler "", "pixelshuffle",
+                                                                       // "pixelshuffledirect", "nearest+conv"
+struct UpSwinBlock {              // one Swin transformer layer (STL) of SwinIR
+  float *ln1_g = nullptr, *ln1_b = nullptr, *ln2_g = nullptr, *ln2_b = nullptr;
+  float* table = nullptr;         // relative-position bias table [225][heads]
+  PackedConv qkv, proj, fc1, fc2; // qkv: 3 heads 32 columns (q scaled by hd^-0.5, heads padded to 32); proj reads that layout
+};
+struct UpSwin {
+  int C = 0, CP = 0;              // embed_dim and the pixel stride of its fp16 operands (C rounded up to 8)
+  int heads = 0, hidden = 0, HP = 0;   // heads, MLP width and its fp16 pixel stride
+  int c4 = 0, c4p = 0;            // 3conv: conv.0 / conv.2 width C / 4 and its pixel stride
+  bool conv3 = false, patch_norm = false;
+  UpSwinTail tail = SW_NONE;
+  int n_up = 0;                   // 2x stages of the pixelshuffle / nearest+conv tails
+  std::vector<int> depths;        // blocks per RSTB
+  std::vector<UpSwinBlock> blocks;
+  float *pn_g = nullptr, *pn_b = nullptr, *norm_g = nullptr, *norm_b = nullptr;   // patch_embed.norm, norm
+};
 
 struct hdrvae_upscaler {
   hdrvae_ctx* ctx = nullptr;      // device / SM count / conv implementation come from the decode context
@@ -371,6 +391,10 @@ struct hdrvae_upscaler {
                                   // Compact: first conv, nb body convs, last conv (nf -> 3 s^2).  SPAN: the fused conv_1,
                                   // block_k.c{1,2,3}_r (k = 1..6), conv_2, then conv_cat (1x1, 4 nf -> nf) and upsampler.0
   std::vector<float*> slopes;     // Compact: PReLU slopes applied after convs[k], k <= nb (cout_pad floats, zero-padded)
+                                  // SwinIR: conv_first, each RSTB's conv (or conv.0/2/4), conv_after_body (1 or 3), then the
+                                  // tail: conv_before_upsample.0, upsample.{2k} | conv_up1/2, conv_hr, conv_last, or upsample.0
+                                  // or conv_last alone
+  UpSwin sw;                      // SwinIR: dimensions and the transformer layers (their linears are not in `convs`)
 };
 
 namespace hdrvae {
@@ -378,16 +402,25 @@ namespace hdrvae {
 // channels per pixel of the Compact last conv's fp32 output: 3 s^2 rounded up to the epilogue's 4-column stores
 static int up_last_channels(const hdrvae_upscaler* up) { return (3 * up->scale * up->scale + 3) / 4 * 4; }
 
-// network grid of a tile of h x w: the reflect-padded tile pixel-unshuffled by the model's factor f
-static int up_net_side(const hdrvae_upscaler* up, int side) { return (side + up->shuffle - 1) / up->shuffle; }
+// network grid of a tile of h x w: the reflect-padded tile pixel-unshuffled by the model's factor f (RRDBNet), or the
+// tile reflect-padded to a multiple of SwinIR's 8-pixel window
+static constexpr int kSwinWin = 8;
+static int up_net_side(const hdrvae_upscaler* up, int side) {
+  if (up->arch == UP_SWINIR) return (side + kSwinWin - 1) / kSwinWin * kSwinWin;
+  return (side + up->shuffle - 1) / up->shuffle;
+}
 
-// torch's reflect pad needs pad < side; a tile side for which the pad to a multiple of f fails is refused
+// torch's reflect pad needs pad < side; a tile side for which the pad to a multiple of f (or of the window) fails is refused
 static int up_check_sides(const hdrvae_upscaler* up, int h, int w) {
-  const int f = up->shuffle;
+  const int f = up->arch == UP_SWINIR ? kSwinWin : up->shuffle;
   for (int side : {h, w}) {
     const int pad = (f - side % f) % f;
-    HDRVAE_REQUIRE(pad < side, "upscaler: a tile side of %d pixels is too short for the reflect pad of %d pixels that the "
-                   "model's %dx pixel unshuffle needs (the pad must be shorter than the side)", side, pad, f);
+    if (up->arch == UP_SWINIR)
+      HDRVAE_REQUIRE(pad < side, "upscaler: a tile side of %d pixels is too short for the reflect pad of %d pixels that "
+                     "SwinIR's %d-pixel windows need (the pad must be shorter than the side)", side, pad, f);
+    else
+      HDRVAE_REQUIRE(pad < side, "upscaler: a tile side of %d pixels is too short for the reflect pad of %d pixels that the "
+                     "model's %dx pixel unshuffle needs (the pad must be shorter than the side)", side, pad, f);
   }
   return 0;
 }
@@ -396,6 +429,8 @@ struct UpPlan {                   // workspace of one forward over n tiles of h 
   size_t img8, cat0, cat1, f_feat, f_a, f_b, f_c, u0, u1, u2, u3;   // RRDBNet
   size_t act0, act1, last;                                          // Compact (SPAN: last)
   size_t sp_r0, sp_r1, sp_d, sp_t0, sp_t1, sp_cat;                  // SPAN
+  size_t sw_f, sw_b0, sw_b1, sw_a16, sw_b16, sw_qkv, sw_o, sw_hid, sw_t0, sw_t1, sw_u0, sw_ua, sw_ub, sw_big, sw_last,
+         sw_out;                                                    // SwinIR
   size_t total;
 };
 static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
@@ -422,6 +457,28 @@ static UpPlan up_make_plan(const hdrvae_upscaler* up, int n, int h, int w) {
       pl.sp_t1 = take(P * nf * 2);
       pl.sp_cat = take(P * 4 * nf * 2); // [f | b6 | b1 | b5_2]: conv_cat's input, the channel order of torch.cat
       pl.last = take(P * up_last_channels(up) * 4);
+      break;
+    }
+    case UP_SWINIR: {
+      const UpSwin& sw = up->sw;
+      const size_t s2 = (size_t)up->scale * up->scale;
+      pl.sw_f = take(P * sw.C * 4);                 // conv_first's output (the long skip), fp32
+      pl.sw_b0 = take(P * sw.C * 4);                // RSTB input / output stream, fp32
+      pl.sw_b1 = take(P * sw.C * 4);                // the STL stream inside an RSTB, fp32
+      pl.sw_a16 = take(P * sw.CP * 2);              // LayerNorm outputs and the stream's fp16 copy
+      pl.sw_b16 = take(P * sw.CP * 2);              // conv_after_body's output (the tail's input), fp16
+      pl.sw_qkv = take(P * sw.heads * 3 * 32 * 2);  // q | k | v, 32 channels per head
+      pl.sw_o = take(P * sw.heads * 32 * 2);        // attention output, 32 channels per head
+      pl.sw_hid = take(P * sw.HP * 2);              // GELU(fc1)
+      pl.sw_t0 = take(sw.conv3 ? P * sw.c4p * 2 : 0);   // 3conv: conv.0 / conv.2 outputs
+      pl.sw_t1 = take(sw.conv3 ? P * sw.c4p * 2 : 0);
+      const bool up64 = sw.tail == SW_PIXELSHUFFLE || sw.tail == SW_NEAREST;
+      pl.sw_u0 = take(up64 ? P * 64 * 2 : 0);       // conv_before_upsample
+      pl.sw_ua = take(up64 ? P * s2 * 64 * 2 : 0);  // 64-channel fp16 stages of the tail, ping-pong
+      pl.sw_ub = take(up64 ? P * s2 * 64 * 2 : 0);
+      pl.sw_big = take(sw.tail == SW_PIXELSHUFFLE ? P * (s2 / 4) * 256 * 2 : 0);   // upsample.{2k}'s 256 channels
+      pl.sw_last = take(sw.tail == SW_DIRECT ? P * up_last_channels(up) * 4 : sw.tail == SW_NONE ? P * 16 : 0);
+      pl.sw_out = take(P * s2 * 16);                // float4 output of the padded tile (cropped into out4)
       break;
     }
     case UP_RRDB:
@@ -603,25 +660,186 @@ static int up_forward_span(hdrvae_upscaler* up, int n, int h, int w, uint8_t* ws
   return run_conv(ctx, up->convs[21], io, n, h, w, impl, s);
 }
 
+// SwinIR forward on n tiles of h x w (fp16 [n][hp][wp][8] x - mean in pl.img8, hp / wp: h / w reflect-padded to a multiple
+// of 8) -> fp32 [n][s h][s w][4] at out4.  Tokens are the NHWC pixels of the padded tile in raster order, so patch embed /
+// unembed are no-ops.  Per STL: LayerNorm -> qkv (1x1 conv) -> window attention (shift 4 in odd blocks) -> proj + the
+// residual, in place on the fp32 stream -> LayerNorm -> fc1 + GELU -> fc2 + the residual (the last STL of an RSTB also
+// writes the stream's fp16 copy, the RSTB conv's operand).  The RSTB conv (or the 3conv triple) adds the RSTB input.
+// After the last RSTB: norm, conv_after_body + conv_first's output, then the tail on the padded grid; the +mean of the
+// output is in the last conv's bias (or, for the 1x form, in the base add of the input).  A padded tile's output is cut
+// out of the padded grid's with up_crop_kernel.
+static int up_forward_swinir(hdrvae_upscaler* up, const float* img, int H, int W, const int4* tiles, int n, int h, int w,
+                             uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
+  hdrvae_ctx* ctx = up->ctx;
+  const int impl = ctx->conv_impl;
+  const UpSwin& sw = up->sw;
+  const int hp = up_net_side(up, h), wp = up_net_side(up, w), sc = up->scale;
+  const long long P = (long long)n * hp * wp;
+  const bool crop = hp != h || wp != w;
+  float* F = reinterpret_cast<float*>(ws + pl.sw_f);
+  float* B0 = reinterpret_cast<float*>(ws + pl.sw_b0);
+  float* S = reinterpret_cast<float*>(ws + pl.sw_b1);
+  uint8_t* a16 = ws + pl.sw_a16;
+  uint8_t* b16 = ws + pl.sw_b16;
+  const PackedConv* conv = up->convs.data();          // walked in the order up_pack_swinir packed them
+  {
+    ConvIO io; io.x = ws + pl.img8; io.x_channels = 8; io.y = F; io.y_dtype = DT_F32; io.y_channels = sw.C;
+    HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hp, wp, impl, s));
+  }
+  const float* rin = F;                               // RSTB input (fp32 stream)
+  if (sw.patch_norm) {
+    HDRVAE_TRY(launch_layernorm(F, P, sw.C, sw.pn_g, sw.pn_b, B0, DT_F32, sw.C, s));
+    rin = B0;
+  }
+  // 3x3 conv (or conv.0 / conv.2 / conv.4 with LeakyReLU 0.2 between) of the fp16 tensor x, + the fp32 residual -> fp32 y
+  // [P][C] (the residual shares y's addressing), and its fp16 copy y16 [P][CP] when given
+  auto res_conv = [&](const void* x, const float* residual, float* y, void* y16) -> int {
+    if (sw.conv3) {
+      ConvIO io; io.x = x; io.x_channels = sw.CP; io.y = ws + pl.sw_t0; io.y_dtype = DT_F16; io.y_channels = sw.c4p;
+      io.lrelu = 0.2f;
+      HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hp, wp, impl, s));
+      ConvIO io2; io2.x = ws + pl.sw_t0; io2.x_channels = sw.c4p; io2.y = ws + pl.sw_t1; io2.y_dtype = DT_F16;
+      io2.y_channels = sw.c4p; io2.lrelu = 0.2f;
+      HDRVAE_TRY(run_conv(ctx, *conv++, io2, n, hp, wp, impl, s));
+      x = ws + pl.sw_t1;
+    }
+    ConvIO io; io.x = x; io.x_channels = sw.conv3 ? sw.c4p : sw.CP; io.y = y; io.y_dtype = DT_F32; io.y_channels = sw.C;
+    io.residual = residual; io.res_dtype = DT_F32;
+    if (y16 != nullptr) { io.y2 = y16; io.y2_channels = sw.CP; io.y2_chan_off = 0; }
+    return run_conv(ctx, *conv++, io, n, hp, wp, impl, s);
+  };
+  size_t bi = 0;
+  for (size_t r = 0; r < sw.depths.size(); ++r) {
+    for (int j = 0; j < sw.depths[r]; ++j, ++bi) {
+      const UpSwinBlock& b = sw.blocks[bi];
+      const float* xin = j == 0 ? rin : S;
+      HDRVAE_TRY(launch_layernorm(xin, P, sw.C, b.ln1_g, b.ln1_b, a16, DT_F16, sw.CP, s));
+      {
+        ConvIO io; io.x = a16; io.x_channels = sw.CP; io.y = ws + pl.sw_qkv; io.y_dtype = DT_F16;
+        HDRVAE_TRY(run_conv(ctx, b.qkv, io, n, hp, wp, impl, s));
+      }
+      HDRVAE_TRY(launch_window_attention(ws + pl.sw_qkv, n, hp, wp, sw.heads, b.table, (j & 1) ? kSwinWin / 2 : 0,
+                                         ws + pl.sw_o, s));
+      {
+        ConvIO io; io.x = ws + pl.sw_o; io.x_channels = sw.heads * 32; io.y = S; io.y_dtype = DT_F32; io.y_channels = sw.C;
+        io.residual = xin; io.res_dtype = DT_F32;
+        HDRVAE_TRY(run_conv(ctx, b.proj, io, n, hp, wp, impl, s));
+      }
+      HDRVAE_TRY(launch_layernorm(S, P, sw.C, b.ln2_g, b.ln2_b, a16, DT_F16, sw.CP, s));
+      {
+        ConvIO io; io.x = a16; io.x_channels = sw.CP; io.y = ws + pl.sw_hid; io.y_dtype = DT_F16; io.y_channels = sw.HP;
+        io.act = ACT_GELU;
+        HDRVAE_TRY(run_conv(ctx, b.fc1, io, n, hp, wp, impl, s));
+      }
+      {
+        ConvIO io; io.x = ws + pl.sw_hid; io.x_channels = sw.HP; io.y = S; io.y_dtype = DT_F32; io.y_channels = sw.C;
+        io.residual = S; io.res_dtype = DT_F32;
+        if (j + 1 == sw.depths[r]) { io.y2 = a16; io.y2_channels = sw.CP; io.y2_chan_off = 0; }
+        HDRVAE_TRY(run_conv(ctx, b.fc2, io, n, hp, wp, impl, s));
+      }
+    }
+    // RSTB end: conv(stream) + RSTB input, in place on B0 (the first RSTB's input may be conv_first's output F, kept)
+    HDRVAE_TRY(res_conv(a16, rin, B0, nullptr));
+    rin = B0;
+  }
+  HDRVAE_TRY(launch_layernorm(rin, P, sw.C, sw.norm_g, sw.norm_b, a16, DT_F16, sw.CP, s));
+  HDRVAE_TRY(res_conv(a16, F, S, b16));                   // conv_after_body + conv_first's output (fp16 copy: the tail's input)
+  float* o4 = crop ? reinterpret_cast<float*>(ws + pl.sw_out) : out4;   // [n][s hp][s wp] float4
+  const int hs = sc * hp, wsd = sc * wp;
+  switch (sw.tail) {
+    case SW_PIXELSHUFFLE:
+    case SW_NEAREST: {
+      uint8_t* cur = ws + pl.sw_u0;
+      uint8_t* pp[2] = {ws + pl.sw_ua, ws + pl.sw_ub};
+      {
+        ConvIO io; io.x = b16; io.x_channels = sw.CP; io.y = cur; io.y_dtype = DT_F16; io.lrelu = 0.01f;   // nn.LeakyReLU()
+        HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hp, wp, impl, s));
+      }
+      for (int k = 0; k < sw.n_up; ++k) {
+        const int gh = hp << k, gw = wp << k;
+        uint8_t* nxt = pp[k & 1];
+        if (sw.tail == SW_PIXELSHUFFLE) {
+          ConvIO io; io.x = cur; io.y = ws + pl.sw_big; io.y_dtype = DT_F16;
+          HDRVAE_TRY(run_conv(ctx, *conv++, io, n, gh, gw, impl, s));
+          HDRVAE_TRY(launch_pixel_shuffle2_f16(ws + pl.sw_big, n, gh, gw, 64, nxt, s));
+        } else {
+          ConvIO io; io.x = cur; io.y = nxt; io.y_dtype = DT_F16; io.lrelu = 0.2f;     // nearest 2x folded into the load
+          HDRVAE_TRY(run_conv(ctx, *conv++, io, n, gh, gw, impl, s));
+        }
+        cur = nxt;
+      }
+      if (sw.tail == SW_NEAREST) {
+        uint8_t* nxt = pp[sw.n_up & 1];
+        ConvIO io; io.x = cur; io.y = nxt; io.y_dtype = DT_F16; io.lrelu = 0.2f;
+        HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hs, wsd, impl, s));
+        cur = nxt;
+      }
+      ConvIO io; io.x = cur; io.y = o4; io.y_dtype = DT_F32; io.y_channels = 4; io.n_store = 4;
+      HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hs, wsd, impl, s));
+      break;
+    }
+    case SW_DIRECT: {
+      const int cl = up_last_channels(up);
+      ConvIO io; io.x = b16; io.x_channels = sw.CP; io.y = ws + pl.sw_last; io.y_dtype = DT_F32; io.y_channels = cl;
+      HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hp, wp, impl, s));
+      const long long opx = P * sc * sc;
+      ProfScope prof("upscaler pixel shuffle", 0.0, (double)P * cl * 4 + opx * 16, s);
+      up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float*>(ws + pl.sw_last), cl, nullptr, H, W,
+                                                          tiles, n, hp, wp, sc, reinterpret_cast<float4*>(o4));
+      HDRVAE_LAUNCHED();
+      break;
+    }
+    case SW_NONE: {
+      // x + conv_last(res): conv_last on the padded grid, cut to the tile, then the base add of the (clamped) input pixel
+      float* last = reinterpret_cast<float*>(ws + pl.sw_last);
+      ConvIO io; io.x = b16; io.x_channels = sw.CP; io.y = crop ? o4 : last; io.y_dtype = DT_F32; io.y_channels = 4;
+      io.n_store = 4;
+      HDRVAE_TRY(run_conv(ctx, *conv++, io, n, hp, wp, impl, s));
+      const long long opx = (long long)n * h * w;
+      if (crop) {
+        ProfScope prof("upscaler crop padded tiles", 0.0, opx * 32.0, s);
+        up_crop_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float4*>(o4), hp, wp, n, h, w,
+                                                    reinterpret_cast<float4*>(last));
+        HDRVAE_LAUNCHED();
+      }
+      ProfScope prof("upscaler pixel shuffle + base", 0.0, opx * 28.0 + opx * 16, s);
+      up_shuffle_base_kernel<<<up_grid(opx), 256, 0, s>>>(last, 4, img, H, W, tiles, n, h, w, 1,
+                                                          reinterpret_cast<float4*>(out4));
+      HDRVAE_LAUNCHED();
+      return 0;
+    }
+  }
+  if (crop) {
+    const long long opx = (long long)n * sc * sc * h * w;
+    ProfScope prof("upscaler crop padded tiles", 0.0, opx * 32.0, s);
+    up_crop_kernel<<<up_grid(opx), 256, 0, s>>>(reinterpret_cast<const float4*>(o4), hs, wsd, n, sc * h, sc * w,
+                                                reinterpret_cast<float4*>(out4));
+    HDRVAE_LAUNCHED();
+  }
+  return 0;
+}
+
 // The network on n tiles of h x w cut from img [.][H][W][3] at the origins of `tiles` (image, y0, x0, clamp to [-1, 1])
 // -> fp32 [n][s h][s w][4] at out4
 static int up_run_model(hdrvae_upscaler* up, const float* img, int H, int W, const int4* tiles, int n, int h, int w,
                         uint8_t* ws, const UpPlan& pl, float* out4, cudaStream_t s) {
   {
     const int f = up->shuffle;
-    const long long npx = (long long)n * up_net_side(up, h) * up_net_side(up, w);
+    const int hq = up_net_side(up, h), wq = up_net_side(up, w);
+    const long long npx = (long long)n * hq * wq;
     ProfScope prof("upscaler extract tiles", 0.0, (double)npx * (f * f * 12 + up_in_channels(f) * 2), s);
     uint4* x = reinterpret_cast<uint4*>(ws + pl.img8);
     const float3 m = up->mean;
-    if (f == 1) up_extract_tiles_kernel<1><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
-    else if (f == 2) up_extract_tiles_kernel<2><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
-    else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, 0, m, x);
+    if (f == 1) up_extract_tiles_kernel<1><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, hq, wq, 0, m, x);
+    else if (f == 2) up_extract_tiles_kernel<2><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, hq, wq, 0, m, x);
+    else up_extract_tiles_kernel<4><<<up_grid(npx), 256, 0, s>>>(img, H, W, tiles, n, h, w, hq, wq, 0, m, x);
     HDRVAE_LAUNCHED();
   }
   switch (up->arch) {
     case UP_RRDB: return up_forward_rrdb(up, n, h, w, ws, pl, out4, s);
     case UP_COMPACT: HDRVAE_TRY(up_forward_compact(up, n, h, w, ws, pl, s)); break;
     case UP_SPAN: HDRVAE_TRY(up_forward_span(up, n, h, w, ws, pl, s)); break;
+    case UP_SWINIR: return up_forward_swinir(up, img, H, W, tiles, n, h, w, ws, pl, out4, s);
   }
   const int sc = up->scale, cl = up_last_channels(up);
   const long long opx = (long long)n * sc * sc * h * w;
@@ -991,6 +1209,235 @@ static int up_pack_span(hdrvae_upscaler* up, cudaStream_t s) {
   return 0;
 }
 
+// SwinIR (spandrel's "SwinIR": JingyunLiang/SwinIR network_swinir.py) with 3 input channels, embed_dim C <= 256, head dim
+// C / heads <= 32, window 8, any RSTB count and depths, any MLP width, resi_connection "1conv" / "3conv", with or without
+// patch_embed.norm, no absolute_pos_embed, and the upsamplers "pixelshuffle" (2x, 4x), "pixelshuffledirect" (2x, 4x),
+// "nearest+conv" (2x, 4x) and "" (1x).  The stored relative_position_index and attn_mask buffers are not read: the index is
+// a function of the window, and the mask is computed for each tile's padded size (window_attention_kernel).  HAT shares
+// SwinIR's key prefix and is refused by its own keys.
+static const char* kSwinKey = "layers.0.residual_group.blocks.0.attn.relative_position_bias_table";
+static int up_pack_swinir(hdrvae_upscaler* up, cudaStream_t s) {
+  hdrvae_ctx* st = &up->store;
+  UpSwin& sw = up->sw;
+  const char* A = "SwinIR";
+  for (const auto& kv : st->shapes) {
+    const std::string& k = kv.first;
+    HDRVAE_REQUIRE(k.find("conv_block") == std::string::npos && k.find("overlap_attn") == std::string::npos &&
+                   k.find("relative_position_index_SA") == std::string::npos,
+                   "SwinIR upscaler: %s has shape %s: a HAT model (conv_block / overlap_attn / relative_position_index_SA "
+                   "keys); HAT is not supported", k.c_str(), up_shape_str(kv.second).c_str());
+    HDRVAE_REQUIRE(k != "absolute_pos_embed", "SwinIR upscaler: absolute_pos_embed has shape %s; models with ape (an "
+                   "absolute position embedding) are not supported", up_shape_str(kv.second).c_str());
+  }
+  auto shape = [&](const std::string& k) -> const std::vector<int64_t>* {
+    auto it = st->shapes.find(k);
+    return it == st->shapes.end() ? nullptr : &it->second;
+  };
+  auto host = [&](const std::string& k, std::vector<float>* out) -> int {
+    size_t cnt = 1;
+    for (int64_t d : st->shapes[k]) cnt *= (size_t)d;
+    out->resize(cnt);
+    HDRVAE_CUDA_OK(cudaMemcpy(out->data(), st->raw[k], cnt * sizeof(float), cudaMemcpyDeviceToHost));
+    return 0;
+  };
+  // a device copy of the staged tensor `k` that outlives the staging (LayerNorm parameters, bias tables)
+  auto keep = [&](const std::string& k, size_t cnt, float** out) -> int {
+    HDRVAE_TRY(dev_alloc(st, cnt * sizeof(float), (void**)out));
+    HDRVAE_CUDA_OK(cudaMemcpyAsync(*out, st->raw[k], cnt * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return 0;
+  };
+  // host fp32 weights [cout][cin][ks][ks] and bias [cout] packed for the conv kernel (kept under the fp32 state-dict map, so
+  // that up_finish_load frees them with the rest)
+  auto pack_host = [&](const std::string& k, const std::vector<float>& wf, const std::vector<float>& bf, int cout, int cin,
+                       int ks, PackedConv* pc) -> int {
+    float *dw = nullptr, *db = nullptr;
+    HDRVAE_TRY(dev_alloc(st, wf.size() * sizeof(float), (void**)&dw));
+    HDRVAE_TRY(dev_alloc(st, bf.size() * sizeof(float), (void**)&db));
+    st->raw[k + ".packed.weight"] = dw;
+    st->raw[k + ".packed.bias"] = db;
+    HDRVAE_CUDA_OK(cudaMemcpy(dw, wf.data(), wf.size() * sizeof(float), cudaMemcpyHostToDevice));
+    HDRVAE_CUDA_OK(cudaMemcpy(db, bf.data(), bf.size() * sizeof(float), cudaMemcpyHostToDevice));
+    return pack_conv(st, dw, db, cout, cin, ks, false, 1.f, DT_F16, pc, s);
+  };
+  // nn.Linear `k` [out][in] + bias [out], packed as a 1x1 conv
+  auto linear = [&](const std::string& k, int out, int in, PackedConv* pc) -> int {
+    HDRVAE_TRY(up_need(st, A, k + ".weight", {out, in}));
+    HDRVAE_TRY(up_need(st, A, k + ".bias", {out}));
+    return pack_conv(st, st->raw[k + ".weight"], st->raw[k + ".bias"], out, in, 1, false, 1.f, DT_F16, pc, s);
+  };
+  // + mean in the bias of the conv that produces the output colours (channel o belongs to colour o / per)
+  auto add_mean = [&](PackedConv* pc, int cout, int per) -> int {
+    std::vector<float> b(cout);
+    HDRVAE_CUDA_OK(cudaMemcpy(b.data(), pc->bias, cout * sizeof(float), cudaMemcpyDeviceToHost));
+    const float m[3] = {up->mean.x, up->mean.y, up->mean.z};
+    for (int o = 0; o < cout; ++o) b[o] += m[o / per];
+    HDRVAE_CUDA_OK(cudaMemcpy(pc->bias, b.data(), cout * sizeof(float), cudaMemcpyHostToDevice));
+    return 0;
+  };
+  const std::vector<int64_t>* cf = shape("conv_first.weight");
+  HDRVAE_REQUIRE(cf != nullptr && cf->size() == 4 && (*cf)[0] >= 1 && (*cf)[0] <= 256 && (*cf)[1] == 3 && (*cf)[2] == 3 &&
+                 (*cf)[3] == 3, "SwinIR upscaler: conv_first.weight has shape %s; want [embed_dim,3,3,3] with embed_dim "
+                 "<= 256 (3 input channels)", up_shape_str(st, "conv_first.weight").c_str());
+  const int C = (int)(*cf)[0];
+  sw.C = C;
+  sw.CP = (C + 7) / 8 * 8;
+  const std::vector<int64_t>* tb = shape(kSwinKey);
+  HDRVAE_REQUIRE(tb->size() == 2 && (*tb)[0] == 225 && (*tb)[1] >= 1, "SwinIR upscaler: %s has shape %s; want [225,heads] "
+                 "(window size 8: (2 ws - 1)^2 rows)", kSwinKey, up_shape_str(*tb).c_str());
+  sw.heads = (int)(*tb)[1];
+  HDRVAE_REQUIRE(C % sw.heads == 0 && C / sw.heads <= 32, "SwinIR upscaler: %s has shape %s: embed_dim %d over %d heads; "
+                 "the head dimension must divide embed_dim and be at most 32", kSwinKey, up_shape_str(*tb).c_str(), C, sw.heads);
+  const int hd = C / sw.heads;
+  const std::string b00 = "layers.0.residual_group.blocks.0.";
+  const std::vector<int64_t>* f1 = shape(b00 + "mlp.fc1.weight");
+  HDRVAE_REQUIRE(f1 != nullptr && f1->size() == 2 && (*f1)[0] >= 1 && (*f1)[1] == C, "SwinIR upscaler: %smlp.fc1.weight has "
+                 "shape %s; want [hidden,%d]", b00.c_str(), up_shape_str(st, b00 + "mlp.fc1.weight").c_str(), C);
+  sw.hidden = (int)(*f1)[0];
+  sw.HP = (sw.hidden + 7) / 8 * 8;
+  sw.conv3 = shape("layers.0.conv.weight") == nullptr && shape("layers.0.conv.0.weight") != nullptr;
+  sw.c4 = C / 4;
+  sw.c4p = (sw.c4 + 7) / 8 * 8;
+  HDRVAE_REQUIRE(!sw.conv3 || sw.c4 >= 1, "SwinIR upscaler: embed_dim %d is too small for resi_connection \"3conv\"", C);
+  sw.patch_norm = shape("patch_embed.norm.weight") != nullptr;
+  // RSTBs layers.i and their blocks layers.i.residual_group.blocks.j
+  int nl = 0;
+  for (const auto& kv : st->shapes) {
+    int i = -1;
+    if (sscanf(kv.first.c_str(), "layers.%d.", &i) == 1) nl = std::max(nl, i + 1);
+  }
+  sw.depths.assign(nl, 0);
+  for (const auto& kv : st->shapes) {
+    int i = -1, j = -1;
+    if (sscanf(kv.first.c_str(), "layers.%d.residual_group.blocks.%d.", &i, &j) == 2 && i >= 0 && j >= 0)
+      sw.depths[i] = std::max(sw.depths[i], j + 1);
+  }
+  for (int i = 0; i < nl; ++i)
+    HDRVAE_REQUIRE(sw.depths[i] >= 1, "SwinIR upscaler state dict lacks layers.%d.residual_group.blocks.0.* (every RSTB "
+                   "needs at least one Swin transformer layer)", i);
+  // upsampler and scale
+  int scale = 1;
+  if (shape("conv_up1.weight") != nullptr) {
+    sw.tail = SW_NEAREST;
+    sw.n_up = shape("conv_up2.weight") != nullptr ? 2 : 1;
+  } else if (shape("conv_before_upsample.0.weight") != nullptr) {
+    sw.tail = SW_PIXELSHUFFLE;
+    HDRVAE_TRY(up_need(st, A, "upsample.0.weight", {256, 64, 3, 3}));
+    HDRVAE_REQUIRE(shape("upsample.4.weight") == nullptr, "SwinIR upscaler: upsample.4.weight has shape %s: a third 2x stage "
+                   "(an 8x SwinIR) is not supported; SwinIR runs at 1x, 2x and 4x", up_shape_str(st, "upsample.4.weight").c_str());
+    sw.n_up = shape("upsample.2.weight") != nullptr ? 2 : 1;
+  } else if (shape("upsample.0.weight") != nullptr) {
+    sw.tail = SW_DIRECT;
+    const std::vector<int64_t>* u = shape("upsample.0.weight");
+    const int64_t c = u->size() == 4 && (*u)[1] == C && (*u)[2] == 3 && (*u)[3] == 3 ? (*u)[0] : 0;
+    HDRVAE_REQUIRE(c == 12 || c == 48, "SwinIR upscaler: upsample.0.weight has shape %s; want [3*scale^2,%d,3,3] with "
+                   "scale 2 or 4", up_shape_str(*u).c_str(), C);
+    scale = c == 12 ? 2 : 4;
+  } else {
+    sw.tail = SW_NONE;
+  }
+  if (sw.tail == SW_NEAREST || sw.tail == SW_PIXELSHUFFLE) scale = 1 << sw.n_up;
+  up->scale = scale;
+  up->mean = make_float3(0.4488f, 0.4371f, 0.4040f);       // in_chans 3: the RGB mean; img_range 1
+  // packing, in launch order
+  auto res_convs = [&](const std::string& k) -> int {     // RSTB conv / conv_after_body: 1conv or 3conv
+    if (!sw.conv3) {
+      up->convs.emplace_back();
+      return up_pack(st, A, k, C, C, 3, false, 1.f, &up->convs.back(), s);
+    }
+    up->convs.emplace_back();
+    HDRVAE_TRY(up_pack(st, A, k + ".0", sw.c4, C, 3, false, 1.f, &up->convs.back(), s));
+    up->convs.emplace_back();
+    HDRVAE_TRY(up_pack(st, A, k + ".2", sw.c4, sw.c4, 1, false, 1.f, &up->convs.back(), s));
+    up->convs.emplace_back();
+    return up_pack(st, A, k + ".4", C, sw.c4, 3, false, 1.f, &up->convs.back(), s);
+  };
+  up->convs.reserve(2 + 3 * (size_t)nl + 3 + 6);
+  up->convs.emplace_back();
+  HDRVAE_TRY(up_pack(st, A, "conv_first", C, 3, 3, false, 1.f, &up->convs.back(), s));
+  if (sw.patch_norm) {
+    HDRVAE_TRY(up_need(st, A, "patch_embed.norm.weight", {C}));
+    HDRVAE_TRY(up_need(st, A, "patch_embed.norm.bias", {C}));
+    HDRVAE_TRY(keep("patch_embed.norm.weight", C, &sw.pn_g));
+    HDRVAE_TRY(keep("patch_embed.norm.bias", C, &sw.pn_b));
+  }
+  const float qscale = (float)(1.0 / sqrt((double)hd));
+  const int QK = sw.heads * 32;                            // columns of q (and of k, v, and the attention output)
+  for (int i = 0; i < nl; ++i) {
+    for (int j = 0; j < sw.depths[i]; ++j) {
+      const std::string b = "layers." + std::to_string(i) + ".residual_group.blocks." + std::to_string(j) + ".";
+      UpSwinBlock blk;
+      for (const char* nm : {"norm1.weight", "norm1.bias", "norm2.weight", "norm2.bias"}) HDRVAE_TRY(up_need(st, A, b + nm, {C}));
+      HDRVAE_TRY(up_need(st, A, b + "attn.relative_position_bias_table", {225, sw.heads}));
+      HDRVAE_TRY(keep(b + "norm1.weight", C, &blk.ln1_g)); HDRVAE_TRY(keep(b + "norm1.bias", C, &blk.ln1_b));
+      HDRVAE_TRY(keep(b + "norm2.weight", C, &blk.ln2_g)); HDRVAE_TRY(keep(b + "norm2.bias", C, &blk.ln2_b));
+      HDRVAE_TRY(keep(b + "attn.relative_position_bias_table", 225 * (size_t)sw.heads, &blk.table));
+      // qkv [3C][C] -> [3][heads][32][C], q rows and bias x hd^-0.5, rows d >= hd of a head zero
+      HDRVAE_TRY(up_need(st, A, b + "attn.qkv.weight", {3 * C, C}));
+      HDRVAE_TRY(up_need(st, A, b + "attn.qkv.bias", {3 * C}));
+      std::vector<float> w, bias;
+      HDRVAE_TRY(host(b + "attn.qkv.weight", &w));
+      HDRVAE_TRY(host(b + "attn.qkv.bias", &bias));
+      std::vector<float> wq((size_t)3 * QK * C, 0.f), bq((size_t)3 * QK, 0.f);
+      for (int q = 0; q < 3; ++q)
+        for (int hh = 0; hh < sw.heads; ++hh)
+          for (int d = 0; d < hd; ++d) {
+            const int src = q * C + hh * hd + d, dst = (q * sw.heads + hh) * 32 + d;
+            const float f = q == 0 ? qscale : 1.f;
+            for (int c = 0; c < C; ++c) wq[(size_t)dst * C + c] = w[(size_t)src * C + c] * f;
+            bq[dst] = bias[src] * f;
+          }
+      HDRVAE_TRY(pack_host(b + "attn.qkv", wq, bq, 3 * QK, C, 1, &blk.qkv));
+      // proj [C][C] -> [C][heads * 32]: input channel h hd + d moves to h 32 + d
+      HDRVAE_TRY(up_need(st, A, b + "attn.proj.weight", {C, C}));
+      HDRVAE_TRY(up_need(st, A, b + "attn.proj.bias", {C}));
+      HDRVAE_TRY(host(b + "attn.proj.weight", &w));
+      HDRVAE_TRY(host(b + "attn.proj.bias", &bias));
+      std::vector<float> wp((size_t)C * QK, 0.f);
+      for (int o = 0; o < C; ++o)
+        for (int hh = 0; hh < sw.heads; ++hh)
+          for (int d = 0; d < hd; ++d) wp[(size_t)o * QK + hh * 32 + d] = w[(size_t)o * C + hh * hd + d];
+      HDRVAE_TRY(pack_host(b + "attn.proj", wp, bias, C, QK, 1, &blk.proj));
+      HDRVAE_TRY(linear(b + "mlp.fc1", sw.hidden, C, &blk.fc1));
+      HDRVAE_TRY(linear(b + "mlp.fc2", C, sw.hidden, &blk.fc2));
+      sw.blocks.push_back(blk);
+    }
+    HDRVAE_TRY(res_convs("layers." + std::to_string(i) + ".conv"));
+  }
+  HDRVAE_TRY(up_need(st, A, "norm.weight", {C}));
+  HDRVAE_TRY(up_need(st, A, "norm.bias", {C}));
+  HDRVAE_TRY(keep("norm.weight", C, &sw.norm_g));
+  HDRVAE_TRY(keep("norm.bias", C, &sw.norm_b));
+  HDRVAE_TRY(res_convs("conv_after_body"));
+  auto add = [&](const std::string& k, int cout, int cin, bool upsample) -> int {
+    up->convs.emplace_back();
+    return up_pack(st, A, k, cout, cin, 3, upsample, 1.f, &up->convs.back(), s);
+  };
+  switch (sw.tail) {
+    case SW_PIXELSHUFFLE:
+      HDRVAE_TRY(add("conv_before_upsample.0", 64, C, false));
+      for (int k = 0; k < sw.n_up; ++k) HDRVAE_TRY(add("upsample." + std::to_string(2 * k), 256, 64, false));
+      HDRVAE_TRY(add("conv_last", 3, 64, false));
+      HDRVAE_TRY(add_mean(&up->convs.back(), 3, 1));
+      break;
+    case SW_NEAREST:
+      HDRVAE_TRY(add("conv_before_upsample.0", 64, C, false));
+      for (int k = 1; k <= sw.n_up; ++k) HDRVAE_TRY(add("conv_up" + std::to_string(k), 64, 64, true));
+      HDRVAE_TRY(add("conv_hr", 64, 64, false));
+      HDRVAE_TRY(add("conv_last", 3, 64, false));
+      HDRVAE_TRY(add_mean(&up->convs.back(), 3, 1));
+      break;
+    case SW_DIRECT:
+      HDRVAE_TRY(add("upsample.0", 3 * scale * scale, C, false));
+      HDRVAE_TRY(add_mean(&up->convs.back(), 3 * scale * scale, scale * scale));
+      break;
+    case SW_NONE:
+      HDRVAE_TRY(add("conv_last", 3, C, false));          // the mean comes back with the input in the base add
+      break;
+  }
+  up->nb = nl;
+  return 0;
+}
+
 // ESRGAN / RRDBNet (nf 64, gc 32) in Real-ESRGAN names (staging mapped the old-arch keys): conv_first, nb RRDBs of three
 // dense blocks (conv1 .. conv5), conv_body, n_up upsampling convs, conv_hr, conv_last.  n_up, top_*: up_count_upconvs.
 static int up_pack_rrdb(hdrvae_upscaler* up, int n_up, const std::string& top_key, const std::string& top_shape,
@@ -1002,7 +1449,8 @@ static int up_pack_rrdb(hdrvae_upscaler* up, int n_up, const std::string& top_ke
     if (sscanf(kv.first.c_str(), "body.%d.", &bi) == 1) nb = std::max(nb, bi + 1);
   }
   HDRVAE_REQUIRE(nb >= 1, "upscaler state dict holds no RRDB blocks (body.N.rdbK.convJ / model.1.sub.N.RDBK.convJ.0) and is "
-                 "no Real-ESRGAN Compact model (body.0.weight without conv_first) or SPAN model (conv_1.sk.weight)");
+                 "no Real-ESRGAN Compact model (body.0.weight without conv_first) or SPAN model (conv_1.sk.weight), nor a "
+                 "SwinIR model (%s)", kSwinKey);
   up->nb = nb;
   // the layout: u upsampling convs (counted on load) and the pixel-unshuffle factor f from conv_first's 3 f^2 input channels
   HDRVAE_REQUIRE(n_up >= 0, "RRDBNet: %s has shape %s; an old-arch RRDBNet's last top-level conv sits at index 3u + 4 "
@@ -1092,16 +1540,19 @@ int hdrvae_upscaler_load_weights(hdrvae_upscaler* up, const hdrvae_weight_desc* 
     st->raw[name] = f;
     st->shapes[name] = shp;
   }
-  // Compact: body.0.weight and no conv_first (in either layout); SPAN: conv_1.sk.weight; anything else is an RRDBNet
+  // Compact: body.0.weight and no conv_first (in either layout); SPAN: conv_1.sk.weight; SwinIR (and HAT, which its loader
+  // refuses): the first block's relative-position bias table; anything else is an RRDBNet
   bool has_conv_first = false;
   for (const auto& kv : st->shapes) has_conv_first = has_conv_first || kv.first.compare(0, 11, "conv_first.") == 0;
   UpArch arch = UP_RRDB;
   if (st->shapes.count("body.0.weight") && !has_conv_first) arch = UP_COMPACT;
   else if (st->shapes.count("conv_1.sk.weight")) arch = UP_SPAN;
+  else if (st->shapes.count(kSwinKey)) arch = UP_SWINIR;
   switch (arch) {
     case UP_RRDB: HDRVAE_TRY(up_pack_rrdb(up, n_up, top_key, top_shape, s)); break;
     case UP_COMPACT: HDRVAE_TRY(up_pack_compact(up, s)); break;
     case UP_SPAN: HDRVAE_TRY(up_pack_span(up, s)); break;
+    case UP_SWINIR: HDRVAE_TRY(up_pack_swinir(up, s)); break;
   }
   up->arch = arch;
   return up_finish_load(up, staging, s);

@@ -291,7 +291,7 @@ class HdrVaeEngine:
           out2 / out2_chan_off / out2_scale: second, 16-bit output y * out2_scale into a slice of out2 [B,OH,OW,Y2]
                            (without out2_chan_off, out2 has y's pixel stride and channel offset);
           residual2 (float32), res_scale: t = conv + bias + res_scale * residual + residual2;
-          lrelu, prelu (Cout slopes), act (N.ACT_SILU / N.ACT_GATE): the activation of t.
+          lrelu, prelu (Cout slopes), act (N.ACT_SILU / N.ACT_GATE / N.ACT_GELU): the activation of t.
         The device tensors given here are used in place (no copies), so they may alias one another as in the upscalers."""
         B, H, W, xc = x_nhwc.shape
         cout = weight.shape[0]

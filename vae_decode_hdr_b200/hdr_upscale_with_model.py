@@ -7,12 +7,13 @@ recombination all run in libhdrvae.so on the GPU (vae_decode_hdr_b200/csrc/upsca
 a CUDA device or without the library the node raises.
 
 Model loading stays what it is in ComfyUI (folder_paths + spandrel, :73-77); the node only reads
-`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Three architectures run:
+`descriptor.model.state_dict()`, `descriptor.scale` and `descriptor.architecture.name`.  Four architectures run:
 RRDBNet (ESRGAN: nf 64, gc 32) at 1x, 2x and 4x -- the plain form with 0, 1 or 2 upsampling convs and the pixel-unshuffle
-form (RealESRGAN_x2plus) --, Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x, and SPAN (nf <= 64) at
-1x, 2x and 4x, which gets the logit reversal like every architecture outside the reference's atanh list.  An RRDBNet of
-another scale (8x), or one whose `descriptor.scale` disagrees with its weights, fails before any GPU work; any other
-architecture is rejected by the library with an error naming the tensor that does not fit; a Compact or SPAN model whose
+form (RealESRGAN_x2plus) --, Real-ESRGAN Compact (SRVGGNetCompact with PReLU) at 1x, 2x and 4x, SPAN (nf <= 64) at
+1x, 2x and 4x, which gets the logit reversal like every architecture outside the reference's atanh list, and SwinIR
+(window 8, embed_dim <= 256) at 1x, 2x and 4x, which gets atanh.  An RRDBNet of another scale (8x), or one whose
+`descriptor.scale` disagrees with its weights, fails before any GPU work; any other architecture (HAT among them) is
+rejected by the library with an error naming the tensor that does not fit; a Compact, SPAN or SwinIR model whose
 `descriptor.scale` disagrees with its weights is an error too.
 """
 from __future__ import annotations
@@ -24,7 +25,8 @@ from typing import Any, Tuple
 
 import torch
 
-from .upscaler import UPSCALE_METHODS, HdrUpscalerEngine, is_compact_state_dict, reversal_for_architecture, rrdbnet_scale
+from .upscaler import (SWIN_KEY, UPSCALE_METHODS, HdrUpscalerEngine, is_compact_state_dict, reversal_for_architecture,
+                       rrdbnet_scale)
 
 
 def _model_filenames():
@@ -88,7 +90,8 @@ class HDRUpscaleWithModel:
         """Packs the descriptor's weights; the engine's scale (read from the weights) must be `descriptor.scale`."""
         scale = getattr(descriptor, "scale", 4)
         sd = descriptor.model.state_dict()
-        if not is_compact_state_dict(sd):
+        # (SWIN_KEY: SwinIR, or HAT, which the library refuses by name; neither has an RRDBNet's scale rule)
+        if not is_compact_state_dict(sd) and SWIN_KEY not in sd:
             # RRDBNet: the scale follows from the key layout, so both checks fail before any weights reach the GPU (an
             # unrecognised layout goes on to the library, whose error names the tensor that does not fit)
             weights = rrdbnet_scale(sd)

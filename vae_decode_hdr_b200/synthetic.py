@@ -214,3 +214,120 @@ def random_span_state_dict(seed: int = 0, nf: int = 48, s: int = 4, norm: bool =
         else:
             sd[name] = (torch.rand(shape, generator=g) * 2 - 1) * 0.05
     return sd
+
+
+SWINIR_UPSAMPLERS = ("pixelshuffle", "pixelshuffledirect", "nearest+conv", "")
+
+
+def swinir_param_shapes(embed_dim: int = 180, depths=(6, 6, 6, 6, 6, 6), heads: int = 6, mlp_ratio: float = 2.0,
+                        upsampler: str = "pixelshuffle", s: int = 4, resi_connection: str = "1conv",
+                        patch_norm: bool = True, img_size: int = 64) -> List[Tuple[str, Tuple[int, ...]]]:
+    """SwinIR (JingyunLiang/SwinIR network_swinir.py, spandrel's "SwinIR") state-dict keys in module order, 3 input channels,
+    window 8, no ape, num_feat 64 in the tails.  Each Swin transformer layer holds its attn_mask buffer when it shifts
+    (odd blocks; [(img_size / 8)^2, 64, 64]) and every layer its relative_position_index buffer [64, 64]."""
+    if upsampler not in SWINIR_UPSAMPLERS:
+        raise ValueError(f"upsampler must be one of {SWINIR_UPSAMPLERS}")
+    C, ws = embed_dim, 8
+    hidden = int(C * mlp_ratio)
+    out: List[Tuple[str, Tuple[int, ...]]] = []
+
+    def conv(name, cout, cin, k):
+        out.append((f"{name}.weight", (cout, cin, k, k)))
+        out.append((f"{name}.bias", (cout,)))
+
+    def lin(name, cout, cin):
+        out.append((f"{name}.weight", (cout, cin)))
+        out.append((f"{name}.bias", (cout,)))
+
+    def resi(name):
+        if resi_connection == "1conv":
+            conv(name, C, C, 3)
+        else:
+            conv(f"{name}.0", C // 4, C, 3)
+            conv(f"{name}.2", C // 4, C // 4, 1)
+            conv(f"{name}.4", C, C // 4, 3)
+    conv("conv_first", C, 3, 3)
+    if patch_norm:
+        out.append(("patch_embed.norm.weight", (C,)))
+        out.append(("patch_embed.norm.bias", (C,)))
+    for i, depth in enumerate(depths):
+        for j in range(depth):
+            b = f"layers.{i}.residual_group.blocks.{j}"
+            if j % 2:
+                out.append((f"{b}.attn_mask", ((img_size // ws) ** 2, ws * ws, ws * ws)))
+            out.append((f"{b}.norm1.weight", (C,)))
+            out.append((f"{b}.norm1.bias", (C,)))
+            out.append((f"{b}.attn.relative_position_bias_table", ((2 * ws - 1) ** 2, heads)))
+            out.append((f"{b}.attn.relative_position_index", (ws * ws, ws * ws)))
+            lin(f"{b}.attn.qkv", 3 * C, C)
+            lin(f"{b}.attn.proj", C, C)
+            out.append((f"{b}.norm2.weight", (C,)))
+            out.append((f"{b}.norm2.bias", (C,)))
+            lin(f"{b}.mlp.fc1", hidden, C)
+            lin(f"{b}.mlp.fc2", C, hidden)
+        resi(f"layers.{i}.conv")
+    out.append(("norm.weight", (C,)))
+    out.append(("norm.bias", (C,)))
+    resi("conv_after_body")
+    if upsampler == "pixelshuffle":
+        conv("conv_before_upsample.0", 64, C, 3)
+        for k in range(int(math.log2(s))):
+            conv(f"upsample.{2 * k}", 256, 64, 3)
+        conv("conv_last", 3, 64, 3)
+    elif upsampler == "pixelshuffledirect":
+        conv("upsample.0", 3 * s * s, C, 3)
+    elif upsampler == "nearest+conv":
+        conv("conv_before_upsample.0", 64, C, 3)
+        conv("conv_up1", 64, 64, 3)
+        if s == 4:
+            conv("conv_up2", 64, 64, 3)
+        conv("conv_hr", 64, 64, 3)
+        conv("conv_last", 3, 64, 3)
+    else:
+        conv("conv_last", 3, C, 3)
+    return out
+
+
+def _swin_buffers(name: str, shape: Tuple[int, ...]) -> torch.Tensor:
+    """SwinIR's relative_position_index and attn_mask buffers as the published module computes them at construction."""
+    ws = 8
+    if name.endswith("relative_position_index"):
+        r = torch.arange(ws * ws)
+        dy = (r[:, None] // ws - r[None, :] // ws) + ws - 1
+        dx = (r[:, None] % ws - r[None, :] % ws) + ws - 1
+        return dy * (2 * ws - 1) + dx
+    res = int(round(math.sqrt(shape[0]))) * ws                      # attn_mask of an img_size x img_size input, shift 4
+    img = torch.zeros(res, res)
+    cnt = 0
+    for hs in (slice(0, -ws), slice(-ws, -ws // 2), slice(-ws // 2, None)):
+        for wsl in (slice(0, -ws), slice(-ws, -ws // 2), slice(-ws // 2, None)):
+            img[hs, wsl] = cnt
+            cnt += 1
+    win = img.view(res // ws, ws, res // ws, ws).permute(0, 2, 1, 3).reshape(-1, ws * ws)
+    m = win[:, None, :] - win[:, :, None]
+    return m.masked_fill(m != 0, -100.0).masked_fill(m == 0, 0.0)
+
+
+def random_swinir_state_dict(seed: int = 0, embed_dim: int = 180, depths=(6, 6, 6, 6, 6, 6), heads: int = 6,
+                             mlp_ratio: float = 2.0, upsampler: str = "pixelshuffle", s: int = 4,
+                             resi_connection: str = "1conv", patch_norm: bool = True) -> Dict[str, torch.Tensor]:
+    """Random SwinIR weights, fp32, CPU, in spandrel's keys and shapes (swinir_param_shapes), buffers included: unit-gain
+    convs and linears (U(+-sqrt(3 / fan_in))), proj and fc2 at half that gain, LayerNorm gains 1 +- 0.2 and shifts +-0.1,
+    bias tables U(+-1), biases U(+-0.05)."""
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    sd: Dict[str, torch.Tensor] = {}
+    for name, shape in swinir_param_shapes(embed_dim, depths, heads, mlp_ratio, upsampler, s, resi_connection, patch_norm):
+        u = torch.rand(shape, generator=g) * 2 - 1
+        if name.endswith(("relative_position_index", "attn_mask")):
+            sd[name] = _swin_buffers(name, shape)
+        elif name.endswith("relative_position_bias_table"):
+            sd[name] = u
+        elif "norm" in name.rsplit(".", 2)[-2] or name.startswith("norm."):
+            sd[name] = 1.0 + 0.2 * u if name.endswith("weight") else 0.1 * u
+        elif name.endswith("weight"):
+            fan_in = math.prod(shape[1:])
+            gain = 0.5 if (".attn.proj." in name or ".mlp.fc2." in name) else 1.0
+            sd[name] = u * gain * math.sqrt(3.0 / fan_in)
+        else:
+            sd[name] = 0.05 * u
+    return sd

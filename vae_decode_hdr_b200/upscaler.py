@@ -26,9 +26,21 @@ def reversal_for_architecture(name: str) -> str:
 
 def is_compact_state_dict(state_dict) -> bool:
     """The Real-ESRGAN Compact (SRVGGNetCompact) key layout, as the library recognises it: `body.0.weight` and no
-    `conv_first.*`.  The library then checks for SPAN (`conv_1.sk.weight`); every other model it runs is an RRDBNet (see
-    `rrdbnet_scale`)."""
+    `conv_first.*`.  The library then checks for SPAN (`conv_1.sk.weight`) and SwinIR (`SWIN_KEY`); every other model it
+    runs is an RRDBNet (see `rrdbnet_scale`)."""
     return "body.0.weight" in state_dict and not any(k.startswith("conv_first.") for k in state_dict)
+
+
+# The first Swin transformer layer's relative-position bias table: the key by which the library recognises SwinIR.  HAT
+# state dicts have it too; the library refuses them by their own keys.
+SWIN_KEY = "layers.0.residual_group.blocks.0.attn.relative_position_bias_table"
+_HAT_MARKS = ("conv_block", "overlap_attn", "relative_position_index_SA")
+
+
+def is_swinir_state_dict(state_dict) -> bool:
+    """The SwinIR key layout as the library recognises it: `SWIN_KEY` and none of HAT's own keys (`conv_block`,
+    `overlap_attn`, `relative_position_index_SA`)."""
+    return SWIN_KEY in state_dict and not any(m in k for k in state_dict for m in _HAT_MARKS)
 
 
 _OLD_TOP = re.compile(r"model\.(\d+)\.(weight|bias)$")
@@ -59,9 +71,11 @@ def rrdbnet_scale(state_dict) -> Optional[int]:
 class HdrUpscalerEngine:
     """One upscaler model packed for the tcgen05 conv kernel on one GPU: an RRDBNet (ESRGAN: nf 64, gc 32; 0, 1 or 2
     upsampling convs, pixel-unshuffle factor 1, 2 or 4, scale 1, 2 or 4), a Real-ESRGAN Compact (SRVGGNetCompact,
-    PReLU, 1x / 2x / 4x) or a SPAN (nf <= 64, 1x / 2x / 4x; the library fuses every Conv3XC from its conv.* and sk
-    tensors and ignores eval_conv.*).  `scale` is the model's, read from the library; `blocks` is the RRDB count, the
-    Compact's body-conv count or SPAN's 6."""
+    PReLU, 1x / 2x / 4x), a SPAN (nf <= 64, 1x / 2x / 4x; the library fuses every Conv3XC from its conv.* and sk
+    tensors and ignores eval_conv.*) or a SwinIR (embed_dim <= 256, head dim <= 32, window 8, 1conv / 3conv, upsampler
+    "pixelshuffle", "pixelshuffledirect" or "nearest+conv" at 2x / 4x, or "" at 1x; the stored relative_position_index
+    and attn_mask buffers are not read).  `scale` is the model's, read from the library; `blocks` is the RRDB count, the
+    Compact's body-conv count, SPAN's 6 or SwinIR's RSTB count."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device="cuda"):
         self.lib = N.load_library()
